@@ -47,7 +47,10 @@ def ncu_traffic():
 def parse():
     ap = argparse.ArgumentParser()
     ap.add_argument('--gpus', type=int, default=1)
-    ap.add_argument('--steps', type=int, default=5)
+    ap.add_argument('--steps', type=int, default=5,
+                    help='timed steps of the headline evaluation (and of every shape with --mode restarts); the side '
+                         'measurements reported beside the headline (other_window_settings, frozen_regime) time the '
+                         'fixed number of steps each reports as its "steps"')
     ap.add_argument('--warmup', type=int, default=3)
     ap.add_argument('--impl', default='ours', choices=['ours', 'reference'])
     ap.add_argument('--n', type=int, default=100000)
@@ -69,7 +72,29 @@ def parse():
                          'independent restarts / hyper-parameter batches, one replica per GPU, no communication')
     ap.add_argument('--shape', default='sweep', help='restarts mode: sweep | toy | ou | hrir | crude | all')
     ap.add_argument('--no-cpu-baseline', action='store_true')
-    return ap.parse_args()
+    ap.add_argument('--dump-outputs', metavar='DIR',
+                    help='write what the last timed step returned -- elbo, terms (7), grad (every variable) -- as '
+                         'DIR/<name>.npy in float64; the inputs are seeded, so two builds can be compared output for output')
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    if args.dump_outputs and (args.impl != 'ours' or args.mode != 'sharded'):
+        ap.error('--dump-outputs needs --impl ours --mode sharded')
+    return args
+
+
+def dump_outputs(out_dir, budget=64 << 20, **arrays):
+    """Writes every array as out_dir/<name>.npy in float64, at most `budget` bytes in all: above it the largest array
+    is replaced by a fixed, seeded sample of its entries (in index order), the same for every run at that shape."""
+    arrays = {k: np.asarray(v, dtype=np.float64) for k, v in arrays.items()}
+    big = max(arrays, key=lambda k: arrays[k].size)
+    room = (budget - 8 * sum(a.size for k, a in arrays.items() if k != big)) // 8
+    if arrays[big].size > room:
+        keep = np.sort(np.random.default_rng(0).choice(arrays[big].size, room, replace=False))
+        arrays[big] = arrays[big].ravel()[keep]
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + '.npy'), a)
 
 
 # ----------------------------------------------------------------------------- clocks
@@ -334,6 +359,8 @@ def run_ours(args):
     last = (last[0], _np(last[1]), _np(last[2]))               # the gradient buffer g_h is reused by later steps
     clocks = sampler.stop()
     eng.set_option('profile', 0)
+    if args.dump_outputs and rank == 0:       # every rank holds the same all-reduced result
+        dump_outputs(args.dump_outputs, elbo=last[0], terms=last[1], grad=last[2])
     dev = torch.tensor(dev_ms, dtype=torch.float64, device='cuda')
     if dist is not None:
         dist.all_reduce(dev, op=dist.ReduceOp.MAX)
@@ -378,7 +405,7 @@ def run_ours(args):
         alt_dev = torch.tensor(ms, dtype=torch.float64, device='cuda')
         if dist is not None:
             dist.all_reduce(alt_dev, op=dist.ReduceOp.MAX)
-        other.append({'cull': alt, 'value': len(ms) / (float(alt_dev.sum().item()) * 1e-3), 'unit': UNIT,
+        other.append({'cull': alt, 'value': len(ms) / (float(alt_dev.sum().item()) * 1e-3), 'unit': UNIT, 'steps': len(ms),
                       'gemm_flops_per_step': alt_tm['gemm_flops'],
                       'gemm_tflops': g_fl / (g_ms * 1e-3) / 1e12 if g_ms > 0 else None,
                       'elbo_rel_diff_vs_headline': abs(alt_out[0] - last[0]) / abs(last[0]),
@@ -509,7 +536,7 @@ def run_ours(args):
         'elbo': last[0],
         'elbo_rel_diff_vs_n1': elbo_vs_n1, 'grad_rel_diff_vs_n1': grad_vs_n1,
         'other_window_settings': other,
-        'frozen_regime': {'value': frozen_value, 'unit': UNIT,
+        'frozen_regime': {'value': frozen_value, 'unit': UNIT, 'steps': len(fms),
                           'note': 'Psi sums frozen by precompute(); gradient w.r.t. log s2, log s2_f, mu_u, var_u'},
         'next_rows': {'fpi_ms_per_round': fpi_ms, 'elbo_smf_ms_per_sample': smf_ms,
                       'predict_f_ms': pred_ms, 'predict_f_shape': '2048 test inputs x 8 filter samples',
@@ -572,7 +599,7 @@ def run_restarts(args):
     sampler = ClockSampler(local_rank)
     sampler.start()
     for shape in shapes:
-        steps = args.steps if shape == 'sweep' else max(args.steps, 50)
+        steps = args.steps
         if world > 1:
             torch.cuda.synchronize()
             dist.barrier()
