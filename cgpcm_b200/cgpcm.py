@@ -640,16 +640,35 @@ class VCGPCM(CGPCM):
         elbos = [self._evaluate_smf(x)[0] for x in samples_h]
         return np.mean(elbos), np.std(elbos) / len(samples_h) ** .5
 
-    def sample(self, iters=200, burn=None):
-        """Samples from the posterior over filters by elliptical slice sampling (``src/core/cgpcm.py:848-872``)."""
-        from .sample import ESS
+    def sample(self, iters=200, burn=None, chains=1):
+        """Samples from the posterior over filters by elliptical slice sampling (``src/core/cgpcm.py:848-872``).
+        ``chains > 1``: that many chains from the mean of q(u), each with a generator seeded from the model's, whose
+        proposals are scored together (``Engine.elbo_smf_batch``, precomputed regime); returns one list of ``iters``
+        states per chain."""
+        from .sample import ESS, MultiESS
         if burn is None:
             burn = iters
-        ess = ESS(lambda x: self._evaluate_smf(x)[2], self.sample_prior, rng=self._rng)
-        ess.move(self.vars['mu_u'].value.reshape(-1, 1))
-        if burn > 0:
-            ess.sample(burn)
-        return ess.sample(iters)
+        if chains == 1:
+            ess = ESS(lambda x: self._evaluate_smf(x)[2], self.sample_prior, rng=self._rng)
+            ess.move(self.vars['mu_u'].value.reshape(-1, 1))
+            if burn > 0:
+                ess.sample(burn)
+            return ess.sample(iters)
+        if chains < 1:
+            raise ValueError('chains must be >= 1')
+        rngs = [np.random.RandomState(int(s)) for s in self._rng.randint(0, 2 ** 31 - 1, size=int(chains))]
+        mu = self.vars['mu_u'].value.reshape(-1, 1)
+
+        def run():
+            p = self._pack()
+            mess = MultiESS(lambda xs: self.engine.elbo_smf_batch(p, np.stack([x.ravel() for x in xs]), reg=config.reg,
+                                                                  want_elbo=False)[2],
+                            [lambda r=r: self._prior_factor() @ r.randn(self.nh, 1) for r in rngs],
+                            x_inits=[mu.copy() for _ in rngs], rngs=rngs)
+            if burn > 0:
+                mess.sample(burn)
+            return mess.sample(iters)
+        return self._with_frozen_stats(run)
 
     def predict_f(self, t, samples_h=50, precompute=True):
         """Predict the function at ``t`` (``src/core/cgpcm.py:781-846``).  ``samples_h`` numeric: that many draws

@@ -34,6 +34,7 @@
 #include "linalg.cuh"
 #include "predict_kernels.cuh"
 #include "psi_kernels.cuh"
+#include "smf_batch.cuh"
 
 using namespace cg;
 
@@ -185,6 +186,12 @@ struct cgpcm_handle {
   double* axx_part = nullptr;
   long axx_part_elems = 0;
   double* cheb_d = nullptr;    // Chebyshev table of the pair-hoisted BVN branch (bvn.cuh)
+  // batched SMF scoring (cgpcm_elbo_smf_batch): one allocation for the samples, W = H_B A of a chunk, the slice partials
+  // and C1 slabs, the factor slabs and the per-sample scalars; info words of the factorisations
+  double* smf_buf = nullptr;
+  long smf_elems = 0;
+  int* smf_info = nullptr;
+  int smf_info_count = 0;
   int axx_slices = 0;
   int axx_slices_opt = 0;      // option "axx_slices": 0 = automatic (axx_sweep)
   double* ypart = nullptr;     // [slices][nhp][ld] private Y accumulators
@@ -1160,6 +1167,8 @@ int cgpcm_destroy(cgpcm_handle* h) {
     if (p) cudaFree(p);
   if (h->wfac) cudaFree(h->wfac);
   if (h->wdesc) cudaFree(h->wdesc);
+  if (h->smf_buf) cudaFree(h->smf_buf);
+  if (h->smf_info) cudaFree(h->smf_info);
   if (h->info) cudaFree(h->info);
   for (auto& e : h->ev)
     if (e) cudaEventDestroy(e);
@@ -1440,6 +1449,79 @@ int cgpcm_psi(cgpcm_handle* h, const double hyp[3], double* sum_Axx, double* Ahh
 
 namespace cgimpl {
 
+// q(u) from the packed parameters in params_d: L from var_u (np.tril_indices order, src/core/tf_util.py:419-447),
+// var = L L^T + reg I (src/core/cgpcm.py:444-445, also into M_LVAR for its factorisation), m2 = var + mu mu^T
+// (src/core/distribution.py:35-42)
+int qu_moments(cgpcm_handle* h, double reg) {
+  const int nh = h->nh, nhp = h->nhp;
+  const long ld = h->ld, l2 = ld * ld;
+  double* Lq = h->M(M_LQ);
+  double* mu = h->V(V_MU);
+  const double* pd = h->params_d;
+  ew(h->st, l2, [=] __device__(long idx) {
+    int i = (int)(idx / ld), j = (int)(idx % ld);
+    Lq[idx] = (i < nh && j <= i) ? pd[5 + nh + (long)i * (i + 1) / 2 + j] : 0.0;
+    if (idx < ld) mu[idx] = idx < nh ? pd[5 + idx] : 0.0;
+  });
+  L(h);
+  if (mm(h, Lq, false, Lq, true, h->M(M_VAR), nhp, nhp, nhp)) return -2;
+  double* var = h->M(M_VAR);
+  double* lvar = h->M(M_LVAR);
+  double* m2 = h->M(M_M2);
+  ew(h->st, l2, [=] __device__(long idx) {
+    int i = (int)(idx / ld), j = (int)(idx % ld);
+    double v = var[idx] + ((i == j && i < nh) ? reg : 0.0);
+    var[idx] = v;
+    lvar[idx] = v;
+    m2[idx] = v + mu[i] * mu[j];
+  });
+  L(h);
+  return 0;
+}
+
+// The KL pieces (src/core/distribution.py:60-76) need the factor / inverse of So = iKh + reg I and of the q(u)
+// covariance: two chains queued on the side streams (So behind the Kh chain, var behind the Kx chain); the caller joins
+// both before kl_scalars.
+int kl_fork(cgpcm_handle* h, double reg) {
+  const int nh = h->nh, nhp = h->nhp;
+  const long ld = h->ld, l2 = ld * ld;
+  if (side_fork(h, 0)) return -2;
+  if (side_fork(h, 1)) return -2;
+  {
+    double* so = h->M(M_SO);
+    const double* ikh = h->M(M_IKH);
+    ew(h->side[0], l2, [=] __device__(long idx) {
+      int i = (int)(idx / ld), j = (int)(idx % ld);
+      so[idx] = ikh[idx] + ((i == j && i < nh) ? reg : 0.0);
+    });
+    h->launches++;
+  }
+  if (chol_inv_on(h, 1, h->M(M_SO), h->M(M_ISO), nh, nhp, h->sc + S_LOGDET_SO, 4)) return -2;
+  if (chol_inv_on(h, 2, h->M(M_LVAR), h->M(M_IVAR), nh, nhp, h->sc + S_LOGDET_VAR, 5)) return -2;
+  return 0;
+}
+
+void kl_scalars(cgpcm_handle* h) {
+  const int nh = h->nh;
+  frob(h, h->M(M_ISO), h->M(M_VAR), nh, nh, h->sc + S_TR_ISO_VAR);
+  matvec(h, h->M(M_ISO), nh, nh, 0, h->V(V_MU), 1.0, h->V(V_ISOMU));
+  dot(h, h->V(V_MU), h->V(V_ISOMU), nh, h->sc + S_MU_ISO_MU);
+}
+
+// The ELBO terms that do not depend on the optimal q(z): tm[0], tm[1], tm[4], tm[5], tm[6] (tm[2], tm[3] are left to
+// the caller).  hs: the device scalars after the final all-reduce.
+void fixed_terms(const cgpcm_handle* h, const double* hs, double s2, double r, double sum_b, double tr_bhh_m2,
+                 double* tm) {
+  const double Ng = hs[S_COUNT + 0], sum_y2 = hs[S_COUNT + 1];
+  const double KL = 0.5 * (hs[S_TR_ISO_VAR] + hs[S_MU_ISO_MU] - h->nh + hs[S_LOGDET_SO] - hs[S_LOGDET_VAR]);
+  tm[0] = -0.5 * Ng * log(2.0 * 3.14159265358979323846 * s2) - 0.5 * sum_y2 / s2;
+  tm[1] = 0.5 * hs[S_LOGDET_KX];
+  tm[2] = tm[3] = 0.0;
+  tm[4] = -0.5 * r * sum_b;
+  tm[5] = -0.5 * r * tr_bhh_m2;
+  tm[6] = -KL;
+}
+
 // The whole evaluation.  mode FULL: hyper-parameters from params; mode FROZEN: Psi sums from the frozen
 // state (precompute), prior kernels still from params (they stay symbolic in the reference too).
 // `freeze`: run the forward Psi sums only and store them (cgpcm_precompute).
@@ -1506,34 +1588,12 @@ int evaluate_once(cgpcm_handle* h, const double* params_host, int mode, uint32_t
   const double* tl = h->fwd_tail;               // device: [N (all ranks), sum y^2 (all ranks)]
   const bool smf = sample_host != nullptr;
   if (!freeze) {
-    // q(u): L from var_u (np.tril_indices order, src/core/tf_util.py:419-447), var = L L^T + reg I
-    // (src/core/cgpcm.py:444-445), m2 = var + mu mu^T (src/core/distribution.py:35-42)
-    double* Lq = h->M(M_LQ);
-    double* mu = h->V(V_MU);
-    const double* pd = h->params_d;
-    ew(st, l2, [=] __device__(long idx) {
-      int i = (int)(idx / ld), j = (int)(idx % ld);
-      Lq[idx] = (i < nh && j <= i) ? pd[5 + nh + (long)i * (i + 1) / 2 + j] : 0.0;
-      if (idx < ld) mu[idx] = idx < nh ? pd[5 + idx] : 0.0;
-    });
-    L(h);
-    if (mm(h, Lq, false, Lq, true, h->M(M_VAR), nhp, nhp, nhp)) return -2;
-    double* var = h->M(M_VAR);
-    double* lvar = h->M(M_LVAR);
-    double* m2 = h->M(M_M2);
-    double* smp = h->V(V_SMP);
     if (smf) {
+      double* smp = h->V(V_SMP);
       CK(cudaMemsetAsync(smp, 0, ld * sizeof(double), st));
       CK(cudaMemcpyAsync(smp, sample_host, nh * sizeof(double), cudaMemcpyHostToDevice, st));
     }
-    ew(st, l2, [=] __device__(long idx) {
-      int i = (int)(idx / ld), j = (int)(idx % ld);
-      double v = var[idx] + ((i == j && i < nh) ? reg : 0.0);
-      var[idx] = v;
-      lvar[idx] = v;
-      m2[idx] = v + mu[i] * mu[j];
-    });
-    L(h);
+    if (qu_moments(h, reg)) return -2;
   }
   CK(cudaEventRecord(h->ev[1], st));
 
@@ -1552,19 +1612,7 @@ int evaluate_once(cgpcm_handle* h, const double* params_host, int mode, uint32_t
       // the main stream's view of iKh / iKx: events recorded now, BEFORE the KL chains are queued behind them
       if (prior_join(h)) return -2;
     }
-    if (side_fork(h, 0)) return -2;
-    if (side_fork(h, 1)) return -2;
-    {
-      double* so = h->M(M_SO);
-      const double* ikh = h->M(M_IKH);
-      ew(h->side[0], l2, [=] __device__(long idx) {
-        int i = (int)(idx / ld), j = (int)(idx % ld);
-        so[idx] = ikh[idx] + ((i == j && i < nh) ? reg : 0.0);
-      });
-      h->launches++;
-    }
-    if (chol_inv_on(h, 1, h->M(M_SO), h->M(M_ISO), nh, nhp, h->sc + S_LOGDET_SO, 4)) return -2;
-    if (chol_inv_on(h, 2, h->M(M_LVAR), h->M(M_IVAR), nh, nhp, h->sc + S_LOGDET_VAR, 5)) return -2;
+    if (kl_fork(h, reg)) return -2;
     kl_pending = true;
   } else {
     if (prior_join(h)) return -2;
@@ -1727,9 +1775,7 @@ int evaluate_once(cgpcm_handle* h, const double* params_host, int mode, uint32_t
     if (side_join(h, 0)) return -2;
     if (side_join(h, 1)) return -2;
   }
-  frob(h, h->M(M_ISO), h->M(M_VAR), nh, nh, h->sc + S_TR_ISO_VAR);
-  matvec(h, h->M(M_ISO), nh, nh, 0, h->V(V_MU), 1.0, h->V(V_ISOMU));
-  dot(h, h->V(V_MU), h->V(V_ISOMU), nh, h->sc + S_MU_ISO_MU);
+  kl_scalars(h);
   CK(cudaEventRecord(h->ev[4], st));
 
   // ---- 5. backward sweep
@@ -1932,15 +1978,10 @@ int evaluate_once(cgpcm_handle* h, const double* params_host, int mode, uint32_t
   double sum_b, tr_bhh_m2 = hs[S_TR_BHH_M2];
   if (full) sum_b = Ng * a - Ng * hs[S_TR_IKH_AHH] - hs[S_TR_IKX_AXX] + hs[S_TR_IKH_Q];
   else sum_b = h->f_sum_b;
-  const double KL = 0.5 * (hs[S_TR_ISO_VAR] + hs[S_MU_ISO_MU] - nh + hs[S_LOGDET_SO] - hs[S_LOGDET_VAR]);
   double tm[7];
-  tm[0] = -0.5 * Ng * log(2.0 * 3.14159265358979323846 * s2) - 0.5 * sum_y2 / s2;
-  tm[1] = 0.5 * hs[S_LOGDET_KX];
+  fixed_terms(h, hs, s2, r, sum_b, tr_bhh_m2, tm);
   tm[2] = -0.5 * hs[S_LOGDET_P];
   tm[3] = 0.5 * hs[S_LAM_LBAR];
-  tm[4] = -0.5 * r * sum_b;
-  tm[5] = -0.5 * r * tr_bhh_m2;
-  tm[6] = -KL;
   double e = 0.0;
   for (int i = 0; i < 7; ++i) e += tm[i];
   if (terms) memcpy(terms, tm, sizeof tm);
@@ -2756,6 +2797,195 @@ int akm_run(cgpcm_handle* h, const double* params_host, double reg, const double
   return 0;
 }
 
+// Samples per internal batch of smf_batch_run: a function of the handle's shape only (the W GEMM always runs with this
+// many rows, zero rows past the batch, so that its launch does not depend on the number of samples).  Seven ld x ld
+// slabs per sample (SMF_SLICES partials, C1, the factors of P and P0) within ~1 GB.
+int smf_bcap(const cgpcm_handle* h) {
+  const double per = (SMF_SLICES + 3.0) * (double)h->ld * h->ld * sizeof(double);
+  const int b = (int)std::min(64.0, 1e9 / per) / 8 * 8;
+  return std::max(8, b);
+}
+
+// VCGPCM.elbo(smf=True, sample=h_b) and the slice sampler's log-likelihood (src/core/cgpcm.py:527-531,594-608,848-872)
+// for B samples in the frozen regime.  Per call: the terms that do not depend on the sample (the prior, q(u) and
+// its KL, the frozen sums), as evaluate_once forms them.  Per batch of <= smf_bcap samples: per chunk W = H_B A (the
+// small-left GEMM over the resident or regenerated Ahx block) and C1_b += W_b^T W_b (smf_c1_kernel), one all-reduce
+// of the C1 slabs, then the factorisations of P_b (want_p) and P0_b (want_p0) in one launch.
+int smf_batch_run(cgpcm_handle* h, const double* params_host, double reg, const double* samples_host, int B,
+                  bool want_p, bool want_p0, double* elbo_out, double* terms_out, double* loglik_out) {
+  const int nh = h->nh, nx = h->nx, nhp = h->nhp;
+  const long ld = h->ld, l2 = ld * ld;
+  const long np = 5 + nh + (long)nh * (nh + 1) / 2;
+  for (long i = 0; i < np; ++i)
+    if (!std::isfinite(params_host[i])) { h->err = "non-finite parameter"; return -4; }
+  for (long i = 0; i < (long)B * nh; ++i)
+    if (!std::isfinite(samples_host[i])) {
+      char b[96];
+      snprintf(b, sizeof b, "non-finite value in sample %ld", i / nh);
+      h->err = b;
+      return -4;
+    }
+  if (!h->frozen) { h->err = "cgpcm_elbo_smf_batch requires cgpcm_precompute"; return -1; }
+  if (!want_p && !want_p0) return 0;
+  const double s2 = exp(params_host[0]), s2f = exp(params_host[1]);
+  const double alpha = exp(params_host[2]), gamma = exp(params_host[3]), omega = exp(params_host[4]);
+  const double r = s2f / s2, c0 = sqrt(s2f) / s2;
+  if (ensure_sweep_buffers(h)) return -2;
+  h->launches = 0;
+  h->pev_used = 0;
+  h->prof_open = false;
+  h->gemm_flops = h->gemm_flops_exec = 0.0;
+  h->gemm_launches = 0;
+  PsiConst c;
+  psi_make_const(alpha, gamma, omega, h->causal, h->cull, &c, h->causal_id);
+  std::vector<Chunk> chunks;
+  plan_chunks(h, h->fc, chunks);
+  if (ensure_ypart(h, y_slices_used(chunks))) return -2;
+  if (plan_store(h, chunks, false)) return -2;
+  const int bcap = smf_bcap(h);
+  const int passes = (want_p ? 1 : 0) + (want_p0 ? 1 : 0);
+  long wcols = 0;
+  for (const Chunk& ch : chunks) wcols = std::max<long>(wcols, (long)ch.nc * ch.kwp);
+  // [hs: bcap x nhp][out: bcap x 5 (+ pad)][part: bcap x SMF_SLICES slabs][c1: bcap slabs][work: 2 bcap slabs][W]
+  const long o_hs = 0, o_out = o_hs + (long)bcap * nhp, o_part = o_out + round_up(bcap * 5, 8);
+  const long o_c1 = o_part + (long)bcap * SMF_SLICES * l2, o_work = o_c1 + (long)bcap * l2;
+  const long o_w = o_work + 2L * bcap * l2, need = o_w + (long)bcap * wcols;
+  if (need > h->smf_elems) {
+    if (h->smf_buf) cudaFree(h->smf_buf);
+    h->smf_buf = nullptr; h->smf_elems = 0;
+    CK(cudaMalloc(&h->smf_buf, need * sizeof(double)));
+    h->smf_elems = need;
+  }
+  if (2 * bcap > h->smf_info_count) {
+    if (h->smf_info) cudaFree(h->smf_info);
+    h->smf_info = nullptr; h->smf_info_count = 0;
+    CK(cudaMalloc(&h->smf_info, 2 * bcap * sizeof(int)));
+    h->smf_info_count = 2 * bcap;
+  }
+  double* d_hs = h->smf_buf + o_hs;
+  double* d_out = h->smf_buf + o_out;
+  double* d_part = h->smf_buf + o_part;
+  double* d_c1 = h->smf_buf + o_c1;
+  double* d_work = h->smf_buf + o_work;
+  double* d_w = h->smf_buf + o_w;
+
+  cudaStream_t st = h->st;
+  CK(cudaEventRecord(h->ev[0], st));
+  CK(cudaMemsetAsync(h->info, 0, 4 * sizeof(int), st));
+  CK(cudaMemcpyAsync(h->params_d, params_host, np * sizeof(double), cudaMemcpyHostToDevice, st));
+  // ---- the terms that do not depend on the sample (evaluate_once, MODE_FROZEN)
+  if (prior_stage(h, c, reg, true, true)) return -2;
+  if (qu_moments(h, reg)) return -2;
+  if (prior_join(h)) return -2;
+  if (kl_fork(h, reg)) return -2;
+  frob(h, h->M(M_F_BHH), h->M(M_M2), nh, nh, h->sc + S_TR_BHH_M2);
+  {
+    double tail[2] = {(double)h->n_local, h->sum_y2_local};
+    CK(cudaMemcpyAsync(h->fwd_tail, tail, sizeof tail, cudaMemcpyHostToDevice, st));
+  }
+  if (allreduce(h, h->fwd_tail, 2)) return -2;
+  if (side_join(h, 0)) return -2;
+  if (side_join(h, 1)) return -2;
+  kl_scalars(h);
+  double hs[S_COUNT + 16];
+  int info[4];
+  CK(cudaMemcpyAsync(hs, h->sc, sizeof hs, cudaMemcpyDeviceToHost, st));
+  CK(cudaMemcpyAsync(info, h->info, sizeof info, cudaMemcpyDeviceToHost, st));
+  CK(cudaStreamSynchronize(st));
+  if (info[0]) {
+    h->prior_valid = false;
+    static const char* names[] = {"?", "Kh", "Kx", "P", "iKh + reg I (prior of q(u))", "q(u) covariance"};
+    const int tag = info[0] / 100000;
+    char b[160];
+    snprintf(b, sizeof b, "matrix %s is not positive definite (pivot %d)", tag >= 1 && tag <= 5 ? names[tag] : "?",
+             info[0] % 100000);
+    h->err = b;
+    return -3;
+  }
+  double tm[7];
+  fixed_terms(h, hs, s2, r, h->f_sum_b, hs[S_TR_BHH_M2], tm);
+
+  // ---- batches of samples
+  std::vector<double> hsm((size_t)bcap * nhp), res((size_t)bcap * 5);
+  std::vector<int> inf((size_t)2 * bcap);
+  const long wstride = wcols;
+  for (int b0 = 0; b0 < B; b0 += bcap) {
+    const int nb = std::min(bcap, B - b0);
+    std::fill(hsm.begin(), hsm.end(), 0.0);
+    for (int b = 0; b < nb; ++b)
+      for (int i = 0; i < nh; ++i) hsm[(size_t)b * nhp + i] = samples_host[(size_t)(b0 + b) * nh + i];
+    // (pageable source: staged before the call returns)
+    CK(cudaMemcpyAsync(d_hs, hsm.data(), hsm.size() * sizeof(double), cudaMemcpyHostToDevice, st));
+    CK(cudaMemsetAsync(d_part, 0, (size_t)nb * SMF_SLICES * l2 * sizeof(double), st));
+    const bool stor = h->use_store;
+    const bool have_a = stor && h->storeA_frozen_valid;
+    for (const Chunk& ch : chunks) {
+      double* Ab = stor ? h->storeA + ch.off : h->wsA;
+      if (!have_a && gen_chunk(h, h->fc, ch, false, Ab)) return -2;
+      const long cols = (long)ch.nc * ch.kwp;
+      // W[b][(n,k)] = sum_i h_b[i] A[i][(n,k)]
+      if (gemm(h, true, false, false, bcap, (int)cols, nhp, 1.0, d_hs, nhp, Ab, cols, 0.0, d_w, wstride)) return -2;
+      SmfC1Args g;
+      g.W = d_w; g.w_stride = wstride; g.kwp = ch.kwp; g.nc = ch.nc;
+      g.part = d_part; g.l2 = l2; g.ld = ld; g.win = (long)ch.k_lo * ld + ch.k_lo;
+      const int T = (ch.kwp + SMF_T - 1) / SMF_T;
+      prof_close(h);
+      smf_c1_kernel<<<dim3(T * (T + 1) / 2, SMF_SLICES, nb), 128, 0, st>>>(g);
+      h->gemm_flops += (double)nb * ch.nc * ch.kwp * (ch.kwp + 1.0);
+      L(h);
+    }
+    if (stor) h->storeA_frozen_valid = true;
+    smf_reduce_kernel<<<148 * 4, 256, 0, st>>>(d_part, (long)nb * l2, l2, ld, nx, d_c1);
+    L(h);
+    if (allreduce(h, d_c1, (long)nb * l2)) return -2;
+    SmfAlgArgs a;
+    a.kx = h->M(M_KX); a.sxx = h->M(M_F_AXX); a.c1 = d_c1; a.fy = h->M(M_F_Y); a.bhh = h->M(M_F_BHH);
+    a.hs = d_hs; a.work = d_work; a.out = d_out; a.info = h->smf_info;
+    a.ld = ld; a.l2 = l2; a.ldh = nhp; a.nh = nh; a.nx = nx;
+    a.r = r; a.c0 = c0; a.reg = reg; a.want_p = want_p; a.passes = passes;
+    CK(cudaMemsetAsync(h->smf_info, 0, 2 * bcap * sizeof(int), st));
+    smf_algebra_kernel<<<dim3(nb, passes), SMF_ALG_THREADS, 2 * nx * sizeof(double), st>>>(a);
+    L(h);
+    CK(cudaGetLastError());
+    CK(cudaMemcpyAsync(res.data(), d_out, (size_t)nb * 5 * sizeof(double), cudaMemcpyDeviceToHost, st));
+    CK(cudaMemcpyAsync(inf.data(), h->smf_info, (size_t)nb * 2 * sizeof(int), cudaMemcpyDeviceToHost, st));
+    CK(cudaStreamSynchronize(st));
+    for (int b = 0; b < nb; ++b)
+      for (int k = 0; k < 2; ++k)
+        if (inf[2 * b + k]) {
+          char m[160];
+          snprintf(m, sizeof m, "matrix %s of sample %d is not positive definite (pivot %d)", k == 0 ? "P" : "P0 (no jitter)",
+                   b0 + b, inf[2 * b + k]);
+          h->err = m;
+          return -3;
+        }
+    for (int b = 0; b < nb; ++b) {
+      const double* o = &res[(size_t)b * 5];
+      if (want_p) {
+        double t[7];
+        memcpy(t, tm, sizeof t);
+        t[2] = -0.5 * o[0];
+        t[3] = 0.5 * o[1];
+        double e = 0.0;
+        for (int i = 0; i < 7; ++i) e += t[i];
+        if (elbo_out) elbo_out[b0 + b] = e;
+        if (terms_out) memcpy(terms_out + (size_t)(b0 + b) * 7, t, sizeof t);
+      }
+      if (want_p0) loglik_out[b0 + b] = -0.5 * o[2] + 0.5 * o[3] - 0.5 * r * o[4];
+    }
+  }
+  CK(cudaEventRecord(h->ev[6], st));
+  CK(cudaStreamSynchronize(st));
+  float ms = 0;
+  cudaEventElapsedTime(&ms, h->ev[0], h->ev[6]);
+  memset(h->timing, 0, sizeof h->timing);
+  h->timing[0] = ms;
+  h->timing[6] = (double)h->launches;
+  h->timing[7] = h->gemm_flops;
+  h->timing[8] = (double)h->gemm_launches;
+  return 0;
+}
+
 }  // namespace cgimpl
 
 extern "C" {
@@ -2818,6 +3048,34 @@ int cgpcm_elbo_smf(cgpcm_handle* h, const double* params, int32_t mode, double r
   if (is_device_ptr(elbo)) cudaMemcpy(elbo, &e, sizeof e, cudaMemcpyHostToDevice); else *elbo = e;
   if (terms) { if (is_device_ptr(terms)) cudaMemcpy(terms, tm, sizeof tm, cudaMemcpyHostToDevice); else memcpy(terms, tm, sizeof tm); }
   if (loglik) { if (is_device_ptr(loglik)) cudaMemcpy(loglik, &ll, sizeof ll, cudaMemcpyHostToDevice); else *loglik = ll; }
+  return 0;
+}
+
+int cgpcm_elbo_smf_batch(cgpcm_handle* h, const double* params, double reg, const double* samples, int32_t n_samples,
+                         double* elbo, double* terms, double* loglik) {
+  if (!h || !params || !samples) return -1;
+  if (n_samples < 1) { h->err = "n_samples must be >= 1"; return -1; }
+  if (!h->t) { h->err = "cgpcm_set_data has not been called"; return -1; }
+  if (!std::isfinite(reg) || reg < 0) { h->err = "reg must be finite and >= 0"; return -4; }
+  CK(cudaSetDevice(h->device));
+  const long np = 5 + h->nh + (long)h->nh * (h->nh + 1) / 2;
+  const long ns = (long)n_samples * h->nh;
+  std::vector<double> host, smp(ns);
+  if (fetch_params(h, params, np, host)) return -2;
+  if (is_device_ptr(samples)) CK(cudaMemcpy(smp.data(), samples, ns * sizeof(double), cudaMemcpyDeviceToHost));
+  else memcpy(smp.data(), samples, ns * sizeof(double));
+  const bool want_p = elbo || terms;
+  std::vector<double> e(want_p ? n_samples : 0), tm(want_p ? 7L * n_samples : 0), ll(loglik ? n_samples : 0);
+  int rc = smf_batch_run(h, host.data(), reg, smp.data(), n_samples, want_p, loglik != nullptr,
+                         want_p ? e.data() : nullptr, want_p ? tm.data() : nullptr, loglik ? ll.data() : nullptr);
+  if (rc) return rc;
+  auto put = [&](double* dst, const std::vector<double>& v) -> int {
+    if (!dst || v.empty()) return 0;
+    if (is_device_ptr(dst)) CK(cudaMemcpy(dst, v.data(), v.size() * sizeof(double), cudaMemcpyHostToDevice));
+    else memcpy(dst, v.data(), v.size() * sizeof(double));
+    return 0;
+  };
+  if (put(elbo, e) || put(terms, tm) || put(loglik, ll)) return -2;
   return 0;
 }
 

@@ -129,6 +129,21 @@ class Engine(object):
                                             _lib.ptr(elbo), _lib.ptr(terms), _lib.ptr(ll)))
         return float(elbo[0]), terms, float(ll[0])
 
+    def elbo_smf_batch(self, params, samples, reg=1e-8, want_elbo=True):
+        """``elbo_smf`` in the precomputed regime for every row of ``samples`` ([B, nh]) in one call:
+        ``(elbo[B], terms[B, 7], log_lik[B])``.  ``want_elbo=False`` skips the jittered factorisation and returns
+        ``(None, None, log_lik)`` (what the slice sampler needs).  A sample's values do not depend on the batch."""
+        samples = np.ascontiguousarray(np.asarray(samples, dtype=np.float64))
+        if samples.ndim != 2 or samples.shape[1] != self.nh or samples.shape[0] < 1 or \
+                int(params.shape[0]) != n_params(self.nh):
+            raise ValueError('shape mismatch in elbo_smf_batch')
+        B = samples.shape[0]
+        elbo, terms = (np.empty(B), np.empty((B, 7))) if want_elbo else (None, None)
+        ll = np.empty(B)
+        self._ck(_lib.lib().cgpcm_elbo_smf_batch(self._h, _lib.ptr(params), float(reg), _lib.ptr(samples), B,
+                                                  _lib.ptr(elbo), _lib.ptr(terms), _lib.ptr(ll)))
+        return elbo, terms, ll
+
     def predict_f(self, params, t_star, samples, smf=False, reg=1e-8):
         """Posterior ``(mean, var)`` of the function at ``t_star`` averaged over the filter ``samples`` ([B, nh])
         (``src/core/cgpcm.py:781-846``); needs the frozen statistics."""

@@ -126,6 +126,18 @@ int cgpcm_elbo_grad(cgpcm_handle* h, const double* params, int32_t mode, uint32_
 int cgpcm_elbo_smf(cgpcm_handle* h, const double* params, int32_t mode, double reg, const double* sample, double* elbo,
                    double* terms, double* loglik);
 
+/* cgpcm_elbo_smf in MODE_FROZEN for many filter samples in one call (src/core/cgpcm.py:527-531,594-608,848-872):
+ * samples[n_samples][nh] -> elbo[n_samples], terms[n_samples][7], loglik[n_samples].  The optimal q(z) of every sample
+ * comes from C1_b = sum_n w_bn w_bn^T with w_bn = A_n^T h_b (H = h_b h_b^T has rank one), contracted for a batch of
+ * samples at a time over the frozen regime's Ahx blocks.  elbo and terms may both be NULL (then P_b, the jittered
+ * matrix, is not factorised), loglik may be NULL; any n_samples >= 1 (split internally into batches).  A sample's
+ * results are bitwise the same whatever batch it is scored in and at whatever position; they agree with
+ * cgpcm_elbo_smf(MODE_FROZEN) up to the rounding of the other summation order.  Requires cgpcm_precompute (-1
+ * otherwise); -4 for a non-finite parameter or sample; -3 when P_b or P0_b is not positive definite
+ * (cgpcm_last_error names the sample). */
+int cgpcm_elbo_smf_batch(cgpcm_handle* h, const double* params, double reg, const double* samples, int32_t n_samples,
+                         double* elbo, double* terms, double* loglik);
+
 /* mod.predict_f(t, samples_h) (src/core/cgpcm.py:781-846): posterior mean[n_star] and variance[n_star] of the function
  * at the test inputs t_star, averaged over the filter samples samples[n_samples][nh].  smf = 0: the optimal q(z) of
  * q(u) (the reference's numeric samples_h: draws from q(u)); smf = 1: the optimal q(z | h) of every sample (the
