@@ -22,7 +22,8 @@ MODE_FROZEN, MODE_FULL = 0, 1
 
 EXPORTS = ['cgpcm_create', 'cgpcm_destroy', 'cgpcm_last_error', 'cgpcm_device_count', 'cgpcm_comm_unique_id', 'cgpcm_comm_init',
            'cgpcm_set_data', 'cgpcm_set_option', 'cgpcm_psi', 'cgpcm_precompute', 'cgpcm_frozen_mats', 'cgpcm_elbo_grad', 'cgpcm_elbo_smf', 'cgpcm_elbo_smf_batch', 'cgpcm_predict_f', 'cgpcm_kernel_samples', 'cgpcm_filter_samples', 'cgpcm_akm_sample', 'cgpcm_fpi', 'cgpcm_fpi_qz', 'cgpcm_elbo_qz',
-           'cgpcm_last_timing', 'cgpcm_bvn_cdf', 'cgpcm_dgemm', 'cgpcm_dgemm_tri', 'cgpcm_dgemm_sym', 'cgpcm_cholinv', 'cgpcm_math_test', 'cgpcm_math_test_fast']
+           'cgpcm_last_timing', 'cgpcm_bvn_cdf', 'cgpcm_dgemm', 'cgpcm_dgemm_tri', 'cgpcm_dgemm_sym', 'cgpcm_cholinv', 'cgpcm_math_test', 'cgpcm_math_test_fast',
+           'cgpcm_smf_c1_test', 'cgpcm_smf_algebra_test']
 
 
 def _sources():
@@ -94,6 +95,9 @@ def lib():
     L.cgpcm_cholinv.argtypes = [dp, dp, dp, i32, i64, ctypes.POINTER(i32)]
     L.cgpcm_math_test.argtypes = [dp, i64, dp, dp, ctypes.POINTER(i32)]
     L.cgpcm_math_test_fast.argtypes = [dp, i64, dp, dp]
+    L.cgpcm_smf_c1_test.argtypes = [dp, i64, i32, i32, dp, i32, i64, dp, vp]
+    L.cgpcm_smf_algebra_test.argtypes = [dp, dp, dp, dp, dp, dp, i32, i32, i32, i64, i32, dbl, dbl, dbl, i32, i32, dp,
+                                         vp, vp]
     for name in EXPORTS:
         if name != 'cgpcm_last_error':
             getattr(L, name).restype = ctypes.c_int

@@ -565,10 +565,10 @@ constexpr int CHUNK_AUTO_MAX = 2048;
 inline int chunk_cap(const cgpcm_handle* h) { return h->chunk_auto ? CHUNK_AUTO_MAX : h->chunk; }
 
 void plan_chunks(cgpcm_handle* h, const PsiConst& c, std::vector<Chunk>& out) {
-  if (!h->chunk_auto) { plan_chunks_fixed(h, c, h->chunk, out); return; }
+  if (!h->chunk_auto) plan_chunks_fixed(h, c, h->chunk, out);
   double best = INFINITY;
   std::vector<Chunk> cand;
-  for (int pass = 0; pass < 6; ++pass) {
+  for (int pass = 0; h->chunk_auto && pass < 6; ++pass) {
     const int chunk = pass / 2 == 0 ? 512 : pass / 2 == 1 ? 1024 : CHUNK_AUTO_MAX;
     plan_chunks_fixed(h, c, chunk, cand, (pass & 1) != 0);
     double cost = 0.0;
@@ -2925,17 +2925,13 @@ int smf_batch_run(cgpcm_handle* h, const double* params_host, double reg, const 
       const long cols = (long)ch.nc * ch.kwp;
       // W[b][(n,k)] = sum_i h_b[i] A[i][(n,k)]
       if (gemm(h, true, false, false, bcap, (int)cols, nhp, 1.0, d_hs, nhp, Ab, cols, 0.0, d_w, wstride)) return -2;
-      SmfC1Args g;
-      g.W = d_w; g.w_stride = wstride; g.kwp = ch.kwp; g.nc = ch.nc;
-      g.part = d_part; g.l2 = l2; g.ld = ld; g.win = (long)ch.k_lo * ld + ch.k_lo;
-      const int T = (ch.kwp + SMF_T - 1) / SMF_T;
       prof_close(h);
-      smf_c1_kernel<<<dim3(T * (T + 1) / 2, SMF_SLICES, nb), 128, 0, st>>>(g);
+      smf_c1_launch(st, d_w, wstride, ch.kwp, ch.nc, ch.k_lo, d_part, ld, nb);
       h->gemm_flops += (double)nb * ch.nc * ch.kwp * (ch.kwp + 1.0);
       L(h);
     }
     if (stor) h->storeA_frozen_valid = true;
-    smf_reduce_kernel<<<148 * 4, 256, 0, st>>>(d_part, (long)nb * l2, l2, ld, nx, d_c1);
+    smf_reduce_launch(st, d_part, ld, nx, nb, d_c1);
     L(h);
     if (allreduce(h, d_c1, (long)nb * l2)) return -2;
     SmfAlgArgs a;
@@ -2944,7 +2940,7 @@ int smf_batch_run(cgpcm_handle* h, const double* params_host, double reg, const 
     a.ld = ld; a.l2 = l2; a.ldh = nhp; a.nh = nh; a.nx = nx;
     a.r = r; a.c0 = c0; a.reg = reg; a.want_p = want_p; a.passes = passes;
     CK(cudaMemsetAsync(h->smf_info, 0, 2 * bcap * sizeof(int), st));
-    smf_algebra_kernel<<<dim3(nb, passes), SMF_ALG_THREADS, 2 * nx * sizeof(double), st>>>(a);
+    smf_algebra_launch(st, a, nb);
     L(h);
     CK(cudaGetLastError());
     CK(cudaMemcpyAsync(res.data(), d_out, (size_t)nb * 5 * sizeof(double), cudaMemcpyDeviceToHost, st));
@@ -3448,6 +3444,60 @@ int cgpcm_cholinv(double* A, double* Ainv, double* logdet, int n, int64_t ld, in
   if (W) cudaFree(W);
   if (ld_d) cudaFree(ld_d);
   if (info) cudaFree(info);
+  return rc;
+}
+
+int cgpcm_smf_c1_test(const double* W, int64_t w_stride, int B, int nwin, const int64_t* windows, int nx, int64_t ld,
+                      double* c1, void* stream) {
+  if (!W || !windows || !c1 || B < 1 || nwin < 1 || nx < 1 || (ld % 8) || round_up(nx, 8) > ld) return -1;
+  for (int w = 0; w < nwin; ++w) {
+    const int64_t k_lo = windows[4 * w], kwp = windows[4 * w + 1], nc = windows[4 * w + 2], off = windows[4 * w + 3];
+    if (kwp < 8 || kwp % 8 || nc < 8 || nc % 8 || k_lo < 0 || k_lo % 2 || k_lo + kwp > round_up(nx, 8) || off < 0 ||
+        off + nc * kwp > w_stride)
+      return -1;
+  }
+  cudaStream_t st = (cudaStream_t)stream;
+  double* part = nullptr;
+  const size_t bytes = (size_t)B * SMF_SLICES * ld * ld * sizeof(double);
+  if (cudaMalloc(&part, bytes) != cudaSuccess) { cudaGetLastError(); return -2; }
+  int rc = cudaMemsetAsync(part, 0, bytes, st) == cudaSuccess ? 0 : -2;
+  for (int w = 0; w < nwin && !rc; ++w) {
+    const int64_t* win = windows + 4 * w;
+    smf_c1_launch(st, W + win[3], w_stride, (int)win[1], (int)win[2], (int)win[0], part, ld, B);
+    if (cudaGetLastError() != cudaSuccess) rc = -2;
+  }
+  if (!rc) {
+    smf_reduce_launch(st, part, ld, nx, B, c1);
+    if (cudaGetLastError() != cudaSuccess) rc = -2;
+  }
+  if (cudaStreamSynchronize(st) != cudaSuccess) rc = -2;
+  cudaFree(part);
+  return rc;
+}
+
+int cgpcm_smf_algebra_test(const double* kx, const double* sum_Bxx, const double* c1, const double* sum_Ahx_y,
+                           const double* sum_Bhh, const double* samples, int B, int nx, int nh, int64_t ld, int ldh,
+                           double r, double c0, double reg, int want_p, int want_p0, double* out, int* info,
+                           void* stream) {
+  if (!kx || !sum_Bxx || !c1 || !sum_Ahx_y || !sum_Bhh || !samples || !out || !info || B < 1 || nx < 1 || nh < 1 ||
+      ld < nx || ld < nh || ldh < nh || (!want_p && !want_p0) || 2L * nx * sizeof(double) > 48 * 1024)
+    return -1;
+  cudaStream_t st = (cudaStream_t)stream;
+  const int passes = (want_p ? 1 : 0) + (want_p0 ? 1 : 0);
+  double* work = nullptr;
+  if (cudaMalloc(&work, (size_t)B * passes * ld * ld * sizeof(double)) != cudaSuccess) { cudaGetLastError(); return -2; }
+  SmfAlgArgs a;
+  a.kx = kx; a.sxx = sum_Bxx; a.c1 = c1; a.fy = sum_Ahx_y; a.bhh = sum_Bhh;
+  a.hs = samples; a.work = work; a.out = out; a.info = info;
+  a.ld = ld; a.l2 = ld * ld; a.ldh = ldh; a.nh = nh; a.nx = nx;
+  a.r = r; a.c0 = c0; a.reg = reg; a.want_p = want_p != 0; a.passes = passes;
+  int rc = cudaMemsetAsync(info, 0, 2 * (size_t)B * sizeof(int), st) == cudaSuccess ? 0 : -2;
+  if (!rc) {
+    smf_algebra_launch(st, a, B);
+    if (cudaGetLastError() != cudaSuccess) rc = -2;
+  }
+  if (cudaStreamSynchronize(st) != cudaSuccess) rc = -2;
+  cudaFree(work);
   return rc;
 }
 

@@ -202,4 +202,23 @@ __global__ void __launch_bounds__(SMF_ALG_THREADS) smf_algebra_kernel(const SmfA
   }
 }
 
+// Launch shapes of the three kernels, shared by smf_batch_run and the C-ABI test hooks.
+// part[b][z] += W_b^T W_b of one window (k_lo, kwp) over nc padded observations, for samples b < nb.
+inline void smf_c1_launch(cudaStream_t st, const double* W, long w_stride, int kwp, int nc, int k_lo, double* part,
+                          long ld, int nb) {
+  SmfC1Args g;
+  g.W = W; g.w_stride = w_stride; g.kwp = kwp; g.nc = nc;
+  g.part = part; g.l2 = ld * ld; g.ld = ld; g.win = (long)k_lo * ld + k_lo;
+  const int T = (kwp + SMF_T - 1) / SMF_T;
+  smf_c1_kernel<<<dim3(T * (T + 1) / 2, SMF_SLICES, nb), 128, 0, st>>>(g);
+}
+
+inline void smf_reduce_launch(cudaStream_t st, const double* part, long ld, int nx, int nb, double* c1) {
+  smf_reduce_kernel<<<148 * 4, 256, 0, st>>>(part, (long)nb * ld * ld, ld * ld, ld, nx, c1);
+}
+
+inline void smf_algebra_launch(cudaStream_t st, const SmfAlgArgs& a, int nb) {
+  smf_algebra_kernel<<<dim3(nb, a.passes), SMF_ALG_THREADS, 2 * a.nx * sizeof(double), st>>>(a);
+}
+
 }  // namespace cg

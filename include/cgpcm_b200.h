@@ -234,6 +234,24 @@ int cgpcm_math_test(const double* x, int64_t n, double* out_exp, double* out_erf
 /* cgpcm_math_test_fast: the variants the separable Psi kernels use: out_exp[i] = exp(min(x[i], 0)) with results below
  * 2^-1021 flushed to 0 (one integer add scales by 2^n), out_erfcx[i] = erfcx(|x[i]|) = exp(x^2) erfc(|x|). */
 int cgpcm_math_test_fast(const double* x, int64_t n, double* out_exp, double* out_erfcx);
+/* The kernels of cgpcm_elbo_smf_batch (csrc/smf_batch.cuh) with the launch shapes that call uses.  Device pointers only,
+ * except `windows`; stream: a cudaStream_t or NULL; both return after the stream has drained.
+ * cgpcm_smf_c1_test: c1[b] (B slabs of ld x ld) = sum over the windows of W_w,b^T W_w,b placed at (k_lo, k_lo), lower
+ * triangle of the leading nx x nx block, 0 elsewhere.  windows: host int64 [nwin][4] = (k_lo, kwp, nc, w_offset);
+ * window w reads W_w,b(n, k) = W[w_offset + b * w_stride + n * kwp + k] for n < nc, k < kwp.  The windows are added into
+ * zeroed per-slice partials in list order, then the slices are summed.  -1 unless kwp and nc are positive multiples of 8,
+ * k_lo is even, k_lo + kwp <= round_up(nx, 8) <= ld, ld % 8 == 0 and w_offset + nc * kwp <= w_stride.
+ * cgpcm_smf_algebra_test: per sample b (samples[b * ldh + i], i < nh), with S_b = sum_Bxx + C1_b (lower triangles of
+ * the nx x nx blocks at leading dimension ld are read) and lam_b = c0 sum_Ahx_y^T h_b (sum_Ahx_y: nh x nx at ld):
+ * out[b][0..1] = log det P_b, |L^-1 lam_b|^2 of P_b = Kx + r S_b + reg I (want_p), out[b][2..3] the same for
+ * P0_b = Kx + r S_b and out[b][4] = h_b^T sum_Bhh h_b (want_p0); entries of a pass not run are not written.
+ * info[b][0 / 1] (int, device) = pivot + 1 of a failed factorisation of P_b / P0_b, else 0.  nx <= 3072. */
+int cgpcm_smf_c1_test(const double* W, int64_t w_stride, int B, int nwin, const int64_t* windows, int nx, int64_t ld,
+                      double* c1, void* stream);
+int cgpcm_smf_algebra_test(const double* kx, const double* sum_Bxx, const double* c1, const double* sum_Ahx_y,
+                           const double* sum_Bhh, const double* samples, int B, int nx, int nh, int64_t ld, int ldh,
+                           double r, double c0, double reg, int want_p, int want_p0, double* out, int* info,
+                           void* stream);
 
 #ifdef __cplusplus
 }

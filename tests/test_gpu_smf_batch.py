@@ -2,6 +2,7 @@
 samples per call (rank-one contraction C1_b = sum_n w_bn w_bn^T, w_bn = A_n^T h_b) against the oracle and against the
 single-sample cgpcm_elbo_smf in MODE_FROZEN; bitwise independence of the batch; VCGPCM.sample(chains=C)."""
 import os
+import re
 import socket
 import subprocess
 import sys
@@ -18,7 +19,7 @@ from oracle import model as om
 from tests.cases import make_case, ulp_noise
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-CASES = ['toy_small', 'toy_test', 'sweep_hi', 'crude', 'toy_acausal_model', 'toy_small_cid']
+CASES = ['toy_small', 'toy_test', 'sweep_hi', 'crude', 'toy_acausal_model', 'toy_small_cid', 'ou', 'hrir']
 
 
 def _engine(c, **opts):
@@ -67,6 +68,30 @@ def test_batch_matches_oracle_and_single_sample(name):
     # loglik only / elbo only
     _, _, ll2 = eng.elbo_smf_batch(c['params'], S, reg=c['reg'], want_elbo=False)
     assert np.array_equal(ll2, ll)
+
+
+def test_batch_with_narrow_windows_matches_oracle(capfd, monkeypatch):
+    """'sweep_wide': 3000 observations over 40 inducing inputs in chunks of 256 observations, so the chunks contract
+    narrow windows, at k_lo > 0 past the first, and neighbouring chunks add overlapping windows into the same C1 slab."""
+    c = make_case('sweep_wide')
+    monkeypatch.setenv('CGPCM_DEBUG_PLAN', '1')
+    eng = _engine(c, chunk=256)
+    eng.precompute(*c['hyp'], reg=c['reg'])
+    capfd.readouterr()
+    S = _samples(c, 2)
+    e, t, ll = eng.elbo_smf_batch(c['params'], S, reg=c['reg'])
+    plan = [tuple(int(v) for v in m) for m in re.findall(r'\((\d+) x (\d+) @(\d+)\)', capfd.readouterr().err)]
+    assert len(plan) > 1 and all(kwp < c['nx'] for _, kwp, _ in plan) and any(k_lo > 0 for _, _, k_lo in plan), plan
+    om.PW_DISTS_EXACT = True
+    try:
+        (e0, t0, ll0), (en, tn, lln) = ulp_noise(
+            lambda p, th: om.elbo_smf(p, c['t'], c['y'], th, c['tx'], c['reg'], S[0]), c['params'], c['th'], trials=1)
+    finally:
+        om.PW_DISTS_EXACT = False
+    scale = max(abs(e0), np.abs(t0).max())
+    assert abs(e[0] - e0) <= 1e-9 * scale + 3 * en and np.abs(t[0] - t0).max() <= 1e-9 * scale + 3 * tn
+    assert abs(ll[0] - ll0) <= 1e-9 * max(abs(ll0), np.abs(t0[2:4]).max()) + 3 * lln
+    _check_against_single(eng, c, S, e, t, ll)
 
 
 def test_batch_invariance_is_bitwise():
