@@ -693,6 +693,22 @@ class VCGPCM(CGPCM):
         return UncertainData(mean=Data(t, mu), lower=Data(t, mu - 2 * std), upper=Data(t, mu + 2 * std),
                              std=Data(t, std))
 
+    def predict_f_samples(self, t, samples_h=50):
+        """Predictive mean and variance of the function at ``t`` for each filter sample: ``(mean[n, B], var[n, B])``.
+        ``samples_h`` as in :meth:`predict_f`: a number draws that many samples from q(u), all under the optimal q(z)
+        of q(u); a list of filter samples (e.g. the states of :meth:`sample`, flattened over chains) gives each its
+        own q(z | h_b).  :meth:`predict_f`'s mean and variance are the row means ``mean.mean(1)`` and ``var.mean(1)``;
+        the variance of the mixture of the samples' predictive distributions is ``var.mean(1) + mean.var(1)``."""
+        t = np.asarray(getattr(t, 'x', t), dtype=np.float64).ravel()
+        if np.isscalar(samples_h) or isinstance(samples_h, (int, np.integer)):
+            samples, smf = [self.sample_q() for _ in range(int(samples_h))], False
+        else:
+            samples, smf = list(samples_h), True
+        samples = np.stack([np.asarray(x, dtype=np.float64).ravel() for x in samples])
+        _, _, mean, var = self._with_frozen_stats(
+            lambda: self.engine.predict_f_batch(self._pack(), t, samples, smf=smf, reg=config.reg))
+        return mean, var
+
     def predict_k(self, t, samples_h=200, psd=False, normalise=True):
         """Predict the kernel, or the PSD via the kernel approximation, at lags ``t``
         (``src/core/cgpcm.py:610-661``): Monte-Carlo over filter samples (numeric ``samples_h``: draws from q(u)).

@@ -2354,12 +2354,94 @@ int qz_run(cgpcm_handle* h, const double* params_host, const double* qz_mean, co
   return 0;
 }
 
+// The moments of q(u) as predict_f uses them: mu (V_MU), var = L L^T + reg I (M_VAR), and tr(Ahh iKh) (S_TR_IKH_AHH).
+int predict_qu(cgpcm_handle* h, double reg) {
+  const int nh = h->nh, nhp = h->nhp;
+  const long ld = h->ld, l2 = ld * ld;
+  cudaStream_t st = h->st;
+  double* Lq = h->M(M_LQ);
+  double* mu = h->V(V_MU);
+  double* var = h->M(M_VAR);
+  const double* pd = h->params_d;
+  ew(st, l2, [=] __device__(long idx) {
+    int i = (int)(idx / ld), j = (int)(idx % ld);
+    Lq[idx] = (i < nh && j <= i) ? pd[5 + nh + (long)i * (i + 1) / 2 + j] : 0.0;
+    if (idx < ld) mu[idx] = idx < nh ? pd[5 + idx] : 0.0;
+  });
+  L(h);
+  if (mm(h, Lq, false, Lq, true, var, nhp, nhp, nhp)) return -2;
+  ew(st, l2, [=] __device__(long idx) {
+    int i = (int)(idx / ld), j = (int)(idx % ld);
+    if (i == j && i < nh) var[idx] += reg;
+  });
+  L(h);
+  frob(h, h->M(M_AHH), h->M(M_IKH), nh, nh, h->sc + S_TR_IKH_AHH);
+  return 0;
+}
+
+// One optimal q(z) of predict_f: Hm = m m^T (smf: m = a filter sample) or var + m m^T (m = mu of q(u)), C1 over the
+// frozen statistics, P = Kx + r (sum_Bxx + C1) + reg I, P^-1 in M_PINV and xm = P^-1 c0 sum_Ahx_y^T m.
+int predict_qz(cgpcm_handle* h, const std::vector<Chunk>& chunks, int smf, const double* mvec, const double* var,
+               double r, double c0, double reg, double* xm) {
+  const int nh = h->nh, nx = h->nx, nxp = h->nxp;
+  const long ld = h->ld, l2 = ld * ld;
+  cudaStream_t st = h->st;
+  double* Hm = h->M(M_H);
+  const int smf_ = smf;
+  ew(st, l2, [=] __device__(long idx) {
+    int i = (int)(idx / ld), j = (int)(idx % ld);
+    Hm[idx] = smf_ ? mvec[i] * mvec[j] : var[idx] + mvec[i] * mvec[j];
+  });
+  L(h);
+  if (frozen_c1(h, chunks, Hm)) return -2;
+  if (allreduce(h, h->M(M_C1), l2)) return -2;
+  double* Pm = h->M(M_LP);
+  const double* kx = h->M(M_KX);
+  const double* fb = h->M(M_F_AXX);
+  const double* c1 = h->M(M_C1);
+  ew(st, l2, [=] __device__(long idx) {
+    int i = (int)(idx / ld), j = (int)(idx % ld);
+    Pm[idx] = kx[idx] + r * (fb[idx] + c1[idx]) + ((i == j && i < nx) ? reg : 0.0);
+  });
+  L(h);
+  if (chol_inv(h, Pm, h->M(M_PINV), nx, nxp, nullptr, 3)) return -2;
+  matvec(h, h->M(M_F_Y), nx, nh, 1, mvec, c0, h->V(V_LAM));
+  matvec(h, h->M(M_PINV), nx, nx, 0, h->V(V_LAM), 1.0, xm);
+  return 0;
+}
+
+// Test-side blocks of a chunk of nv test points at tc: A* (h->wsA, [i][n][k] at kw = nxp), T = iKh A* (h->wsT) and
+// Bxx*_n = Axx*_n - A*_n^T iKh A*_n (dense [n][nx][nx] in X).
+int predict_chunk_blocks(cgpcm_handle* h, const PsiConst& cd, const BvnTab& T, const double* tc, int nv, double* X) {
+  const int nh = h->nh, nx = h->nx, nhp = h->nhp, nxp = h->nxp;
+  const long ld = h->ld;
+  cudaStream_t st = h->st;
+  const int nc = round_up(nv, 8);
+  const long cols = (long)nc * nxp;
+  {
+    const int threads = std::min(256, round_up(nxp, 32));
+    dim3 grid(nhp, (nc + AHX_NSUB - 1) / AHX_NSUB);
+    ahx_gen_kernel<<<grid, threads, 0, st>>>(tc, tc, nv, nc, h->th, nh, h->tx, nx, 0, nxp, h->wsA, nullptr, ld,
+                                             (long)nhp * ld, cd);
+    L(h);
+  }
+  if (gemm(h, true, false, false, nhp, (int)cols, nhp, 1.0, h->M(M_IKH), ld, h->wsA, cols, 0.0, h->wsT, cols)) return -2;
+  axx_user_kernel<<<148 * 8, 256, 0, st>>>(tc, nv, h->tx, nx, X, cd, T);
+  L(h);
+  {
+    dim3 grid((nx + 31) / 32, (nx + 31) / 32, nv);
+    bxx_star_kernel<<<grid, 256, 0, st>>>(h->wsA, h->wsT, nh, nc, nxp, nx, X);
+    L(h);
+  }
+  return 0;
+}
+
 // VCGPCM.predict_f (src/core/cgpcm.py:781-846) for given filter samples: posterior mean and variance of the function
 // at the test inputs, averaged over the samples.  smf = 0: one optimal q(z) from the moments of q(u); smf = 1: the
 // optimal q(z | h) per sample.  Training side: the frozen regime's sweeps; test side: predict_kernels.cuh.
 int predict_run(cgpcm_handle* h, const double* params_host, double reg, const double* tstar_host, long n_star,
                 const double* samples_host, int B, int smf, double* mu_out, double* var_out) {
-  const int nh = h->nh, nx = h->nx, nhp = h->nhp, nxp = h->nxp;
+  const int nh = h->nh, nx = h->nx, nxp = h->nxp;
   const long ld = h->ld, l2 = ld * ld;
   const long np = 5 + nh + (long)nh * (nh + 1) / 2;
   for (long i = 0; i < np; ++i)
@@ -2416,54 +2498,16 @@ int predict_run(cgpcm_handle* h, const double* params_host, double reg, const do
   PCK(cudaMemsetAsync(d_acc, 0, (size_t)2 * std::max<long>(n_star, 1) * sizeof(double), st));
   PRC(prior_stage(h, c, reg, true));
   if (!h->gram_valid) PRC(plan_store(h, chunks, false));
-  // q(u) moments
-  double* Lq = h->M(M_LQ);
-  double* mu = h->V(V_MU);
-  double* var = h->M(M_VAR);
-  double* Hm = h->M(M_H);
-  {
-    const double* pd = h->params_d;
-    ew(st, l2, [=] __device__(long idx) {
-      int i = (int)(idx / ld), j = (int)(idx % ld);
-      Lq[idx] = (i < nh && j <= i) ? pd[5 + nh + (long)i * (i + 1) / 2 + j] : 0.0;
-      if (idx < ld) mu[idx] = idx < nh ? pd[5 + idx] : 0.0;
-    });
-    L(h);
-    PRC(mm(h, Lq, false, Lq, true, var, nhp, nhp, nhp));
-    ew(st, l2, [=] __device__(long idx) {
-      int i = (int)(idx / ld), j = (int)(idx % ld);
-      if (i == j && i < nh) var[idx] += reg;
-    });
-    L(h);
-  }
-  frob(h, h->M(M_AHH), h->M(M_IKH), nh, nh, h->sc + S_TR_IKH_AHH);
+  PRC(predict_qu(h, reg));
+  const double* mu = h->V(V_MU);
+  const double* var = h->M(M_VAR);
   const double a_val = (h->causal ? 0.5 : 1.0) * sqrt(3.14159265358979323846 / (2.0 * alpha));
   // ---- training side: q(z) (once, or per sample) and the per-sample scalar q1
   for (int b = 0; b < std::max(B, nq); ++b) {
     const double* hb = d_h + (long)b * ld;
     if (b < nq) {
-      const double* mvec = smf ? hb : mu;
-      const int smf_ = smf;
-      ew(st, l2, [=] __device__(long idx) {
-        int i = (int)(idx / ld), j = (int)(idx % ld);
-        Hm[idx] = smf_ ? mvec[i] * mvec[j] : var[idx] + mvec[i] * mvec[j];
-      });
-      L(h);
-      PRC(frozen_c1(h, chunks, Hm));
-      PRC(allreduce(h, h->M(M_C1), l2));
-      double* Pm = h->M(M_LP);
-      const double* kx = h->M(M_KX);
-      const double* fb = h->M(M_F_AXX);
-      const double* c1 = h->M(M_C1);
-      ew(st, l2, [=] __device__(long idx) {
-        int i = (int)(idx / ld), j = (int)(idx % ld);
-        Pm[idx] = kx[idx] + r * (fb[idx] + c1[idx]) + ((i == j && i < nx) ? reg : 0.0);
-      });
-      L(h);
-      PRC(chol_inv(h, Pm, h->M(M_PINV), nx, nxp, nullptr, 3));
       double* xm = d_xm + (long)b * ld;
-      matvec(h, h->M(M_F_Y), nx, nh, 1, mvec, c0, h->V(V_LAM));
-      matvec(h, h->M(M_PINV), nx, nx, 0, h->V(V_LAM), 1.0, xm);
+      PRC(predict_qz(h, chunks, smf, smf ? hb : mu, var, r, c0, reg, xm));
       double* mxb = d_mx + (long)b * l2;
       const double* xv = h->M(M_PINV);
       const double* ikx = h->M(M_IKX);
@@ -2487,23 +2531,7 @@ int predict_run(cgpcm_handle* h, const double* params_host, double reg, const do
   for (long p0 = 0; p0 < n_star; p0 += TC) {
     const int nv = (int)std::min<long>(TC, n_star - p0);
     const int nc = round_up(nv, 8);
-    const long cols = (long)nc * nxp;
-    const double* tc = d_t + p0;
-    {
-      const int threads = std::min(256, round_up(nxp, 32));
-      dim3 grid(nhp, (nc + AHX_NSUB - 1) / AHX_NSUB);
-      ahx_gen_kernel<<<grid, threads, 0, st>>>(tc, tc, nv, nc, h->th, nh, h->tx, nx, 0, nxp, h->wsA, nullptr, ld,
-                                               (long)nhp * ld, cd);
-      L(h);
-    }
-    PRC(gemm(h, true, false, false, nhp, (int)cols, nhp, 1.0, h->M(M_IKH), ld, h->wsA, cols, 0.0, h->wsT, cols));
-    axx_user_kernel<<<148 * 8, 256, 0, st>>>(tc, nv, h->tx, nx, d_x, cd, T);
-    L(h);
-    {
-      dim3 grid((nx + 31) / 32, (nx + 31) / 32, nv);
-      bxx_star_kernel<<<grid, 256, 0, st>>>(h->wsA, h->wsT, nh, nc, nxp, nx, d_x);
-      L(h);
-    }
+    PRC(predict_chunk_blocks(h, cd, T, d_t + p0, nv, d_x));
     for (int b = 0; b < B; ++b) {
       const int qb = smf ? b : 0;
       predict_point_kernel<<<nv, 256, nx * sizeof(double), st>>>(h->wsA, nh, nc, nxp, nx, d_h + (long)b * ld,
@@ -2806,6 +2834,39 @@ int smf_bcap(const cgpcm_handle* h) {
   return std::max(8, b);
 }
 
+// The per-batch C1 stage of the batched SMF paths: stage nb <= bcap samples (host, nb x nh) into d_hs (bcap x nhp,
+// zero rows past nb), then per chunk W = H_B A (the small-left GEMM over the resident or regenerated Ahx block, always
+// bcap rows) and part_b += W_b^T W_b (smf_c1_kernel), the slice sum into the C1 slabs and one all-reduce of them.
+int smf_c1_stage(cgpcm_handle* h, const std::vector<Chunk>& chunks, const double* samples_host, int nb, int bcap,
+                 std::vector<double>& hsm, double* d_hs, double* d_part, double* d_c1, double* d_w, long wstride) {
+  const int nh = h->nh, nx = h->nx, nhp = h->nhp;
+  const long ld = h->ld, l2 = ld * ld;
+  cudaStream_t st = h->st;
+  hsm.assign((size_t)bcap * nhp, 0.0);
+  for (int b = 0; b < nb; ++b)
+    for (int i = 0; i < nh; ++i) hsm[(size_t)b * nhp + i] = samples_host[(size_t)b * nh + i];
+  // (pageable source: staged before the call returns)
+  CK(cudaMemcpyAsync(d_hs, hsm.data(), hsm.size() * sizeof(double), cudaMemcpyHostToDevice, st));
+  CK(cudaMemsetAsync(d_part, 0, (size_t)nb * SMF_SLICES * l2 * sizeof(double), st));
+  const bool stor = h->use_store;
+  const bool have_a = stor && h->storeA_frozen_valid;
+  for (const Chunk& ch : chunks) {
+    double* Ab = stor ? h->storeA + ch.off : h->wsA;
+    if (!have_a && gen_chunk(h, h->fc, ch, false, Ab)) return -2;
+    const long cols = (long)ch.nc * ch.kwp;
+    // W[b][(n,k)] = sum_i h_b[i] A[i][(n,k)]
+    if (gemm(h, true, false, false, bcap, (int)cols, nhp, 1.0, d_hs, nhp, Ab, cols, 0.0, d_w, wstride)) return -2;
+    prof_close(h);
+    smf_c1_launch(st, d_w, wstride, ch.kwp, ch.nc, ch.k_lo, d_part, ld, nb);
+    h->gemm_flops += (double)nb * ch.nc * ch.kwp * (ch.kwp + 1.0);
+    L(h);
+  }
+  if (stor) h->storeA_frozen_valid = true;
+  smf_reduce_launch(st, d_part, ld, nx, nb, d_c1);
+  L(h);
+  return allreduce(h, d_c1, (long)nb * l2);
+}
+
 // VCGPCM.elbo(smf=True, sample=h_b) and the slice sampler's log-likelihood (src/core/cgpcm.py:527-531,594-608,848-872)
 // for B samples in the frozen regime.  Per call: the terms that do not depend on the sample (the prior, q(u) and
 // its KL, the frozen sums), as evaluate_once forms them.  Per batch of <= smf_bcap samples: per chunk W = H_B A (the
@@ -2911,29 +2972,8 @@ int smf_batch_run(cgpcm_handle* h, const double* params_host, double reg, const 
   const long wstride = wcols;
   for (int b0 = 0; b0 < B; b0 += bcap) {
     const int nb = std::min(bcap, B - b0);
-    std::fill(hsm.begin(), hsm.end(), 0.0);
-    for (int b = 0; b < nb; ++b)
-      for (int i = 0; i < nh; ++i) hsm[(size_t)b * nhp + i] = samples_host[(size_t)(b0 + b) * nh + i];
-    // (pageable source: staged before the call returns)
-    CK(cudaMemcpyAsync(d_hs, hsm.data(), hsm.size() * sizeof(double), cudaMemcpyHostToDevice, st));
-    CK(cudaMemsetAsync(d_part, 0, (size_t)nb * SMF_SLICES * l2 * sizeof(double), st));
-    const bool stor = h->use_store;
-    const bool have_a = stor && h->storeA_frozen_valid;
-    for (const Chunk& ch : chunks) {
-      double* Ab = stor ? h->storeA + ch.off : h->wsA;
-      if (!have_a && gen_chunk(h, h->fc, ch, false, Ab)) return -2;
-      const long cols = (long)ch.nc * ch.kwp;
-      // W[b][(n,k)] = sum_i h_b[i] A[i][(n,k)]
-      if (gemm(h, true, false, false, bcap, (int)cols, nhp, 1.0, d_hs, nhp, Ab, cols, 0.0, d_w, wstride)) return -2;
-      prof_close(h);
-      smf_c1_launch(st, d_w, wstride, ch.kwp, ch.nc, ch.k_lo, d_part, ld, nb);
-      h->gemm_flops += (double)nb * ch.nc * ch.kwp * (ch.kwp + 1.0);
-      L(h);
-    }
-    if (stor) h->storeA_frozen_valid = true;
-    smf_reduce_launch(st, d_part, ld, nx, nb, d_c1);
-    L(h);
-    if (allreduce(h, d_c1, (long)nb * l2)) return -2;
+    if (smf_c1_stage(h, chunks, samples_host + (size_t)b0 * nh, nb, bcap, hsm, d_hs, d_part, d_c1, d_w, wstride))
+      return -2;
     SmfAlgArgs a;
     a.kx = h->M(M_KX); a.sxx = h->M(M_F_AXX); a.c1 = d_c1; a.fy = h->M(M_F_Y); a.bhh = h->M(M_F_BHH);
     a.hs = d_hs; a.work = d_work; a.out = d_out; a.info = h->smf_info;
@@ -2972,6 +3012,233 @@ int smf_batch_run(cgpcm_handle* h, const double* params_host, double reg, const 
   }
   CK(cudaEventRecord(h->ev[6], st));
   CK(cudaStreamSynchronize(st));
+  float ms = 0;
+  cudaEventElapsedTime(&ms, h->ev[0], h->ev[6]);
+  memset(h->timing, 0, sizeof h->timing);
+  h->timing[0] = ms;
+  h->timing[6] = (double)h->launches;
+  h->timing[7] = h->gemm_flops;
+  h->timing[8] = (double)h->gemm_launches;
+  return 0;
+}
+
+// Samples per internal batch of predict_batch_run: a function of the handle's shape only (every launch of the batch
+// is shaped for this many samples).  Per sample: the C1 partials and slab and the two slabs of smf_posterior_kernel
+// (SMF_SLICES + 3 ld x ld), and V_b of a test chunk (chunk x nxp), within ~1 GB.
+int predict_bcap(const cgpcm_handle* h) {
+  const double per = ((SMF_SLICES + 3.0) * (double)h->ld * h->ld + (double)h->chunk * h->nxp) * sizeof(double);
+  const int b = (int)std::min(64.0, 1e9 / per) / 8 * 8;
+  return std::max(8, b);
+}
+
+// predict_f's moments for each of B filter samples (and their average, as predict_run forms it) in the frozen regime.
+// Training side: smf = 0, the one q(z) of q(u) (predict_qz, as predict_run); smf = 1, per batch of bcap samples the C1
+// stage of smf_batch_run and smf_posterior_kernel (P_b, xm_b, mx_b, q1_b).  Test side, per chunk of test points: A* and
+// Bxx* once (predict_chunk_blocks), then per batch V = H_B A* (small-left GEMM), Qb = <Bxx*, mx_b> (predict_qb_kernel),
+// v^T mx_b v and v . xm_b (predict_quad_kernel) and predict_finish_kernel.  With smf = 1 the samples go in groups whose
+// mx slabs fit ~1 GB; A* and Bxx* are rebuilt per group.
+int predict_batch_run(cgpcm_handle* h, const double* params_host, double reg, const double* tstar_host, long n_star,
+                      const double* samples_host, int B, int smf, double* mu_out, double* var_out, double* mean_s_out,
+                      double* var_s_out) {
+  const int nh = h->nh, nx = h->nx, nhp = h->nhp, nxp = h->nxp;
+  const long ld = h->ld, l2 = ld * ld;
+  const long np = 5 + nh + (long)nh * (nh + 1) / 2;
+  for (long i = 0; i < np; ++i)
+    if (!std::isfinite(params_host[i])) { h->err = "non-finite parameter"; return -4; }
+  for (long i = 0; i < n_star; ++i)
+    if (!std::isfinite(tstar_host[i])) { h->err = "non-finite test input"; return -4; }
+  for (long i = 0; i < (long)B * nh; ++i)
+    if (!std::isfinite(samples_host[i])) {
+      char b[96];
+      snprintf(b, sizeof b, "non-finite value in sample %ld", i / nh);
+      h->err = b;
+      return -4;
+    }
+  if (!h->frozen) { h->err = "cgpcm_predict_f_batch requires cgpcm_precompute"; return -1; }
+  const double s2 = exp(params_host[0]), s2f = exp(params_host[1]);
+  const double alpha = exp(params_host[2]), gamma = exp(params_host[3]), omega = exp(params_host[4]);
+  const double r = s2f / s2, c0 = sqrt(s2f) / s2;
+  if (ensure_sweep_buffers(h)) return -2;
+  h->launches = 0;
+  h->pev_used = 0;
+  h->prof_open = false;
+  h->gemm_flops = h->gemm_flops_exec = 0.0;
+  h->gemm_launches = 0;
+  PsiConst c;
+  psi_make_const(alpha, gamma, omega, h->causal, h->cull, &c, h->causal_id);
+  PsiConst cd = c;                       // test-side statistics are evaluated densely (no windows)
+  cd.cull = 746.0;
+  BvnTab T;
+  bvn_make_tab(gamma / (alpha + gamma + omega), &T);
+  std::vector<Chunk> chunks;
+  plan_chunks(h, h->fc, chunks);
+  if (ensure_ypart(h, y_slices_used(chunks))) return -2;
+  cudaStream_t st = h->st;
+  const int TC = std::min<long>(h->chunk, n_star);
+  const int TCP = round_up(TC, 8);
+  const int bcap = predict_bcap(h);
+  const int gcap = smf ? std::max(bcap, std::min(round_up(B, bcap), (int)(1e9 / (l2 * 8.0)) / bcap * bcap))
+                       : round_up(B, bcap);
+  const int nq = smf ? gcap : 1;         // q(z) slabs held at a time
+  long wcols = 0;
+  for (const Chunk& ch : chunks) wcols = std::max<long>(wcols, (long)ch.nc * ch.kwp);
+  const bool per_sample = mean_s_out || var_s_out;
+  // [t][acc 2 n*][per-sample 2 n* B][X][hs][q1][xm][mx][part][c1][work][W][V][qpart][quad][lin]
+  long off = 0;
+  auto take = [&](long n) { const long o = off; off += (n + 1) / 2 * 2; return o; };     // 16-byte aligned
+  const long o_t = take(n_star), o_acc = take(2 * n_star), o_ps = take(per_sample ? 2 * n_star * B : 0);
+  const long o_x = take((long)TC * nx * nx), o_hs = take((long)gcap * nhp), o_q1 = take(gcap);
+  const long o_xm = take((long)nq * ld), o_mx = take((long)nq * l2);
+  const long o_part = take(smf ? (long)bcap * SMF_SLICES * l2 : 0), o_c1 = take(smf ? (long)bcap * l2 : 0);
+  const long o_work = take(smf ? 2L * bcap * l2 : 0), o_w = take(smf ? (long)bcap * wcols : 0);
+  const long vstride = (long)TCP * nxp;
+  const long o_v = take((long)bcap * vstride), o_qp = take((long)PQ_SLICES * TC * bcap);
+  const long o_quad = take((long)TC * bcap), o_lin = take((long)TC * bcap);
+  double* buf = nullptr;
+  int* d_info = nullptr;
+  auto cleanup = [&]() {
+    if (buf) cudaFree(buf);
+    if (d_info) cudaFree(d_info);
+  };
+#define PCK(call) do { cudaError_t e_ = (call); if (e_ != cudaSuccess) { char b_[256]; snprintf(b_, sizeof b_, \
+    "CUDA error %s in predict_f_batch (%s)", cudaGetErrorString(e_), #call); h->err = b_; cleanup(); return -2; } } while (0)
+#define PRC(call) do { if (call) { cleanup(); return -2; } } while (0)
+  PCK(cudaMalloc(&buf, (size_t)off * sizeof(double)));
+  PCK(cudaMalloc(&d_info, (size_t)bcap * sizeof(int)));
+  double *d_t = buf + o_t, *d_acc = buf + o_acc, *d_ps = buf + o_ps, *d_x = buf + o_x, *d_hs = buf + o_hs;
+  double *d_q1 = buf + o_q1, *d_xm = buf + o_xm, *d_mx = buf + o_mx, *d_part = buf + o_part, *d_c1 = buf + o_c1;
+  double *d_work = buf + o_work, *d_w = buf + o_w, *d_v = buf + o_v, *d_qp = buf + o_qp, *d_quad = buf + o_quad;
+  double* d_lin = buf + o_lin;
+  PCK(cudaEventRecord(h->ev[0], st));
+  PCK(cudaMemsetAsync(h->info, 0, 4 * sizeof(int), st));
+  PCK(cudaMemcpyAsync(h->params_d, params_host, np * sizeof(double), cudaMemcpyHostToDevice, st));
+  PCK(cudaMemcpyAsync(d_t, tstar_host, n_star * sizeof(double), cudaMemcpyHostToDevice, st));
+  PCK(cudaMemsetAsync(d_acc, 0, (size_t)2 * n_star * sizeof(double), st));
+  PRC(prior_stage(h, c, reg, true));
+  if (smf || !h->gram_valid) PRC(plan_store(h, chunks, false));
+  PRC(predict_qu(h, reg));
+  const double a_val = (h->causal ? 0.5 : 1.0) * sqrt(3.14159265358979323846 / (2.0 * alpha));
+  if (!smf) {
+    // the one q(z) of q(u), as predict_run forms it; mx in the dense nx x nx layout of the test-side kernels
+    PRC(predict_qz(h, chunks, 0, h->V(V_MU), h->M(M_VAR), r, c0, reg, d_xm));
+    const double* xv = h->M(M_PINV);
+    const double* ikx = h->M(M_IKX);
+    const double* xm = d_xm;
+    double* mx = d_mx;
+    ew(st, (long)nx * nx, [=] __device__(long idx) {
+      const int i = (int)(idx / nx), j = (int)(idx % nx);
+      const long e = (long)i * ld + j;
+      mx[idx] = xv[e] + xm[i] * xm[j] - ikx[e];
+    });
+    L(h);
+  }
+  {
+    // a failed factorisation of the prior or of the shared q(z)
+    int info[4];
+    PCK(cudaMemcpyAsync(info, h->info, sizeof info, cudaMemcpyDeviceToHost, st));
+    PCK(cudaStreamSynchronize(st));
+    if (info[0]) {
+      h->prior_valid = false;
+      static const char* names[] = {"?", "Kh", "Kx", "P of q(z)", "?", "?"};
+      const int tag = info[0] / 100000;
+      char b[160];
+      snprintf(b, sizeof b, "matrix %s is not positive definite (pivot %d)", tag >= 1 && tag <= 5 ? names[tag] : "?",
+               info[0] % 100000);
+      h->err = b;
+      cleanup();
+      return -3;
+    }
+  }
+  std::vector<double> hsm;
+  std::vector<int> inf(bcap);
+  const double w = 1.0 / B;
+  for (int g0 = 0; g0 < B; g0 += gcap) {
+    const int gn = std::min(gcap, B - g0);
+    const int nbat = (gn + bcap - 1) / bcap;
+    // ---- training side of the group
+    for (int bi = 0; bi < nbat; ++bi) {
+      const int b0 = g0 + bi * bcap, nb = std::min(bcap, B - b0);
+      double* hs = d_hs + (long)bi * bcap * nhp;
+      double* q1 = d_q1 + (long)bi * bcap;
+      if (smf) {
+        PRC(smf_c1_stage(h, chunks, samples_host + (size_t)b0 * nh, nb, bcap, hsm, hs, d_part, d_c1, d_w, wcols));
+        SmfPostArgs a;
+        a.kx = h->M(M_KX); a.sxx = h->M(M_F_AXX); a.c1 = d_c1; a.fy = h->M(M_F_Y); a.ahh = h->M(M_AHH);
+        a.ikx = h->M(M_IKX); a.tr = h->sc + S_TR_IKH_AHH; a.hs = hs; a.work = d_work;
+        a.mx = d_mx + (long)bi * bcap * l2; a.xm = d_xm + (long)bi * bcap * ld; a.q1 = q1; a.info = d_info;
+        a.ld = ld; a.l2 = l2; a.ldh = nhp; a.nh = nh; a.nx = nx; a.nb = nb;
+        a.r = r; a.c0 = c0; a.reg = reg; a.a = a_val;
+        PCK(cudaMemsetAsync(d_info, 0, bcap * sizeof(int), st));
+        smf_posterior_launch(st, a, bcap);
+        L(h);
+        PCK(cudaGetLastError());
+        PCK(cudaMemcpyAsync(inf.data(), d_info, bcap * sizeof(int), cudaMemcpyDeviceToHost, st));
+        PCK(cudaStreamSynchronize(st));
+        for (int b = 0; b < nb; ++b)
+          if (inf[b]) {
+            char m[160];
+            snprintf(m, sizeof m, "matrix P of sample %d is not positive definite (pivot %d)", b0 + b, inf[b]);
+            h->err = m;
+            cleanup();
+            return -3;
+          }
+      } else {
+        hsm.assign((size_t)bcap * nhp, 0.0);
+        for (int b = 0; b < nb; ++b)
+          for (int i = 0; i < nh; ++i) hsm[(size_t)b * nhp + i] = samples_host[(size_t)(b0 + b) * nh + i];
+        // (pageable source: staged before the call returns)
+        PCK(cudaMemcpyAsync(hs, hsm.data(), hsm.size() * sizeof(double), cudaMemcpyHostToDevice, st));
+        predict_q1_kernel<<<bcap, 256, 0, st>>>(h->M(M_AHH), ld, hs, nhp, nh, nb, a_val, h->sc + S_TR_IKH_AHH, q1);
+        L(h);
+      }
+    }
+    // ---- test side of the group, chunk by chunk
+    for (long p0 = 0; p0 < n_star; p0 += TC) {
+      const int nv = (int)std::min<long>(TC, n_star - p0);
+      const long cols = (long)round_up(nv, 8) * nxp;
+      PRC(predict_chunk_blocks(h, cd, T, d_t + p0, nv, d_x));
+      if (!smf) {
+        predict_qb_launch(st, d_x, (long)nx * nx, d_mx, l2, 1, nv, TC, 1, d_qp, bcap);     // one column
+        L(h);
+      }
+      for (int bi = 0; bi < nbat; ++bi) {
+        const int b0 = g0 + bi * bcap, nb = std::min(bcap, B - b0);
+        const double* hs = d_hs + (long)bi * bcap * nhp;
+        // V[b][(n,k)] = sum_i h_b[i] A*[i][(n,k)]
+        PRC(gemm(h, true, false, false, bcap, (int)cols, nhp, 1.0, hs, nhp, h->wsA, cols, 0.0, d_v, vstride));
+        prof_close(h);
+        const double* mx = smf ? d_mx + (long)bi * bcap * l2 : d_mx;
+        const double* xm = smf ? d_xm + (long)bi * bcap * ld : d_xm;
+        if (smf) {
+          predict_qb_launch(st, d_x, (long)nx * nx, mx, l2, nb, nv, TC, bcap, d_qp, bcap);
+          L(h);
+        }
+        PredQuadArgs qa;
+        qa.V = d_v; qa.v_stride = vstride; qa.ldv = nxp;
+        qa.mx = mx; qa.mx_stride = smf ? l2 : 0; qa.xm = xm; qa.xm_stride = smf ? ld : 0;
+        qa.nv = nv; qa.nx = nx; qa.nb = nb; qa.quad = d_quad; qa.lin = d_lin; qa.ldo = bcap;
+        predict_quad_launch(st, qa, bcap);
+        L(h);
+        predict_finish_kernel<<<(nv + 127) / 128, 128, 0, st>>>(
+            d_qp, TC, bcap, smf ? 1 : 0, d_quad, d_lin, bcap, d_q1 + (long)bi * bcap, nv, nb, sqrt(s2f), s2f, w,
+            mean_s_out ? d_ps + p0 * B + b0 : nullptr, var_s_out ? d_ps + (n_star + p0) * B + b0 : nullptr, B,
+            d_acc + p0, d_acc + n_star + p0);
+        L(h);
+      }
+    }
+    PCK(cudaGetLastError());
+  }
+  if (mu_out) PCK(cudaMemcpyAsync(mu_out, d_acc, n_star * sizeof(double), cudaMemcpyDefault, st));
+  if (var_out) PCK(cudaMemcpyAsync(var_out, d_acc + n_star, n_star * sizeof(double), cudaMemcpyDefault, st));
+  if (mean_s_out) PCK(cudaMemcpyAsync(mean_s_out, d_ps, n_star * B * sizeof(double), cudaMemcpyDefault, st));
+  if (var_s_out) PCK(cudaMemcpyAsync(var_s_out, d_ps + n_star * B, n_star * B * sizeof(double), cudaMemcpyDefault, st));
+  prof_close(h);
+  PCK(cudaEventRecord(h->ev[6], st));
+  PCK(cudaStreamSynchronize(st));
+  PCK(cudaGetLastError());
+  cleanup();
+#undef PCK
+#undef PRC
   float ms = 0;
   cudaEventElapsedTime(&ms, h->ev[0], h->ev[6]);
   memset(h->timing, 0, sizeof h->timing);
@@ -3090,6 +3357,26 @@ int cgpcm_predict_f(cgpcm_handle* h, const double* params, double reg, const dou
   if (is_device_ptr(samples)) CK(cudaMemcpy(smp.data(), samples, smp.size() * sizeof(double), cudaMemcpyDeviceToHost));
   else memcpy(smp.data(), samples, smp.size() * sizeof(double));
   return predict_run(h, host.data(), reg, ts.data(), n_star, smp.data(), n_samples, smf, mean, var);
+}
+
+int cgpcm_predict_f_batch(cgpcm_handle* h, const double* params, double reg, const double* t_star, int64_t n_star,
+                          const double* samples, int32_t n_samples, int32_t smf, double* mean, double* var,
+                          double* mean_s, double* var_s) {
+  if (!h || !params || n_star < 0 || !samples || (n_star > 0 && !t_star)) return -1;
+  if (n_samples < 1) { h->err = "n_samples must be >= 1"; return -1; }
+  if (!h->t) { h->err = "cgpcm_set_data has not been called"; return -1; }
+  if (!std::isfinite(reg) || reg < 0) { h->err = "reg must be finite and >= 0"; return -4; }
+  if (n_star == 0) return 0;
+  CK(cudaSetDevice(h->device));
+  const long np = 5 + h->nh + (long)h->nh * (h->nh + 1) / 2;
+  std::vector<double> host, ts(n_star), smp((size_t)n_samples * h->nh);
+  if (fetch_params(h, params, np, host)) return -2;
+  if (is_device_ptr(t_star)) CK(cudaMemcpy(ts.data(), t_star, n_star * sizeof(double), cudaMemcpyDeviceToHost));
+  else memcpy(ts.data(), t_star, n_star * sizeof(double));
+  if (is_device_ptr(samples)) CK(cudaMemcpy(smp.data(), samples, smp.size() * sizeof(double), cudaMemcpyDeviceToHost));
+  else memcpy(smp.data(), samples, smp.size() * sizeof(double));
+  return predict_batch_run(h, host.data(), reg, ts.data(), n_star, smp.data(), n_samples, smf ? 1 : 0, mean, var,
+                           mean_s, var_s);
 }
 
 int cgpcm_kernel_samples(cgpcm_handle* h, const double* params, double reg, const double* t, int64_t n,
@@ -3498,6 +3785,70 @@ int cgpcm_smf_algebra_test(const double* kx, const double* sum_Bxx, const double
   }
   if (cudaStreamSynchronize(st) != cudaSuccess) rc = -2;
   cudaFree(work);
+  return rc;
+}
+
+int cgpcm_smf_posterior_test(const double* kx, const double* sum_Bxx, const double* c1, const double* sum_Ahx_y,
+                             const double* Ahh, const double* iKx, const double* tr_ahh_ikh, const double* samples,
+                             int B, int nslots, int nx, int nh, int64_t ld, int ldh, double r, double c0, double reg,
+                             double a, double* mx, double* xm, double* q1, int* info, void* stream) {
+  if (!kx || !sum_Bxx || !c1 || !sum_Ahx_y || !Ahh || !iKx || !tr_ahh_ikh || !samples || !mx || !xm || !q1 || !info ||
+      B < 1 || nslots < B || nx < 1 || nh < 1 || ld < nx || ld < nh || ldh < nh || 3L * nx * sizeof(double) > 48 * 1024)
+    return -1;
+  cudaStream_t st = (cudaStream_t)stream;
+  const long l2 = ld * ld;
+  double* work = nullptr;
+  if (cudaMalloc(&work, (size_t)B * 2 * l2 * sizeof(double)) != cudaSuccess) { cudaGetLastError(); return -2; }
+  SmfPostArgs g;
+  g.kx = kx; g.sxx = sum_Bxx; g.c1 = c1; g.fy = sum_Ahx_y; g.ahh = Ahh; g.ikx = iKx; g.tr = tr_ahh_ikh; g.hs = samples;
+  g.work = work; g.mx = mx; g.xm = xm; g.q1 = q1; g.info = info;
+  g.ld = ld; g.l2 = l2; g.ldh = ldh; g.nh = nh; g.nx = nx; g.nb = B;
+  g.r = r; g.c0 = c0; g.reg = reg; g.a = a;
+  int rc = cudaMemsetAsync(info, 0, (size_t)B * sizeof(int), st) == cudaSuccess ? 0 : -2;
+  if (!rc) {
+    smf_posterior_launch(st, g, nslots);
+    if (cudaGetLastError() != cudaSuccess) rc = -2;
+  }
+  if (cudaStreamSynchronize(st) != cudaSuccess) rc = -2;
+  cudaFree(work);
+  return rc;
+}
+
+int cgpcm_predict_quad_test(const double* V, int64_t v_stride, int ldv, const double* mx, int64_t mx_stride,
+                            const double* xm, int64_t xm_stride, const double* bxx, int nv, int nx, int B, int nslots,
+                            double* quad, double* lin, double* qb, void* stream) {
+  if (!V || !mx || !xm || !quad || !lin || (qb && !bxx) || nv < 1 || nx < 1 || B < 1 || nslots < B || ldv < nx ||
+      (B > 1 && v_stride < (int64_t)(nv - 1) * ldv + nx) || mx_stride < 0 || (mx_stride > 0 && mx_stride < (int64_t)nx * nx) ||
+      xm_stride < 0 || (xm_stride > 0 && xm_stride < nx))
+    return -1;
+  cudaStream_t st = (cudaStream_t)stream;
+  int rc = 0;
+  PredQuadArgs g;
+  g.V = V; g.v_stride = v_stride; g.ldv = ldv; g.mx = mx; g.mx_stride = mx_stride; g.xm = xm; g.xm_stride = xm_stride;
+  g.nv = nv; g.nx = nx; g.nb = B; g.quad = quad; g.lin = lin; g.ldo = B;
+  predict_quad_launch(st, g, nslots);
+  if (cudaGetLastError() != cudaSuccess) rc = -2;
+  double* part = nullptr;
+  if (!rc && qb) {
+    // Qb = the PQ_SLICES partials summed in order, as predict_finish_kernel sums them
+    const size_t n = (size_t)PQ_SLICES * nv * B;
+    if (cudaMalloc(&part, n * sizeof(double)) != cudaSuccess) { cudaGetLastError(); rc = -2; }
+    if (!rc) {
+      predict_qb_launch(st, bxx, (long)nx * nx, mx, mx_stride, B, nv, nv, nslots, part, B);
+      if (cudaGetLastError() != cudaSuccess) rc = -2;
+    }
+    if (!rc) {
+      const int zs = PQ_SLICES;
+      ew(st, (long)nv * B, [=] __device__(long idx) {
+        double s = 0.0;
+        for (int z = 0; z < zs; ++z) s += part[(long)z * nv * B + idx];
+        qb[idx] = s;
+      });
+      if (cudaGetLastError() != cudaSuccess) rc = -2;
+    }
+  }
+  if (cudaStreamSynchronize(st) != cudaSuccess) rc = -2;
+  if (part) cudaFree(part);
   return rc;
 }
 

@@ -9,6 +9,8 @@
 #pragma once
 #include <cuda_runtime.h>
 
+#include "dgemm_dmma.cuh"
+
 namespace cg {
 
 // X[n][k][l] -= sum_i A[i][n][k] * T[i][n][l]   (A, T in the chunk layout [i][n][kw], X dense [n][nx][nx]).
@@ -90,6 +92,217 @@ __global__ void __launch_bounds__(256) predict_point_kernel(const double* __rest
     acc_mu[n] += w * m1;
     acc_var[n] += w * (m2 - m1 * m1);
   }
+}
+
+// ---- Batched prediction (cgpcm_predict_f_batch): the test side for a batch of samples per launch.  Per chunk of test
+// points, with V_b = H_B A* (one row v_nb = A*_n^T h_b per point, from the small-left GEMM):
+//     Qb[n][b]   = <Bxx*_n, mx_b>            (predict_qb_kernel: points x samples x nx^2, Bxx* read once per batch)
+//     quad[n][b] = v_nb^T mx_b v_nb,  lin[n][b] = v_nb . xm_b      (predict_quad_kernel)
+//     mean_nb = sqrt(s2_f) lin,  var_nb = s2_f (q1_b + Qb + quad) - mean_nb^2      (predict_finish_kernel)
+// Launch shapes are functions of the chunk and the internal batch size only, and every sum over k runs in an order
+// fixed by nx, so a sample's moments are bitwise the same in any batch and at any position.
+constexpr int PQ_T = 32;                 // rows (points) and columns of an output tile
+constexpr int PQ_BK = 32;                // k per shared-memory stage
+constexpr int PQ_LDS = PQ_BK + 4;        // == 4 (mod 8): conflict-free fragment loads
+constexpr int PQ_SLICES = 8;             // fixed k slices of the Qb contraction (partials summed in order)
+
+struct PredQbArgs {
+  const double* X;      // Bxx*_n(k, l) at X[n * K + k * nx + l]  (K = nx^2)
+  const double* mx;     // mx_b(k, l) at mx[b * mx_stride + k * nx + l]
+  long mx_stride;
+  long K;
+  int nv, ncol;         // points of the chunk, valid sample columns
+  double* q;            // partials: slice z at q[(z * nrow + n) * ldq + b]
+  int nrow, ldq;
+};
+
+// grid (point tiles, sample tiles, PQ_SLICES), 128 threads: 4 warps own the 16 x 16 quadrants of a 32 x 32 tile
+// (2 x 2 DMMA m8n8k4 tiles each).  Slice z contracts k-tiles [z per, (z + 1) per) in order.
+__global__ void __launch_bounds__(128) predict_qb_kernel(const PredQbArgs g) {
+  __shared__ __align__(16) double As[PQ_T * PQ_LDS];
+  __shared__ __align__(16) double Bs[PQ_T * PQ_LDS];
+  const int r0 = blockIdx.x * PQ_T, s0 = blockIdx.y * PQ_T, z = blockIdx.z;
+  const long kt = (g.K + PQ_BK - 1) / PQ_BK, per = (kt + PQ_SLICES - 1) / PQ_SLICES;
+  const long k_begin = z * per * PQ_BK, k_end = min(g.K, (z + 1) * per * PQ_BK);
+  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  const int wi = warp >> 1, wj = warp & 1, grp = lane >> 2, tig = lane & 3;
+  double acc[2][2][2];
+#pragma unroll
+  for (int x = 0; x < 2; ++x)
+#pragma unroll
+    for (int y = 0; y < 2; ++y) acc[x][y][0] = acc[x][y][1] = 0.0;
+  for (long k0 = k_begin; k0 < k_end; k0 += PQ_BK) {
+#pragma unroll
+    for (int q = 0; q < PQ_T * PQ_BK / 128; ++q) {
+      const int e = q * 128 + tid, rr = e >> 5, cc = e & 31;
+      const long k = k0 + cc;
+      const bool kok = k < k_end;
+      As[rr * PQ_LDS + cc] = (kok && r0 + rr < g.nv) ? g.X[(long)(r0 + rr) * g.K + k] : 0.0;
+      Bs[rr * PQ_LDS + cc] = (kok && s0 + rr < g.ncol) ? g.mx[(long)(s0 + rr) * g.mx_stride + k] : 0.0;
+    }
+    __syncthreads();
+#pragma unroll
+    for (int k4 = 0; k4 < PQ_BK / 4; ++k4) {
+      double fa[2], fb[2];
+#pragma unroll
+      for (int x = 0; x < 2; ++x) {
+        fa[x] = As[(wi * 16 + x * 8 + grp) * PQ_LDS + k4 * 4 + tig];
+        fb[x] = Bs[(wj * 16 + x * 8 + grp) * PQ_LDS + k4 * 4 + tig];
+      }
+#pragma unroll
+      for (int x = 0; x < 2; ++x)
+#pragma unroll
+        for (int y = 0; y < 2; ++y) dmma_8x8x4(acc[x][y][0], acc[x][y][1], fa[x], fb[y]);
+    }
+    __syncthreads();
+  }
+  double* Q = g.q + (long)z * g.nrow * g.ldq;
+#pragma unroll
+  for (int x = 0; x < 2; ++x) {
+    const int row = r0 + wi * 16 + x * 8 + grp;
+    if (row >= g.nv) continue;
+#pragma unroll
+    for (int y = 0; y < 2; ++y)
+#pragma unroll
+      for (int u = 0; u < 2; ++u) {
+        const int col = s0 + wj * 16 + y * 8 + tig * 2 + u;
+        if (col < g.ncol) Q[(long)row * g.ldq + col] = acc[x][y][u];
+      }
+  }
+}
+
+struct PredQuadArgs {
+  const double* V;      // v_nb(k) at V[b * v_stride + n * ldv + k]
+  long v_stride;
+  int ldv;
+  const double* mx;     // mx_b(k, l) at mx[b * mx_stride + k * nx + l]  (stride 0: one q(z) for every sample)
+  long mx_stride;
+  const double* xm;     // xm_b at xm[b * xm_stride]
+  long xm_stride;
+  int nv, nx, nb;
+  double* quad;         // [n][b] at n * ldo + b
+  double* lin;
+  int ldo;
+};
+
+// grid (point tiles, samples), 128 threads.  Per 32-column tile of Y = V_b mx_b (DMMA, warps on 16 x 16 quadrants as
+// above), the epilogue multiplies Y element-wise with V_b and adds it into per-row partials; column tiles in order,
+// then the four lanes of a row (fixed butterfly) and the two column-half warps in order.  Samples b >= nb return.
+__global__ void __launch_bounds__(128) predict_quad_kernel(const PredQuadArgs g) {
+  __shared__ __align__(16) double Vs[PQ_T * PQ_LDS];
+  __shared__ __align__(16) double Ms[PQ_T * PQ_LDS];
+  __shared__ double red[2][PQ_T];
+  const int b = blockIdx.y;
+  if (b >= g.nb) return;
+  const int r0 = blockIdx.x * PQ_T, nx = g.nx;
+  const double* Vb = g.V + (long)b * g.v_stride;
+  const double* Mb = g.mx + (long)b * g.mx_stride;
+  const double* Xb = g.xm + (long)b * g.xm_stride;
+  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  const int wi = warp >> 1, wj = warp & 1, grp = lane >> 2, tig = lane & 3;
+  double rp[2] = {0.0, 0.0};
+  for (int c0 = 0; c0 < nx; c0 += PQ_T) {
+    double acc[2][2][2];
+#pragma unroll
+    for (int x = 0; x < 2; ++x)
+#pragma unroll
+      for (int y = 0; y < 2; ++y) acc[x][y][0] = acc[x][y][1] = 0.0;
+    for (int k0 = 0; k0 < nx; k0 += PQ_BK) {
+#pragma unroll
+      for (int q = 0; q < PQ_T * PQ_BK / 128; ++q) {
+        const int e = q * 128 + tid, hi = e >> 5, lo = e & 31;
+        // Vs[row][k] = V(r0 + row, k0 + k);  Ms[col][k] = mx(k0 + k, c0 + col)
+        Vs[hi * PQ_LDS + lo] = (r0 + hi < g.nv && k0 + lo < nx) ? Vb[(long)(r0 + hi) * g.ldv + k0 + lo] : 0.0;
+        Ms[lo * PQ_LDS + hi] = (k0 + hi < nx && c0 + lo < nx) ? Mb[(long)(k0 + hi) * nx + c0 + lo] : 0.0;
+      }
+      __syncthreads();
+#pragma unroll
+      for (int k4 = 0; k4 < PQ_BK / 4; ++k4) {
+        double fa[2], fb[2];
+#pragma unroll
+        for (int x = 0; x < 2; ++x) {
+          fa[x] = Vs[(wi * 16 + x * 8 + grp) * PQ_LDS + k4 * 4 + tig];
+          fb[x] = Ms[(wj * 16 + x * 8 + grp) * PQ_LDS + k4 * 4 + tig];
+        }
+#pragma unroll
+        for (int x = 0; x < 2; ++x)
+#pragma unroll
+          for (int y = 0; y < 2; ++y) dmma_8x8x4(acc[x][y][0], acc[x][y][1], fa[x], fb[y]);
+      }
+      __syncthreads();
+    }
+#pragma unroll
+    for (int x = 0; x < 2; ++x) {
+      const int row = r0 + wi * 16 + x * 8 + grp;
+      if (row >= g.nv) continue;
+#pragma unroll
+      for (int y = 0; y < 2; ++y)
+#pragma unroll
+        for (int u = 0; u < 2; ++u) {
+          const int col = c0 + wj * 16 + y * 8 + tig * 2 + u;
+          if (col < nx) rp[x] += acc[x][y][u] * Vb[(long)row * g.ldv + col];
+        }
+    }
+  }
+#pragma unroll
+  for (int x = 0; x < 2; ++x) {
+    rp[x] += __shfl_xor_sync(0xffffffffu, rp[x], 1);
+    rp[x] += __shfl_xor_sync(0xffffffffu, rp[x], 2);
+    if (tig == 0) red[wj][wi * 16 + x * 8 + grp] = rp[x];
+  }
+  // lin: warp w takes rows w, w + 4, ..; lanes stride k, then a fixed shuffle tree
+  for (int rr = warp; rr < PQ_T; rr += 4) {
+    const int row = r0 + rr;
+    if (row >= g.nv) continue;
+    double s = 0.0;
+    for (int k = lane; k < nx; k += 32) s += Vb[(long)row * g.ldv + k] * Xb[k];
+#pragma unroll
+    for (int off = 16; off > 0; off >>= 1) s += __shfl_down_sync(0xffffffffu, s, off);
+    if (lane == 0) g.lin[(long)row * g.ldo + b] = s;
+  }
+  __syncthreads();
+  if (tid < PQ_T && r0 + tid < g.nv) g.quad[(long)(r0 + tid) * g.ldo + b] = red[0][tid] + red[1][tid];
+}
+
+// Launch shapes of the test-side kernels, shared by predict_batch_run and the C-ABI test hook.  The grids depend on the
+// chunk's point count (nrow: its capacity, nv: valid points) and the batch's sample slots (nslots) only.
+// q[z][n][b] (z < PQ_SLICES, n < nv, b < ncol) = partial <Bxx*_n, mx_b> over k slice z.
+inline void predict_qb_launch(cudaStream_t st, const double* X, long K, const double* mx, long mx_stride, int ncol,
+                              int nv, int nrow, int nslots, double* q, int ldq) {
+  PredQbArgs g;
+  g.X = X; g.K = K; g.mx = mx; g.mx_stride = mx_stride; g.nv = nv; g.ncol = ncol; g.q = q; g.nrow = nrow; g.ldq = ldq;
+  predict_qb_kernel<<<dim3((nv + PQ_T - 1) / PQ_T, (nslots + PQ_T - 1) / PQ_T, PQ_SLICES), 128, 0, st>>>(g);
+}
+
+inline void predict_quad_launch(cudaStream_t st, const PredQuadArgs& g, int nslots) {
+  predict_quad_kernel<<<dim3((g.nv + PQ_T - 1) / PQ_T, nslots), 128, 0, st>>>(g);
+}
+
+// One thread per point of the chunk: per-sample moments for b < nb in ascending b, and the running averages
+//   mean_s[n][b] = m1 = sqrt(s2f) lin,  var_s[n][b] = m2 - m1^2,  m2 = s2f (q1_b + Qb + quad),
+//   acc_mu[n] += w m1,  acc_var[n] += w (m2 - m1^2)          (the accumulation of predict_point_kernel)
+// Qb = the PQ_SLICES partials of column b * q_col summed in order (q_col = 0: one q(z) for every sample).
+__global__ void predict_finish_kernel(const double* __restrict__ qpart, int nrow, int ldq, int q_col,
+                                      const double* __restrict__ quad, const double* __restrict__ lin, int ldo,
+                                      const double* __restrict__ q1, int nv, int nb, double sqrt_s2f, double s2f,
+                                      double w, double* __restrict__ mean_s, double* __restrict__ var_s, long lds,
+                                      double* __restrict__ acc_mu, double* __restrict__ acc_var) {
+  const int n = blockIdx.x * blockDim.x + threadIdx.x;
+  if (n >= nv) return;
+  double am = acc_mu[n], av = acc_var[n];
+  for (int b = 0; b < nb; ++b) {
+    double qb = 0.0;
+    for (int z = 0; z < PQ_SLICES; ++z) qb += qpart[((long)z * nrow + n) * ldq + b * q_col];
+    const double m1 = sqrt_s2f * lin[(long)n * ldo + b];
+    const double m2 = s2f * (q1[b] + qb + quad[(long)n * ldo + b]);
+    const double v = m2 - m1 * m1;
+    if (mean_s) mean_s[(long)n * lds + b] = m1;
+    if (var_s) var_s[(long)n * lds + b] = v;
+    am += w * m1;
+    av += w * v;
+  }
+  acc_mu[n] = am;
+  acc_var[n] = av;
 }
 
 }  // namespace cg

@@ -202,6 +202,159 @@ __global__ void __launch_bounds__(SMF_ALG_THREADS) smf_algebra_kernel(const SmfA
   }
 }
 
+// h^T M h (M: nh x nh at leading dimension ld) for the whole block, valid in thread 0: one warp per row (fixed shuffle
+// tree), rows in a fixed order per warp, warps added in order.  wsum: blockDim.x / 32 doubles of shared memory.
+__device__ double block_quad_form(const double* M, long ld, const double* hb, int nh, double* wsum) {
+  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5, nw = blockDim.x >> 5;
+  double acc = 0.0;
+  for (int i = warp; i < nh; i += nw) {
+    double s = 0.0;
+    for (int k = lane; k < nh; k += 32) s += M[(long)i * ld + k] * hb[k];
+#pragma unroll
+    for (int off = 16; off > 0; off >>= 1) s += __shfl_down_sync(0xffffffffu, s, off);
+    acc += hb[i] * s;
+  }
+  if (lane == 0) wsum[warp] = acc;
+  __syncthreads();
+  double s = 0.0;
+  if (tid == 0)
+    for (int w = 0; w < nw; ++w) s += wsum[w];
+  return s;
+}
+
+struct SmfPostArgs {
+  const double* kx;     // Kx (with its jitter), ld x ld
+  const double* sxx;    // frozen sum_Bxx
+  const double* c1;     // [b] slabs (lower triangle)
+  const double* fy;     // frozen sum_Ahx_y, nh x nx at leading dimension ld
+  const double* ahh;    // frozen Ahh, nh x nh at leading dimension ld
+  const double* ikx;    // iKx, ld x ld
+  const double* tr;     // device scalar tr(Ahh iKh)
+  const double* hs;     // samples [b][ldh]
+  double* work;         // [b][2] ld x ld slabs: Cholesky factor L of P_b, then L^-1
+  double* mx;           // [b] at stride l2: mx_b = P_b^-1 + xm_b xm_b^T - iKx, full nx x nx at leading dimension nx
+  double* xm;           // [b] at stride ld: xm_b = P_b^-1 lam_b
+  double* q1;           // [b]: a + h_b^T Ahh h_b - tr(Ahh iKh)
+  int* info;            // [b]: pivot + 1 of a failed factorisation of P_b, else 0
+  long ld, l2;
+  int ldh, nh, nx, nb;
+  double r, c0, reg, a;
+};
+
+// The per-sample optimal q(z | h_b) of predict_f (SMF) and the scalar q1_b, one CTA per sample (b < nb):
+// P_b = Kx + r (sum_Bxx + C1_b) + reg I, its right-looking Cholesky factorisation (stored as L in the first work slab)
+// fused with the forward solve of lam_b = c0 sum_Ahx_y^T h_b, the backward solve for xm_b, Z = L^-1 by the same
+// right-looking sweep (second slab), then mx_b[k][l] = sum_{i >= max(k, l)} Z[i][k] Z[i][l] + xm_k xm_l - iKx[k][l]
+// (both triangles from the same value).  Every sum runs in an order fixed by nx alone.  Dynamic shared memory:
+// 3 nx doubles.
+__global__ void __launch_bounds__(SMF_ALG_THREADS) smf_posterior_kernel(const SmfPostArgs g) {
+  extern __shared__ double sh[];
+  double* col = sh;           // column j of the factor below the diagonal
+  double* zv = sh + g.nx;     // right-hand side / solution
+  double* dg = sh + 2 * g.nx; // diagonal of the factor
+  __shared__ double wsum[SMF_ALG_THREADS / 32];
+  const int b = blockIdx.x;
+  if (b >= g.nb) return;
+  const int n = g.nx, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  constexpr int NW = SMF_ALG_THREADS / 32;
+  const long ld = g.ld;
+  double* P = g.work + (long)b * 2 * g.l2;
+  double* Z = P + g.l2;
+  const double* c1 = g.c1 + (long)b * g.l2;
+  const double* hb = g.hs + (long)b * g.ldh;
+  for (long idx = tid; idx < (long)n * n; idx += blockDim.x) {
+    const int i = (int)(idx / n), j = (int)(idx - (long)i * n);
+    const long e = (long)i * ld + j;
+    if (j <= i) {
+      const double s = g.sxx[e] + c1[e];
+      P[e] = g.kx[e] + g.r * s + (i == j ? g.reg : 0.0);
+    }
+    Z[e] = i == j ? 1.0 : 0.0;
+  }
+  for (int k = tid; k < n; k += blockDim.x) {
+    double s = 0.0;
+    for (int i = 0; i < g.nh; ++i) s += g.fy[(long)i * ld + k] * hb[i];
+    zv[k] = g.c0 * s;
+  }
+  __syncthreads();
+  int fail = 0;
+  for (int j = 0; j < n; ++j) {
+    const double d = P[(long)j * ld + j];
+    if (!(d > 0.0)) { fail = j + 1; break; }       // the same value in every thread: a uniform exit
+    const double l = sqrt(d);
+    for (int i = j + 1 + tid; i < n; i += blockDim.x) {
+      const double v = P[(long)i * ld + j] / l;
+      col[i] = v;
+      P[(long)i * ld + j] = v;
+    }
+    if (tid == 0) {
+      zv[j] = zv[j] / l;
+      dg[j] = l;
+    }
+    __syncthreads();
+    const double zj = zv[j];
+    for (int i = j + 1 + warp; i < n; i += NW) {
+      const double lij = col[i];
+      double* row = P + (long)i * ld;
+      for (int k = j + 1 + lane; k <= i; k += 32) row[k] -= lij * col[k];
+      if (lane == 0) zv[i] -= lij * zj;
+    }
+    __syncthreads();
+  }
+  if (fail) {
+    if (tid == 0) g.info[b] = fail;
+    return;
+  }
+  // backward solve L^T x = z (x overwrites zv)
+  for (int j = n - 1; j >= 0; --j) {
+    if (tid == 0) zv[j] = zv[j] / dg[j];
+    __syncthreads();
+    const double xj = zv[j];
+    for (int i = tid; i < j; i += blockDim.x) zv[i] -= P[(long)j * ld + i] * xj;
+    __syncthreads();
+  }
+  // Z = L^-1 (lower): row j is final once divided by L[j][j]; then it updates the rows below it
+  for (int j = 0; j < n; ++j) {
+    const double l = dg[j];
+    for (int c = tid; c <= j; c += blockDim.x) Z[(long)j * ld + c] /= l;
+    __syncthreads();
+    const double* zj = Z + (long)j * ld;
+    for (int i = j + 1 + warp; i < n; i += NW) {
+      const double lij = P[(long)i * ld + j];
+      double* row = Z + (long)i * ld;
+      for (int c = lane; c <= j; c += 32) row[c] -= lij * zj[c];
+    }
+    __syncthreads();
+  }
+  double* mxb = g.mx + (long)b * g.l2;
+  for (long idx = tid; idx < (long)n * n; idx += blockDim.x) {
+    const int k = (int)(idx / n), l = (int)(idx - (long)k * n);
+    if (l > k) continue;
+    double s = 0.0;
+    for (int i = k; i < n; ++i) s += Z[(long)i * ld + k] * Z[(long)i * ld + l];
+    const double v = s + zv[k] * zv[l] - g.ikx[(long)k * ld + l];
+    mxb[(long)k * n + l] = v;
+    mxb[(long)l * n + k] = v;
+  }
+  for (int k = tid; k < n; k += blockDim.x) g.xm[(long)b * ld + k] = zv[k];
+  const double q = block_quad_form(g.ahh, ld, hb, g.nh, wsum);
+  if (tid == 0) {
+    g.q1[b] = g.a + q - g.tr[0];
+    g.info[b] = 0;
+  }
+}
+
+// q1_b = a + h_b^T Ahh h_b - tr(Ahh iKh) for b < nb: the per-sample scalar of predict_f when q(z) is shared (smf = 0)
+__global__ void __launch_bounds__(256) predict_q1_kernel(const double* __restrict__ ahh, long ld,
+                                                         const double* __restrict__ hs, int ldh, int nh, int nb, double a,
+                                                         const double* __restrict__ tr, double* __restrict__ q1) {
+  __shared__ double wsum[8];
+  const int b = blockIdx.x;
+  if (b >= nb) return;
+  const double q = block_quad_form(ahh, ld, hs + (long)b * ldh, nh, wsum);
+  if (threadIdx.x == 0) q1[b] = a + q - tr[0];
+}
+
 // Launch shapes of the three kernels, shared by smf_batch_run and the C-ABI test hooks.
 // part[b][z] += W_b^T W_b of one window (k_lo, kwp) over nc padded observations, for samples b < nb.
 inline void smf_c1_launch(cudaStream_t st, const double* W, long w_stride, int kwp, int nc, int k_lo, double* part,
@@ -219,6 +372,11 @@ inline void smf_reduce_launch(cudaStream_t st, const double* part, long ld, int 
 
 inline void smf_algebra_launch(cudaStream_t st, const SmfAlgArgs& a, int nb) {
   smf_algebra_kernel<<<dim3(nb, a.passes), SMF_ALG_THREADS, 2 * a.nx * sizeof(double), st>>>(a);
+}
+
+// one CTA per sample slot of the batch (samples b >= a.nb return at once)
+inline void smf_posterior_launch(cudaStream_t st, const SmfPostArgs& a, int nslots) {
+  smf_posterior_kernel<<<nslots, SMF_ALG_THREADS, 3 * a.nx * sizeof(double), st>>>(a);
 }
 
 }  // namespace cg

@@ -157,6 +157,28 @@ class Engine(object):
                                              int(bool(smf)), _lib.ptr(mean), _lib.ptr(var)))
         return mean, var
 
+    def predict_f_batch(self, params, t_star, samples, smf=True, reg=1e-8, per_sample=True):
+        """Predictive moments of the function at ``t_star`` for every filter sample ([B, nh]) in one call:
+        ``(mean[n], var[n], mean_s[n, B], var_s[n, B])``.  ``mean_s[:, b]`` and ``var_s[:, b]`` are the mean and
+        variance under sample b's q(z) (``smf=True``: q(z | h_b); ``smf=False``: the one q(z) of q(u)); ``mean`` and
+        ``var`` are their sample averages, what :meth:`predict_f` returns.  ``per_sample=False`` returns ``None`` for
+        the last two.  A sample's moments do not depend on the other samples of the call; needs the frozen statistics."""
+        t_star = np.ascontiguousarray(np.asarray(t_star, dtype=np.float64).ravel())
+        samples = np.ascontiguousarray(np.asarray(samples, dtype=np.float64))
+        if samples.ndim == 1:
+            samples = samples.reshape(1, -1)
+        if samples.ndim != 2 or samples.shape[1] != self.nh or samples.shape[0] < 1 or \
+                int(params.shape[0]) != n_params(self.nh):
+            raise ValueError('shape mismatch in predict_f_batch')
+        n, B = t_star.shape[0], samples.shape[0]
+        mean, var = np.empty(n), np.empty(n)
+        mean_s, var_s = (np.empty((n, B)), np.empty((n, B))) if per_sample else (None, None)
+        if n:
+            self._ck(_lib.lib().cgpcm_predict_f_batch(self._h, _lib.ptr(params), float(reg), _lib.ptr(t_star), n,
+                                                       _lib.ptr(samples), B, int(bool(smf)), _lib.ptr(mean),
+                                                       _lib.ptr(var), _lib.ptr(mean_s), _lib.ptr(var_s)))
+        return mean, var, mean_s, var_s
+
     def kernel_samples(self, params, t, samples, reg=1e-8):
         """Kernel samples ``k[n, b]`` of ``predict_k`` at lags ``t`` for filter ``samples`` ([B, nh])
         (``src/core/cgpcm.py:610-634``), before normalisation."""

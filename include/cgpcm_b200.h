@@ -145,6 +145,21 @@ int cgpcm_elbo_smf_batch(cgpcm_handle* h, const double* params, double reg, cons
 int cgpcm_predict_f(cgpcm_handle* h, const double* params, double reg, const double* t_star, int64_t n_star,
                     const double* samples, int32_t n_samples, int32_t smf, double* mean, double* var);
 
+/* predict_f's moments per filter sample: for every test input n and sample b, the predictive mean and variance of the
+ * function under that sample's q(z) (smf = 1: q(z | h_b); smf = 0: the one q(z) of q(u)):
+ * mean_s[n * n_samples + b], var_s[n * n_samples + b] (the layout of cgpcm_kernel_samples), and their averages over
+ * the samples mean[n_star], var[n_star] -- what cgpcm_predict_f returns for the same arguments, added per sample in
+ * ascending b with weight 1 / n_samples.  The law of total variance gives the mixture variance of the samples as
+ * mean_b(var_s) + var_b(mean_s).  Any output may be NULL; host or device pointers.  The samples are processed in
+ * internal batches whose size depends on the handle's shape only, and no sum runs across samples except the average:
+ * a sample's mean_s / var_s are bitwise the same whatever other samples share the call and in any position.  Uses the
+ * statistics frozen by cgpcm_precompute (-1 otherwise); -1 when n_samples < 1; -4 for a non-finite parameter, sample or
+ * test input; -3 when some P_b is not positive definite (cgpcm_last_error names the sample and the pivot); n_star = 0
+ * returns 0 and writes nothing. */
+int cgpcm_predict_f_batch(cgpcm_handle* h, const double* params, double reg, const double* t_star, int64_t n_star,
+                          const double* samples, int32_t n_samples, int32_t smf, double* mean, double* var,
+                          double* mean_s, double* var_s);
+
 /* The Monte-Carlo kernel samples of mod.predict_k(t, samples_h) (src/core/cgpcm.py:610-634; centre statistics
  * _a_center / _Ahh_center :164-166,190-192), before normalisation / FFT / percentiles (host post-processing):
  * out[p * n_samples + b] = s2_f (a_c(t_p) + tr((h_b h_b^T - iKh) Ahh_c(t_p))) for lags t[n] and filter samples
@@ -252,6 +267,24 @@ int cgpcm_smf_algebra_test(const double* kx, const double* sum_Bxx, const double
                            const double* sum_Bhh, const double* samples, int B, int nx, int nh, int64_t ld, int ldh,
                            double r, double c0, double reg, int want_p, int want_p0, double* out, int* info,
                            void* stream);
+/* The kernels of cgpcm_predict_f_batch (csrc/smf_batch.cuh, csrc/predict_kernels.cuh) with its launch shapes; device
+ * pointers only; they return after the stream has drained.  nslots >= B: the sample slots the grid is shaped for (the
+ * internal batch size; slots b >= B do nothing).
+ * cgpcm_smf_posterior_test: per sample b, P_b = Kx + r (sum_Bxx + C1_b) + reg I (lower triangles read, ld x ld),
+ * lam_b = c0 sum_Ahx_y^T h_b, xm[b * ld + k] = (P_b^-1 lam_b)[k], mx[b * ld * ld + k * nx + l] =
+ * (P_b^-1 + xm xm^T - iKx)[k][l] (full nx x nx), q1[b] = a + h_b^T Ahh h_b - tr_ahh_ikh[0] (a device scalar).
+ * info[b] = pivot + 1 of a failed factorisation of P_b (its other outputs are not written), else 0.  nx <= 2048.
+ * cgpcm_predict_quad_test: per point n < nv and sample b < B, with v = V[b * v_stride + n * ldv + k],
+ * M_b = mx[b * mx_stride + k * nx + l] and x_b = xm[b * xm_stride + k] (stride 0: one matrix for every sample):
+ * quad[n * B + b] = v^T M_b v, lin[n * B + b] = v . x_b and, when qb is not NULL, qb[n * B + b] = <Bxx_n, M_b> with
+ * Bxx_n = bxx[n * nx * nx + k * nx + l]. */
+int cgpcm_smf_posterior_test(const double* kx, const double* sum_Bxx, const double* c1, const double* sum_Ahx_y,
+                             const double* Ahh, const double* iKx, const double* tr_ahh_ikh, const double* samples,
+                             int B, int nslots, int nx, int nh, int64_t ld, int ldh, double r, double c0, double reg,
+                             double a, double* mx, double* xm, double* q1, int* info, void* stream);
+int cgpcm_predict_quad_test(const double* V, int64_t v_stride, int ldv, const double* mx, int64_t mx_stride,
+                            const double* xm, int64_t xm_stride, const double* bxx, int nv, int nx, int B, int nslots,
+                            double* quad, double* lin, double* qb, void* stream);
 
 #ifdef __cplusplus
 }
