@@ -21,9 +21,10 @@ GRAD_ALL = 0x7f
 MODE_FROZEN, MODE_FULL = 0, 1
 
 EXPORTS = ['cgpcm_create', 'cgpcm_destroy', 'cgpcm_last_error', 'cgpcm_device_count', 'cgpcm_comm_unique_id', 'cgpcm_comm_init',
-           'cgpcm_set_data', 'cgpcm_set_option', 'cgpcm_psi', 'cgpcm_precompute', 'cgpcm_frozen_mats', 'cgpcm_elbo_grad', 'cgpcm_elbo_smf', 'cgpcm_elbo_smf_batch', 'cgpcm_predict_f', 'cgpcm_predict_f_batch', 'cgpcm_kernel_samples', 'cgpcm_filter_samples', 'cgpcm_akm_sample', 'cgpcm_fpi', 'cgpcm_fpi_qz', 'cgpcm_elbo_qz',
+           'cgpcm_set_data', 'cgpcm_set_option', 'cgpcm_psi', 'cgpcm_precompute', 'cgpcm_frozen_mats', 'cgpcm_elbo_grad', 'cgpcm_elbo_smf', 'cgpcm_elbo_smf_batch', 'cgpcm_predict_f', 'cgpcm_predict_f_batch', 'cgpcm_predict_f_cov', 'cgpcm_kernel_samples', 'cgpcm_filter_samples', 'cgpcm_akm_sample', 'cgpcm_fpi', 'cgpcm_fpi_qz', 'cgpcm_elbo_qz',
            'cgpcm_last_timing', 'cgpcm_bvn_cdf', 'cgpcm_dgemm', 'cgpcm_dgemm_tri', 'cgpcm_dgemm_sym', 'cgpcm_cholinv', 'cgpcm_math_test', 'cgpcm_math_test_fast',
-           'cgpcm_smf_c1_test', 'cgpcm_smf_algebra_test', 'cgpcm_smf_posterior_test', 'cgpcm_predict_quad_test']
+           'cgpcm_smf_c1_test', 'cgpcm_smf_algebra_test', 'cgpcm_smf_posterior_test', 'cgpcm_predict_quad_test',
+           'cgpcm_predict_pair_test']
 
 
 def _sources():
@@ -82,6 +83,7 @@ def lib():
     L.cgpcm_elbo_smf_batch.argtypes = [vp, dp, dbl, dp, ctypes.c_int32, dp, dp, dp]
     L.cgpcm_predict_f.argtypes = [vp, dp, dbl, dp, i64, dp, ctypes.c_int32, ctypes.c_int32, dp, dp]
     L.cgpcm_predict_f_batch.argtypes = [vp, dp, dbl, dp, i64, dp, ctypes.c_int32, ctypes.c_int32, dp, dp, dp, dp]
+    L.cgpcm_predict_f_cov.argtypes = [vp, dp, dbl, dp, i64, dp, ctypes.c_int32, ctypes.c_int32, dp, dp, dp, dp, dp]
     L.cgpcm_kernel_samples.argtypes = [vp, dp, dbl, dp, i64, dp, ctypes.c_int32, dp]
     L.cgpcm_filter_samples.argtypes = [vp, dp, dbl, dp, i64, dp, ctypes.c_int32, dp, dp]
     L.cgpcm_akm_sample.argtypes = [vp, dp, dbl, dp, i64, dp, dp, dp, dp]
@@ -102,6 +104,7 @@ def lib():
     L.cgpcm_smf_posterior_test.argtypes = [dp, dp, dp, dp, dp, dp, dp, dp, i32, i32, i32, i32, i64, i32, dbl, dbl, dbl,
                                            dbl, dp, dp, dp, vp, vp]
     L.cgpcm_predict_quad_test.argtypes = [dp, i64, i32, dp, i64, dp, i64, dp, i32, i32, i32, i32, dp, dp, dp, vp]
+    L.cgpcm_predict_pair_test.argtypes = [dp, i32, dp, i32, dp, i32, dp, i32, i32, dp, i64, i32, dp, vp]
     for name in EXPORTS:
         if name != 'cgpcm_last_error':
             getattr(L, name).restype = ctypes.c_int

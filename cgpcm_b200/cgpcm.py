@@ -709,6 +709,37 @@ class VCGPCM(CGPCM):
             lambda: self.engine.predict_f_batch(self._pack(), t, samples, smf=smf, reg=config.reg))
         return mean, var
 
+    def _filter_batch(self, samples_h):
+        if np.isscalar(samples_h) or isinstance(samples_h, (int, np.integer)):
+            samples, smf = [self.sample_q() for _ in range(int(samples_h))], False
+        else:
+            samples, smf = list(samples_h), True
+        return np.stack([np.asarray(x, dtype=np.float64).ravel() for x in samples]), smf
+
+    def predict_f_cov(self, t, samples_h=50, per_sample=False):
+        """Joint predictive distribution of the function at ``t`` (at most 4096 inputs): ``(mean[n], cov[n, n])`` with
+        ``cov`` the covariance of the mixture of the samples' predictive distributions, ``cov_avg + Cov_b(mean_s)``;
+        ``cov_avg``, the sample average of the per-sample covariances, has :meth:`predict_f`'s variance on its
+        diagonal.  ``samples_h`` as in :meth:`predict_f_samples`.  ``per_sample=True`` also returns
+        ``(mean_s[n, B], cov_s[B, n, n])``, each sample's mean and covariance."""
+        t = np.asarray(getattr(t, 'x', t), dtype=np.float64).ravel()
+        samples, smf = self._filter_batch(samples_h)
+        mean, cov, mean_s, cov_s, _ = self._with_frozen_stats(lambda: self.engine.predict_f_cov(
+            self._pack(), t, samples, smf=smf, reg=config.reg, per_sample=per_sample))
+        mix = cov + np.atleast_2d(np.cov(mean_s, bias=True))
+        return (mean, mix, mean_s, cov_s) if per_sample else (mean, mix)
+
+    def sample_f(self, t, samples_h=50):
+        """Posterior sample paths of the function at ``t`` (at most 4096 inputs), one per filter sample: ``[n, B]``,
+        column b a draw from the joint predictive distribution under sample b's q(z) (``samples_h`` as in
+        :meth:`predict_f_samples`).  The standard normal noise comes from the model's generator, so every rank draws
+        the same paths."""
+        t = np.asarray(getattr(t, 'x', t), dtype=np.float64).ravel()
+        samples, smf = self._filter_batch(samples_h)
+        noise = self._rng.randn(t.shape[0], samples.shape[0])
+        return self._with_frozen_stats(lambda: self.engine.predict_f_cov(
+            self._pack(), t, samples, smf=smf, reg=config.reg, noise=noise))[4]
+
     def predict_k(self, t, samples_h=200, psd=False, normalise=True):
         """Predict the kernel, or the PSD via the kernel approximation, at lags ``t``
         (``src/core/cgpcm.py:610-661``): Monte-Carlo over filter samples (numeric ``samples_h``: draws from q(u)).

@@ -3249,6 +3249,378 @@ int predict_batch_run(cgpcm_handle* h, const double* params_host, double reg, co
   return 0;
 }
 
+// Points per side of a pair tile of predict_cov_run: a function of nx only.  The tile's pair blocks (P^2 nx^2) and its
+// fold (P nxp)^2 stay within ~1 GB.
+int pcov_tile(const cgpcm_handle* h) {
+  const int tp = (int)sqrt(6e7 / ((double)h->nxp * h->nxp)) / 8 * 8;
+  return std::max(8, std::min(64, tp));
+}
+
+// The joint predictive covariance of f at n_star <= 4096 test inputs for each of B filter samples, and draws of f
+// (cgpcm_predict_f_cov).  Training side as predict_batch_run: smf = 0 the one q(z) of q(u) (predict_qz); smf = 1 per
+// batch of predict_bcap samples the C1 stage and smf_posterior_kernel.  Test side, once: A* and T = iKh A* for all test
+// inputs.  Per group of samples (their covariance slabs within ~4 GB):
+//   per batch   V = H_B A* (small-left GEMM), the means (predict_quad_kernel's v . xm_b), and per sample the rank-one
+//               term R_b = (V_b mx_b) V_b^T into C_b (two GEMMs);
+//   per tile    of P x Q points with p >= q: the fold A*_p^T T_q (one GEMM), the pair blocks Bxx* (axx_pair_kernel), the
+//               centre statistics at the tile's lags (ahh_center_kernel) and, per batch, <Ahh_c, hh_b - iKh> (GEMM),
+//               <Bxx*, mx_b> (predict_qb_kernel) and pcov_finish_kernel;
+//   then        cov += C_b / B in ascending b, and per sample chol(C_b + reg I) (identity on the padding) and the draw.
+// Every launch is shaped by the handle, n_star and the internal batch size, and no sum runs across samples except cov,
+// so a sample's mean, C_b and draw are bitwise the same in any batch and at any position.
+int predict_cov_run(cgpcm_handle* h, const double* params_host, double reg, const double* tstar_host, long n_star,
+                    const double* samples_host, int B, int smf, const double* noise_host, double* mean_s_out,
+                    double* cov_s_out, double* cov_out, double* draws_out) {
+  const int nh = h->nh, nx = h->nx, nhp = h->nhp, nxp = h->nxp;
+  const long ld = h->ld, l2 = ld * ld;
+  const long np = 5 + nh + (long)nh * (nh + 1) / 2;
+  for (long i = 0; i < np; ++i)
+    if (!std::isfinite(params_host[i])) { h->err = "non-finite parameter"; return -4; }
+  for (long i = 0; i < n_star; ++i)
+    if (!std::isfinite(tstar_host[i])) { h->err = "non-finite test input"; return -4; }
+  for (long i = 0; i < (long)B * nh; ++i)
+    if (!std::isfinite(samples_host[i])) {
+      char b[96];
+      snprintf(b, sizeof b, "non-finite value in sample %ld", i / nh);
+      h->err = b;
+      return -4;
+    }
+  if (noise_host)
+    for (long i = 0; i < n_star * B; ++i)
+      if (!std::isfinite(noise_host[i])) { h->err = "non-finite noise"; return -4; }
+  if (!h->frozen) { h->err = "cgpcm_predict_f_cov requires cgpcm_precompute"; return -1; }
+  const bool want_draws = draws_out && noise_host;
+  const double s2 = exp(params_host[0]), s2f = exp(params_host[1]);
+  const double alpha = exp(params_host[2]), gamma = exp(params_host[3]), omega = exp(params_host[4]);
+  const double r = s2f / s2, c0 = sqrt(s2f) / s2;
+  if (ensure_sweep_buffers(h)) return -2;
+  h->launches = 0;
+  h->pev_used = 0;
+  h->prof_open = false;
+  h->gemm_flops = h->gemm_flops_exec = 0.0;
+  h->gemm_launches = 0;
+  PsiConst c;
+  psi_make_const(alpha, gamma, omega, h->causal, h->cull, &c, h->causal_id);
+  PsiConst cd = c;                       // test-side statistics are evaluated densely (no windows)
+  cd.cull = 746.0;
+  BvnTab T;
+  bvn_make_tab(gamma / (alpha + gamma + omega), &T);
+  std::vector<Chunk> chunks;
+  plan_chunks(h, h->fc, chunks);
+  if (ensure_ypart(h, y_slices_used(chunks))) return -2;
+  cudaStream_t st = h->st;
+  const int n = (int)n_star, npad = round_up(n, 8);
+  const long n2 = (long)npad * npad;
+  const int TP = pcov_tile(h);
+  const int TPP = TP * TP;               // pairs of a full tile (a multiple of 8)
+  const int nhl = round_up(nh, 2);
+  const long KH = (long)nh * nhl;
+  const int bcap = predict_bcap(h);
+  const double per = 8.0 * ((double)n2 + (double)KH + (double)nxp * nxp + (smf ? (double)l2 : 0.0));
+  const int gcap = std::max(bcap, std::min(round_up(B, bcap), (int)std::min(1e6, 4e9 / per) / bcap * bcap));
+  const int nq = smf ? gcap : 1;         // q(z) slabs held at a time
+  long wcols = 0;
+  for (const Chunk& ch : chunks) wcols = std::max<long>(wcols, (long)ch.nc * ch.kwp);
+  const long acols = (long)npad * nxp;   // columns of A* / T: [i][p][k]
+  long off = 0;
+  auto take = [&](long cnt) { const long o = off; off += (cnt + 1) / 2 * 2; return o; };     // 16-byte aligned
+  const long o_t = take(n), o_a = take((long)nhp * acols), o_ta = take((long)nhp * acols);
+  const long o_mean = take((long)n * B), o_draw = take(want_draws ? (long)n * B : 0);
+  const long o_noise = take(want_draws ? (long)B * npad : 0), o_cov = take(cov_out ? n2 : 0);
+  const long o_x = take((long)TPP * nx * nx), o_g = take((long)TPP * nxp * nxp);
+  const long o_ac = take(TPP), o_lag = take(TPP), o_AC = take((long)TPP * KH);
+  const long o_gf = take((long)TPP * bcap), o_qp = take((long)PQ_SLICES * TPP * bcap);
+  const long o_hs = take((long)gcap * nhp), o_q1 = take(gcap), o_xm = take((long)nq * ld), o_mx = take((long)nq * l2);
+  const long o_mxp = take((long)nq * nxp * nxp), o_hh = take((long)gcap * KH), o_c = take((long)gcap * n2);
+  const long o_part = take(smf ? (long)bcap * SMF_SLICES * l2 : 0), o_c1 = take(smf ? (long)bcap * l2 : 0);
+  const long o_work = take(smf ? 2L * bcap * l2 : 0), o_w = take(smf ? (long)bcap * wcols : 0);
+  const long o_v = take((long)bcap * acols), o_y = take(acols);
+  const long o_quad = take((long)npad * bcap), o_lin = take((long)npad * bcap);
+  const long o_k = take(want_draws ? n2 : 0), o_f = take(want_draws ? npad : 0);
+  double* buf = nullptr;
+  int* d_info = nullptr;
+  auto cleanup = [&]() {
+    if (buf) cudaFree(buf);
+    if (d_info) cudaFree(d_info);
+  };
+#define PCK(call) do { cudaError_t e_ = (call); if (e_ != cudaSuccess) { char b_[256]; snprintf(b_, sizeof b_, \
+    "CUDA error %s in predict_f_cov (%s)", cudaGetErrorString(e_), #call); h->err = b_; cleanup(); return -2; } } while (0)
+#define PRC(call) do { if (call) { cleanup(); return -2; } } while (0)
+  PCK(cudaMalloc(&buf, (size_t)off * sizeof(double)));
+  PCK(cudaMalloc(&d_info, (size_t)(gcap + bcap) * sizeof(int)));
+  double *d_t = buf + o_t, *d_A = buf + o_a, *d_TA = buf + o_ta, *d_mean = buf + o_mean, *d_draw = buf + o_draw;
+  double *d_noise = buf + o_noise, *d_cov = buf + o_cov, *d_x = buf + o_x, *d_g = buf + o_g, *d_ac = buf + o_ac;
+  double *d_lag = buf + o_lag, *d_AC = buf + o_AC, *d_gf = buf + o_gf, *d_qp = buf + o_qp, *d_hs = buf + o_hs;
+  double *d_q1 = buf + o_q1, *d_xm = buf + o_xm, *d_mx = buf + o_mx, *d_mxp = buf + o_mxp, *d_hh = buf + o_hh;
+  double *d_c = buf + o_c, *d_part = buf + o_part, *d_c1 = buf + o_c1, *d_work = buf + o_work, *d_w = buf + o_w;
+  double *d_v = buf + o_v, *d_y = buf + o_y, *d_quad = buf + o_quad, *d_lin = buf + o_lin, *d_k = buf + o_k;
+  double* d_f = buf + o_f;
+  int* d_pinfo = d_info + bcap;          // per sample of the group: the factorisation of C_b + reg I
+  PCK(cudaEventRecord(h->ev[0], st));
+  PCK(cudaMemsetAsync(h->info, 0, 4 * sizeof(int), st));
+  PCK(cudaMemcpyAsync(h->params_d, params_host, np * sizeof(double), cudaMemcpyHostToDevice, st));
+  PCK(cudaMemcpyAsync(d_t, tstar_host, n * sizeof(double), cudaMemcpyHostToDevice, st));
+  if (cov_out) PCK(cudaMemsetAsync(d_cov, 0, (size_t)n2 * sizeof(double), st));
+  std::vector<double> noise_t;
+  if (want_draws) {
+    // noise[p][b] -> one zero-padded column per sample
+    noise_t.assign((size_t)B * npad, 0.0);
+    for (int b = 0; b < B; ++b)
+      for (int p = 0; p < n; ++p) noise_t[(size_t)b * npad + p] = noise_host[(size_t)p * B + b];
+    PCK(cudaMemcpyAsync(d_noise, noise_t.data(), noise_t.size() * sizeof(double), cudaMemcpyHostToDevice, st));
+  }
+  PRC(prior_stage(h, c, reg, true));
+  if (smf || !h->gram_valid) PRC(plan_store(h, chunks, false));
+  PRC(predict_qu(h, reg));
+  if (!smf) {
+    PRC(predict_qz(h, chunks, 0, h->V(V_MU), h->M(M_VAR), r, c0, reg, d_xm));
+    const double* xv = h->M(M_PINV);
+    const double* ikx = h->M(M_IKX);
+    const double* xm = d_xm;
+    double* mx = d_mx;
+    double* mxp = d_mxp;
+    const int nxp_ = nxp;
+    ew(st, (long)nxp * nxp, [=] __device__(long idx) {
+      const int i = (int)(idx / nxp_), j = (int)(idx % nxp_);
+      const long e = (long)i * ld + j;
+      const double v = (i < nx && j < nx) ? xv[e] + xm[i] * xm[j] - ikx[e] : 0.0;
+      if (i < nx && j < nx) mx[(long)i * nx + j] = v;
+      mxp[idx] = v;
+    });
+    L(h);
+  }
+  {
+    int info[4];
+    PCK(cudaMemcpyAsync(info, h->info, sizeof info, cudaMemcpyDeviceToHost, st));
+    PCK(cudaStreamSynchronize(st));
+    if (info[0]) {
+      h->prior_valid = false;
+      static const char* names[] = {"?", "Kh", "Kx", "P of q(z)", "?", "?"};
+      const int tag = info[0] / 100000;
+      char b[160];
+      snprintf(b, sizeof b, "matrix %s is not positive definite (pivot %d)", tag >= 1 && tag <= 5 ? names[tag] : "?",
+               info[0] % 100000);
+      h->err = b;
+      cleanup();
+      return -3;
+    }
+  }
+  // ---- test side, once: A* and T = iKh A* for every test input
+  {
+    const int threads = std::min(256, round_up(nxp, 32));
+    dim3 grid(nhp, (npad + AHX_NSUB - 1) / AHX_NSUB);
+    ahx_gen_kernel<<<grid, threads, 0, st>>>(d_t, d_t, n, npad, h->th, nh, h->tx, nx, 0, nxp, d_A, nullptr, ld,
+                                             (long)nhp * ld, cd);
+    L(h);
+  }
+  PRC(gemm(h, true, false, false, nhp, (int)acols, nhp, 1.0, h->M(M_IKH), ld, d_A, acols, 0.0, d_TA, acols));
+  std::vector<double> hsm;
+  std::vector<int> inf(std::max(bcap, gcap));
+  const double w = 1.0 / B;
+  const int ntile = (n + TP - 1) / TP;
+  for (int g0 = 0; g0 < B; g0 += gcap) {
+    const int gn = std::min(gcap, B - g0);
+    const int nbat = (gn + bcap - 1) / bcap;
+    // ---- training side of the group
+    for (int bi = 0; bi < nbat; ++bi) {
+      const int b0 = g0 + bi * bcap, nb = std::min(bcap, B - b0);
+      double* hs = d_hs + (long)bi * bcap * nhp;
+      if (smf) {
+        PRC(smf_c1_stage(h, chunks, samples_host + (size_t)b0 * nh, nb, bcap, hsm, hs, d_part, d_c1, d_w, wcols));
+        SmfPostArgs a;
+        a.kx = h->M(M_KX); a.sxx = h->M(M_F_AXX); a.c1 = d_c1; a.fy = h->M(M_F_Y); a.ahh = h->M(M_AHH);
+        a.ikx = h->M(M_IKX); a.tr = h->sc + S_TR_IKH_AHH; a.hs = hs; a.work = d_work;
+        a.mx = d_mx + (long)bi * bcap * l2; a.xm = d_xm + (long)bi * bcap * ld; a.q1 = d_q1 + (long)bi * bcap;
+        a.info = d_info; a.ld = ld; a.l2 = l2; a.ldh = nhp; a.nh = nh; a.nx = nx; a.nb = nb;
+        a.r = r; a.c0 = c0; a.reg = reg; a.a = 0.0;
+        PCK(cudaMemsetAsync(d_info, 0, bcap * sizeof(int), st));
+        smf_posterior_launch(st, a, bcap);
+        L(h);
+        PCK(cudaGetLastError());
+        PCK(cudaMemcpyAsync(inf.data(), d_info, bcap * sizeof(int), cudaMemcpyDeviceToHost, st));
+        PCK(cudaStreamSynchronize(st));
+        for (int b = 0; b < nb; ++b)
+          if (inf[b]) {
+            char m[160];
+            snprintf(m, sizeof m, "matrix P of sample %d is not positive definite (pivot %d)", b0 + b, inf[b]);
+            h->err = m;
+            cleanup();
+            return -3;
+          }
+        // mx_b in the padded nxp x nxp layout of the rank-one GEMMs
+        const double* mx = d_mx + (long)bi * bcap * l2;
+        double* mxp = d_mxp + (long)bi * bcap * nxp * nxp;
+        const int nxp_ = nxp;
+        const long pp = (long)nxp * nxp;
+        ew(st, (long)nb * pp, [=] __device__(long idx) {
+          const int b = (int)(idx / pp);
+          const long e = idx - (long)b * pp;
+          const int i = (int)(e / nxp_), j = (int)(e % nxp_);
+          mxp[idx] = (i < nx && j < nx) ? mx[(long)b * l2 + (long)i * nx + j] : 0.0;
+        });
+        L(h);
+      } else {
+        hsm.assign((size_t)bcap * nhp, 0.0);
+        for (int b = 0; b < nb; ++b)
+          for (int i = 0; i < nh; ++i) hsm[(size_t)b * nhp + i] = samples_host[(size_t)(b0 + b) * nh + i];
+        // (pageable source: staged before the call returns)
+        PCK(cudaMemcpyAsync(hs, hsm.data(), hsm.size() * sizeof(double), cudaMemcpyHostToDevice, st));
+      }
+    }
+    // HH[b] = h_b h_b^T - iKh (rows past the group are zero)
+    hh_build_kernel<<<148 * 4, 256, 0, st>>>(d_hs, nhp, gn, nbat * bcap, h->M(M_IKH), ld, nh, nhl, d_hh);
+    L(h);
+    // ---- per batch: V = H_B A*, the means, R_b = V_b mx_b V_b^T into C_b
+    for (int bi = 0; bi < nbat; ++bi) {
+      const int b0 = g0 + bi * bcap, nb = std::min(bcap, B - b0);
+      const double* hs = d_hs + (long)bi * bcap * nhp;
+      PRC(gemm(h, true, false, false, bcap, (int)acols, nhp, 1.0, hs, nhp, d_A, acols, 0.0, d_v, acols));
+      prof_close(h);
+      PredQuadArgs qa;
+      qa.V = d_v; qa.v_stride = acols; qa.ldv = nxp;
+      qa.mx = smf ? d_mx + (long)bi * bcap * l2 : d_mx; qa.mx_stride = smf ? l2 : 0;
+      qa.xm = smf ? d_xm + (long)bi * bcap * ld : d_xm; qa.xm_stride = smf ? ld : 0;
+      qa.nv = n; qa.nx = nx; qa.nb = nb; qa.quad = d_quad; qa.lin = d_lin; qa.ldo = bcap;
+      predict_quad_launch(st, qa, bcap);
+      L(h);
+      {
+        const double* lin = d_lin;
+        double* mean = d_mean + b0;
+        const double sq = sqrt(s2f);
+        const int nb_ = nb, Bn = B, bc = bcap;
+        ew(st, (long)n * nb, [=] __device__(long idx) {
+          const int p = (int)(idx / nb_), b = (int)(idx % nb_);
+          mean[(long)p * Bn + b] = sq * lin[(long)p * bc + b];
+        });
+        L(h);
+      }
+      for (int b = 0; b < nb; ++b) {
+        const double* Vb = d_v + (long)b * acols;
+        const double* mxp = d_mxp + (smf ? (long)(bi * bcap + b) * nxp * nxp : 0);
+        double* Cb = d_c + (long)(bi * bcap + b) * n2;
+        PRC(gemm(h, true, false, false, npad, nxp, nxp, 1.0, Vb, nxp, mxp, nxp, 0.0, d_y, nxp));
+        PRC(gemm(h, true, true, false, npad, npad, nxp, 1.0, d_y, nxp, Vb, nxp, 0.0, Cb, npad));
+      }
+    }
+    // ---- pair tiles p >= q
+    for (int pt = 0; pt < ntile; ++pt)
+      for (int qt = 0; qt <= pt; ++qt) {
+        const int p0 = pt * TP, q0 = qt * TP;
+        const int P = std::min(TP, n - p0), Q = std::min(TP, n - q0);
+        const int npairs = P * Q, npp = round_up(npairs, 8);
+        const long ldg = (long)TP * nxp;
+        // G(i, k; j, l) = sum_m A*[m][(p0 + i, k)] T[m][(q0 + j, l)]
+        PRC(gemm(h, false, false, false, P * nxp, Q * nxp, nhp, 1.0, d_A + (long)p0 * nxp, acols,
+                 d_TA + (long)q0 * nxp, acols, 0.0, d_g, ldg));
+        prof_close(h);
+        axx_pair_launch(st, d_t + p0, P, d_t + q0, Q, h->tx, nx, d_g, ldg, nxp, d_x, cd, T);
+        L(h);
+        {
+          const double* tt = d_t;
+          double* lag = d_lag;
+          ew(st, npairs, [=] __device__(long e) { lag[e] = tt[p0 + e / Q] - tt[q0 + e % Q]; });
+          L(h);
+        }
+        if (npp > npairs) PCK(cudaMemsetAsync(d_AC + (long)npairs * KH, 0, (size_t)(npp - npairs) * KH * sizeof(double), st));
+        ahh_center_kernel<<<148 * 8, 256, 0, st>>>(d_lag, npairs, h->th, nh, nhl, alpha, gamma, h->causal, d_AC, d_ac);
+        L(h);
+        if (!smf) {
+          predict_qb_launch(st, d_x, (long)nx * nx, d_mx, l2, 1, npairs, TPP, 1, d_qp, bcap);     // one column
+          L(h);
+        }
+        for (int bi = 0; bi < nbat; ++bi) {
+          const int b0 = g0 + bi * bcap, nb = std::min(bcap, B - b0);
+          // gf[e][b] = sum_(i,j) Ahh_c(lag_e)[i][j] HH_b[i][j]
+          PRC(gemm(h, true, true, false, npp, bcap, (int)KH, 1.0, d_AC, KH, d_hh + (long)bi * bcap * KH, KH, 0.0, d_gf,
+                   bcap));
+          prof_close(h);
+          if (smf) {
+            predict_qb_launch(st, d_x, (long)nx * nx, d_mx + (long)bi * bcap * l2, l2, nb, npairs, TPP, bcap, d_qp, bcap);
+            L(h);
+          }
+          pcov_finish_kernel<<<(int)std::min<long>(((long)npairs * nb + 255) / 256, 148 * 16), 256, 0, st>>>(
+              d_qp, TPP, bcap, smf ? 1 : 0, d_gf, bcap, d_ac, npairs, Q, p0, q0, nb, d_mean + b0, B, s2f,
+              d_c + (long)bi * bcap * n2, n2, npad);
+          L(h);
+        }
+      }
+    PCK(cudaGetLastError());
+    // ---- cov += C_b / B in ascending b; the per-sample outputs
+    if (cov_out) {
+      const double* C = d_c;
+      double* cv = d_cov;
+      const int gn_ = gn;
+      ew(st, n2, [=] __device__(long idx) {
+        double s = cv[idx];
+        for (int b = 0; b < gn_; ++b) s += w * C[(long)b * n2 + idx];
+        cv[idx] = s;
+      });
+      L(h);
+    }
+    if (cov_s_out)
+      for (int b = 0; b < gn; ++b)
+        PCK(cudaMemcpy2DAsync(cov_s_out + (size_t)(g0 + b) * n * n, (size_t)n * sizeof(double), d_c + (long)b * n2,
+                              (size_t)npad * sizeof(double), (size_t)n * sizeof(double), n, cudaMemcpyDefault, st));
+    if (want_draws) {
+      PCK(cudaMemsetAsync(d_pinfo, 0, (size_t)gn * sizeof(int), st));
+      for (int b = 0; b < gn; ++b) {
+        const double* Cb = d_c + (long)b * n2;
+        double* Kp = d_k;
+        const int nn = n, ldn = npad;
+        ew(st, n2, [=] __device__(long idx) {
+          const int rr = (int)(idx / ldn), qq = (int)(idx - (long)rr * ldn);
+          double v = (rr == qq) ? 1.0 : 0.0;                  // identity on the padding block
+          if (rr < nn && qq < nn) v = Cb[idx] + (rr == qq ? reg : 0.0);
+          Kp[idx] = v;
+        });
+        L(h);
+        cudaError_t e = potrf_lower(st, d_k, npad, npad, d_pinfo + b, 7, h->M(M_XW));
+        L(h, 2 * ((npad + LA_NB - 1) / LA_NB));
+        if (e != cudaSuccess) { h->err = "potrf launch failed"; cleanup(); return -2; }
+        matvec_kernel<<<(npad + 7) / 8, 256, 0, st>>>(d_k, npad, npad, npad, 0, d_noise + (long)(g0 + b) * npad, 1.0, d_f);
+        L(h);
+        const double* fv = d_f;
+        const double* mean = d_mean + g0 + b;
+        double* dr = d_draw + g0 + b;
+        const int Bn = B;
+        ew(st, n, [=] __device__(long p) { dr[p * Bn] = mean[p * Bn] + fv[p]; });
+        L(h);
+      }
+      PCK(cudaMemcpyAsync(inf.data(), d_pinfo, (size_t)gn * sizeof(int), cudaMemcpyDeviceToHost, st));
+      PCK(cudaStreamSynchronize(st));
+      for (int b = 0; b < gn; ++b)
+        if (inf[b]) {
+          char m[160];
+          snprintf(m, sizeof m, "matrix C_b + reg I of sample %d is not positive definite (pivot %d)", g0 + b,
+                   inf[b] % 100000);
+          h->err = m;
+          cleanup();
+          return -3;
+        }
+    }
+  }
+  if (mean_s_out) PCK(cudaMemcpyAsync(mean_s_out, d_mean, (size_t)n * B * sizeof(double), cudaMemcpyDefault, st));
+  if (want_draws) PCK(cudaMemcpyAsync(draws_out, d_draw, (size_t)n * B * sizeof(double), cudaMemcpyDefault, st));
+  if (cov_out)
+    PCK(cudaMemcpy2DAsync(cov_out, (size_t)n * sizeof(double), d_cov, (size_t)npad * sizeof(double),
+                          (size_t)n * sizeof(double), n, cudaMemcpyDefault, st));
+  prof_close(h);
+  PCK(cudaEventRecord(h->ev[6], st));
+  PCK(cudaStreamSynchronize(st));
+  PCK(cudaGetLastError());
+  cleanup();
+#undef PCK
+#undef PRC
+  float ms = 0;
+  cudaEventElapsedTime(&ms, h->ev[0], h->ev[6]);
+  memset(h->timing, 0, sizeof h->timing);
+  h->timing[0] = ms;
+  h->timing[6] = (double)h->launches;
+  h->timing[7] = h->gemm_flops;
+  h->timing[8] = (double)h->gemm_launches;
+  return 0;
+}
+
 }  // namespace cgimpl
 
 extern "C" {
@@ -3377,6 +3749,31 @@ int cgpcm_predict_f_batch(cgpcm_handle* h, const double* params, double reg, con
   else memcpy(smp.data(), samples, smp.size() * sizeof(double));
   return predict_batch_run(h, host.data(), reg, ts.data(), n_star, smp.data(), n_samples, smf ? 1 : 0, mean, var,
                            mean_s, var_s);
+}
+
+int cgpcm_predict_f_cov(cgpcm_handle* h, const double* params, double reg, const double* t_star, int64_t n_star,
+                        const double* samples, int32_t n_samples, int32_t smf, double* mean_s, double* cov_s,
+                        double* cov, const double* noise, double* draws) {
+  if (!h || !params || n_star < 0 || !samples || (n_star > 0 && !t_star)) return -1;
+  if (n_samples < 1) { h->err = "n_samples must be >= 1"; return -1; }
+  if (n_star > 4096) { h->err = "predict_f_cov: at most 4096 test inputs"; return -1; }
+  if (draws && !noise) { h->err = "predict_f_cov: draws need noise"; return -1; }
+  if (!h->t) { h->err = "cgpcm_set_data has not been called"; return -1; }
+  if (!std::isfinite(reg) || reg < 0) { h->err = "reg must be finite and >= 0"; return -4; }
+  if (n_star == 0) return 0;
+  CK(cudaSetDevice(h->device));
+  const long np = 5 + h->nh + (long)h->nh * (h->nh + 1) / 2;
+  std::vector<double> host, ts(n_star), smp((size_t)n_samples * h->nh), ns(draws ? (size_t)n_star * n_samples : 0);
+  if (fetch_params(h, params, np, host)) return -2;
+  auto fetch = [&](const double* src, std::vector<double>& dst) -> int {
+    if (is_device_ptr(src)) CK(cudaMemcpy(dst.data(), src, dst.size() * sizeof(double), cudaMemcpyDeviceToHost));
+    else memcpy(dst.data(), src, dst.size() * sizeof(double));
+    return 0;
+  };
+  if (fetch(t_star, ts) || fetch(samples, smp)) return -2;
+  if (draws && fetch(noise, ns)) return -2;
+  return predict_cov_run(h, host.data(), reg, ts.data(), n_star, smp.data(), n_samples, smf ? 1 : 0,
+                         draws ? ns.data() : nullptr, mean_s, cov_s, cov, draws);
 }
 
 int cgpcm_kernel_samples(cgpcm_handle* h, const double* params, double reg, const double* t, int64_t n,
@@ -3849,6 +4246,24 @@ int cgpcm_predict_quad_test(const double* V, int64_t v_stride, int ldv, const do
   }
   if (cudaStreamSynchronize(st) != cudaSuccess) rc = -2;
   if (part) cudaFree(part);
+  return rc;
+}
+
+int cgpcm_predict_pair_test(const double* tp, int np_, const double* tq, int nq, const double* tx, int nx,
+                            const double hyp[3], int causal, int causal_id, const double* G, int64_t ldg, int gk,
+                            double* X, void* stream) {
+  if (!tp || !tq || !tx || !hyp || !X || np_ < 1 || nq < 1 || nx < 1 || (G && (gk < nx || ldg < (int64_t)nq * gk)))
+    return -1;
+  for (int i = 0; i < 3; ++i)
+    if (!std::isfinite(hyp[i]) || hyp[i] <= 0) return -4;
+  cudaStream_t st = (cudaStream_t)stream;
+  PsiConst c;
+  psi_make_const(hyp[0], hyp[1], hyp[2], causal ? 1 : 0, 0.0, &c, causal_id);      // cull 0: dense (746)
+  BvnTab T;
+  bvn_make_tab(hyp[1] / (hyp[0] + hyp[1] + hyp[2]), &T);
+  axx_pair_launch(st, tp, np_, tq, nq, tx, nx, G, (long)ldg, gk, X, c, T);
+  int rc = cudaGetLastError() == cudaSuccess ? 0 : -2;
+  if (cudaStreamSynchronize(st) != cudaSuccess) rc = -2;
   return rc;
 }
 

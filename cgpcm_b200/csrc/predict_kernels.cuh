@@ -10,6 +10,7 @@
 #include <cuda_runtime.h>
 
 #include "dgemm_dmma.cuh"
+#include "psi_kernels.cuh"
 
 namespace cg {
 
@@ -303,6 +304,71 @@ __global__ void predict_finish_kernel(const double* __restrict__ qpart, int nrow
   }
   acc_mu[n] = am;
   acc_var[n] = av;
+}
+
+// ---- Joint predictive covariance (cgpcm_predict_f_cov): the expectation of f_p f_q under sample b's q(z) is
+//     E[f_p f_q | h_b] = s2_f (a_c(t_p - t_q) + <Ahh_c(t_p - t_q), h_b h_b^T - iKh> + <Bxx*(p, q), mx_b> + v_p^T mx_b v_q)
+//     Bxx*(p, q) = Axx(t_p, t_q) - A*_p^T iKh A*_q,   v_p = A*_p^T h_b
+// Axx(t_p, t_q) is the closed form of Axx with the two inputs on the two factors of the double integral: substituting
+// s1 = t_p - tau1, s2 = t_q - tau2 leaves the quadratic form unchanged and only moves the linear terms, so it is
+// axx_user_kernel's arithmetic with dk = t_p - tx_k and dl = t_q - tx_l (tests/pair_oracle.py).  The centre
+// statistics a_c, Ahh_c at the lag are those of predict_k / the AKM sampler (ahh_center_kernel).  Work runs over tiles
+// of P x Q point pairs, p >= q; pair e = i Q + j stands for (p0 + i, q0 + j).
+
+// X[e][k][l] = Axx(tp[i], tq[j])[k][l] - G(i, k; j, l)   (e = i nq + j, dense [pair][nx][nx]; G optional:
+// G(i, k; j, l) at G[(i gk + k) ldg + j gk + l], the fold A*_p^T iKh A*_q as one GEMM lays it out).  Evaluated densely
+// (c.cull = 746: a skipped element is exactly 0).  Grid-stride, any grid.
+__global__ void axx_pair_kernel(const double* __restrict__ tp, int np_, const double* __restrict__ tq, int nq,
+                                const double* __restrict__ tx, int nx, const double* __restrict__ G, long ldg, int gk,
+                                double* __restrict__ X, const PsiConst c, const BvnTab T) {
+  const long per = (long)nx * nx;
+  const long total = (long)np_ * nq * per;
+  for (long idx = (long)blockIdx.x * blockDim.x + threadIdx.x; idx < total; idx += (long)gridDim.x * blockDim.x) {
+    const long e = idx / per;
+    const int r = (int)(idx - e * per);
+    const int k = r / nx, l = r - k * nx;
+    const int i = (int)(e / nq), j = (int)(e - (long)i * nq);
+    const double dk = tp[i] - tx[k], dl = tq[j] - tx[l];
+    const double Gx = -c.g1 * (dk * dk + dl * dl) + c.g2 * dk * dl;
+    double v = 0.0;
+    if (Gx >= -c.cull) {
+      v = c.pref_xx * exp(Gx);
+      if (c.causal) {
+        double x1 = c.p * dk + c.q * dl, x2 = c.q * dk + c.p * dl;
+        if (c.causal_id) { x1 -= fmax(dk, 0.0) * c.isq11; x2 -= fmax(dl, 0.0) * c.isq11; }
+        v *= bvnd_tab(-x1, -x2, T);
+      }
+    }
+    if (G) v -= G[((long)i * gk + k) * ldg + (long)j * gk + l];
+    X[idx] = v;
+  }
+}
+
+inline void axx_pair_launch(cudaStream_t st, const double* tp, int np_, const double* tq, int nq, const double* tx,
+                            int nx, const double* G, long ldg, int gk, double* X, const PsiConst& c, const BvnTab& T) {
+  axx_pair_kernel<<<148 * 8, 256, 0, st>>>(tp, np_, tq, nq, tx, nx, G, ldg, gk, X, c, T);
+}
+
+// One thread per (pair, sample) of a tile with p >= q:
+//   C_b[p][q] = C_b[q][p] = s2f (ac[e] + gf[e][b] + Qb + R) - m_p m_q
+// with R = v_p^T mx_b v_q already in C_b[p][q] (the rank-one GEMMs), Qb the PQ_SLICES partials of column b * q_col
+// summed in order, gf[e][b] = <Ahh_c, h_b h_b^T - iKh> and m the per-sample means at m[p * ldm + b].
+__global__ void pcov_finish_kernel(const double* __restrict__ qpart, int nrow, int ldq, int q_col,
+                                   const double* __restrict__ gf, int ldgf, const double* __restrict__ ac, int npairs,
+                                   int nq, int p0, int q0, int nb, const double* __restrict__ m, long ldm, double s2f,
+                                   double* __restrict__ C, long cstride, long ldc) {
+  const long total = (long)npairs * nb;
+  for (long idx = (long)blockIdx.x * blockDim.x + threadIdx.x; idx < total; idx += (long)gridDim.x * blockDim.x) {
+    const int e = (int)(idx / nb), b = (int)(idx - (long)e * nb);
+    const int p = p0 + e / nq, q = q0 + e % nq;
+    if (p < q) continue;
+    double qb = 0.0;
+    for (int z = 0; z < PQ_SLICES; ++z) qb += qpart[((long)z * nrow + e) * ldq + b * q_col];
+    double* Cb = C + (long)b * cstride;
+    const double v = s2f * (ac[e] + gf[(long)e * ldgf + b] + qb + Cb[(long)p * ldc + q]) - m[(long)p * ldm + b] * m[(long)q * ldm + b];
+    Cb[(long)p * ldc + q] = v;
+    Cb[(long)q * ldc + p] = v;
+  }
 }
 
 }  // namespace cg

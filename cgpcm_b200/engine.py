@@ -179,6 +179,37 @@ class Engine(object):
                                                        _lib.ptr(var), _lib.ptr(mean_s), _lib.ptr(var_s)))
         return mean, var, mean_s, var_s
 
+    def predict_f_cov(self, params, t_star, samples, smf=True, reg=1e-8, per_sample=False, noise=None):
+        """Joint predictive covariance of the function at ``t_star`` (at most 4096 inputs) for every filter sample
+        ([B, nh]) in one call: ``(mean[n], cov[n, n], mean_s[n, B], cov_s[B, n, n], draws[n, B])``.  ``cov_s[b]`` is the
+        covariance of f under sample b's q(z) (``smf`` as in :meth:`predict_f_batch`; its diagonal is that method's
+        ``var_s[:, b]``); ``mean`` and ``cov`` are the sample averages (``diag(cov)`` is :meth:`predict_f`'s variance).
+        The mixture covariance of the samples is ``cov + np.cov(mean_s, bias=True)``.  ``per_sample=False`` returns
+        ``None`` for ``cov_s``.  With standard normal ``noise`` ([n, B]), ``draws[:, b] = mean_s[:, b] +
+        chol(cov_s[b] + reg I) noise[:, b]``, else ``None``.  A sample's outputs do not depend on the other samples of
+        the call; needs the frozen statistics."""
+        t_star = np.ascontiguousarray(np.asarray(t_star, dtype=np.float64).ravel())
+        samples = np.ascontiguousarray(np.asarray(samples, dtype=np.float64))
+        if samples.ndim == 1:
+            samples = samples.reshape(1, -1)
+        if samples.ndim != 2 or samples.shape[1] != self.nh or samples.shape[0] < 1 or \
+                int(params.shape[0]) != n_params(self.nh):
+            raise ValueError('shape mismatch in predict_f_cov')
+        n, B = t_star.shape[0], samples.shape[0]
+        draws = None
+        if noise is not None:
+            noise = np.ascontiguousarray(np.asarray(noise, dtype=np.float64))
+            if noise.shape != (n, B):
+                raise ValueError('noise must have shape (n_star, B)')
+            draws = np.empty((n, B))
+        mean_s, cov = np.empty((n, B)), np.empty((n, n))
+        cov_s = np.empty((B, n, n)) if per_sample else None
+        if n:
+            self._ck(_lib.lib().cgpcm_predict_f_cov(self._h, _lib.ptr(params), float(reg), _lib.ptr(t_star), n,
+                                                     _lib.ptr(samples), B, int(bool(smf)), _lib.ptr(mean_s),
+                                                     _lib.ptr(cov_s), _lib.ptr(cov), _lib.ptr(noise), _lib.ptr(draws)))
+        return mean_s.mean(1), cov, mean_s, cov_s, draws
+
     def kernel_samples(self, params, t, samples, reg=1e-8):
         """Kernel samples ``k[n, b]`` of ``predict_k`` at lags ``t`` for filter ``samples`` ([B, nh])
         (``src/core/cgpcm.py:610-634``), before normalisation."""

@@ -160,6 +160,31 @@ int cgpcm_predict_f_batch(cgpcm_handle* h, const double* params, double reg, con
                           const double* samples, int32_t n_samples, int32_t smf, double* mean, double* var,
                           double* mean_s, double* var_s);
 
+/* The joint predictive covariance of the function at n_star <= 4096 test inputs, per filter sample, and posterior
+ * draws of f.  For sample b, under the q(z) of cgpcm_predict_f_batch (smf = 1: q(z | h_b); smf = 0: the one q(z) of
+ * q(u)):
+ *   mean_s[p * n_samples + b]       the predictive mean, as cgpcm_predict_f_batch;
+ *   cov_s[(b * n_star + p) * n_star + q] = C_b[p][q] = E[f_p f_q | h_b] - mean_s[p][b] mean_s[q][b], full and exactly
+ *                                   symmetric; diag(C_b) is cgpcm_predict_f_batch's var_s[:, b];
+ *   cov[p * n_star + q]             (1 / n_samples) sum_b C_b, added in ascending b; its diagonal is cgpcm_predict_f's
+ *                                   var.  By the law of total covariance the covariance of the mixture of the samples'
+ *                                   predictive distributions is cov + Cov_b(mean_s);
+ *   draws[p * n_samples + b]        mean_s[:, b] + chol(C_b + reg I) noise[:, b] for the caller's standard normal
+ *                                   noise[p * n_samples + b] (so that draws follow the host generator).
+ * With E[f_p f_q | h] = s2_f (a_c(t_p - t_q) + <Ahh_c(t_p - t_q), h h^T - iKh> + <Axx(t_p, t_q), mx>
+ *                             + <(h h^T - iKh) Ahx_q mx, Ahx_p>),  mx = x_m2 - iKx,
+ * a_c / Ahh_c the centre statistics of cgpcm_kernel_samples at the lag and Axx(t_p, t_q) the Axx statistic with the two
+ * inputs on its two factors.  Every output may be NULL (draws then needs no noise; draws without noise is -1); host or
+ * device pointers.  C_b + reg I is only factorised when draws is requested.  Internal batch sizes depend on the
+ * handle's shape and n_star only and no sum runs across samples except cov: a sample's mean_s, C_b and draw are bitwise
+ * the same in any batch and at any position.  Uses the statistics frozen by cgpcm_precompute (-1 otherwise); -1 when
+ * n_samples < 1 or n_star > 4096; -4 for a non-finite parameter, sample, test input or noise; -3 when some P_b or some
+ * C_b + reg I is not positive definite (cgpcm_last_error names the sample and the pivot); n_star = 0 returns 0 and
+ * writes nothing. */
+int cgpcm_predict_f_cov(cgpcm_handle* h, const double* params, double reg, const double* t_star, int64_t n_star,
+                        const double* samples, int32_t n_samples, int32_t smf, double* mean_s, double* cov_s,
+                        double* cov, const double* noise, double* draws);
+
 /* The Monte-Carlo kernel samples of mod.predict_k(t, samples_h) (src/core/cgpcm.py:610-634; centre statistics
  * _a_center / _Ahh_center :164-166,190-192), before normalisation / FFT / percentiles (host post-processing):
  * out[p * n_samples + b] = s2_f (a_c(t_p) + tr((h_b h_b^T - iKh) Ahh_c(t_p))) for lags t[n] and filter samples
@@ -285,6 +310,15 @@ int cgpcm_smf_posterior_test(const double* kx, const double* sum_Bxx, const doub
 int cgpcm_predict_quad_test(const double* V, int64_t v_stride, int ldv, const double* mx, int64_t mx_stride,
                             const double* xm, int64_t xm_stride, const double* bxx, int nv, int nx, int B, int nslots,
                             double* quad, double* lin, double* qb, void* stream);
+/* The pair-block kernel of cgpcm_predict_f_cov (axx_pair_kernel, csrc/predict_kernels.cuh) with its launch shape; device
+ * pointers only; returns after the stream has drained.  For i < np, j < nq, k, l < nx, with hyp = (alpha, gamma, omega)
+ * on the host and the model's causal / causal_id flags:
+ *   X[((i * nq + j) * nx + k) * nx + l] = Axx(tp[i], tq[j])[k][l] - G[(i * gk + k) * ldg + j * gk + l]
+ * (G may be NULL: no fold; ldg >= nq gk, gk >= nx), Axx(t1, t2) the Axx statistic with dk = t1 - tx_k, dl = t2 - tx_l,
+ * evaluated densely.  -1 for bad shapes, -4 for a non-positive or non-finite hyper-parameter. */
+int cgpcm_predict_pair_test(const double* tp, int np, const double* tq, int nq, const double* tx, int nx,
+                            const double hyp[3], int causal, int causal_id, const double* G, int64_t ldg, int gk,
+                            double* X, void* stream);
 
 #ifdef __cplusplus
 }
