@@ -393,6 +393,141 @@ void dot(cgpcm_handle* h, const double* a, const double* b, int n, double* out) 
 
 void zero(cgpcm_handle* h, double* p, long n) { cudaMemsetAsync(p, 0, n * sizeof(double), h->st); }
 
+// ---- bookkeeping shared by the runs -------------------------------------------------------------
+
+// Device scratch of one call: take(n) reserves a slice of n elements (aligned to 256 bytes, as cudaMalloc aligns; the
+// DMMA paths need 16) and returns its byte offset, alloc() makes one cudaMalloc, and the destructor frees it.
+struct Scratch {
+  size_t bytes = 0;
+  char* base = nullptr;
+  Scratch() = default;
+  Scratch(const Scratch&) = delete;
+  Scratch& operator=(const Scratch&) = delete;
+  ~Scratch() { if (base) cudaFree(base); }
+  size_t take(size_t n, size_t elem = sizeof(double)) {
+    const size_t o = bytes;
+    bytes += (n * elem + 255) / 256 * 256;
+    return o;
+  }
+  cudaError_t alloc() { return bytes ? cudaMalloc(&base, bytes) : cudaSuccess; }
+  template <class T = double> T* at(size_t off) const { return (T*)(base + off); }
+};
+
+// The hyper-parameters of params_host[0..4] (log s2, log s2_f, log alpha, log gamma, log omega) and the two ratios of
+// the bound: r = s2_f / s2, c0 = sqrt(s2_f) / s2.
+struct Hyp {
+  double s2, s2f, alpha, gamma, omega, r, c0;
+};
+Hyp hyp_of(const double* p) {
+  Hyp q;
+  q.s2 = exp(p[0]); q.s2f = exp(p[1]);
+  q.alpha = exp(p[2]); q.gamma = exp(p[3]); q.omega = exp(p[4]);
+  q.r = q.s2f / q.s2; q.c0 = sqrt(q.s2f) / q.s2;
+  return q;
+}
+
+// Start of a run: reset the launch, profile and GEMM counters, record ev[0] and clear the info word.
+int begin_run(cgpcm_handle* h) {
+  h->launches = 0;
+  h->pev_used = 0;
+  h->prof_open = false;
+  h->gemm_flops = h->gemm_flops_exec = 0.0;
+  h->gemm_launches = 0;
+  CK(cudaEventRecord(h->ev[0], h->st));
+  CK(cudaMemsetAsync(h->info, 0, 4 * sizeof(int), h->st));
+  return 0;
+}
+
+// End of a run: close the profiled GEMM run, record ev[6], wait for the stream and fetch the info word.
+int end_run(cgpcm_handle* h, int& info) {
+  int w[4];
+  CK(cudaMemcpyAsync(w, h->info, sizeof w, cudaMemcpyDeviceToHost, h->st));
+  prof_close(h);
+  CK(cudaEventRecord(h->ev[6], h->st));
+  CK(cudaStreamSynchronize(h->st));
+  CK(cudaGetLastError());
+  info = w[0];
+  return 0;
+}
+
+// cgpcm_last_timing of a run: [0] ev[0] -> ev[6] in ms, [6] launches, [7] GEMM flops, [8] GEMM launches, [9] executed
+// GEMM flops; the rest 0.
+void record_timing(cgpcm_handle* h) {
+  float ms = 0;
+  cudaEventElapsedTime(&ms, h->ev[0], h->ev[6]);
+  memset(h->timing, 0, sizeof h->timing);
+  h->timing[0] = ms;
+  h->timing[6] = (double)h->launches;
+  h->timing[7] = h->gemm_flops;
+  h->timing[8] = (double)h->gemm_launches;
+  h->timing[9] = h->gemm_flops_exec;
+}
+
+// A failed factorisation reported by the info word (tag * 100000 + pivot), named from the run's table: the prior
+// kernels are refactored next time, and the run returns -3.
+template <int N>
+int pd_error(cgpcm_handle* h, int info, const char* const (&names)[N]) {
+  if (!info) return 0;
+  h->prior_valid = false;
+  const int tag = info / 100000;
+  char b[160];
+  snprintf(b, sizeof b, "matrix %s is not positive definite (pivot %d)", tag >= 1 && tag < N ? names[tag] : "?",
+           info % 100000);
+  h->err = b;
+  return -3;
+}
+
+// A failed per-sample factorisation (the prior is not involved).
+int sample_pd_error(cgpcm_handle* h, const char* what, int sample, int pivot) {
+  char b[160];
+  snprintf(b, sizeof b, "matrix %s of sample %d is not positive definite (pivot %d)", what, sample, pivot);
+  h->err = b;
+  return -3;
+}
+
+// -4 with `msg` unless p[0..n) are all finite.
+int check_finite(cgpcm_handle* h, const double* p, long n, const char* msg) {
+  for (long i = 0; i < n; ++i)
+    if (!std::isfinite(p[i])) { h->err = msg; return -4; }
+  return 0;
+}
+
+// The same for B samples of nh values, naming the first sample with a non-finite value.
+int check_samples(cgpcm_handle* h, const double* s, long B, int nh) {
+  for (long i = 0; i < B * nh; ++i)
+    if (!std::isfinite(s[i])) {
+      char b[96];
+      snprintf(b, sizeof b, "non-finite value in sample %ld", i / nh);
+      h->err = b;
+      return -4;
+    }
+  return 0;
+}
+
+// n values of a user buffer (host or device) into v.
+int to_host(cgpcm_handle* h, const double* src, long n, std::vector<double>& v) {
+  v.resize(n);
+  if (is_device_ptr(src)) CK(cudaMemcpy(v.data(), src, n * sizeof(double), cudaMemcpyDeviceToHost));
+  else memcpy(v.data(), src, n * sizeof(double));
+  return 0;
+}
+
+// n host values into a user buffer (host or device; nothing when dst is NULL).
+int put(cgpcm_handle* h, double* dst, const double* src, long n) {
+  if (!dst || n == 0) return 0;
+  if (is_device_ptr(dst)) CK(cudaMemcpy(dst, src, n * sizeof(double), cudaMemcpyHostToDevice));
+  else memcpy(dst, src, n * sizeof(double));
+  return 0;
+}
+
+// Shared argument checks of the entry points: the data (`data`: h->t, or h->th where only the inducing inputs are
+// needed) has been set and reg is usable.
+int check_call(cgpcm_handle* h, const double* data, double reg) {
+  if (!data) { h->err = "cgpcm_set_data has not been called"; return -1; }
+  if (!std::isfinite(reg) || reg < 0) { h->err = "reg must be finite and >= 0"; return -4; }
+  return 0;
+}
+
 cudaEvent_t prof_event(cgpcm_handle* h, int kind) {
   if ((h->pev_used & 1) == 0) {
     if (h->pev_kind.size() <= h->pev_used / 2) h->pev_kind.resize(h->pev_used / 2 + 1);
@@ -1353,11 +1488,6 @@ int export_mat(cgpcm_handle* h, const double* src, int r, int c, double* dst) {
   return 0;
 }
 
-// Psi sums at hyper-parameters c: fills M_AXX0 (+tangents), M_Q, M_Y, M_C1 (with H given) ...
-struct EvalScalars {
-  double n_glob, sum_y2;
-};
-
 }  // namespace cgimpl
 
 extern "C" {
@@ -1370,12 +1500,11 @@ int cgpcm_psi(cgpcm_handle* h, const double hyp[3], double* sum_Axx, double* Ahh
     if (!std::isfinite(hyp[i]) || hyp[i] <= 0) { h->err = "hyper-parameters must be positive and finite"; return -4; }
   CK(cudaSetDevice(h->device));
   if (ensure_sweep_buffers(h)) return -2;
-  h->launches = 0;
   PsiConst c;
   psi_make_const(hyp[0], hyp[1], hyp[2], h->causal, h->cull, &c, h->causal_id);
   BvnTab T;
   bvn_make_tab(hyp[1] / (hyp[0] + hyp[1] + hyp[2]), &T);
-  CK(cudaEventRecord(h->ev[0], h->st));
+  if (begin_run(h)) return -2;
   const long ld = h->ld;
   h->prior_valid = false;      // the slots of the prior kernels are overwritten below (without jitter)
   prior_kernels_kernel<<<148 * 2, 256, 0, h->st>>>(h->th, h->nh, ld, h->tx, h->nx, ld, 0.0, h->M(M_KH0), h->M(M_LH),
@@ -1410,38 +1539,31 @@ int cgpcm_psi(cgpcm_handle* h, const double hyp[3], double* sum_Axx, double* Ahh
   }
   if (Ahx && h->n_local > 0) {
     double* dst = Ahx;
-    double* tmp = nullptr;
+    Scratch tmp;                  // staging for a host destination
     long total = h->n_local * h->nh * h->nx;
-    if (!is_device_ptr(Ahx)) { CK(cudaMalloc(&tmp, total * sizeof(double))); dst = tmp; }
+    if (!is_device_ptr(Ahx)) { tmp.take(total); CK(tmp.alloc()); dst = tmp.at(0); }
     ahx_user_kernel<<<148 * 8, 256, 0, h->st>>>(h->t, (int)h->n_local, h->th, h->nh, h->tx, h->nx, dst, c);
     L(h);
-    if (tmp) {
-      CK(cudaMemcpyAsync(Ahx, tmp, total * sizeof(double), cudaMemcpyDeviceToHost, h->st));
+    if (dst != Ahx) {
+      CK(cudaMemcpyAsync(Ahx, dst, total * sizeof(double), cudaMemcpyDeviceToHost, h->st));
       CK(cudaStreamSynchronize(h->st));
-      cudaFree(tmp);
     }
   }
   if (Axx && h->n_local > 0) {
     double* dst = Axx;
-    double* tmp = nullptr;
+    Scratch tmp;
     long total = h->n_local * h->nx * h->nx;
-    if (!is_device_ptr(Axx)) { CK(cudaMalloc(&tmp, total * sizeof(double))); dst = tmp; }
+    if (!is_device_ptr(Axx)) { tmp.take(total); CK(tmp.alloc()); dst = tmp.at(0); }
     axx_user_kernel<<<148 * 8, 256, 0, h->st>>>(h->t, (int)h->n_local, h->tx, h->nx, dst, c, T);
     L(h);
-    if (tmp) {
-      CK(cudaMemcpyAsync(Axx, tmp, total * sizeof(double), cudaMemcpyDeviceToHost, h->st));
+    if (dst != Axx) {
+      CK(cudaMemcpyAsync(Axx, dst, total * sizeof(double), cudaMemcpyDeviceToHost, h->st));
       CK(cudaStreamSynchronize(h->st));
-      cudaFree(tmp);
     }
   }
-  CK(cudaEventRecord(h->ev[1], h->st));
-  CK(cudaStreamSynchronize(h->st));
-  float ms = 0;
-  cudaEventElapsedTime(&ms, h->ev[0], h->ev[1]);
-  memset(h->timing, 0, sizeof h->timing);
-  h->timing[0] = ms;
-  h->timing[6] = (double)h->launches;
-  CK(cudaGetLastError());
+  int info;
+  if (end_run(h, info)) return -2;
+  record_timing(h);
   return 0;
 }
 
@@ -1551,20 +1673,12 @@ int evaluate_once(cgpcm_handle* h, const double* params_host, int mode, uint32_t
   const long ld = h->ld, l2 = ld * ld;
   const long nvar = (long)nh * (nh + 1) / 2;
   const long np = 5 + nh + nvar;
-  for (long i = 0; i < (freeze ? 5 : np); ++i)
-    if (!std::isfinite(params_host[i])) { h->err = "non-finite parameter"; return -4; }
-  const double s2 = exp(params_host[0]), s2f = exp(params_host[1]);
-  const double alpha = exp(params_host[2]), gamma = exp(params_host[3]), omega = exp(params_host[4]);
-  const double r = s2f / s2, c0 = sqrt(s2f) / s2;
+  if (check_finite(h, params_host, freeze ? 5 : np, "non-finite parameter")) return -4;
+  const Hyp hp = hyp_of(params_host);
+  const double s2 = hp.s2, alpha = hp.alpha, gamma = hp.gamma, omega = hp.omega, r = hp.r, c0 = hp.c0;
   const bool full = (mode == CGPCM_MODE_FULL) || freeze;
   if (!full && !h->frozen) { h->err = "MODE_FROZEN requires cgpcm_precompute"; return -1; }
   if (ensure_sweep_buffers(h)) return -2;
-  h->launches = 0;
-  h->pev_used = 0;
-  h->prof_open = false;
-  h->gemm_flops = 0.0;
-  h->gemm_flops_exec = 0.0;
-  h->gemm_launches = 0;
 
   PsiConst c;
   psi_make_const(alpha, gamma, omega, h->causal, h->cull, &c, h->causal_id);
@@ -1575,8 +1689,7 @@ int evaluate_once(cgpcm_handle* h, const double* params_host, int mode, uint32_t
   plan_chunks(h, ca, chunks);
 
   cudaStream_t st = h->st;
-  CK(cudaEventRecord(h->ev[0], st));
-  CK(cudaMemsetAsync(h->info, 0, 4 * sizeof(int), st));
+  if (begin_run(h)) return -2;
   if (!freeze) CK(cudaMemcpyAsync(h->params_d, params_host, np * sizeof(double), cudaMemcpyHostToDevice, st));
 
   // ---- 1. prologue (a full-regime evaluation always rebuilds the prior kernels; the precomputed regime reuses them).
@@ -1680,14 +1793,9 @@ int evaluate_once(cgpcm_handle* h, const double* params_host, int mode, uint32_t
       L(h);
     }
     CK(cudaStreamSynchronize(st));
-    if (info[0]) h->prior_valid = false;
-    if (info[0]) {
-      char b[128];
-      snprintf(b, sizeof b, "matrix %s is not positive definite (pivot %d)", info[0] / 100000 == 1 ? "Kh" : "Kx",
-               info[0] % 100000);
-      h->err = b;
-      return -3;
-    }
+    // the precomputation factorises Kh, Kx and (option "tri") the window blocks of iKx, reported as Kx
+    static const char* names[] = {"?", "Kh", "Kx", "?", "?", "?", "Kx"};
+    if (pd_error(h, info[0], names)) return -3;
     const double Ng = hs[S_COUNT + 0];
     const double a = (h->causal ? 0.5 : 1.0) * sqrt(3.14159265358979323846 / (2.0 * alpha));
     {
@@ -1954,27 +2062,15 @@ int evaluate_once(cgpcm_handle* h, const double* params_host, int mode, uint32_t
 
   // ---- collect
   double hs[S_COUNT + 16];
-  int info[4];
+  int info;
   CK(cudaMemcpyAsync(hs, h->sc, sizeof hs, cudaMemcpyDeviceToHost, st));
-  CK(cudaMemcpyAsync(info, h->info, sizeof info, cudaMemcpyDeviceToHost, st));
   if (want_grad) CK(cudaMemcpyAsync(grad, h->gvar_d, np * sizeof(double), cudaMemcpyDefault, st));
-  prof_close(h);
-  CK(cudaEventRecord(h->ev[6], st));
-  CK(cudaStreamSynchronize(st));
-  CK(cudaGetLastError());
+  if (end_run(h, info)) return -2;
   const double Ng = hs[S_COUNT + 0], sum_y2 = hs[S_COUNT + 1];
-  if (info[0]) h->prior_valid = false;
-  if (info[0]) {
-    static const char* names[] = {"?", "Kh", "Kx", "P", "iKh + reg I (prior of q(u))", "q(u) covariance",
-                                  "iKx (a window block)", "-C1bar (a window block)"};
-    int tag = info[0] / 100000;
-    char b[160];
-    snprintf(b, sizeof b, "matrix %s is not positive definite (pivot %d)", tag >= 1 && tag <= 7 ? names[tag] : "?",
-             info[0] % 100000);
-    h->err = b;
-    h->last_info_tag = tag;
-    return -3;
-  }
+  static const char* names[] = {"?", "Kh", "Kx", "P", "iKh + reg I (prior of q(u))", "q(u) covariance",
+                                "iKx (a window block)", "-C1bar (a window block)"};
+  h->last_info_tag = info / 100000;
+  if (pd_error(h, info, names)) return -3;
   double sum_b, tr_bhh_m2 = hs[S_TR_BHH_M2];
   if (full) sum_b = Ng * a - Ng * hs[S_TR_IKH_AHH] - hs[S_TR_IKX_AXX] + hs[S_TR_IKH_Q];
   else sum_b = h->f_sum_b;
@@ -2008,11 +2104,13 @@ int evaluate_once(cgpcm_handle* h, const double* params_host, int mode, uint32_t
       if (grad_mask & CGPCM_GRAD_GAMMA) g5[3] = gamma * gg;
       if (grad_mask & CGPCM_GRAD_OMEGA) g5[4] = omega * go;
     }
-    if (is_device_ptr(grad)) CK(cudaMemcpy(grad, g5, sizeof g5, cudaMemcpyHostToDevice));
-    else memcpy(grad, g5, sizeof g5);
+    return put(h, grad, g5, 5);
   }
   return 0;
 }
+
+int predict_qz(cgpcm_handle* h, const std::vector<Chunk>& chunks, int smf, const double* mvec, const double* var,
+               double r, double c0, double reg, double* xm);
 
 // VCGPCM.fpi(num, z=True, high_reg) followed by convert(z=True) (src/core/cgpcm.py:479-516,577-592) on the frozen
 // Psi statistics: num rounds of  q(u) -> optimal q(z) -> optimal q(u)  (Normal.from_natural,
@@ -2027,57 +2125,32 @@ int fpi_run(cgpcm_handle* h, const double* params_host, int num, int high_reg, d
   const long ld = h->ld, l2 = ld * ld;
   const long nvar = (long)nh * (nh + 1) / 2;
   const long np = 5 + nh + nvar;
-  for (long i = 0; i < np; ++i)
-    if (!std::isfinite(params_host[i])) { h->err = "non-finite parameter"; return -4; }
+  if (check_finite(h, params_host, np, "non-finite parameter")) return -4;
   if (!h->frozen) { h->err = "cgpcm_fpi requires cgpcm_precompute"; return -1; }
-  const double s2 = exp(params_host[0]), s2f = exp(params_host[1]);
-  const double alpha = exp(params_host[2]), gamma = exp(params_host[3]), omega = exp(params_host[4]);
-  const double r = s2f / s2, c0 = sqrt(s2f) / s2;
+  const Hyp hp = hyp_of(params_host);
+  const double r = hp.r, c0 = hp.c0;
   const double hr = high_reg ? 1e-4 : 0.0;
   if (ensure_sweep_buffers(h)) return -2;
-  h->launches = 0;
-  h->pev_used = 0;
-  h->prof_open = false;
-  h->gemm_flops = h->gemm_flops_exec = 0.0;
-  h->gemm_launches = 0;
   PsiConst c;
-  psi_make_const(alpha, gamma, omega, h->causal, h->cull, &c, h->causal_id);
+  psi_make_const(hp.alpha, hp.gamma, hp.omega, h->causal, h->cull, &c, h->causal_id);
   std::vector<Chunk> chunks;
   plan_chunks(h, h->fc, chunks);
   cudaStream_t st = h->st;
-  CK(cudaEventRecord(h->ev[0], st));
-  CK(cudaMemsetAsync(h->info, 0, 4 * sizeof(int), st));
+  if (begin_run(h)) return -2;
   CK(cudaMemcpyAsync(h->params_d, params_host, np * sizeof(double), cudaMemcpyHostToDevice, st));
   if (prior_stage(h, c, reg, true)) return -2;
   if (!h->gram_valid && plan_store(h, chunks, false)) return -2;
-  double* Lq = h->M(M_LQ);
   double* mu = h->V(V_MU);
   double* muz = h->V(V_MUZ);
   double* var = h->M(M_VAR);
-  double* Hm = h->M(M_H);
-  {
-    const double* pd = h->params_d;
-    ew(st, l2, [=] __device__(long idx) {
-      int i = (int)(idx / ld), j = (int)(idx % ld);
-      Lq[idx] = (i < nh && j <= i) ? pd[5 + nh + (long)i * (i + 1) / 2 + j] : 0.0;
-      if (idx < ld) mu[idx] = idx < nh ? pd[5 + idx] : 0.0;
-    });
-    L(h);
-    if (mm(h, Lq, false, Lq, true, var, nhp, nhp, nhp)) return -2;
-    ew(st, l2, [=] __device__(long idx) {
-      int i = (int)(idx / ld), j = (int)(idx % ld);
-      if (i == j && i < nh) var[idx] += reg;      // self.h = Normal(reg(L L^T), mu_u)  (cgpcm.py:444-445)
-    });
-    L(h);
-  }
+  // self.h = Normal(reg(L L^T), mu_u)  (cgpcm.py:444-445)
+  if (qu_moments(h, reg)) return -2;
   const bool start_z = qz_mean != nullptr && qz_chol != nullptr;
   if (start_z) {
     // q(z) from the caller: mean, and covariance reg(Lz Lz^T) into M_PINV (the slot the q(z) covariance lives in)
     const long nvz = (long)nx * (nx + 1) / 2;
-    for (long i = 0; i < nx; ++i)
-      if (!std::isfinite(qz_mean[i])) { h->err = "non-finite mu_z"; return -4; }
-    for (long i = 0; i < nvz; ++i)
-      if (!std::isfinite(qz_chol[i])) { h->err = "non-finite var_z"; return -4; }
+    if (check_finite(h, qz_mean, nx, "non-finite mu_z")) return -4;
+    if (check_finite(h, qz_chol, nvz, "non-finite var_z")) return -4;
     CK(cudaMemsetAsync(muz, 0, ld * sizeof(double), st));
     CK(cudaMemcpyAsync(muz, qz_mean, nx * sizeof(double), cudaMemcpyHostToDevice, st));
     CK(cudaMemcpyAsync(h->gvar_d, qz_chol, nvz * sizeof(double), cudaMemcpyHostToDevice, st));
@@ -2097,30 +2170,7 @@ int fpi_run(cgpcm_handle* h, const double* params_host, int num, int high_reg, d
     L(h);
   }
   // one half round each: A = optimal q(z) given q(u) (z = True), B = optimal q(u) given q(z) (z = False)
-  auto half_a = [&](double hrz) -> int {
-    ew(st, l2, [=] __device__(long idx) {
-      int i = (int)(idx / ld), j = (int)(idx % ld);
-      Hm[idx] = var[idx] + mu[i] * mu[j];
-    });
-    L(h);
-    if (frozen_c1(h, chunks, Hm)) return -2;
-    if (allreduce(h, h->M(M_C1), l2)) return -2;
-    {
-      double* Pm = h->M(M_LP);
-      const double* kx = h->M(M_KX);
-      const double* fb = h->M(M_F_AXX);      // frozen sum_Bxx
-      const double* c1 = h->M(M_C1);
-      ew(st, l2, [=] __device__(long idx) {
-        int i = (int)(idx / ld), j = (int)(idx % ld);
-        Pm[idx] = kx[idx] + r * (fb[idx] + c1[idx]) + ((i == j && i < nx) ? hrz + reg : 0.0);
-      });
-      L(h);
-    }
-    if (chol_inv(h, h->M(M_LP), h->M(M_PINV), nx, nxp, nullptr, 3)) return -2;
-    matvec(h, h->M(M_F_Y), nx, nh, 1, mu, c0, h->V(V_LAM));                  // lam = c0 Y^T mean_u
-    matvec(h, h->M(M_PINV), nx, nx, 0, h->V(V_LAM), 1.0, muz);               // mean_z = var_z lam
-    return 0;
-  };
+  auto half_a = [&](double hrz) -> int { return predict_qz(h, chunks, 0, mu, var, r, c0, hrz + reg, muz); };
   auto half_b = [&](double hru) -> int {
     {
       double* W = h->M(M_WX);
@@ -2183,30 +2233,11 @@ int fpi_run(cgpcm_handle* h, const double* params_host, int num, int high_reg, d
   };
   if (emit(mu, var, nh, nhp, mu_u, var_u, 5)) return -2;
   if (emit(muz, h->M(M_PINV), nx, nxp, mu_z, var_z, 3)) return -2;
-  int info[4];
-  CK(cudaMemcpyAsync(info, h->info, sizeof info, cudaMemcpyDeviceToHost, st));
-  prof_close(h);
-  CK(cudaEventRecord(h->ev[6], st));
-  CK(cudaStreamSynchronize(st));
-  CK(cudaGetLastError());
-  if (info[0]) h->prior_valid = false;
-  if (info[0]) {
-    static const char* names[] = {"?", "Kh", "Kx", "P of q(z)", "P of q(u)", "a q covariance"};
-    int tag = info[0] / 100000;
-    char b[160];
-    snprintf(b, sizeof b, "matrix %s is not positive definite (pivot %d)", tag >= 1 && tag <= 5 ? names[tag] : "?",
-             info[0] % 100000);
-    h->err = b;
-    return -3;
-  }
-  float ms = 0;
-  cudaEventElapsedTime(&ms, h->ev[0], h->ev[6]);
-  memset(h->timing, 0, sizeof h->timing);
-  h->timing[0] = ms;
-  h->timing[6] = (double)h->launches;
-  h->timing[7] = h->gemm_flops;
-  h->timing[8] = (double)h->gemm_launches;
-  h->timing[9] = h->gemm_flops_exec;
+  int info;
+  if (end_run(h, info)) return -2;
+  static const char* names[] = {"?", "Kh", "Kx", "P of q(z)", "P of q(u)", "a q covariance"};
+  if (pd_error(h, info, names)) return -3;
+  record_timing(h);
   return 0;
 }
 
@@ -2219,29 +2250,19 @@ int qz_run(cgpcm_handle* h, const double* params_host, const double* qz_mean, co
   const int nh = h->nh, nx = h->nx, nhp = h->nhp, nxp = h->nxp;
   const long ld = h->ld, l2 = ld * ld;
   const long nvz = (long)nx * (nx + 1) / 2;
-  for (long i = 0; i < 5; ++i)
-    if (!std::isfinite(params_host[i])) { h->err = "non-finite parameter"; return -4; }
-  for (long i = 0; i < nx; ++i)
-    if (!std::isfinite(qz_mean[i])) { h->err = "non-finite mu_z"; return -4; }
-  for (long i = 0; i < nvz; ++i)
-    if (!std::isfinite(qz_chol[i])) { h->err = "non-finite var_z"; return -4; }
+  if (check_finite(h, params_host, 5, "non-finite parameter")) return -4;
+  if (check_finite(h, qz_mean, nx, "non-finite mu_z")) return -4;
+  if (check_finite(h, qz_chol, nvz, "non-finite var_z")) return -4;
   if (!h->frozen) { h->err = "cgpcm_elbo_qz requires cgpcm_precompute"; return -1; }
-  const double s2 = exp(params_host[0]), s2f = exp(params_host[1]);
-  const double alpha = exp(params_host[2]), gamma = exp(params_host[3]), omega = exp(params_host[4]);
-  const double r = s2f / s2, c0 = sqrt(s2f) / s2;
+  const Hyp hp = hyp_of(params_host);
+  const double r = hp.r, c0 = hp.c0;
   if (ensure_sweep_buffers(h)) return -2;
-  h->launches = 0;
-  h->pev_used = 0;
-  h->prof_open = false;
-  h->gemm_flops = h->gemm_flops_exec = 0.0;
-  h->gemm_launches = 0;
   PsiConst c;
-  psi_make_const(alpha, gamma, omega, h->causal, h->cull, &c, h->causal_id);
+  psi_make_const(hp.alpha, hp.gamma, hp.omega, h->causal, h->cull, &c, h->causal_id);
   std::vector<Chunk> chunks;
   plan_chunks(h, h->fc, chunks);
   cudaStream_t st = h->st;
-  CK(cudaEventRecord(h->ev[0], st));
-  CK(cudaMemsetAsync(h->info, 0, 4 * sizeof(int), st));
+  if (begin_run(h)) return -2;
   if (prior_stage(h, c, reg, true)) return -2;
   if (!h->gram_valid && plan_store(h, chunks, false)) return -2;
   double* muz = h->V(V_MUZ);
@@ -2305,23 +2326,11 @@ int qz_run(cgpcm_handle* h, const double* params_host, const double* qz_mean, co
   matvec(h, h->M(M_ISO), nx, nx, 0, muz, 1.0, h->V(V_ISOMU));
   dot(h, muz, h->V(V_ISOMU), nx, h->sc + S_MU_ISO_MU);
   double hs[S_COUNT + 16];
-  int info[4];
+  int info;
   CK(cudaMemcpyAsync(hs, h->sc, sizeof hs, cudaMemcpyDeviceToHost, st));
-  CK(cudaMemcpyAsync(info, h->info, sizeof info, cudaMemcpyDeviceToHost, st));
-  prof_close(h);
-  CK(cudaEventRecord(h->ev[6], st));
-  CK(cudaStreamSynchronize(st));
-  CK(cudaGetLastError());
-  if (info[0]) h->prior_valid = false;
-  if (info[0]) {
-    static const char* names[] = {"?", "Kh", "Kx", "P of q(u)", "iKx + reg I (prior of q(z))", "q(z) covariance"};
-    int tag = info[0] / 100000;
-    char b[160];
-    snprintf(b, sizeof b, "matrix %s is not positive definite (pivot %d)", tag >= 1 && tag <= 5 ? names[tag] : "?",
-             info[0] % 100000);
-    h->err = b;
-    return -3;
-  }
+  if (end_run(h, info)) return -2;
+  static const char* names[] = {"?", "Kh", "Kx", "P of q(u)", "iKx + reg I (prior of q(z))", "q(z) covariance"};
+  if (pd_error(h, info, names)) return -3;
   // N and sum y^2 of all ranks
   double tail[2] = {(double)h->n_local, h->sum_y2_local};
   if (h->world > 1) {
@@ -2332,7 +2341,7 @@ int qz_run(cgpcm_handle* h, const double* params_host, const double* qz_mean, co
   }
   const double KL = 0.5 * (hs[S_TR_ISO_VAR] + hs[S_MU_ISO_MU] - nx + hs[S_LOGDET_SO] - hs[S_LOGDET_VAR]);
   double tm[7];
-  tm[0] = -0.5 * tail[0] * log(2.0 * 3.14159265358979323846 * s2) - 0.5 * tail[1] / s2;
+  tm[0] = -0.5 * tail[0] * log(2.0 * 3.14159265358979323846 * hp.s2) - 0.5 * tail[1] / hp.s2;
   tm[1] = 0.5 * hs[S_LOGDET_KH];
   tm[2] = -0.5 * hs[S_LOGDET_P];
   tm[3] = 0.5 * hs[S_LAM_LBAR];
@@ -2343,39 +2352,14 @@ int qz_run(cgpcm_handle* h, const double* params_host, const double* qz_mean, co
   for (int i = 0; i < 7; ++i) e += tm[i];
   if (terms) memcpy(terms, tm, sizeof tm);
   if (elbo) *elbo = e;
-  float ms = 0;
-  cudaEventElapsedTime(&ms, h->ev[0], h->ev[6]);
-  memset(h->timing, 0, sizeof h->timing);
-  h->timing[0] = ms;
-  h->timing[6] = (double)h->launches;
-  h->timing[7] = h->gemm_flops;
-  h->timing[8] = (double)h->gemm_launches;
-  h->timing[9] = h->gemm_flops_exec;
+  record_timing(h);
   return 0;
 }
 
 // The moments of q(u) as predict_f uses them: mu (V_MU), var = L L^T + reg I (M_VAR), and tr(Ahh iKh) (S_TR_IKH_AHH).
 int predict_qu(cgpcm_handle* h, double reg) {
-  const int nh = h->nh, nhp = h->nhp;
-  const long ld = h->ld, l2 = ld * ld;
-  cudaStream_t st = h->st;
-  double* Lq = h->M(M_LQ);
-  double* mu = h->V(V_MU);
-  double* var = h->M(M_VAR);
-  const double* pd = h->params_d;
-  ew(st, l2, [=] __device__(long idx) {
-    int i = (int)(idx / ld), j = (int)(idx % ld);
-    Lq[idx] = (i < nh && j <= i) ? pd[5 + nh + (long)i * (i + 1) / 2 + j] : 0.0;
-    if (idx < ld) mu[idx] = idx < nh ? pd[5 + idx] : 0.0;
-  });
-  L(h);
-  if (mm(h, Lq, false, Lq, true, var, nhp, nhp, nhp)) return -2;
-  ew(st, l2, [=] __device__(long idx) {
-    int i = (int)(idx / ld), j = (int)(idx % ld);
-    if (i == j && i < nh) var[idx] += reg;
-  });
-  L(h);
-  frob(h, h->M(M_AHH), h->M(M_IKH), nh, nh, h->sc + S_TR_IKH_AHH);
+  if (qu_moments(h, reg)) return -2;
+  frob(h, h->M(M_AHH), h->M(M_IKH), h->nh, h->nh, h->sc + S_TR_IKH_AHH);
   return 0;
 }
 
@@ -2444,70 +2428,52 @@ int predict_run(cgpcm_handle* h, const double* params_host, double reg, const do
   const int nh = h->nh, nx = h->nx, nxp = h->nxp;
   const long ld = h->ld, l2 = ld * ld;
   const long np = 5 + nh + (long)nh * (nh + 1) / 2;
-  for (long i = 0; i < np; ++i)
-    if (!std::isfinite(params_host[i])) { h->err = "non-finite parameter"; return -4; }
-  for (long i = 0; i < n_star; ++i)
-    if (!std::isfinite(tstar_host[i])) { h->err = "non-finite test input"; return -4; }
-  for (long i = 0; i < (long)B * nh; ++i)
-    if (!std::isfinite(samples_host[i])) { h->err = "non-finite sample"; return -4; }
+  if (check_finite(h, params_host, np, "non-finite parameter")) return -4;
+  if (check_finite(h, tstar_host, n_star, "non-finite test input")) return -4;
+  if (check_samples(h, samples_host, B, nh)) return -4;
   if (!h->frozen) { h->err = "cgpcm_predict_f requires cgpcm_precompute"; return -1; }
-  const double s2 = exp(params_host[0]), s2f = exp(params_host[1]);
-  const double alpha = exp(params_host[2]), gamma = exp(params_host[3]), omega = exp(params_host[4]);
-  const double r = s2f / s2, c0 = sqrt(s2f) / s2;
+  const Hyp hp = hyp_of(params_host);
+  const double r = hp.r, c0 = hp.c0, s2f = hp.s2f;
   if (ensure_sweep_buffers(h)) return -2;
-  h->launches = 0;
-  h->pev_used = 0;
-  h->prof_open = false;
-  h->gemm_flops = h->gemm_flops_exec = 0.0;
-  h->gemm_launches = 0;
   PsiConst c;
-  psi_make_const(alpha, gamma, omega, h->causal, h->cull, &c, h->causal_id);
+  psi_make_const(hp.alpha, hp.gamma, hp.omega, h->causal, h->cull, &c, h->causal_id);
   PsiConst cd = c;                       // test-side statistics are evaluated densely (no windows)
   cd.cull = 746.0;
   BvnTab T;
-  bvn_make_tab(gamma / (alpha + gamma + omega), &T);
+  bvn_make_tab(hp.gamma / (hp.alpha + hp.gamma + hp.omega), &T);
   std::vector<Chunk> chunks;
   plan_chunks(h, h->fc, chunks);
   cudaStream_t st = h->st;
   const int TC = std::min<long>(h->chunk, std::max<long>(n_star, 1));
   const int nq = smf ? B : 1;            // distinct q(z)
-  // scratch of this call
-  double *d_t = nullptr, *d_x = nullptr, *d_mx = nullptr, *d_vec = nullptr, *d_q1 = nullptr, *d_acc = nullptr;
-  auto cleanup = [&]() {
-    double* ps[] = {d_t, d_x, d_mx, d_vec, d_q1, d_acc};
-    for (double* q : ps) if (q) cudaFree(q);
-  };
-#define PCK(call) do { cudaError_t e_ = (call); if (e_ != cudaSuccess) { char b_[256]; snprintf(b_, sizeof b_, \
-    "CUDA error %s in predict_f (%s)", cudaGetErrorString(e_), #call); h->err = b_; cleanup(); return -2; } } while (0)
-#define PRC(call) do { if (call) { cleanup(); return -2; } } while (0)
-  PCK(cudaMalloc(&d_t, (size_t)std::max<long>(n_star, 1) * sizeof(double)));
-  PCK(cudaMalloc(&d_x, (size_t)TC * nx * nx * sizeof(double)));
-  PCK(cudaMalloc(&d_mx, (size_t)nq * l2 * sizeof(double)));
-  PCK(cudaMalloc(&d_vec, (size_t)(B + nq) * ld * sizeof(double)));      // samples h_b, then x_mean per q(z)
-  PCK(cudaMalloc(&d_q1, (size_t)B * sizeof(double)));
-  PCK(cudaMalloc(&d_acc, (size_t)2 * std::max<long>(n_star, 1) * sizeof(double)));
+  Scratch s;
+  const size_t o_t = s.take(std::max<long>(n_star, 1)), o_x = s.take((size_t)TC * nx * nx);
+  const size_t o_mx = s.take((size_t)nq * l2), o_vec = s.take((size_t)(B + nq) * ld);   // samples h_b, then xm per q(z)
+  const size_t o_q1 = s.take(B), o_acc = s.take(2 * std::max<long>(n_star, 1));
+  CK(s.alloc());
+  double *d_t = s.at(o_t), *d_x = s.at(o_x), *d_mx = s.at(o_mx), *d_vec = s.at(o_vec), *d_q1 = s.at(o_q1);
+  double* d_acc = s.at(o_acc);
   double* d_h = d_vec;
   double* d_xm = d_vec + (long)B * ld;
-  PCK(cudaEventRecord(h->ev[0], st));
-  PCK(cudaMemsetAsync(h->info, 0, 4 * sizeof(int), st));
-  PCK(cudaMemcpyAsync(h->params_d, params_host, np * sizeof(double), cudaMemcpyHostToDevice, st));
-  PCK(cudaMemcpyAsync(d_t, tstar_host, n_star * sizeof(double), cudaMemcpyHostToDevice, st));
-  PCK(cudaMemsetAsync(d_vec, 0, (size_t)(B + nq) * ld * sizeof(double), st));
-  PCK(cudaMemcpy2DAsync(d_h, ld * sizeof(double), samples_host, nh * sizeof(double), nh * sizeof(double), B,
-                        cudaMemcpyHostToDevice, st));
-  PCK(cudaMemsetAsync(d_acc, 0, (size_t)2 * std::max<long>(n_star, 1) * sizeof(double), st));
-  PRC(prior_stage(h, c, reg, true));
-  if (!h->gram_valid) PRC(plan_store(h, chunks, false));
-  PRC(predict_qu(h, reg));
+  if (begin_run(h)) return -2;
+  CK(cudaMemcpyAsync(h->params_d, params_host, np * sizeof(double), cudaMemcpyHostToDevice, st));
+  CK(cudaMemcpyAsync(d_t, tstar_host, n_star * sizeof(double), cudaMemcpyHostToDevice, st));
+  CK(cudaMemsetAsync(d_vec, 0, (size_t)(B + nq) * ld * sizeof(double), st));
+  CK(cudaMemcpy2DAsync(d_h, ld * sizeof(double), samples_host, nh * sizeof(double), nh * sizeof(double), B,
+                       cudaMemcpyHostToDevice, st));
+  CK(cudaMemsetAsync(d_acc, 0, (size_t)2 * std::max<long>(n_star, 1) * sizeof(double), st));
+  if (prior_stage(h, c, reg, true)) return -2;
+  if (!h->gram_valid && plan_store(h, chunks, false)) return -2;
+  if (predict_qu(h, reg)) return -2;
   const double* mu = h->V(V_MU);
   const double* var = h->M(M_VAR);
-  const double a_val = (h->causal ? 0.5 : 1.0) * sqrt(3.14159265358979323846 / (2.0 * alpha));
+  const double a_val = (h->causal ? 0.5 : 1.0) * sqrt(3.14159265358979323846 / (2.0 * hp.alpha));
   // ---- training side: q(z) (once, or per sample) and the per-sample scalar q1
   for (int b = 0; b < std::max(B, nq); ++b) {
     const double* hb = d_h + (long)b * ld;
     if (b < nq) {
       double* xm = d_xm + (long)b * ld;
-      PRC(predict_qz(h, chunks, smf, smf ? hb : mu, var, r, c0, reg, xm));
+      if (predict_qz(h, chunks, smf, smf ? hb : mu, var, r, c0, reg, xm)) return -2;
       double* mxb = d_mx + (long)b * l2;
       const double* xv = h->M(M_PINV);
       const double* ikx = h->M(M_IKX);
@@ -2531,7 +2497,7 @@ int predict_run(cgpcm_handle* h, const double* params_host, double reg, const do
   for (long p0 = 0; p0 < n_star; p0 += TC) {
     const int nv = (int)std::min<long>(TC, n_star - p0);
     const int nc = round_up(nv, 8);
-    PRC(predict_chunk_blocks(h, cd, T, d_t + p0, nv, d_x));
+    if (predict_chunk_blocks(h, cd, T, d_t + p0, nv, d_x)) return -2;
     for (int b = 0; b < B; ++b) {
       const int qb = smf ? b : 0;
       predict_point_kernel<<<nv, 256, nx * sizeof(double), st>>>(h->wsA, nh, nc, nxp, nx, d_h + (long)b * ld,
@@ -2541,32 +2507,13 @@ int predict_run(cgpcm_handle* h, const double* params_host, double reg, const do
       L(h);
     }
   }
-  if (mu_out) PCK(cudaMemcpyAsync(mu_out, d_acc, n_star * sizeof(double), cudaMemcpyDefault, st));
-  if (var_out) PCK(cudaMemcpyAsync(var_out, d_acc + n_star, n_star * sizeof(double), cudaMemcpyDefault, st));
-  int info[4];
-  PCK(cudaMemcpyAsync(info, h->info, sizeof info, cudaMemcpyDeviceToHost, st));
-  prof_close(h);
-  PCK(cudaEventRecord(h->ev[6], st));
-  PCK(cudaStreamSynchronize(st));
-  PCK(cudaGetLastError());
-  cleanup();
-#undef PCK
-#undef PRC
-  if (info[0]) h->prior_valid = false;
-  if (info[0]) {
-    static const char* names[] = {"?", "Kh", "Kx", "P of q(z)", "?", "?"};
-    int tag = info[0] / 100000;
-    char b[160];
-    snprintf(b, sizeof b, "matrix %s is not positive definite (pivot %d)", tag >= 1 && tag <= 5 ? names[tag] : "?",
-             info[0] % 100000);
-    h->err = b;
-    return -3;
-  }
-  float ms = 0;
-  cudaEventElapsedTime(&ms, h->ev[0], h->ev[6]);
-  memset(h->timing, 0, sizeof h->timing);
-  h->timing[0] = ms;
-  h->timing[6] = (double)h->launches;
+  if (mu_out) CK(cudaMemcpyAsync(mu_out, d_acc, n_star * sizeof(double), cudaMemcpyDefault, st));
+  if (var_out) CK(cudaMemcpyAsync(var_out, d_acc + n_star, n_star * sizeof(double), cudaMemcpyDefault, st));
+  int info;
+  if (end_run(h, info)) return -2;
+  static const char* names[] = {"?", "Kh", "Kx", "P of q(z)"};
+  if (pd_error(h, info, names)) return -3;
+  record_timing(h);
   return 0;
 }
 
@@ -2577,78 +2524,47 @@ int kernel_run(cgpcm_handle* h, const double* params_host, double reg, const dou
                const double* samples_host, int B, double* out) {
   const int nh = h->nh;
   const long ld = h->ld;
-  const long np = 5 + nh + (long)nh * (nh + 1) / 2;
-  for (long i = 0; i < 5; ++i)
-    if (!std::isfinite(params_host[i])) { h->err = "non-finite parameter"; return -4; }
-  for (long i = 0; i < n; ++i)
-    if (!std::isfinite(t_host[i])) { h->err = "non-finite input"; return -4; }
-  for (long i = 0; i < (long)B * nh; ++i)
-    if (!std::isfinite(samples_host[i])) { h->err = "non-finite sample"; return -4; }
-  (void)np;
-  const double s2f = exp(params_host[1]);
-  const double alpha = exp(params_host[2]), gamma = exp(params_host[3]), omega = exp(params_host[4]);
-  h->launches = 0;
-  h->gemm_flops = h->gemm_flops_exec = 0.0;
-  h->gemm_launches = 0;
-  h->pev_used = 0;
-  h->prof_open = false;
+  if (check_finite(h, params_host, 5, "non-finite parameter")) return -4;
+  if (check_finite(h, t_host, n, "non-finite input")) return -4;
+  if (check_samples(h, samples_host, B, nh)) return -4;
+  const Hyp hp = hyp_of(params_host);
+  const double alpha = hp.alpha, gamma = hp.gamma;
   PsiConst c;
-  psi_make_const(alpha, gamma, omega, h->causal, h->cull, &c, h->causal_id);
+  psi_make_const(alpha, gamma, hp.omega, h->causal, h->cull, &c, h->causal_id);
   cudaStream_t st = h->st;
   const int nhl = round_up(nh, 2);
   const long K = (long)nh * nhl;
   const int Bp = round_up(B, 8);
   const int TC = (int)std::min<long>(round_up((int)std::min<long>(n, 1024), 8), 1024);
-  double *d_t = nullptr, *d_hs = nullptr, *d_ac = nullptr, *d_AC = nullptr, *d_HH = nullptr, *d_G = nullptr, *d_out = nullptr;
-  auto cleanup = [&]() {
-    double* ps[] = {d_t, d_hs, d_ac, d_AC, d_HH, d_G, d_out};
-    for (double* q : ps) if (q) cudaFree(q);
-  };
-#define PCK(call) do { cudaError_t e_ = (call); if (e_ != cudaSuccess) { char b_[256]; snprintf(b_, sizeof b_, \
-    "CUDA error %s in kernel_samples (%s)", cudaGetErrorString(e_), #call); h->err = b_; cleanup(); return -2; } } while (0)
-#define PRC(call) do { if (call) { cleanup(); return -2; } } while (0)
-  PCK(cudaMalloc(&d_t, (size_t)n * sizeof(double)));
-  PCK(cudaMalloc(&d_hs, (size_t)B * nh * sizeof(double)));
-  PCK(cudaMalloc(&d_ac, (size_t)TC * sizeof(double)));
-  PCK(cudaMalloc(&d_AC, (size_t)TC * K * sizeof(double)));
-  PCK(cudaMalloc(&d_HH, (size_t)Bp * K * sizeof(double)));
-  PCK(cudaMalloc(&d_G, (size_t)TC * Bp * sizeof(double)));
-  PCK(cudaMalloc(&d_out, (size_t)n * B * sizeof(double)));
-  PCK(cudaEventRecord(h->ev[0], st));
-  PCK(cudaMemsetAsync(h->info, 0, 4 * sizeof(int), st));
-  PCK(cudaMemcpyAsync(d_t, t_host, n * sizeof(double), cudaMemcpyHostToDevice, st));
-  PCK(cudaMemcpyAsync(d_hs, samples_host, (size_t)B * nh * sizeof(double), cudaMemcpyHostToDevice, st));
-  PRC(prior_stage(h, c, reg, true));                          // Kh -> iKh (M_IKH)
+  Scratch s;
+  const size_t o_t = s.take(n), o_hs = s.take((size_t)B * nh), o_ac = s.take(TC), o_AC = s.take((size_t)TC * K);
+  const size_t o_HH = s.take((size_t)Bp * K), o_G = s.take((size_t)TC * Bp), o_out = s.take((size_t)n * B);
+  CK(s.alloc());
+  double *d_t = s.at(o_t), *d_hs = s.at(o_hs), *d_ac = s.at(o_ac), *d_AC = s.at(o_AC), *d_HH = s.at(o_HH);
+  double *d_G = s.at(o_G), *d_out = s.at(o_out);
+  if (begin_run(h)) return -2;
+  CK(cudaMemcpyAsync(d_t, t_host, n * sizeof(double), cudaMemcpyHostToDevice, st));
+  CK(cudaMemcpyAsync(d_hs, samples_host, (size_t)B * nh * sizeof(double), cudaMemcpyHostToDevice, st));
+  if (prior_stage(h, c, reg, true)) return -2;                // Kh -> iKh (M_IKH)
   hh_build_kernel<<<148 * 4, 256, 0, st>>>(d_hs, nh, B, Bp, h->M(M_IKH), ld, nh, nhl, d_HH);
   L(h);
   for (long p0 = 0; p0 < n; p0 += TC) {
     const int nv = (int)std::min<long>(TC, n - p0);
     const int nvp = round_up(nv, 8);
-    if (nvp > nv) PCK(cudaMemsetAsync(d_AC + (long)nv * K, 0, (size_t)(nvp - nv) * K * sizeof(double), st));
+    if (nvp > nv) CK(cudaMemsetAsync(d_AC + (long)nv * K, 0, (size_t)(nvp - nv) * K * sizeof(double), st));
     ahh_center_kernel<<<148 * 8, 256, 0, st>>>(d_t + p0, nv, h->th, nh, nhl, alpha, gamma, h->causal, d_AC, d_ac);
     L(h);
     // G[p][b] = sum_e AC[p][e] HH[b][e]
-    PRC(gemm(h, true, true, false, nvp, Bp, (int)K, 1.0, d_AC, K, d_HH, K, 0.0, d_G, Bp));
-    kernel_finish_kernel<<<148 * 2, 256, 0, st>>>(d_G, Bp, d_ac, nv, B, s2f, d_out + p0 * B);
+    if (gemm(h, true, true, false, nvp, Bp, (int)K, 1.0, d_AC, K, d_HH, K, 0.0, d_G, Bp)) return -2;
+    kernel_finish_kernel<<<148 * 2, 256, 0, st>>>(d_G, Bp, d_ac, nv, B, hp.s2f, d_out + p0 * B);
     L(h);
   }
-  PCK(cudaMemcpyAsync(out, d_out, (size_t)n * B * sizeof(double), cudaMemcpyDefault, st));
-  int info[4];
-  PCK(cudaMemcpyAsync(info, h->info, sizeof info, cudaMemcpyDeviceToHost, st));
-  prof_close(h);
-  PCK(cudaEventRecord(h->ev[6], st));
-  PCK(cudaStreamSynchronize(st));
-  PCK(cudaGetLastError());
-  cleanup();
-#undef PCK
-#undef PRC
-  if (info[0]) h->prior_valid = false;
-  if (info[0]) { h->err = "matrix Kh is not positive definite"; return -3; }
-  float ms = 0;
-  cudaEventElapsedTime(&ms, h->ev[0], h->ev[6]);
-  memset(h->timing, 0, sizeof h->timing);
-  h->timing[0] = ms;
-  h->timing[6] = (double)h->launches;
+  CK(cudaMemcpyAsync(out, d_out, (size_t)n * B * sizeof(double), cudaMemcpyDefault, st));
+  int info;
+  if (end_run(h, info)) return -2;
+  static const char* names[] = {"?", "Kh", "Kx"};
+  if (pd_error(h, info, names)) return -3;
+  record_timing(h);
   return 0;
 }
 
@@ -2659,93 +2575,61 @@ int filter_run(cgpcm_handle* h, const double* params_host, double reg, const dou
                const double* samples_host, int B, const double* noise_host, double* out) {
   const int nh = h->nh, nhp = h->nhp;
   const long ld = h->ld;
-  for (long i = 0; i < 5; ++i)
-    if (!std::isfinite(params_host[i])) { h->err = "non-finite parameter"; return -4; }
-  for (long i = 0; i < n; ++i)
-    if (!std::isfinite(t_host[i])) { h->err = "non-finite input"; return -4; }
-  for (long i = 0; i < (long)B * nh; ++i)
-    if (!std::isfinite(samples_host[i])) { h->err = "non-finite sample"; return -4; }
-  for (long i = 0; i < n * B; ++i)
-    if (!std::isfinite(noise_host[i])) { h->err = "non-finite noise"; return -4; }
+  if (check_finite(h, params_host, 5, "non-finite parameter")) return -4;
+  if (check_finite(h, t_host, n, "non-finite input")) return -4;
+  if (check_samples(h, samples_host, B, nh)) return -4;
+  if (check_finite(h, noise_host, n * B, "non-finite noise")) return -4;
   if (n > 8192) { h->err = "predict_h / predict_psd: at most 8192 inputs"; return -1; }
-  const double alpha = exp(params_host[2]), gamma = exp(params_host[3]), omega = exp(params_host[4]);
-  h->launches = 0;
-  h->gemm_flops = h->gemm_flops_exec = 0.0;
-  h->gemm_launches = 0;
-  h->pev_used = 0;
-  h->prof_open = false;
+  const Hyp hp = hyp_of(params_host);
   PsiConst c;
-  psi_make_const(alpha, gamma, omega, h->causal, h->cull, &c, h->causal_id);
+  psi_make_const(hp.alpha, hp.gamma, hp.omega, h->causal, h->cull, &c, h->causal_id);
   cudaStream_t st = h->st;
   const int ldn = round_up((int)n, 8);
   const int Bp = round_up(B, 8);
-  double *d_t = nullptr, *d_kuh = nullptr, *d_ktt = nullptr, *d_a = nullptr, *d_hs = nullptr, *d_e = nullptr, *d_o = nullptr;
-  auto cleanup = [&]() {
-    double* ps[] = {d_t, d_kuh, d_ktt, d_a, d_hs, d_e, d_o};
-    for (double* q : ps) if (q) cudaFree(q);
-  };
-#define PCK(call) do { cudaError_t e_ = (call); if (e_ != cudaSuccess) { char b_[256]; snprintf(b_, sizeof b_, \
-    "CUDA error %s in filter_samples (%s)", cudaGetErrorString(e_), #call); h->err = b_; cleanup(); return -2; } } while (0)
-#define PRC(call) do { if (call) { cleanup(); return -2; } } while (0)
-  PCK(cudaMalloc(&d_t, (size_t)n * sizeof(double)));
-  PCK(cudaMalloc(&d_kuh, (size_t)nhp * ldn * sizeof(double)));
-  PCK(cudaMalloc(&d_ktt, (size_t)ldn * ldn * sizeof(double)));
-  PCK(cudaMalloc(&d_a, (size_t)nhp * ldn * sizeof(double)));
-  PCK(cudaMalloc(&d_hs, (size_t)nhp * Bp * sizeof(double)));
-  PCK(cudaMalloc(&d_e, (size_t)ldn * Bp * sizeof(double)));
-  PCK(cudaMalloc(&d_o, (size_t)ldn * Bp * sizeof(double)));
-  PCK(cudaEventRecord(h->ev[0], st));
-  PCK(cudaMemsetAsync(h->info, 0, 4 * sizeof(int), st));
-  PCK(cudaMemcpyAsync(d_t, t_host, n * sizeof(double), cudaMemcpyHostToDevice, st));
+  Scratch s;
+  const size_t o_t = s.take(n), o_kuh = s.take((size_t)nhp * ldn), o_ktt = s.take((size_t)ldn * ldn);
+  const size_t o_a = s.take((size_t)nhp * ldn), o_hs = s.take((size_t)nhp * Bp), o_e = s.take((size_t)ldn * Bp);
+  const size_t o_o = s.take((size_t)ldn * Bp);
+  CK(s.alloc());
+  double *d_t = s.at(o_t), *d_kuh = s.at(o_kuh), *d_ktt = s.at(o_ktt), *d_a = s.at(o_a), *d_hs = s.at(o_hs);
+  double *d_e = s.at(o_e), *d_o = s.at(o_o);
+  if (begin_run(h)) return -2;
+  CK(cudaMemcpyAsync(d_t, t_host, n * sizeof(double), cudaMemcpyHostToDevice, st));
   // Hs[i][b] = samples[b][i] (transposed on the host), E[p][b] = noise[p][b]; zero padding
   std::vector<double> hs((size_t)nhp * Bp, 0.0), ee((size_t)ldn * Bp, 0.0);
   for (int b = 0; b < B; ++b)
     for (int i = 0; i < nh; ++i) hs[(size_t)i * Bp + b] = samples_host[(size_t)b * nh + i];
   for (long p2 = 0; p2 < n; ++p2)
     for (int b = 0; b < B; ++b) ee[(size_t)p2 * Bp + b] = noise_host[(size_t)p2 * B + b];
-  PCK(cudaMemcpyAsync(d_hs, hs.data(), hs.size() * sizeof(double), cudaMemcpyHostToDevice, st));
-  PCK(cudaMemcpyAsync(d_e, ee.data(), ee.size() * sizeof(double), cudaMemcpyHostToDevice, st));
-  PRC(prior_stage(h, c, reg, true));                                  // M_LH = chol(reg(Kh)), padded with the identity
-  filter_kernels_kernel<<<148 * 4, 256, 0, st>>>(h->th, nh, nhp, d_t, (int)n, ldn, alpha, gamma, reg, d_kuh, d_ktt);
+  CK(cudaMemcpyAsync(d_hs, hs.data(), hs.size() * sizeof(double), cudaMemcpyHostToDevice, st));
+  CK(cudaMemcpyAsync(d_e, ee.data(), ee.size() * sizeof(double), cudaMemcpyHostToDevice, st));
+  if (prior_stage(h, c, reg, true)) return -2;                        // M_LH = chol(reg(Kh)), padded with the identity
+  filter_kernels_kernel<<<148 * 4, 256, 0, st>>>(h->th, nh, nhp, d_t, (int)n, ldn, hp.alpha, hp.gamma, reg, d_kuh,
+                                                 d_ktt);
   L(h);
   // X = Lh^-1 ;  A = X Kuh ;  S = Ktt - A^T A ;  L = chol(S)
   {
     cudaError_t e = trtri_lower(st, h->M(M_LH), h->M(M_T1), h->M(M_T2), nhp, ld);
     L(h, 20);
-    if (e != cudaSuccess) { h->err = "trtri launch failed"; cleanup(); return -2; }
+    if (e != cudaSuccess) { h->err = "trtri launch failed"; return -2; }
   }
-  PRC(gemm(h, true, false, false, nhp, ldn, nhp, 1.0, h->M(M_T1), ld, d_kuh, ldn, 0.0, d_a, ldn));
-  PRC(gemm(h, false, false, false, ldn, ldn, nhp, -1.0, d_a, ldn, d_a, ldn, 1.0, d_ktt, ldn));
+  if (gemm(h, true, false, false, nhp, ldn, nhp, 1.0, h->M(M_T1), ld, d_kuh, ldn, 0.0, d_a, ldn)) return -2;
+  if (gemm(h, false, false, false, ldn, ldn, nhp, -1.0, d_a, ldn, d_a, ldn, 1.0, d_ktt, ldn)) return -2;
   {
     cudaError_t e = potrf_lower(st, d_ktt, ldn, ldn, h->info, 5, h->M(M_XW));
     L(h, 20);
-    if (e != cudaSuccess) { h->err = "potrf launch failed"; cleanup(); return -2; }
+    if (e != cudaSuccess) { h->err = "potrf launch failed"; return -2; }
   }
   // out = Kuh^T Hs + L E
-  PRC(gemm(h, false, false, false, ldn, Bp, nhp, 1.0, d_kuh, ldn, d_hs, Bp, 0.0, d_o, Bp));
-  PRC(gemm(h, true, false, false, ldn, Bp, ldn, 1.0, d_ktt, ldn, d_e, Bp, 1.0, d_o, Bp));
-  PCK(cudaMemcpy2DAsync(out, (size_t)B * sizeof(double), d_o, (size_t)Bp * sizeof(double), (size_t)B * sizeof(double), n,
-                        cudaMemcpyDefault, st));
-  int info[4];
-  PCK(cudaMemcpyAsync(info, h->info, sizeof info, cudaMemcpyDeviceToHost, st));
-  prof_close(h);
-  PCK(cudaEventRecord(h->ev[6], st));
-  PCK(cudaStreamSynchronize(st));
-  PCK(cudaGetLastError());
-  cleanup();
-#undef PCK
-#undef PRC
-  if (info[0]) h->prior_valid = false;
-  if (info[0]) {
-    h->err = info[0] / 100000 == 5 ? "matrix k_h(t, t) - A^T A + reg I is not positive definite"
-                                   : "matrix Kh is not positive definite";
-    return -3;
-  }
-  float ms = 0;
-  cudaEventElapsedTime(&ms, h->ev[0], h->ev[6]);
-  memset(h->timing, 0, sizeof h->timing);
-  h->timing[0] = ms;
-  h->timing[6] = (double)h->launches;
+  if (gemm(h, false, false, false, ldn, Bp, nhp, 1.0, d_kuh, ldn, d_hs, Bp, 0.0, d_o, Bp)) return -2;
+  if (gemm(h, true, false, false, ldn, Bp, ldn, 1.0, d_ktt, ldn, d_e, Bp, 1.0, d_o, Bp)) return -2;
+  CK(cudaMemcpy2DAsync(out, (size_t)B * sizeof(double), d_o, (size_t)Bp * sizeof(double), (size_t)B * sizeof(double), n,
+                       cudaMemcpyDefault, st));
+  int info;
+  if (end_run(h, info)) return -2;
+  static const char* names[] = {"?", "Kh", "Kx", "?", "?", "k_h(t, t) - A^T A + reg I"};
+  if (pd_error(h, info, names)) return -3;
+  record_timing(h);
   return 0;
 }
 
@@ -2759,31 +2643,22 @@ int akm_run(cgpcm_handle* h, const double* params_host, double reg, const double
   for (long i = 0; i < n; ++i)
     if (!std::isfinite(t_host[i]) || !std::isfinite(e_host[i])) { h->err = "non-finite input"; return -4; }
   if (n > 4096) { h->err = "AKM sample: at most 4096 inputs"; return -1; }
-  const double s2f = exp(params_host[1]);
+  const double s2f = hyp_of(params_host).s2f;
   cudaStream_t st = h->st;
   const int ldn = round_up((int)n, 8);
   std::vector<double> lags((size_t)n * n);
   for (long p2 = 0; p2 < n; ++p2)
     for (long q = 0; q < n; ++q) lags[(size_t)p2 * n + q] = t_host[p2] - t_host[q];
-  double *d_k = nullptr, *d_K = nullptr, *d_e = nullptr, *d_f = nullptr;
-  auto cleanup = [&]() {
-    double* ps[] = {d_k, d_K, d_e, d_f};
-    for (double* q : ps) if (q) cudaFree(q);
-  };
-#define PCK(call) do { cudaError_t e_ = (call); if (e_ != cudaSuccess) { char b_[256]; snprintf(b_, sizeof b_, \
-    "CUDA error %s in akm_sample (%s)", cudaGetErrorString(e_), #call); h->err = b_; cleanup(); return -2; } } while (0)
-  PCK(cudaMalloc(&d_k, (size_t)n * n * sizeof(double)));
-  PCK(cudaMalloc(&d_K, (size_t)ldn * ldn * sizeof(double)));
-  PCK(cudaMalloc(&d_e, (size_t)ldn * sizeof(double)));
-  PCK(cudaMalloc(&d_f, (size_t)ldn * sizeof(double)));
-  {
-    int rc = kernel_run(h, params_host, reg, lags.data(), n * n, h_host, 1, d_k);     // s2_f (a + tr(..)) per lag
-    if (rc) { cleanup(); return rc; }
-  }
-  PCK(cudaEventRecord(h->ev[0], st));
-  PCK(cudaMemsetAsync(h->info, 0, 4 * sizeof(int), st));
-  PCK(cudaMemsetAsync(d_e, 0, (size_t)ldn * sizeof(double), st));
-  PCK(cudaMemcpyAsync(d_e, e_host, (size_t)n * sizeof(double), cudaMemcpyHostToDevice, st));
+  Scratch s;
+  const size_t o_k = s.take((size_t)n * n), o_K = s.take((size_t)ldn * ldn), o_e = s.take(ldn), o_f = s.take(ldn);
+  CK(s.alloc());
+  double *d_k = s.at(o_k), *d_K = s.at(o_K), *d_e = s.at(o_e), *d_f = s.at(o_f);
+  if (int rc = kernel_run(h, params_host, reg, lags.data(), n * n, h_host, 1, d_k)) return rc;   // s2_f (a + tr(..)) per lag
+  // this run's own part: timed from a new ev[0] and added to the kernel_run part; the counters go on
+  CK(cudaEventRecord(h->ev[0], st));
+  CK(cudaMemsetAsync(h->info, 0, 4 * sizeof(int), st));
+  CK(cudaMemsetAsync(d_e, 0, (size_t)ldn * sizeof(double), st));
+  CK(cudaMemcpyAsync(d_e, e_host, (size_t)n * sizeof(double), cudaMemcpyHostToDevice, st));
   {
     const double* kk = d_k;
     double* Kp = d_K;
@@ -2798,30 +2673,23 @@ int akm_run(cgpcm_handle* h, const double* params_host, double reg, const double
     L(h);
   }
   if (K_out)
-    PCK(cudaMemcpy2DAsync(K_out, (size_t)n * sizeof(double), d_K, (size_t)ldn * sizeof(double), (size_t)n * sizeof(double),
-                          n, cudaMemcpyDefault, st));
+    CK(cudaMemcpy2DAsync(K_out, (size_t)n * sizeof(double), d_K, (size_t)ldn * sizeof(double), (size_t)n * sizeof(double),
+                         n, cudaMemcpyDefault, st));
   {
     cudaError_t e = potrf_lower(st, d_K, ldn, ldn, h->info, 6, h->M(M_XW));
     L(h, 2 * ((ldn + LA_NB - 1) / LA_NB));
-    if (e != cudaSuccess) { h->err = "potrf launch failed"; cleanup(); return -2; }
+    if (e != cudaSuccess) { h->err = "potrf launch failed"; return -2; }
   }
   matvec_kernel<<<(ldn + 7) / 8, 256, 0, st>>>(d_K, ldn, ldn, ldn, 0, d_e, sqrt(s2f), d_f);
   L(h);
-  PCK(cudaMemcpyAsync(f_out, d_f, (size_t)n * sizeof(double), cudaMemcpyDefault, st));
-  int info[4];
-  PCK(cudaMemcpyAsync(info, h->info, sizeof info, cudaMemcpyDeviceToHost, st));
-  prof_close(h);
-  PCK(cudaEventRecord(h->ev[6], st));
-  PCK(cudaStreamSynchronize(st));
-  PCK(cudaGetLastError());
-  cleanup();
-#undef PCK
-  if (info[0]) h->prior_valid = false;
-  if (info[0]) { h->err = "AKM covariance a + tr((h h^T - iKh) Ahh) + reg I is not positive definite"; return -3; }
-  float ms = 0;
-  cudaEventElapsedTime(&ms, h->ev[0], h->ev[6]);
-  h->timing[0] += ms;
-  h->timing[6] = (double)h->launches;
+  CK(cudaMemcpyAsync(f_out, d_f, (size_t)n * sizeof(double), cudaMemcpyDefault, st));
+  int info;
+  if (end_run(h, info)) return -2;
+  if (info) h->prior_valid = false;
+  if (info) { h->err = "AKM covariance a + tr((h h^T - iKh) Ahh) + reg I is not positive definite"; return -3; }
+  const double kernel_ms = h->timing[0];
+  record_timing(h);
+  h->timing[0] += kernel_ms;
   return 0;
 }
 
@@ -2834,19 +2702,26 @@ int smf_bcap(const cgpcm_handle* h) {
   return std::max(8, b);
 }
 
-// The per-batch C1 stage of the batched SMF paths: stage nb <= bcap samples (host, nb x nh) into d_hs (bcap x nhp,
-// zero rows past nb), then per chunk W = H_B A (the small-left GEMM over the resident or regenerated Ahx block, always
-// bcap rows) and part_b += W_b^T W_b (smf_c1_kernel), the slice sum into the C1 slabs and one all-reduce of them.
-int smf_c1_stage(cgpcm_handle* h, const std::vector<Chunk>& chunks, const double* samples_host, int nb, int bcap,
-                 std::vector<double>& hsm, double* d_hs, double* d_part, double* d_c1, double* d_w, long wstride) {
-  const int nh = h->nh, nx = h->nx, nhp = h->nhp;
-  const long ld = h->ld, l2 = ld * ld;
-  cudaStream_t st = h->st;
-  hsm.assign((size_t)bcap * nhp, 0.0);
+// nb <= bcap samples (host, nb x nh) into d_hs (bcap x nhp, zero past each sample and past nb)
+int stage_samples(cgpcm_handle* h, const double* samples_host, int nb, int bcap, double* d_hs) {
+  const int nh = h->nh, nhp = h->nhp;
+  std::vector<double> hsm((size_t)bcap * nhp, 0.0);
   for (int b = 0; b < nb; ++b)
     for (int i = 0; i < nh; ++i) hsm[(size_t)b * nhp + i] = samples_host[(size_t)b * nh + i];
   // (pageable source: staged before the call returns)
-  CK(cudaMemcpyAsync(d_hs, hsm.data(), hsm.size() * sizeof(double), cudaMemcpyHostToDevice, st));
+  CK(cudaMemcpyAsync(d_hs, hsm.data(), hsm.size() * sizeof(double), cudaMemcpyHostToDevice, h->st));
+  return 0;
+}
+
+// The per-batch C1 stage of the batched SMF paths: stage nb <= bcap samples into d_hs (stage_samples), then per chunk
+// W = H_B A (the small-left GEMM over the resident or regenerated Ahx block, always bcap rows) and part_b += W_b^T W_b
+// (smf_c1_kernel), the slice sum into the C1 slabs and one all-reduce of them.
+int smf_c1_stage(cgpcm_handle* h, const std::vector<Chunk>& chunks, const double* samples_host, int nb, int bcap,
+                 double* d_hs, double* d_part, double* d_c1, double* d_w, long wstride) {
+  const int nx = h->nx, nhp = h->nhp;
+  const long ld = h->ld, l2 = ld * ld;
+  cudaStream_t st = h->st;
+  if (stage_samples(h, samples_host, nb, bcap, d_hs)) return -2;
   CK(cudaMemsetAsync(d_part, 0, (size_t)nb * SMF_SLICES * l2 * sizeof(double), st));
   const bool stor = h->use_store;
   const bool have_a = stor && h->storeA_frozen_valid;
@@ -2867,6 +2742,31 @@ int smf_c1_stage(cgpcm_handle* h, const std::vector<Chunk>& chunks, const double
   return allreduce(h, d_c1, (long)nb * l2);
 }
 
+// The training side of the batched prediction paths with smf = 1, for the nb <= bcap samples from b0: the C1 stage,
+// smf_posterior_kernel (P_b, xm_b, mx_b and q1_b with the constant term a) and the check of each P_b.
+int smf_posterior_stage(cgpcm_handle* h, const std::vector<Chunk>& chunks, const double* samples_host, int b0, int nb,
+                        int bcap, double* hs, double* part, double* c1, double* w, long wcols, double* work, int* info,
+                        double* mx, double* xm, double* q1, double r, double c0, double reg, double a_val) {
+  cudaStream_t st = h->st;
+  if (smf_c1_stage(h, chunks, samples_host + (size_t)b0 * h->nh, nb, bcap, hs, part, c1, w, wcols)) return -2;
+  SmfPostArgs a;
+  a.kx = h->M(M_KX); a.sxx = h->M(M_F_AXX); a.c1 = c1; a.fy = h->M(M_F_Y); a.ahh = h->M(M_AHH);
+  a.ikx = h->M(M_IKX); a.tr = h->sc + S_TR_IKH_AHH; a.hs = hs; a.work = work;
+  a.mx = mx; a.xm = xm; a.q1 = q1; a.info = info;
+  a.ld = h->ld; a.l2 = h->ld * h->ld; a.ldh = h->nhp; a.nh = h->nh; a.nx = h->nx; a.nb = nb;
+  a.r = r; a.c0 = c0; a.reg = reg; a.a = a_val;
+  CK(cudaMemsetAsync(info, 0, bcap * sizeof(int), st));
+  smf_posterior_launch(st, a, bcap);
+  L(h);
+  CK(cudaGetLastError());
+  std::vector<int> inf(bcap);
+  CK(cudaMemcpyAsync(inf.data(), info, bcap * sizeof(int), cudaMemcpyDeviceToHost, st));
+  CK(cudaStreamSynchronize(st));
+  for (int b = 0; b < nb; ++b)
+    if (inf[b]) return sample_pd_error(h, "P", b0 + b, inf[b]);
+  return 0;
+}
+
 // VCGPCM.elbo(smf=True, sample=h_b) and the slice sampler's log-likelihood (src/core/cgpcm.py:527-531,594-608,848-872)
 // for B samples in the frozen regime.  Per call: the terms that do not depend on the sample (the prior, q(u) and
 // its KL, the frozen sums), as evaluate_once forms them.  Per batch of <= smf_bcap samples: per chunk W = H_B A (the
@@ -2877,28 +2777,15 @@ int smf_batch_run(cgpcm_handle* h, const double* params_host, double reg, const 
   const int nh = h->nh, nx = h->nx, nhp = h->nhp;
   const long ld = h->ld, l2 = ld * ld;
   const long np = 5 + nh + (long)nh * (nh + 1) / 2;
-  for (long i = 0; i < np; ++i)
-    if (!std::isfinite(params_host[i])) { h->err = "non-finite parameter"; return -4; }
-  for (long i = 0; i < (long)B * nh; ++i)
-    if (!std::isfinite(samples_host[i])) {
-      char b[96];
-      snprintf(b, sizeof b, "non-finite value in sample %ld", i / nh);
-      h->err = b;
-      return -4;
-    }
+  if (check_finite(h, params_host, np, "non-finite parameter")) return -4;
+  if (check_samples(h, samples_host, B, nh)) return -4;
   if (!h->frozen) { h->err = "cgpcm_elbo_smf_batch requires cgpcm_precompute"; return -1; }
   if (!want_p && !want_p0) return 0;
-  const double s2 = exp(params_host[0]), s2f = exp(params_host[1]);
-  const double alpha = exp(params_host[2]), gamma = exp(params_host[3]), omega = exp(params_host[4]);
-  const double r = s2f / s2, c0 = sqrt(s2f) / s2;
+  const Hyp hp = hyp_of(params_host);
+  const double r = hp.r, c0 = hp.c0;
   if (ensure_sweep_buffers(h)) return -2;
-  h->launches = 0;
-  h->pev_used = 0;
-  h->prof_open = false;
-  h->gemm_flops = h->gemm_flops_exec = 0.0;
-  h->gemm_launches = 0;
   PsiConst c;
-  psi_make_const(alpha, gamma, omega, h->causal, h->cull, &c, h->causal_id);
+  psi_make_const(hp.alpha, hp.gamma, hp.omega, h->causal, h->cull, &c, h->causal_id);
   std::vector<Chunk> chunks;
   plan_chunks(h, h->fc, chunks);
   if (ensure_ypart(h, y_slices_used(chunks))) return -2;
@@ -2931,8 +2818,7 @@ int smf_batch_run(cgpcm_handle* h, const double* params_host, double reg, const 
   double* d_w = h->smf_buf + o_w;
 
   cudaStream_t st = h->st;
-  CK(cudaEventRecord(h->ev[0], st));
-  CK(cudaMemsetAsync(h->info, 0, 4 * sizeof(int), st));
+  if (begin_run(h)) return -2;
   CK(cudaMemcpyAsync(h->params_d, params_host, np * sizeof(double), cudaMemcpyHostToDevice, st));
   // ---- the terms that do not depend on the sample (evaluate_once, MODE_FROZEN)
   if (prior_stage(h, c, reg, true, true)) return -2;
@@ -2953,27 +2839,17 @@ int smf_batch_run(cgpcm_handle* h, const double* params_host, double reg, const 
   CK(cudaMemcpyAsync(hs, h->sc, sizeof hs, cudaMemcpyDeviceToHost, st));
   CK(cudaMemcpyAsync(info, h->info, sizeof info, cudaMemcpyDeviceToHost, st));
   CK(cudaStreamSynchronize(st));
-  if (info[0]) {
-    h->prior_valid = false;
-    static const char* names[] = {"?", "Kh", "Kx", "P", "iKh + reg I (prior of q(u))", "q(u) covariance"};
-    const int tag = info[0] / 100000;
-    char b[160];
-    snprintf(b, sizeof b, "matrix %s is not positive definite (pivot %d)", tag >= 1 && tag <= 5 ? names[tag] : "?",
-             info[0] % 100000);
-    h->err = b;
-    return -3;
-  }
+  static const char* names[] = {"?", "Kh", "Kx", "P", "iKh + reg I (prior of q(u))", "q(u) covariance"};
+  if (pd_error(h, info[0], names)) return -3;
   double tm[7];
-  fixed_terms(h, hs, s2, r, h->f_sum_b, hs[S_TR_BHH_M2], tm);
+  fixed_terms(h, hs, hp.s2, r, h->f_sum_b, hs[S_TR_BHH_M2], tm);
 
   // ---- batches of samples
-  std::vector<double> hsm((size_t)bcap * nhp), res((size_t)bcap * 5);
+  std::vector<double> res((size_t)bcap * 5);
   std::vector<int> inf((size_t)2 * bcap);
-  const long wstride = wcols;
   for (int b0 = 0; b0 < B; b0 += bcap) {
     const int nb = std::min(bcap, B - b0);
-    if (smf_c1_stage(h, chunks, samples_host + (size_t)b0 * nh, nb, bcap, hsm, d_hs, d_part, d_c1, d_w, wstride))
-      return -2;
+    if (smf_c1_stage(h, chunks, samples_host + (size_t)b0 * nh, nb, bcap, d_hs, d_part, d_c1, d_w, wcols)) return -2;
     SmfAlgArgs a;
     a.kx = h->M(M_KX); a.sxx = h->M(M_F_AXX); a.c1 = d_c1; a.fy = h->M(M_F_Y); a.bhh = h->M(M_F_BHH);
     a.hs = d_hs; a.work = d_work; a.out = d_out; a.info = h->smf_info;
@@ -2988,13 +2864,7 @@ int smf_batch_run(cgpcm_handle* h, const double* params_host, double reg, const 
     CK(cudaStreamSynchronize(st));
     for (int b = 0; b < nb; ++b)
       for (int k = 0; k < 2; ++k)
-        if (inf[2 * b + k]) {
-          char m[160];
-          snprintf(m, sizeof m, "matrix %s of sample %d is not positive definite (pivot %d)", k == 0 ? "P" : "P0 (no jitter)",
-                   b0 + b, inf[2 * b + k]);
-          h->err = m;
-          return -3;
-        }
+        if (inf[2 * b + k]) return sample_pd_error(h, k == 0 ? "P" : "P0 (no jitter)", b0 + b, inf[2 * b + k]);
     for (int b = 0; b < nb; ++b) {
       const double* o = &res[(size_t)b * 5];
       if (want_p) {
@@ -3010,15 +2880,9 @@ int smf_batch_run(cgpcm_handle* h, const double* params_host, double reg, const 
       if (want_p0) loglik_out[b0 + b] = -0.5 * o[2] + 0.5 * o[3] - 0.5 * r * o[4];
     }
   }
-  CK(cudaEventRecord(h->ev[6], st));
-  CK(cudaStreamSynchronize(st));
-  float ms = 0;
-  cudaEventElapsedTime(&ms, h->ev[0], h->ev[6]);
-  memset(h->timing, 0, sizeof h->timing);
-  h->timing[0] = ms;
-  h->timing[6] = (double)h->launches;
-  h->timing[7] = h->gemm_flops;
-  h->timing[8] = (double)h->gemm_launches;
+  int info_end;      // the prior's, checked above
+  if (end_run(h, info_end)) return -2;
+  record_timing(h);
   return 0;
 }
 
@@ -3029,6 +2893,44 @@ int predict_bcap(const cgpcm_handle* h) {
   const double per = ((SMF_SLICES + 3.0) * (double)h->ld * h->ld + (double)h->chunk * h->nxp) * sizeof(double);
   const int b = (int)std::min(64.0, 1e9 / per) / 8 * 8;
   return std::max(8, b);
+}
+
+// The training side shared by all samples of the batched prediction paths: with smf = 0 the one q(z) of q(u)
+// (predict_qz) and mx = P^-1 + xm xm^T - iKx, dense nx x nx as the test-side kernels read it; then the check of the
+// factorisations of the prior and of that q(z).
+int shared_qz_stage(cgpcm_handle* h, const std::vector<Chunk>& chunks, int smf, double r, double c0, double reg,
+                    double* xm, double* mx) {
+  if (!smf) {
+    if (predict_qz(h, chunks, 0, h->V(V_MU), h->M(M_VAR), r, c0, reg, xm)) return -2;
+    const int nx = h->nx;
+    const long ld = h->ld;
+    const double* xv = h->M(M_PINV);
+    const double* ikx = h->M(M_IKX);
+    ew(h->st, (long)nx * nx, [=] __device__(long idx) {
+      const int i = (int)(idx / nx), j = (int)(idx % nx);
+      const long e = (long)i * ld + j;
+      mx[idx] = xv[e] + xm[i] * xm[j] - ikx[e];
+    });
+    L(h);
+  }
+  int info[4];
+  CK(cudaMemcpyAsync(info, h->info, sizeof info, cudaMemcpyDeviceToHost, h->st));
+  CK(cudaStreamSynchronize(h->st));
+  static const char* names[] = {"?", "Kh", "Kx", "P of q(z)"};
+  return pd_error(h, info[0], names);
+}
+
+// nb dense nx x nx mx slabs (ld x ld apart) into the padded nxp x nxp layout of the rank-one GEMMs
+void pad_mx(cgpcm_handle* h, const double* mx, int nb, double* mxp) {
+  const int nx = h->nx, nxp = h->nxp;
+  const long l2 = h->ld * h->ld, pp = (long)nxp * nxp;
+  ew(h->st, (long)nb * pp, [=] __device__(long idx) {
+    const int b = (int)(idx / pp);
+    const long e = idx - (long)b * pp;
+    const int i = (int)(e / nxp), j = (int)(e % nxp);
+    mxp[idx] = (i < nx && j < nx) ? mx[(long)b * l2 + (long)i * nx + j] : 0.0;
+  });
+  L(h);
 }
 
 // predict_f's moments for each of B filter samples (and their average, as predict_run forms it) in the frozen regime.
@@ -3043,33 +2945,19 @@ int predict_batch_run(cgpcm_handle* h, const double* params_host, double reg, co
   const int nh = h->nh, nx = h->nx, nhp = h->nhp, nxp = h->nxp;
   const long ld = h->ld, l2 = ld * ld;
   const long np = 5 + nh + (long)nh * (nh + 1) / 2;
-  for (long i = 0; i < np; ++i)
-    if (!std::isfinite(params_host[i])) { h->err = "non-finite parameter"; return -4; }
-  for (long i = 0; i < n_star; ++i)
-    if (!std::isfinite(tstar_host[i])) { h->err = "non-finite test input"; return -4; }
-  for (long i = 0; i < (long)B * nh; ++i)
-    if (!std::isfinite(samples_host[i])) {
-      char b[96];
-      snprintf(b, sizeof b, "non-finite value in sample %ld", i / nh);
-      h->err = b;
-      return -4;
-    }
+  if (check_finite(h, params_host, np, "non-finite parameter")) return -4;
+  if (check_finite(h, tstar_host, n_star, "non-finite test input")) return -4;
+  if (check_samples(h, samples_host, B, nh)) return -4;
   if (!h->frozen) { h->err = "cgpcm_predict_f_batch requires cgpcm_precompute"; return -1; }
-  const double s2 = exp(params_host[0]), s2f = exp(params_host[1]);
-  const double alpha = exp(params_host[2]), gamma = exp(params_host[3]), omega = exp(params_host[4]);
-  const double r = s2f / s2, c0 = sqrt(s2f) / s2;
+  const Hyp hp = hyp_of(params_host);
+  const double r = hp.r, c0 = hp.c0, s2f = hp.s2f;
   if (ensure_sweep_buffers(h)) return -2;
-  h->launches = 0;
-  h->pev_used = 0;
-  h->prof_open = false;
-  h->gemm_flops = h->gemm_flops_exec = 0.0;
-  h->gemm_launches = 0;
   PsiConst c;
-  psi_make_const(alpha, gamma, omega, h->causal, h->cull, &c, h->causal_id);
+  psi_make_const(hp.alpha, hp.gamma, hp.omega, h->causal, h->cull, &c, h->causal_id);
   PsiConst cd = c;                       // test-side statistics are evaluated densely (no windows)
   cd.cull = 746.0;
   BvnTab T;
-  bvn_make_tab(gamma / (alpha + gamma + omega), &T);
+  bvn_make_tab(hp.gamma / (hp.alpha + hp.gamma + hp.omega), &T);
   std::vector<Chunk> chunks;
   plan_chunks(h, h->fc, chunks);
   if (ensure_ypart(h, y_slices_used(chunks))) return -2;
@@ -3083,74 +2971,32 @@ int predict_batch_run(cgpcm_handle* h, const double* params_host, double reg, co
   long wcols = 0;
   for (const Chunk& ch : chunks) wcols = std::max<long>(wcols, (long)ch.nc * ch.kwp);
   const bool per_sample = mean_s_out || var_s_out;
-  // [t][acc 2 n*][per-sample 2 n* B][X][hs][q1][xm][mx][part][c1][work][W][V][qpart][quad][lin]
-  long off = 0;
-  auto take = [&](long n) { const long o = off; off += (n + 1) / 2 * 2; return o; };     // 16-byte aligned
-  const long o_t = take(n_star), o_acc = take(2 * n_star), o_ps = take(per_sample ? 2 * n_star * B : 0);
-  const long o_x = take((long)TC * nx * nx), o_hs = take((long)gcap * nhp), o_q1 = take(gcap);
-  const long o_xm = take((long)nq * ld), o_mx = take((long)nq * l2);
-  const long o_part = take(smf ? (long)bcap * SMF_SLICES * l2 : 0), o_c1 = take(smf ? (long)bcap * l2 : 0);
-  const long o_work = take(smf ? 2L * bcap * l2 : 0), o_w = take(smf ? (long)bcap * wcols : 0);
+  // [t][acc 2 n*][per-sample 2 n* B][X][hs][q1][xm][mx][part][c1][work][W][V][qpart][quad][lin][info]
+  Scratch s;
+  const size_t o_t = s.take(n_star), o_acc = s.take(2 * n_star), o_ps = s.take(per_sample ? 2 * n_star * B : 0);
+  const size_t o_x = s.take((size_t)TC * nx * nx), o_hs = s.take((size_t)gcap * nhp), o_q1 = s.take(gcap);
+  const size_t o_xm = s.take((size_t)nq * ld), o_mx = s.take((size_t)nq * l2);
+  const size_t o_part = s.take(smf ? (size_t)bcap * SMF_SLICES * l2 : 0), o_c1 = s.take(smf ? (size_t)bcap * l2 : 0);
+  const size_t o_work = s.take(smf ? 2 * (size_t)bcap * l2 : 0), o_w = s.take(smf ? (size_t)bcap * wcols : 0);
   const long vstride = (long)TCP * nxp;
-  const long o_v = take((long)bcap * vstride), o_qp = take((long)PQ_SLICES * TC * bcap);
-  const long o_quad = take((long)TC * bcap), o_lin = take((long)TC * bcap);
-  double* buf = nullptr;
-  int* d_info = nullptr;
-  auto cleanup = [&]() {
-    if (buf) cudaFree(buf);
-    if (d_info) cudaFree(d_info);
-  };
-#define PCK(call) do { cudaError_t e_ = (call); if (e_ != cudaSuccess) { char b_[256]; snprintf(b_, sizeof b_, \
-    "CUDA error %s in predict_f_batch (%s)", cudaGetErrorString(e_), #call); h->err = b_; cleanup(); return -2; } } while (0)
-#define PRC(call) do { if (call) { cleanup(); return -2; } } while (0)
-  PCK(cudaMalloc(&buf, (size_t)off * sizeof(double)));
-  PCK(cudaMalloc(&d_info, (size_t)bcap * sizeof(int)));
-  double *d_t = buf + o_t, *d_acc = buf + o_acc, *d_ps = buf + o_ps, *d_x = buf + o_x, *d_hs = buf + o_hs;
-  double *d_q1 = buf + o_q1, *d_xm = buf + o_xm, *d_mx = buf + o_mx, *d_part = buf + o_part, *d_c1 = buf + o_c1;
-  double *d_work = buf + o_work, *d_w = buf + o_w, *d_v = buf + o_v, *d_qp = buf + o_qp, *d_quad = buf + o_quad;
-  double* d_lin = buf + o_lin;
-  PCK(cudaEventRecord(h->ev[0], st));
-  PCK(cudaMemsetAsync(h->info, 0, 4 * sizeof(int), st));
-  PCK(cudaMemcpyAsync(h->params_d, params_host, np * sizeof(double), cudaMemcpyHostToDevice, st));
-  PCK(cudaMemcpyAsync(d_t, tstar_host, n_star * sizeof(double), cudaMemcpyHostToDevice, st));
-  PCK(cudaMemsetAsync(d_acc, 0, (size_t)2 * n_star * sizeof(double), st));
-  PRC(prior_stage(h, c, reg, true));
-  if (smf || !h->gram_valid) PRC(plan_store(h, chunks, false));
-  PRC(predict_qu(h, reg));
-  const double a_val = (h->causal ? 0.5 : 1.0) * sqrt(3.14159265358979323846 / (2.0 * alpha));
-  if (!smf) {
-    // the one q(z) of q(u), as predict_run forms it; mx in the dense nx x nx layout of the test-side kernels
-    PRC(predict_qz(h, chunks, 0, h->V(V_MU), h->M(M_VAR), r, c0, reg, d_xm));
-    const double* xv = h->M(M_PINV);
-    const double* ikx = h->M(M_IKX);
-    const double* xm = d_xm;
-    double* mx = d_mx;
-    ew(st, (long)nx * nx, [=] __device__(long idx) {
-      const int i = (int)(idx / nx), j = (int)(idx % nx);
-      const long e = (long)i * ld + j;
-      mx[idx] = xv[e] + xm[i] * xm[j] - ikx[e];
-    });
-    L(h);
-  }
-  {
-    // a failed factorisation of the prior or of the shared q(z)
-    int info[4];
-    PCK(cudaMemcpyAsync(info, h->info, sizeof info, cudaMemcpyDeviceToHost, st));
-    PCK(cudaStreamSynchronize(st));
-    if (info[0]) {
-      h->prior_valid = false;
-      static const char* names[] = {"?", "Kh", "Kx", "P of q(z)", "?", "?"};
-      const int tag = info[0] / 100000;
-      char b[160];
-      snprintf(b, sizeof b, "matrix %s is not positive definite (pivot %d)", tag >= 1 && tag <= 5 ? names[tag] : "?",
-               info[0] % 100000);
-      h->err = b;
-      cleanup();
-      return -3;
-    }
-  }
-  std::vector<double> hsm;
-  std::vector<int> inf(bcap);
+  const size_t o_v = s.take((size_t)bcap * vstride), o_qp = s.take((size_t)PQ_SLICES * TC * bcap);
+  const size_t o_quad = s.take((size_t)TC * bcap), o_lin = s.take((size_t)TC * bcap);
+  const size_t o_info = s.take(bcap, sizeof(int));
+  CK(s.alloc());
+  double *d_t = s.at(o_t), *d_acc = s.at(o_acc), *d_ps = s.at(o_ps), *d_x = s.at(o_x), *d_hs = s.at(o_hs);
+  double *d_q1 = s.at(o_q1), *d_xm = s.at(o_xm), *d_mx = s.at(o_mx), *d_part = s.at(o_part), *d_c1 = s.at(o_c1);
+  double *d_work = s.at(o_work), *d_w = s.at(o_w), *d_v = s.at(o_v), *d_qp = s.at(o_qp), *d_quad = s.at(o_quad);
+  double* d_lin = s.at(o_lin);
+  int* d_info = s.at<int>(o_info);
+  if (begin_run(h)) return -2;
+  CK(cudaMemcpyAsync(h->params_d, params_host, np * sizeof(double), cudaMemcpyHostToDevice, st));
+  CK(cudaMemcpyAsync(d_t, tstar_host, n_star * sizeof(double), cudaMemcpyHostToDevice, st));
+  CK(cudaMemsetAsync(d_acc, 0, (size_t)2 * n_star * sizeof(double), st));
+  if (prior_stage(h, c, reg, true)) return -2;
+  if ((smf || !h->gram_valid) && plan_store(h, chunks, false)) return -2;
+  if (predict_qu(h, reg)) return -2;
+  const double a_val = (h->causal ? 0.5 : 1.0) * sqrt(3.14159265358979323846 / (2.0 * hp.alpha));
+  if (int rc = shared_qz_stage(h, chunks, smf, r, c0, reg, d_xm, d_mx)) return rc;
   const double w = 1.0 / B;
   for (int g0 = 0; g0 < B; g0 += gcap) {
     const int gn = std::min(gcap, B - g0);
@@ -3161,33 +3007,12 @@ int predict_batch_run(cgpcm_handle* h, const double* params_host, double reg, co
       double* hs = d_hs + (long)bi * bcap * nhp;
       double* q1 = d_q1 + (long)bi * bcap;
       if (smf) {
-        PRC(smf_c1_stage(h, chunks, samples_host + (size_t)b0 * nh, nb, bcap, hsm, hs, d_part, d_c1, d_w, wcols));
-        SmfPostArgs a;
-        a.kx = h->M(M_KX); a.sxx = h->M(M_F_AXX); a.c1 = d_c1; a.fy = h->M(M_F_Y); a.ahh = h->M(M_AHH);
-        a.ikx = h->M(M_IKX); a.tr = h->sc + S_TR_IKH_AHH; a.hs = hs; a.work = d_work;
-        a.mx = d_mx + (long)bi * bcap * l2; a.xm = d_xm + (long)bi * bcap * ld; a.q1 = q1; a.info = d_info;
-        a.ld = ld; a.l2 = l2; a.ldh = nhp; a.nh = nh; a.nx = nx; a.nb = nb;
-        a.r = r; a.c0 = c0; a.reg = reg; a.a = a_val;
-        PCK(cudaMemsetAsync(d_info, 0, bcap * sizeof(int), st));
-        smf_posterior_launch(st, a, bcap);
-        L(h);
-        PCK(cudaGetLastError());
-        PCK(cudaMemcpyAsync(inf.data(), d_info, bcap * sizeof(int), cudaMemcpyDeviceToHost, st));
-        PCK(cudaStreamSynchronize(st));
-        for (int b = 0; b < nb; ++b)
-          if (inf[b]) {
-            char m[160];
-            snprintf(m, sizeof m, "matrix P of sample %d is not positive definite (pivot %d)", b0 + b, inf[b]);
-            h->err = m;
-            cleanup();
-            return -3;
-          }
+        if (int rc = smf_posterior_stage(h, chunks, samples_host, b0, nb, bcap, hs, d_part, d_c1, d_w, wcols, d_work,
+                                         d_info, d_mx + (long)bi * bcap * l2, d_xm + (long)bi * bcap * ld, q1, r, c0,
+                                         reg, a_val))
+          return rc;
       } else {
-        hsm.assign((size_t)bcap * nhp, 0.0);
-        for (int b = 0; b < nb; ++b)
-          for (int i = 0; i < nh; ++i) hsm[(size_t)b * nhp + i] = samples_host[(size_t)(b0 + b) * nh + i];
-        // (pageable source: staged before the call returns)
-        PCK(cudaMemcpyAsync(hs, hsm.data(), hsm.size() * sizeof(double), cudaMemcpyHostToDevice, st));
+        if (stage_samples(h, samples_host + (size_t)b0 * nh, nb, bcap, hs)) return -2;
         predict_q1_kernel<<<bcap, 256, 0, st>>>(h->M(M_AHH), ld, hs, nhp, nh, nb, a_val, h->sc + S_TR_IKH_AHH, q1);
         L(h);
       }
@@ -3196,7 +3021,7 @@ int predict_batch_run(cgpcm_handle* h, const double* params_host, double reg, co
     for (long p0 = 0; p0 < n_star; p0 += TC) {
       const int nv = (int)std::min<long>(TC, n_star - p0);
       const long cols = (long)round_up(nv, 8) * nxp;
-      PRC(predict_chunk_blocks(h, cd, T, d_t + p0, nv, d_x));
+      if (predict_chunk_blocks(h, cd, T, d_t + p0, nv, d_x)) return -2;
       if (!smf) {
         predict_qb_launch(st, d_x, (long)nx * nx, d_mx, l2, 1, nv, TC, 1, d_qp, bcap);     // one column
         L(h);
@@ -3205,7 +3030,7 @@ int predict_batch_run(cgpcm_handle* h, const double* params_host, double reg, co
         const int b0 = g0 + bi * bcap, nb = std::min(bcap, B - b0);
         const double* hs = d_hs + (long)bi * bcap * nhp;
         // V[b][(n,k)] = sum_i h_b[i] A*[i][(n,k)]
-        PRC(gemm(h, true, false, false, bcap, (int)cols, nhp, 1.0, hs, nhp, h->wsA, cols, 0.0, d_v, vstride));
+        if (gemm(h, true, false, false, bcap, (int)cols, nhp, 1.0, hs, nhp, h->wsA, cols, 0.0, d_v, vstride)) return -2;
         prof_close(h);
         const double* mx = smf ? d_mx + (long)bi * bcap * l2 : d_mx;
         const double* xm = smf ? d_xm + (long)bi * bcap * ld : d_xm;
@@ -3226,26 +3051,15 @@ int predict_batch_run(cgpcm_handle* h, const double* params_host, double reg, co
         L(h);
       }
     }
-    PCK(cudaGetLastError());
+    CK(cudaGetLastError());
   }
-  if (mu_out) PCK(cudaMemcpyAsync(mu_out, d_acc, n_star * sizeof(double), cudaMemcpyDefault, st));
-  if (var_out) PCK(cudaMemcpyAsync(var_out, d_acc + n_star, n_star * sizeof(double), cudaMemcpyDefault, st));
-  if (mean_s_out) PCK(cudaMemcpyAsync(mean_s_out, d_ps, n_star * B * sizeof(double), cudaMemcpyDefault, st));
-  if (var_s_out) PCK(cudaMemcpyAsync(var_s_out, d_ps + n_star * B, n_star * B * sizeof(double), cudaMemcpyDefault, st));
-  prof_close(h);
-  PCK(cudaEventRecord(h->ev[6], st));
-  PCK(cudaStreamSynchronize(st));
-  PCK(cudaGetLastError());
-  cleanup();
-#undef PCK
-#undef PRC
-  float ms = 0;
-  cudaEventElapsedTime(&ms, h->ev[0], h->ev[6]);
-  memset(h->timing, 0, sizeof h->timing);
-  h->timing[0] = ms;
-  h->timing[6] = (double)h->launches;
-  h->timing[7] = h->gemm_flops;
-  h->timing[8] = (double)h->gemm_launches;
+  if (mu_out) CK(cudaMemcpyAsync(mu_out, d_acc, n_star * sizeof(double), cudaMemcpyDefault, st));
+  if (var_out) CK(cudaMemcpyAsync(var_out, d_acc + n_star, n_star * sizeof(double), cudaMemcpyDefault, st));
+  if (mean_s_out) CK(cudaMemcpyAsync(mean_s_out, d_ps, n_star * B * sizeof(double), cudaMemcpyDefault, st));
+  if (var_s_out) CK(cudaMemcpyAsync(var_s_out, d_ps + n_star * B, n_star * B * sizeof(double), cudaMemcpyDefault, st));
+  int info;          // the prior's and the shared q(z)'s, checked above
+  if (end_run(h, info)) return -2;
+  record_timing(h);
   return 0;
 }
 
@@ -3274,37 +3088,21 @@ int predict_cov_run(cgpcm_handle* h, const double* params_host, double reg, cons
   const int nh = h->nh, nx = h->nx, nhp = h->nhp, nxp = h->nxp;
   const long ld = h->ld, l2 = ld * ld;
   const long np = 5 + nh + (long)nh * (nh + 1) / 2;
-  for (long i = 0; i < np; ++i)
-    if (!std::isfinite(params_host[i])) { h->err = "non-finite parameter"; return -4; }
-  for (long i = 0; i < n_star; ++i)
-    if (!std::isfinite(tstar_host[i])) { h->err = "non-finite test input"; return -4; }
-  for (long i = 0; i < (long)B * nh; ++i)
-    if (!std::isfinite(samples_host[i])) {
-      char b[96];
-      snprintf(b, sizeof b, "non-finite value in sample %ld", i / nh);
-      h->err = b;
-      return -4;
-    }
-  if (noise_host)
-    for (long i = 0; i < n_star * B; ++i)
-      if (!std::isfinite(noise_host[i])) { h->err = "non-finite noise"; return -4; }
+  if (check_finite(h, params_host, np, "non-finite parameter")) return -4;
+  if (check_finite(h, tstar_host, n_star, "non-finite test input")) return -4;
+  if (check_samples(h, samples_host, B, nh)) return -4;
+  if (noise_host && check_finite(h, noise_host, n_star * B, "non-finite noise")) return -4;
   if (!h->frozen) { h->err = "cgpcm_predict_f_cov requires cgpcm_precompute"; return -1; }
   const bool want_draws = draws_out && noise_host;
-  const double s2 = exp(params_host[0]), s2f = exp(params_host[1]);
-  const double alpha = exp(params_host[2]), gamma = exp(params_host[3]), omega = exp(params_host[4]);
-  const double r = s2f / s2, c0 = sqrt(s2f) / s2;
+  const Hyp hp = hyp_of(params_host);
+  const double r = hp.r, c0 = hp.c0, s2f = hp.s2f, alpha = hp.alpha, gamma = hp.gamma;
   if (ensure_sweep_buffers(h)) return -2;
-  h->launches = 0;
-  h->pev_used = 0;
-  h->prof_open = false;
-  h->gemm_flops = h->gemm_flops_exec = 0.0;
-  h->gemm_launches = 0;
   PsiConst c;
-  psi_make_const(alpha, gamma, omega, h->causal, h->cull, &c, h->causal_id);
+  psi_make_const(alpha, gamma, hp.omega, h->causal, h->cull, &c, h->causal_id);
   PsiConst cd = c;                       // test-side statistics are evaluated densely (no windows)
   cd.cull = 746.0;
   BvnTab T;
-  bvn_make_tab(gamma / (alpha + gamma + omega), &T);
+  bvn_make_tab(gamma / (alpha + gamma + hp.omega), &T);
   std::vector<Chunk> chunks;
   plan_chunks(h, h->fc, chunks);
   if (ensure_ypart(h, y_slices_used(chunks))) return -2;
@@ -3322,89 +3120,49 @@ int predict_cov_run(cgpcm_handle* h, const double* params_host, double reg, cons
   long wcols = 0;
   for (const Chunk& ch : chunks) wcols = std::max<long>(wcols, (long)ch.nc * ch.kwp);
   const long acols = (long)npad * nxp;   // columns of A* / T: [i][p][k]
-  long off = 0;
-  auto take = [&](long cnt) { const long o = off; off += (cnt + 1) / 2 * 2; return o; };     // 16-byte aligned
-  const long o_t = take(n), o_a = take((long)nhp * acols), o_ta = take((long)nhp * acols);
-  const long o_mean = take((long)n * B), o_draw = take(want_draws ? (long)n * B : 0);
-  const long o_noise = take(want_draws ? (long)B * npad : 0), o_cov = take(cov_out ? n2 : 0);
-  const long o_x = take((long)TPP * nx * nx), o_g = take((long)TPP * nxp * nxp);
-  const long o_ac = take(TPP), o_lag = take(TPP), o_AC = take((long)TPP * KH);
-  const long o_gf = take((long)TPP * bcap), o_qp = take((long)PQ_SLICES * TPP * bcap);
-  const long o_hs = take((long)gcap * nhp), o_q1 = take(gcap), o_xm = take((long)nq * ld), o_mx = take((long)nq * l2);
-  const long o_mxp = take((long)nq * nxp * nxp), o_hh = take((long)gcap * KH), o_c = take((long)gcap * n2);
-  const long o_part = take(smf ? (long)bcap * SMF_SLICES * l2 : 0), o_c1 = take(smf ? (long)bcap * l2 : 0);
-  const long o_work = take(smf ? 2L * bcap * l2 : 0), o_w = take(smf ? (long)bcap * wcols : 0);
-  const long o_v = take((long)bcap * acols), o_y = take(acols);
-  const long o_quad = take((long)npad * bcap), o_lin = take((long)npad * bcap);
-  const long o_k = take(want_draws ? n2 : 0), o_f = take(want_draws ? npad : 0);
-  double* buf = nullptr;
-  int* d_info = nullptr;
-  auto cleanup = [&]() {
-    if (buf) cudaFree(buf);
-    if (d_info) cudaFree(d_info);
-  };
-#define PCK(call) do { cudaError_t e_ = (call); if (e_ != cudaSuccess) { char b_[256]; snprintf(b_, sizeof b_, \
-    "CUDA error %s in predict_f_cov (%s)", cudaGetErrorString(e_), #call); h->err = b_; cleanup(); return -2; } } while (0)
-#define PRC(call) do { if (call) { cleanup(); return -2; } } while (0)
-  PCK(cudaMalloc(&buf, (size_t)off * sizeof(double)));
-  PCK(cudaMalloc(&d_info, (size_t)(gcap + bcap) * sizeof(int)));
-  double *d_t = buf + o_t, *d_A = buf + o_a, *d_TA = buf + o_ta, *d_mean = buf + o_mean, *d_draw = buf + o_draw;
-  double *d_noise = buf + o_noise, *d_cov = buf + o_cov, *d_x = buf + o_x, *d_g = buf + o_g, *d_ac = buf + o_ac;
-  double *d_lag = buf + o_lag, *d_AC = buf + o_AC, *d_gf = buf + o_gf, *d_qp = buf + o_qp, *d_hs = buf + o_hs;
-  double *d_q1 = buf + o_q1, *d_xm = buf + o_xm, *d_mx = buf + o_mx, *d_mxp = buf + o_mxp, *d_hh = buf + o_hh;
-  double *d_c = buf + o_c, *d_part = buf + o_part, *d_c1 = buf + o_c1, *d_work = buf + o_work, *d_w = buf + o_w;
-  double *d_v = buf + o_v, *d_y = buf + o_y, *d_quad = buf + o_quad, *d_lin = buf + o_lin, *d_k = buf + o_k;
-  double* d_f = buf + o_f;
+  Scratch s;
+  const size_t o_t = s.take(n), o_a = s.take((size_t)nhp * acols), o_ta = s.take((size_t)nhp * acols);
+  const size_t o_mean = s.take((size_t)n * B), o_draw = s.take(want_draws ? (size_t)n * B : 0);
+  const size_t o_noise = s.take(want_draws ? (size_t)B * npad : 0), o_cov = s.take(cov_out ? n2 : 0);
+  const size_t o_x = s.take((size_t)TPP * nx * nx), o_g = s.take((size_t)TPP * nxp * nxp);
+  const size_t o_ac = s.take(TPP), o_lag = s.take(TPP), o_AC = s.take((size_t)TPP * KH);
+  const size_t o_gf = s.take((size_t)TPP * bcap), o_qp = s.take((size_t)PQ_SLICES * TPP * bcap);
+  const size_t o_hs = s.take((size_t)gcap * nhp), o_q1 = s.take(gcap), o_xm = s.take((size_t)nq * ld);
+  const size_t o_mx = s.take((size_t)nq * l2), o_mxp = s.take((size_t)nq * nxp * nxp);
+  const size_t o_hh = s.take((size_t)gcap * KH), o_c = s.take((size_t)gcap * n2);
+  const size_t o_part = s.take(smf ? (size_t)bcap * SMF_SLICES * l2 : 0), o_c1 = s.take(smf ? (size_t)bcap * l2 : 0);
+  const size_t o_work = s.take(smf ? 2 * (size_t)bcap * l2 : 0), o_w = s.take(smf ? (size_t)bcap * wcols : 0);
+  const size_t o_v = s.take((size_t)bcap * acols), o_y = s.take(acols);
+  const size_t o_quad = s.take((size_t)npad * bcap), o_lin = s.take((size_t)npad * bcap);
+  const size_t o_k = s.take(want_draws ? n2 : 0), o_f = s.take(want_draws ? npad : 0);
+  const size_t o_info = s.take(gcap + bcap, sizeof(int));
+  CK(s.alloc());
+  double *d_t = s.at(o_t), *d_A = s.at(o_a), *d_TA = s.at(o_ta), *d_mean = s.at(o_mean), *d_draw = s.at(o_draw);
+  double *d_noise = s.at(o_noise), *d_cov = s.at(o_cov), *d_x = s.at(o_x), *d_g = s.at(o_g), *d_ac = s.at(o_ac);
+  double *d_lag = s.at(o_lag), *d_AC = s.at(o_AC), *d_gf = s.at(o_gf), *d_qp = s.at(o_qp), *d_hs = s.at(o_hs);
+  double *d_q1 = s.at(o_q1), *d_xm = s.at(o_xm), *d_mx = s.at(o_mx), *d_mxp = s.at(o_mxp), *d_hh = s.at(o_hh);
+  double *d_c = s.at(o_c), *d_part = s.at(o_part), *d_c1 = s.at(o_c1), *d_work = s.at(o_work), *d_w = s.at(o_w);
+  double *d_v = s.at(o_v), *d_y = s.at(o_y), *d_quad = s.at(o_quad), *d_lin = s.at(o_lin), *d_k = s.at(o_k);
+  double* d_f = s.at(o_f);
+  int* d_info = s.at<int>(o_info);
   int* d_pinfo = d_info + bcap;          // per sample of the group: the factorisation of C_b + reg I
-  PCK(cudaEventRecord(h->ev[0], st));
-  PCK(cudaMemsetAsync(h->info, 0, 4 * sizeof(int), st));
-  PCK(cudaMemcpyAsync(h->params_d, params_host, np * sizeof(double), cudaMemcpyHostToDevice, st));
-  PCK(cudaMemcpyAsync(d_t, tstar_host, n * sizeof(double), cudaMemcpyHostToDevice, st));
-  if (cov_out) PCK(cudaMemsetAsync(d_cov, 0, (size_t)n2 * sizeof(double), st));
+  if (begin_run(h)) return -2;
+  CK(cudaMemcpyAsync(h->params_d, params_host, np * sizeof(double), cudaMemcpyHostToDevice, st));
+  CK(cudaMemcpyAsync(d_t, tstar_host, n * sizeof(double), cudaMemcpyHostToDevice, st));
+  if (cov_out) CK(cudaMemsetAsync(d_cov, 0, (size_t)n2 * sizeof(double), st));
   std::vector<double> noise_t;
   if (want_draws) {
     // noise[p][b] -> one zero-padded column per sample
     noise_t.assign((size_t)B * npad, 0.0);
     for (int b = 0; b < B; ++b)
       for (int p = 0; p < n; ++p) noise_t[(size_t)b * npad + p] = noise_host[(size_t)p * B + b];
-    PCK(cudaMemcpyAsync(d_noise, noise_t.data(), noise_t.size() * sizeof(double), cudaMemcpyHostToDevice, st));
+    CK(cudaMemcpyAsync(d_noise, noise_t.data(), noise_t.size() * sizeof(double), cudaMemcpyHostToDevice, st));
   }
-  PRC(prior_stage(h, c, reg, true));
-  if (smf || !h->gram_valid) PRC(plan_store(h, chunks, false));
-  PRC(predict_qu(h, reg));
-  if (!smf) {
-    PRC(predict_qz(h, chunks, 0, h->V(V_MU), h->M(M_VAR), r, c0, reg, d_xm));
-    const double* xv = h->M(M_PINV);
-    const double* ikx = h->M(M_IKX);
-    const double* xm = d_xm;
-    double* mx = d_mx;
-    double* mxp = d_mxp;
-    const int nxp_ = nxp;
-    ew(st, (long)nxp * nxp, [=] __device__(long idx) {
-      const int i = (int)(idx / nxp_), j = (int)(idx % nxp_);
-      const long e = (long)i * ld + j;
-      const double v = (i < nx && j < nx) ? xv[e] + xm[i] * xm[j] - ikx[e] : 0.0;
-      if (i < nx && j < nx) mx[(long)i * nx + j] = v;
-      mxp[idx] = v;
-    });
-    L(h);
-  }
-  {
-    int info[4];
-    PCK(cudaMemcpyAsync(info, h->info, sizeof info, cudaMemcpyDeviceToHost, st));
-    PCK(cudaStreamSynchronize(st));
-    if (info[0]) {
-      h->prior_valid = false;
-      static const char* names[] = {"?", "Kh", "Kx", "P of q(z)", "?", "?"};
-      const int tag = info[0] / 100000;
-      char b[160];
-      snprintf(b, sizeof b, "matrix %s is not positive definite (pivot %d)", tag >= 1 && tag <= 5 ? names[tag] : "?",
-               info[0] % 100000);
-      h->err = b;
-      cleanup();
-      return -3;
-    }
-  }
+  if (prior_stage(h, c, reg, true)) return -2;
+  if ((smf || !h->gram_valid) && plan_store(h, chunks, false)) return -2;
+  if (predict_qu(h, reg)) return -2;
+  if (int rc = shared_qz_stage(h, chunks, smf, r, c0, reg, d_xm, d_mx)) return rc;
+  if (!smf) pad_mx(h, d_mx, 1, d_mxp);
   // ---- test side, once: A* and T = iKh A* for every test input
   {
     const int threads = std::min(256, round_up(nxp, 32));
@@ -3413,9 +3171,8 @@ int predict_cov_run(cgpcm_handle* h, const double* params_host, double reg, cons
                                              (long)nhp * ld, cd);
     L(h);
   }
-  PRC(gemm(h, true, false, false, nhp, (int)acols, nhp, 1.0, h->M(M_IKH), ld, d_A, acols, 0.0, d_TA, acols));
-  std::vector<double> hsm;
-  std::vector<int> inf(std::max(bcap, gcap));
+  if (gemm(h, true, false, false, nhp, (int)acols, nhp, 1.0, h->M(M_IKH), ld, d_A, acols, 0.0, d_TA, acols)) return -2;
+  std::vector<int> inf(gcap);
   const double w = 1.0 / B;
   const int ntile = (n + TP - 1) / TP;
   for (int g0 = 0; g0 < B; g0 += gcap) {
@@ -3426,45 +3183,13 @@ int predict_cov_run(cgpcm_handle* h, const double* params_host, double reg, cons
       const int b0 = g0 + bi * bcap, nb = std::min(bcap, B - b0);
       double* hs = d_hs + (long)bi * bcap * nhp;
       if (smf) {
-        PRC(smf_c1_stage(h, chunks, samples_host + (size_t)b0 * nh, nb, bcap, hsm, hs, d_part, d_c1, d_w, wcols));
-        SmfPostArgs a;
-        a.kx = h->M(M_KX); a.sxx = h->M(M_F_AXX); a.c1 = d_c1; a.fy = h->M(M_F_Y); a.ahh = h->M(M_AHH);
-        a.ikx = h->M(M_IKX); a.tr = h->sc + S_TR_IKH_AHH; a.hs = hs; a.work = d_work;
-        a.mx = d_mx + (long)bi * bcap * l2; a.xm = d_xm + (long)bi * bcap * ld; a.q1 = d_q1 + (long)bi * bcap;
-        a.info = d_info; a.ld = ld; a.l2 = l2; a.ldh = nhp; a.nh = nh; a.nx = nx; a.nb = nb;
-        a.r = r; a.c0 = c0; a.reg = reg; a.a = 0.0;
-        PCK(cudaMemsetAsync(d_info, 0, bcap * sizeof(int), st));
-        smf_posterior_launch(st, a, bcap);
-        L(h);
-        PCK(cudaGetLastError());
-        PCK(cudaMemcpyAsync(inf.data(), d_info, bcap * sizeof(int), cudaMemcpyDeviceToHost, st));
-        PCK(cudaStreamSynchronize(st));
-        for (int b = 0; b < nb; ++b)
-          if (inf[b]) {
-            char m[160];
-            snprintf(m, sizeof m, "matrix P of sample %d is not positive definite (pivot %d)", b0 + b, inf[b]);
-            h->err = m;
-            cleanup();
-            return -3;
-          }
-        // mx_b in the padded nxp x nxp layout of the rank-one GEMMs
-        const double* mx = d_mx + (long)bi * bcap * l2;
-        double* mxp = d_mxp + (long)bi * bcap * nxp * nxp;
-        const int nxp_ = nxp;
-        const long pp = (long)nxp * nxp;
-        ew(st, (long)nb * pp, [=] __device__(long idx) {
-          const int b = (int)(idx / pp);
-          const long e = idx - (long)b * pp;
-          const int i = (int)(e / nxp_), j = (int)(e % nxp_);
-          mxp[idx] = (i < nx && j < nx) ? mx[(long)b * l2 + (long)i * nx + j] : 0.0;
-        });
-        L(h);
+        if (int rc = smf_posterior_stage(h, chunks, samples_host, b0, nb, bcap, hs, d_part, d_c1, d_w, wcols, d_work,
+                                         d_info, d_mx + (long)bi * bcap * l2, d_xm + (long)bi * bcap * ld,
+                                         d_q1 + (long)bi * bcap, r, c0, reg, 0.0))
+          return rc;
+        pad_mx(h, d_mx + (long)bi * bcap * l2, nb, d_mxp + (long)bi * bcap * nxp * nxp);
       } else {
-        hsm.assign((size_t)bcap * nhp, 0.0);
-        for (int b = 0; b < nb; ++b)
-          for (int i = 0; i < nh; ++i) hsm[(size_t)b * nhp + i] = samples_host[(size_t)(b0 + b) * nh + i];
-        // (pageable source: staged before the call returns)
-        PCK(cudaMemcpyAsync(hs, hsm.data(), hsm.size() * sizeof(double), cudaMemcpyHostToDevice, st));
+        if (stage_samples(h, samples_host + (size_t)b0 * nh, nb, bcap, hs)) return -2;
       }
     }
     // HH[b] = h_b h_b^T - iKh (rows past the group are zero)
@@ -3474,7 +3199,7 @@ int predict_cov_run(cgpcm_handle* h, const double* params_host, double reg, cons
     for (int bi = 0; bi < nbat; ++bi) {
       const int b0 = g0 + bi * bcap, nb = std::min(bcap, B - b0);
       const double* hs = d_hs + (long)bi * bcap * nhp;
-      PRC(gemm(h, true, false, false, bcap, (int)acols, nhp, 1.0, hs, nhp, d_A, acols, 0.0, d_v, acols));
+      if (gemm(h, true, false, false, bcap, (int)acols, nhp, 1.0, hs, nhp, d_A, acols, 0.0, d_v, acols)) return -2;
       prof_close(h);
       PredQuadArgs qa;
       qa.V = d_v; qa.v_stride = acols; qa.ldv = nxp;
@@ -3498,8 +3223,8 @@ int predict_cov_run(cgpcm_handle* h, const double* params_host, double reg, cons
         const double* Vb = d_v + (long)b * acols;
         const double* mxp = d_mxp + (smf ? (long)(bi * bcap + b) * nxp * nxp : 0);
         double* Cb = d_c + (long)(bi * bcap + b) * n2;
-        PRC(gemm(h, true, false, false, npad, nxp, nxp, 1.0, Vb, nxp, mxp, nxp, 0.0, d_y, nxp));
-        PRC(gemm(h, true, true, false, npad, npad, nxp, 1.0, d_y, nxp, Vb, nxp, 0.0, Cb, npad));
+        if (gemm(h, true, false, false, npad, nxp, nxp, 1.0, Vb, nxp, mxp, nxp, 0.0, d_y, nxp)) return -2;
+        if (gemm(h, true, true, false, npad, npad, nxp, 1.0, d_y, nxp, Vb, nxp, 0.0, Cb, npad)) return -2;
       }
     }
     // ---- pair tiles p >= q
@@ -3510,8 +3235,8 @@ int predict_cov_run(cgpcm_handle* h, const double* params_host, double reg, cons
         const int npairs = P * Q, npp = round_up(npairs, 8);
         const long ldg = (long)TP * nxp;
         // G(i, k; j, l) = sum_m A*[m][(p0 + i, k)] T[m][(q0 + j, l)]
-        PRC(gemm(h, false, false, false, P * nxp, Q * nxp, nhp, 1.0, d_A + (long)p0 * nxp, acols,
-                 d_TA + (long)q0 * nxp, acols, 0.0, d_g, ldg));
+        if (gemm(h, false, false, false, P * nxp, Q * nxp, nhp, 1.0, d_A + (long)p0 * nxp, acols,
+                 d_TA + (long)q0 * nxp, acols, 0.0, d_g, ldg)) return -2;
         prof_close(h);
         axx_pair_launch(st, d_t + p0, P, d_t + q0, Q, h->tx, nx, d_g, ldg, nxp, d_x, cd, T);
         L(h);
@@ -3521,7 +3246,7 @@ int predict_cov_run(cgpcm_handle* h, const double* params_host, double reg, cons
           ew(st, npairs, [=] __device__(long e) { lag[e] = tt[p0 + e / Q] - tt[q0 + e % Q]; });
           L(h);
         }
-        if (npp > npairs) PCK(cudaMemsetAsync(d_AC + (long)npairs * KH, 0, (size_t)(npp - npairs) * KH * sizeof(double), st));
+        if (npp > npairs) CK(cudaMemsetAsync(d_AC + (long)npairs * KH, 0, (size_t)(npp - npairs) * KH * sizeof(double), st));
         ahh_center_kernel<<<148 * 8, 256, 0, st>>>(d_lag, npairs, h->th, nh, nhl, alpha, gamma, h->causal, d_AC, d_ac);
         L(h);
         if (!smf) {
@@ -3531,8 +3256,8 @@ int predict_cov_run(cgpcm_handle* h, const double* params_host, double reg, cons
         for (int bi = 0; bi < nbat; ++bi) {
           const int b0 = g0 + bi * bcap, nb = std::min(bcap, B - b0);
           // gf[e][b] = sum_(i,j) Ahh_c(lag_e)[i][j] HH_b[i][j]
-          PRC(gemm(h, true, true, false, npp, bcap, (int)KH, 1.0, d_AC, KH, d_hh + (long)bi * bcap * KH, KH, 0.0, d_gf,
-                   bcap));
+          if (gemm(h, true, true, false, npp, bcap, (int)KH, 1.0, d_AC, KH, d_hh + (long)bi * bcap * KH, KH, 0.0, d_gf,
+                   bcap)) return -2;
           prof_close(h);
           if (smf) {
             predict_qb_launch(st, d_x, (long)nx * nx, d_mx + (long)bi * bcap * l2, l2, nb, npairs, TPP, bcap, d_qp, bcap);
@@ -3544,7 +3269,7 @@ int predict_cov_run(cgpcm_handle* h, const double* params_host, double reg, cons
           L(h);
         }
       }
-    PCK(cudaGetLastError());
+    CK(cudaGetLastError());
     // ---- cov += C_b / B in ascending b; the per-sample outputs
     if (cov_out) {
       const double* C = d_c;
@@ -3559,10 +3284,10 @@ int predict_cov_run(cgpcm_handle* h, const double* params_host, double reg, cons
     }
     if (cov_s_out)
       for (int b = 0; b < gn; ++b)
-        PCK(cudaMemcpy2DAsync(cov_s_out + (size_t)(g0 + b) * n * n, (size_t)n * sizeof(double), d_c + (long)b * n2,
+        CK(cudaMemcpy2DAsync(cov_s_out + (size_t)(g0 + b) * n * n, (size_t)n * sizeof(double), d_c + (long)b * n2,
                               (size_t)npad * sizeof(double), (size_t)n * sizeof(double), n, cudaMemcpyDefault, st));
     if (want_draws) {
-      PCK(cudaMemsetAsync(d_pinfo, 0, (size_t)gn * sizeof(int), st));
+      CK(cudaMemsetAsync(d_pinfo, 0, (size_t)gn * sizeof(int), st));
       for (int b = 0; b < gn; ++b) {
         const double* Cb = d_c + (long)b * n2;
         double* Kp = d_k;
@@ -3576,7 +3301,7 @@ int predict_cov_run(cgpcm_handle* h, const double* params_host, double reg, cons
         L(h);
         cudaError_t e = potrf_lower(st, d_k, npad, npad, d_pinfo + b, 7, h->M(M_XW));
         L(h, 2 * ((npad + LA_NB - 1) / LA_NB));
-        if (e != cudaSuccess) { h->err = "potrf launch failed"; cleanup(); return -2; }
+        if (e != cudaSuccess) { h->err = "potrf launch failed"; return -2; }
         matvec_kernel<<<(npad + 7) / 8, 256, 0, st>>>(d_k, npad, npad, npad, 0, d_noise + (long)(g0 + b) * npad, 1.0, d_f);
         L(h);
         const double* fv = d_f;
@@ -3586,51 +3311,26 @@ int predict_cov_run(cgpcm_handle* h, const double* params_host, double reg, cons
         ew(st, n, [=] __device__(long p) { dr[p * Bn] = mean[p * Bn] + fv[p]; });
         L(h);
       }
-      PCK(cudaMemcpyAsync(inf.data(), d_pinfo, (size_t)gn * sizeof(int), cudaMemcpyDeviceToHost, st));
-      PCK(cudaStreamSynchronize(st));
+      CK(cudaMemcpyAsync(inf.data(), d_pinfo, (size_t)gn * sizeof(int), cudaMemcpyDeviceToHost, st));
+      CK(cudaStreamSynchronize(st));
       for (int b = 0; b < gn; ++b)
-        if (inf[b]) {
-          char m[160];
-          snprintf(m, sizeof m, "matrix C_b + reg I of sample %d is not positive definite (pivot %d)", g0 + b,
-                   inf[b] % 100000);
-          h->err = m;
-          cleanup();
-          return -3;
-        }
+        if (inf[b]) return sample_pd_error(h, "C_b + reg I", g0 + b, inf[b] % 100000);
     }
   }
-  if (mean_s_out) PCK(cudaMemcpyAsync(mean_s_out, d_mean, (size_t)n * B * sizeof(double), cudaMemcpyDefault, st));
-  if (want_draws) PCK(cudaMemcpyAsync(draws_out, d_draw, (size_t)n * B * sizeof(double), cudaMemcpyDefault, st));
+  if (mean_s_out) CK(cudaMemcpyAsync(mean_s_out, d_mean, (size_t)n * B * sizeof(double), cudaMemcpyDefault, st));
+  if (want_draws) CK(cudaMemcpyAsync(draws_out, d_draw, (size_t)n * B * sizeof(double), cudaMemcpyDefault, st));
   if (cov_out)
-    PCK(cudaMemcpy2DAsync(cov_out, (size_t)n * sizeof(double), d_cov, (size_t)npad * sizeof(double),
-                          (size_t)n * sizeof(double), n, cudaMemcpyDefault, st));
-  prof_close(h);
-  PCK(cudaEventRecord(h->ev[6], st));
-  PCK(cudaStreamSynchronize(st));
-  PCK(cudaGetLastError());
-  cleanup();
-#undef PCK
-#undef PRC
-  float ms = 0;
-  cudaEventElapsedTime(&ms, h->ev[0], h->ev[6]);
-  memset(h->timing, 0, sizeof h->timing);
-  h->timing[0] = ms;
-  h->timing[6] = (double)h->launches;
-  h->timing[7] = h->gemm_flops;
-  h->timing[8] = (double)h->gemm_launches;
+    CK(cudaMemcpy2DAsync(cov_out, (size_t)n * sizeof(double), d_cov, (size_t)npad * sizeof(double),
+                         (size_t)n * sizeof(double), n, cudaMemcpyDefault, st));
+  int info;          // the prior's and the shared q(z)'s, checked above
+  if (end_run(h, info)) return -2;
+  record_timing(h);
   return 0;
 }
 
 }  // namespace cgimpl
 
 extern "C" {
-
-static int fetch_params(cgpcm_handle* h, const double* params, long np, std::vector<double>& host) {
-  host.resize(np);
-  if (is_device_ptr(params)) CK(cudaMemcpy(host.data(), params, np * sizeof(double), cudaMemcpyDeviceToHost));
-  else memcpy(host.data(), params, np * sizeof(double));
-  return 0;
-}
 
 int cgpcm_precompute(cgpcm_handle* h, const double hyp[3], double reg) {
   if (!h || !hyp) return -1;
@@ -3651,38 +3351,24 @@ int cgpcm_frozen_mats(cgpcm_handle* h, double* sum_Bxx, double* sum_Bhh, double*
   if (export_mat(h, h->M(M_F_BHH), h->nh, h->nh, sum_Bhh)) return -2;
   if (export_mat(h, h->M(M_F_Y), h->nh, h->nx, sum_Ahx_y)) return -2;
   CK(cudaStreamSynchronize(h->st));
-  if (sum_b) {
-    if (is_device_ptr(sum_b)) CK(cudaMemcpy(sum_b, &h->f_sum_b, sizeof(double), cudaMemcpyHostToDevice));
-    else *sum_b = h->f_sum_b;
-  }
-  return 0;
+  return put(h, sum_b, &h->f_sum_b, 1);
 }
 
 int cgpcm_elbo_smf(cgpcm_handle* h, const double* params, int32_t mode, double reg, const double* sample, double* elbo,
                    double* terms, double* loglik) {
   if (!h || !params || !sample || !elbo) return -1;
   if (mode != CGPCM_MODE_FROZEN && mode != CGPCM_MODE_FULL) { h->err = "bad mode"; return -1; }
-  if (!h->t) { h->err = "cgpcm_set_data has not been called"; return -1; }
-  if (!std::isfinite(reg) || reg < 0) { h->err = "reg must be finite and >= 0"; return -4; }
+  if (int rc = check_call(h, h->t, reg)) return rc;
   CK(cudaSetDevice(h->device));
   const long np = 5 + h->nh + (long)h->nh * (h->nh + 1) / 2;
-  std::vector<double> host, smp(h->nh);
-  if (fetch_params(h, params, np, host)) return -2;
-  if (is_device_ptr(sample)) CK(cudaMemcpy(smp.data(), sample, h->nh * sizeof(double), cudaMemcpyDeviceToHost));
-  else memcpy(smp.data(), sample, h->nh * sizeof(double));
-  for (int i = 0; i < h->nh; ++i)
-    if (!std::isfinite(smp[i])) { h->err = "non-finite sample"; return -4; }
+  std::vector<double> host, smp;
+  if (to_host(h, params, np, host) || to_host(h, sample, h->nh, smp)) return -2;
+  if (check_samples(h, smp.data(), 1, h->nh)) return -4;
   double e = 0.0, tm[7], ll = 0.0;
   int rc = evaluate(h, host.data(), mode, 0u, reg, false, &e, tm, nullptr, smp.data(), &ll);
   if (rc) return rc;
-  float ms = 0;
-  cudaEventElapsedTime(&ms, h->ev[0], h->ev[6]);
-  memset(h->timing, 0, sizeof h->timing);
-  h->timing[0] = ms;
-  h->timing[6] = (double)h->launches;
-  if (is_device_ptr(elbo)) cudaMemcpy(elbo, &e, sizeof e, cudaMemcpyHostToDevice); else *elbo = e;
-  if (terms) { if (is_device_ptr(terms)) cudaMemcpy(terms, tm, sizeof tm, cudaMemcpyHostToDevice); else memcpy(terms, tm, sizeof tm); }
-  if (loglik) { if (is_device_ptr(loglik)) cudaMemcpy(loglik, &ll, sizeof ll, cudaMemcpyHostToDevice); else *loglik = ll; }
+  record_timing(h);
+  if (put(h, elbo, &e, 1) || put(h, terms, tm, 7) || put(h, loglik, &ll, 1)) return -2;
   return 0;
 }
 
@@ -3690,44 +3376,31 @@ int cgpcm_elbo_smf_batch(cgpcm_handle* h, const double* params, double reg, cons
                          double* elbo, double* terms, double* loglik) {
   if (!h || !params || !samples) return -1;
   if (n_samples < 1) { h->err = "n_samples must be >= 1"; return -1; }
-  if (!h->t) { h->err = "cgpcm_set_data has not been called"; return -1; }
-  if (!std::isfinite(reg) || reg < 0) { h->err = "reg must be finite and >= 0"; return -4; }
+  if (int rc = check_call(h, h->t, reg)) return rc;
   CK(cudaSetDevice(h->device));
   const long np = 5 + h->nh + (long)h->nh * (h->nh + 1) / 2;
-  const long ns = (long)n_samples * h->nh;
-  std::vector<double> host, smp(ns);
-  if (fetch_params(h, params, np, host)) return -2;
-  if (is_device_ptr(samples)) CK(cudaMemcpy(smp.data(), samples, ns * sizeof(double), cudaMemcpyDeviceToHost));
-  else memcpy(smp.data(), samples, ns * sizeof(double));
+  std::vector<double> host, smp;
+  if (to_host(h, params, np, host) || to_host(h, samples, (long)n_samples * h->nh, smp)) return -2;
   const bool want_p = elbo || terms;
   std::vector<double> e(want_p ? n_samples : 0), tm(want_p ? 7L * n_samples : 0), ll(loglik ? n_samples : 0);
   int rc = smf_batch_run(h, host.data(), reg, smp.data(), n_samples, want_p, loglik != nullptr,
                          want_p ? e.data() : nullptr, want_p ? tm.data() : nullptr, loglik ? ll.data() : nullptr);
   if (rc) return rc;
-  auto put = [&](double* dst, const std::vector<double>& v) -> int {
-    if (!dst || v.empty()) return 0;
-    if (is_device_ptr(dst)) CK(cudaMemcpy(dst, v.data(), v.size() * sizeof(double), cudaMemcpyHostToDevice));
-    else memcpy(dst, v.data(), v.size() * sizeof(double));
-    return 0;
-  };
-  if (put(elbo, e) || put(terms, tm) || put(loglik, ll)) return -2;
+  if (put(h, elbo, e.data(), e.size()) || put(h, terms, tm.data(), tm.size()) || put(h, loglik, ll.data(), ll.size()))
+    return -2;
   return 0;
 }
 
 int cgpcm_predict_f(cgpcm_handle* h, const double* params, double reg, const double* t_star, int64_t n_star,
                     const double* samples, int32_t n_samples, int32_t smf, double* mean, double* var) {
   if (!h || !params || n_star < 0 || n_samples < 1 || !samples || (n_star > 0 && !t_star)) return -1;
-  if (!h->t) { h->err = "cgpcm_set_data has not been called"; return -1; }
-  if (!std::isfinite(reg) || reg < 0) { h->err = "reg must be finite and >= 0"; return -4; }
+  if (int rc = check_call(h, h->t, reg)) return rc;
   if (n_star == 0) return 0;
   CK(cudaSetDevice(h->device));
   const long np = 5 + h->nh + (long)h->nh * (h->nh + 1) / 2;
-  std::vector<double> host, ts(n_star), smp((size_t)n_samples * h->nh);
-  if (fetch_params(h, params, np, host)) return -2;
-  if (is_device_ptr(t_star)) CK(cudaMemcpy(ts.data(), t_star, n_star * sizeof(double), cudaMemcpyDeviceToHost));
-  else memcpy(ts.data(), t_star, n_star * sizeof(double));
-  if (is_device_ptr(samples)) CK(cudaMemcpy(smp.data(), samples, smp.size() * sizeof(double), cudaMemcpyDeviceToHost));
-  else memcpy(smp.data(), samples, smp.size() * sizeof(double));
+  std::vector<double> host, ts, smp;
+  if (to_host(h, params, np, host) || to_host(h, t_star, n_star, ts) || to_host(h, samples, (long)n_samples * h->nh, smp))
+    return -2;
   return predict_run(h, host.data(), reg, ts.data(), n_star, smp.data(), n_samples, smf, mean, var);
 }
 
@@ -3736,17 +3409,13 @@ int cgpcm_predict_f_batch(cgpcm_handle* h, const double* params, double reg, con
                           double* mean_s, double* var_s) {
   if (!h || !params || n_star < 0 || !samples || (n_star > 0 && !t_star)) return -1;
   if (n_samples < 1) { h->err = "n_samples must be >= 1"; return -1; }
-  if (!h->t) { h->err = "cgpcm_set_data has not been called"; return -1; }
-  if (!std::isfinite(reg) || reg < 0) { h->err = "reg must be finite and >= 0"; return -4; }
+  if (int rc = check_call(h, h->t, reg)) return rc;
   if (n_star == 0) return 0;
   CK(cudaSetDevice(h->device));
   const long np = 5 + h->nh + (long)h->nh * (h->nh + 1) / 2;
-  std::vector<double> host, ts(n_star), smp((size_t)n_samples * h->nh);
-  if (fetch_params(h, params, np, host)) return -2;
-  if (is_device_ptr(t_star)) CK(cudaMemcpy(ts.data(), t_star, n_star * sizeof(double), cudaMemcpyDeviceToHost));
-  else memcpy(ts.data(), t_star, n_star * sizeof(double));
-  if (is_device_ptr(samples)) CK(cudaMemcpy(smp.data(), samples, smp.size() * sizeof(double), cudaMemcpyDeviceToHost));
-  else memcpy(smp.data(), samples, smp.size() * sizeof(double));
+  std::vector<double> host, ts, smp;
+  if (to_host(h, params, np, host) || to_host(h, t_star, n_star, ts) || to_host(h, samples, (long)n_samples * h->nh, smp))
+    return -2;
   return predict_batch_run(h, host.data(), reg, ts.data(), n_star, smp.data(), n_samples, smf ? 1 : 0, mean, var,
                            mean_s, var_s);
 }
@@ -3758,20 +3427,14 @@ int cgpcm_predict_f_cov(cgpcm_handle* h, const double* params, double reg, const
   if (n_samples < 1) { h->err = "n_samples must be >= 1"; return -1; }
   if (n_star > 4096) { h->err = "predict_f_cov: at most 4096 test inputs"; return -1; }
   if (draws && !noise) { h->err = "predict_f_cov: draws need noise"; return -1; }
-  if (!h->t) { h->err = "cgpcm_set_data has not been called"; return -1; }
-  if (!std::isfinite(reg) || reg < 0) { h->err = "reg must be finite and >= 0"; return -4; }
+  if (int rc = check_call(h, h->t, reg)) return rc;
   if (n_star == 0) return 0;
   CK(cudaSetDevice(h->device));
   const long np = 5 + h->nh + (long)h->nh * (h->nh + 1) / 2;
-  std::vector<double> host, ts(n_star), smp((size_t)n_samples * h->nh), ns(draws ? (size_t)n_star * n_samples : 0);
-  if (fetch_params(h, params, np, host)) return -2;
-  auto fetch = [&](const double* src, std::vector<double>& dst) -> int {
-    if (is_device_ptr(src)) CK(cudaMemcpy(dst.data(), src, dst.size() * sizeof(double), cudaMemcpyDeviceToHost));
-    else memcpy(dst.data(), src, dst.size() * sizeof(double));
-    return 0;
-  };
-  if (fetch(t_star, ts) || fetch(samples, smp)) return -2;
-  if (draws && fetch(noise, ns)) return -2;
+  std::vector<double> host, ts, smp, ns;
+  if (to_host(h, params, np, host) || to_host(h, t_star, n_star, ts) || to_host(h, samples, (long)n_samples * h->nh, smp))
+    return -2;
+  if (draws && to_host(h, noise, (long)n_star * n_samples, ns)) return -2;
   return predict_cov_run(h, host.data(), reg, ts.data(), n_star, smp.data(), n_samples, smf ? 1 : 0,
                          draws ? ns.data() : nullptr, mean_s, cov_s, cov, draws);
 }
@@ -3779,147 +3442,115 @@ int cgpcm_predict_f_cov(cgpcm_handle* h, const double* params, double reg, const
 int cgpcm_kernel_samples(cgpcm_handle* h, const double* params, double reg, const double* t, int64_t n,
                          const double* samples, int32_t n_samples, double* out) {
   if (!h || !params || n < 0 || n_samples < 1 || !samples || !out || (n > 0 && !t)) return -1;
-  if (!h->th) { h->err = "cgpcm_set_data has not been called"; return -1; }
-  if (!std::isfinite(reg) || reg < 0) { h->err = "reg must be finite and >= 0"; return -4; }
+  if (int rc = check_call(h, h->th, reg)) return rc;
   if (n == 0) return 0;
   CK(cudaSetDevice(h->device));
-  std::vector<double> host, ts(n), smp((size_t)n_samples * h->nh);
-  if (fetch_params(h, params, 5, host)) return -2;
-  if (is_device_ptr(t)) CK(cudaMemcpy(ts.data(), t, n * sizeof(double), cudaMemcpyDeviceToHost));
-  else memcpy(ts.data(), t, n * sizeof(double));
-  if (is_device_ptr(samples)) CK(cudaMemcpy(smp.data(), samples, smp.size() * sizeof(double), cudaMemcpyDeviceToHost));
-  else memcpy(smp.data(), samples, smp.size() * sizeof(double));
+  std::vector<double> host, ts, smp;
+  if (to_host(h, params, 5, host) || to_host(h, t, n, ts) || to_host(h, samples, (long)n_samples * h->nh, smp)) return -2;
   return kernel_run(h, host.data(), reg, ts.data(), n, smp.data(), n_samples, out);
 }
 
 int cgpcm_filter_samples(cgpcm_handle* h, const double* params, double reg, const double* t, int64_t n,
                          const double* samples, int32_t n_samples, const double* noise, double* out) {
   if (!h || !params || n < 0 || n_samples < 1 || !samples || !noise || !out || (n > 0 && !t)) return -1;
-  if (!h->th) { h->err = "cgpcm_set_data has not been called"; return -1; }
-  if (!std::isfinite(reg) || reg < 0) { h->err = "reg must be finite and >= 0"; return -4; }
+  if (int rc = check_call(h, h->th, reg)) return rc;
   if (n == 0) return 0;
   CK(cudaSetDevice(h->device));
-  std::vector<double> host, ts(n), smp((size_t)n_samples * h->nh), ns((size_t)n * n_samples);
-  if (fetch_params(h, params, 5, host)) return -2;
-  auto fetch = [&](const double* src, std::vector<double>& dst) -> int {
-    if (is_device_ptr(src)) CK(cudaMemcpy(dst.data(), src, dst.size() * sizeof(double), cudaMemcpyDeviceToHost));
-    else memcpy(dst.data(), src, dst.size() * sizeof(double));
-    return 0;
-  };
-  if (fetch(t, ts) || fetch(samples, smp) || fetch(noise, ns)) return -2;
+  std::vector<double> host, ts, smp, ns;
+  if (to_host(h, params, 5, host) || to_host(h, t, n, ts) || to_host(h, samples, (long)n_samples * h->nh, smp) ||
+      to_host(h, noise, n * n_samples, ns))
+    return -2;
   return filter_run(h, host.data(), reg, ts.data(), n, smp.data(), n_samples, ns.data(), out);
 }
 
 int cgpcm_akm_sample(cgpcm_handle* h, const double* params, double reg, const double* t, int64_t n,
                      const double* sample_h, const double* e, double* f, double* K) {
   if (!h || !params || n < 1 || !t || !sample_h || !e || !f) return -1;
-  if (!h->th) { h->err = "cgpcm_set_data has not been called"; return -1; }
-  if (!std::isfinite(reg) || reg < 0) { h->err = "reg must be finite and >= 0"; return -4; }
+  if (int rc = check_call(h, h->th, reg)) return rc;
   CK(cudaSetDevice(h->device));
-  std::vector<double> host, ts(n), hs(h->nh), es(n);
-  if (fetch_params(h, params, 5, host)) return -2;
-  auto fetch = [&](const double* src, std::vector<double>& dst) -> int {
-    if (is_device_ptr(src)) CK(cudaMemcpy(dst.data(), src, dst.size() * sizeof(double), cudaMemcpyDeviceToHost));
-    else memcpy(dst.data(), src, dst.size() * sizeof(double));
-    return 0;
-  };
-  if (fetch(t, ts) || fetch(sample_h, hs) || fetch(e, es)) return -2;
-  for (double v : hs)
-    if (!std::isfinite(v)) { h->err = "non-finite sample"; return -4; }
+  std::vector<double> host, ts, hs, es;
+  if (to_host(h, params, 5, host) || to_host(h, t, n, ts) || to_host(h, sample_h, h->nh, hs) || to_host(h, e, n, es))
+    return -2;
+  if (check_samples(h, hs.data(), 1, h->nh)) return -4;
   return akm_run(h, host.data(), reg, ts.data(), n, hs.data(), es.data(), f, K);
 }
 
 int cgpcm_fpi(cgpcm_handle* h, const double* params, int32_t num, int32_t high_reg, double reg, double* mu_u,
               double* var_u, double* mu_z, double* var_z) {
   if (!h || !params || num < 0) return -1;
-  if (!h->t) { h->err = "cgpcm_set_data has not been called"; return -1; }
-  if (!std::isfinite(reg) || reg < 0) { h->err = "reg must be finite and >= 0"; return -4; }
+  if (int rc = check_call(h, h->t, reg)) return rc;
   CK(cudaSetDevice(h->device));
   const long np = 5 + h->nh + (long)h->nh * (h->nh + 1) / 2;
   std::vector<double> host;
-  if (fetch_params(h, params, np, host)) return -2;
+  if (to_host(h, params, np, host)) return -2;
   return fpi_run(h, host.data(), num, high_reg, reg, mu_u, var_u, mu_z, var_z);
 }
 
 int cgpcm_fpi_qz(cgpcm_handle* h, const double* params, const double* mu_z_in, const double* var_z_in, int32_t num,
                  int32_t high_reg, double reg, double* mu_u, double* var_u, double* mu_z, double* var_z) {
   if (!h || !params || !mu_z_in || !var_z_in || num < 0) return -1;
-  if (!h->t) { h->err = "cgpcm_set_data has not been called"; return -1; }
-  if (!std::isfinite(reg) || reg < 0) { h->err = "reg must be finite and >= 0"; return -4; }
+  if (int rc = check_call(h, h->t, reg)) return rc;
   CK(cudaSetDevice(h->device));
   const long np = 5 + h->nh + (long)h->nh * (h->nh + 1) / 2;
   std::vector<double> host, mz, vz;
-  if (fetch_params(h, params, np, host)) return -2;
-  if (fetch_params(h, mu_z_in, h->nx, mz)) return -2;
-  if (fetch_params(h, var_z_in, (long)h->nx * (h->nx + 1) / 2, vz)) return -2;
+  if (to_host(h, params, np, host) || to_host(h, mu_z_in, h->nx, mz) ||
+      to_host(h, var_z_in, (long)h->nx * (h->nx + 1) / 2, vz))
+    return -2;
   return fpi_run(h, host.data(), num, high_reg, reg, mu_u, var_u, mu_z, var_z, mz.data(), vz.data());
 }
 
 int cgpcm_elbo_qz(cgpcm_handle* h, const double* params, const double* mu_z, const double* var_z, double reg,
                   double* elbo, double* terms) {
   if (!h || !params || !mu_z || !var_z || !elbo) return -1;
-  if (!h->t) { h->err = "cgpcm_set_data has not been called"; return -1; }
-  if (!std::isfinite(reg) || reg < 0) { h->err = "reg must be finite and >= 0"; return -4; }
+  if (int rc = check_call(h, h->t, reg)) return rc;
   CK(cudaSetDevice(h->device));
   std::vector<double> host, mz, vz;
-  if (fetch_params(h, params, 5, host)) return -2;
-  if (fetch_params(h, mu_z, h->nx, mz)) return -2;
-  if (fetch_params(h, var_z, (long)h->nx * (h->nx + 1) / 2, vz)) return -2;
+  if (to_host(h, params, 5, host) || to_host(h, mu_z, h->nx, mz) || to_host(h, var_z, (long)h->nx * (h->nx + 1) / 2, vz))
+    return -2;
   double e = 0.0, tm[7];
   int rc = qz_run(h, host.data(), mz.data(), vz.data(), reg, &e, tm);
-  if (rc == 0) {
-    if (is_device_ptr(elbo)) cudaMemcpy(elbo, &e, sizeof e, cudaMemcpyHostToDevice); else *elbo = e;
-    if (terms) { if (is_device_ptr(terms)) cudaMemcpy(terms, tm, sizeof tm, cudaMemcpyHostToDevice); else memcpy(terms, tm, sizeof tm); }
-  }
-  return rc;
+  if (rc) return rc;
+  return put(h, elbo, &e, 1) || put(h, terms, tm, 7) ? -2 : 0;
 }
 
 int cgpcm_elbo_grad(cgpcm_handle* h, const double* params, int32_t mode, uint32_t grad_mask, double reg, double* elbo,
                     double* terms, double* grad) {
   if (!h || !params || !elbo) return -1;
   if (mode != CGPCM_MODE_FROZEN && mode != CGPCM_MODE_FULL) { h->err = "bad mode"; return -1; }
-  if (!h->t) { h->err = "cgpcm_set_data has not been called"; return -1; }
-  if (!std::isfinite(reg) || reg < 0) { h->err = "reg must be finite and >= 0"; return -4; }
+  if (int rc = check_call(h, h->t, reg)) return rc;
   CK(cudaSetDevice(h->device));
   const long np = 5 + h->nh + (long)h->nh * (h->nh + 1) / 2;
   std::vector<double> host;
-  if (fetch_params(h, params, np, host)) return -2;
+  if (to_host(h, params, np, host)) return -2;
   double e = 0.0, tm[7];
   int rc = evaluate(h, host.data(), mode, grad ? grad_mask : 0u, reg, false, &e, tm, grad);
-  if (rc == 0) {
-    float ms[6] = {0, 0, 0, 0, 0, 0};
-    cudaEventElapsedTime(&ms[0], h->ev[0], h->ev[6]);
-    cudaEventElapsedTime(&ms[1], h->ev[1], h->ev[3]);   // forward sweep (Axx + chunks + all-reduce)
-    cudaEventElapsedTime(&ms[2], h->ev[4], h->ev[5]);   // backward sweep
-    cudaEventElapsedTime(&ms[3], h->ev[3], h->ev[4]);   // M x M algebra between the sweeps
-    cudaEventElapsedTime(&ms[4], h->ev[1], h->ev[2]);   // Axx kernels
-    h->timing[0] = ms[0]; h->timing[1] = ms[1]; h->timing[2] = ms[2]; h->timing[3] = ms[3]; h->timing[4] = ms[4];
-    h->timing[5] = ms[1] - ms[4] + ms[2];
-    if (h->profile) {
-      double tot = 0.0, tot_gen = 0.0;
-      for (size_t i = 0; i + 1 < h->pev_used; i += 2) {
-        float g = 0;
-        cudaEventElapsedTime(&g, h->pev[i], h->pev[i + 1]);
-        if (h->pev_kind[i / 2]) tot_gen += g; else tot += g;
-      }
-      h->timing[5] = tot;
-      h->timing[10] = tot_gen;
+  if (rc) return rc;
+  record_timing(h);
+  float ms[5] = {0, 0, 0, 0, 0};
+  cudaEventElapsedTime(&ms[1], h->ev[1], h->ev[3]);   // forward sweep (Axx + chunks + all-reduce)
+  cudaEventElapsedTime(&ms[2], h->ev[4], h->ev[5]);   // backward sweep
+  cudaEventElapsedTime(&ms[3], h->ev[3], h->ev[4]);   // M x M algebra between the sweeps
+  cudaEventElapsedTime(&ms[4], h->ev[1], h->ev[2]);   // Axx kernels
+  h->timing[1] = ms[1]; h->timing[2] = ms[2]; h->timing[3] = ms[3]; h->timing[4] = ms[4];
+  h->timing[5] = ms[1] - ms[4] + ms[2];
+  if (h->profile) {
+    double tot = 0.0, tot_gen = 0.0;
+    for (size_t i = 0; i + 1 < h->pev_used; i += 2) {
+      float g = 0;
+      cudaEventElapsedTime(&g, h->pev[i], h->pev[i + 1]);
+      if (h->pev_kind[i / 2]) tot_gen += g; else tot += g;
     }
-    h->timing[6] = (double)h->launches;
-    h->timing[7] = h->gemm_flops;
-    h->timing[8] = (double)h->gemm_launches;
-    h->timing[9] = h->gemm_flops_exec;
-    {
-      // this rank's own sweep time, without the waits inside the collectives: what a caller balances shards with
-      float f = 0, b = 0;
-      cudaEventElapsedTime(&f, h->ev[1], h->ev[7]);
-      cudaEventElapsedTime(&b, h->ev[4], h->ev[8]);
-      h->timing[11] = f + b;
-    }
-    if (is_device_ptr(elbo)) cudaMemcpy(elbo, &e, sizeof e, cudaMemcpyHostToDevice); else *elbo = e;
-    if (terms) { if (is_device_ptr(terms)) cudaMemcpy(terms, tm, sizeof tm, cudaMemcpyHostToDevice); else memcpy(terms, tm, sizeof tm); }
+    h->timing[5] = tot;
+    h->timing[10] = tot_gen;
   }
-  return rc;
+  {
+    // this rank's own sweep time, without the waits inside the collectives: what a caller balances shards with
+    float f = 0, b = 0;
+    cudaEventElapsedTime(&f, h->ev[1], h->ev[7]);
+    cudaEventElapsedTime(&b, h->ev[4], h->ev[8]);
+    h->timing[11] = f + b;
+  }
+  return put(h, elbo, &e, 1) || put(h, terms, tm, 7) ? -2 : 0;
 }
 
 int cgpcm_last_timing(cgpcm_handle* h, double out[12]) {
@@ -4109,11 +3740,11 @@ int cgpcm_cholinv(double* A, double* Ainv, double* logdet, int n, int64_t ld, in
   if (!A || n < 1 || ld < n || (ld % 8)) return -1;
   int np = round_up(n, 8);
   if (np > ld) return -1;
-  double *X = nullptr, *W = nullptr, *ld_d = nullptr;
-  int* info = nullptr;
-  int rc = 0;
-  if (cudaMalloc(&X, ld * ld * sizeof(double)) != cudaSuccess || cudaMalloc(&W, ld * ld * sizeof(double)) != cudaSuccess ||
-      cudaMalloc(&ld_d, sizeof(double)) != cudaSuccess || cudaMalloc(&info, sizeof(int)) != cudaSuccess) rc = -2;
+  Scratch s;
+  const size_t o_x = s.take(ld * ld), o_w = s.take(ld * ld), o_ld = s.take(1), o_info = s.take(1, sizeof(int));
+  int rc = s.alloc() == cudaSuccess ? 0 : -2;
+  double *X = s.at(o_x), *W = s.at(o_w), *ld_d = s.at(o_ld);
+  int* info = s.at<int>(o_info);
   if (!rc) {
     cudaMemset(info, 0, sizeof(int));
     if (cholinv(nullptr, A, Ainv, X, W, n, np, ld, logdet ? ld_d : nullptr, info, 1) != cudaSuccess) rc = -2;
@@ -4124,10 +3755,6 @@ int cgpcm_cholinv(double* A, double* Ainv, double* logdet, int n, int64_t ld, in
     if (logdet) cudaMemcpy(logdet, ld_d, sizeof(double), cudaMemcpyDefault);
     if (!rc && hi) rc = -3;
   }
-  if (X) cudaFree(X);
-  if (W) cudaFree(W);
-  if (ld_d) cudaFree(ld_d);
-  if (info) cudaFree(info);
   return rc;
 }
 
@@ -4141,9 +3768,11 @@ int cgpcm_smf_c1_test(const double* W, int64_t w_stride, int B, int nwin, const 
       return -1;
   }
   cudaStream_t st = (cudaStream_t)stream;
-  double* part = nullptr;
+  Scratch s;
   const size_t bytes = (size_t)B * SMF_SLICES * ld * ld * sizeof(double);
-  if (cudaMalloc(&part, bytes) != cudaSuccess) { cudaGetLastError(); return -2; }
+  s.take(bytes, 1);
+  if (s.alloc() != cudaSuccess) { cudaGetLastError(); return -2; }
+  double* part = s.at(0);
   int rc = cudaMemsetAsync(part, 0, bytes, st) == cudaSuccess ? 0 : -2;
   for (int w = 0; w < nwin && !rc; ++w) {
     const int64_t* win = windows + 4 * w;
@@ -4155,7 +3784,6 @@ int cgpcm_smf_c1_test(const double* W, int64_t w_stride, int B, int nwin, const 
     if (cudaGetLastError() != cudaSuccess) rc = -2;
   }
   if (cudaStreamSynchronize(st) != cudaSuccess) rc = -2;
-  cudaFree(part);
   return rc;
 }
 
@@ -4168,8 +3796,10 @@ int cgpcm_smf_algebra_test(const double* kx, const double* sum_Bxx, const double
     return -1;
   cudaStream_t st = (cudaStream_t)stream;
   const int passes = (want_p ? 1 : 0) + (want_p0 ? 1 : 0);
-  double* work = nullptr;
-  if (cudaMalloc(&work, (size_t)B * passes * ld * ld * sizeof(double)) != cudaSuccess) { cudaGetLastError(); return -2; }
+  Scratch s;
+  s.take((size_t)B * passes * ld * ld);
+  if (s.alloc() != cudaSuccess) { cudaGetLastError(); return -2; }
+  double* work = s.at(0);
   SmfAlgArgs a;
   a.kx = kx; a.sxx = sum_Bxx; a.c1 = c1; a.fy = sum_Ahx_y; a.bhh = sum_Bhh;
   a.hs = samples; a.work = work; a.out = out; a.info = info;
@@ -4181,7 +3811,6 @@ int cgpcm_smf_algebra_test(const double* kx, const double* sum_Bxx, const double
     if (cudaGetLastError() != cudaSuccess) rc = -2;
   }
   if (cudaStreamSynchronize(st) != cudaSuccess) rc = -2;
-  cudaFree(work);
   return rc;
 }
 
@@ -4194,8 +3823,10 @@ int cgpcm_smf_posterior_test(const double* kx, const double* sum_Bxx, const doub
     return -1;
   cudaStream_t st = (cudaStream_t)stream;
   const long l2 = ld * ld;
-  double* work = nullptr;
-  if (cudaMalloc(&work, (size_t)B * 2 * l2 * sizeof(double)) != cudaSuccess) { cudaGetLastError(); return -2; }
+  Scratch s;
+  s.take((size_t)B * 2 * l2);
+  if (s.alloc() != cudaSuccess) { cudaGetLastError(); return -2; }
+  double* work = s.at(0);
   SmfPostArgs g;
   g.kx = kx; g.sxx = sum_Bxx; g.c1 = c1; g.fy = sum_Ahx_y; g.ahh = Ahh; g.ikx = iKx; g.tr = tr_ahh_ikh; g.hs = samples;
   g.work = work; g.mx = mx; g.xm = xm; g.q1 = q1; g.info = info;
@@ -4207,7 +3838,6 @@ int cgpcm_smf_posterior_test(const double* kx, const double* sum_Bxx, const doub
     if (cudaGetLastError() != cudaSuccess) rc = -2;
   }
   if (cudaStreamSynchronize(st) != cudaSuccess) rc = -2;
-  cudaFree(work);
   return rc;
 }
 
@@ -4225,11 +3855,12 @@ int cgpcm_predict_quad_test(const double* V, int64_t v_stride, int ldv, const do
   g.nv = nv; g.nx = nx; g.nb = B; g.quad = quad; g.lin = lin; g.ldo = B;
   predict_quad_launch(st, g, nslots);
   if (cudaGetLastError() != cudaSuccess) rc = -2;
-  double* part = nullptr;
+  Scratch s;
   if (!rc && qb) {
     // Qb = the PQ_SLICES partials summed in order, as predict_finish_kernel sums them
-    const size_t n = (size_t)PQ_SLICES * nv * B;
-    if (cudaMalloc(&part, n * sizeof(double)) != cudaSuccess) { cudaGetLastError(); rc = -2; }
+    s.take((size_t)PQ_SLICES * nv * B);
+    if (s.alloc() != cudaSuccess) { cudaGetLastError(); rc = -2; }
+    double* part = s.at(0);
     if (!rc) {
       predict_qb_launch(st, bxx, (long)nx * nx, mx, mx_stride, B, nv, nv, nslots, part, B);
       if (cudaGetLastError() != cudaSuccess) rc = -2;
@@ -4245,7 +3876,6 @@ int cgpcm_predict_quad_test(const double* V, int64_t v_stride, int ldv, const do
     }
   }
   if (cudaStreamSynchronize(st) != cudaSuccess) rc = -2;
-  if (part) cudaFree(part);
   return rc;
 }
 
