@@ -21,7 +21,7 @@ GRAD_ALL = 0x7f
 MODE_FROZEN, MODE_FULL = 0, 1
 
 EXPORTS = ['cgpcm_create', 'cgpcm_destroy', 'cgpcm_last_error', 'cgpcm_device_count', 'cgpcm_comm_unique_id', 'cgpcm_comm_init',
-           'cgpcm_set_data', 'cgpcm_set_option', 'cgpcm_psi', 'cgpcm_precompute', 'cgpcm_frozen_mats', 'cgpcm_elbo_grad', 'cgpcm_elbo_smf', 'cgpcm_elbo_smf_batch', 'cgpcm_predict_f', 'cgpcm_predict_f_batch', 'cgpcm_predict_f_cov', 'cgpcm_kernel_samples', 'cgpcm_filter_samples', 'cgpcm_akm_sample', 'cgpcm_fpi', 'cgpcm_fpi_qz', 'cgpcm_elbo_qz',
+           'cgpcm_set_data', 'cgpcm_set_option', 'cgpcm_psi', 'cgpcm_precompute', 'cgpcm_frozen_mats', 'cgpcm_elbo_grad', 'cgpcm_elbo_smf', 'cgpcm_elbo_smf_batch', 'cgpcm_predict_f', 'cgpcm_predict_f_batch', 'cgpcm_predict_f_cov', 'cgpcm_predict_logpdf', 'cgpcm_kernel_samples', 'cgpcm_filter_samples', 'cgpcm_akm_sample', 'cgpcm_fpi', 'cgpcm_fpi_qz', 'cgpcm_elbo_qz',
            'cgpcm_last_timing', 'cgpcm_bvn_cdf', 'cgpcm_dgemm', 'cgpcm_dgemm_tri', 'cgpcm_dgemm_sym', 'cgpcm_cholinv', 'cgpcm_math_test', 'cgpcm_math_test_fast',
            'cgpcm_smf_c1_test', 'cgpcm_smf_algebra_test', 'cgpcm_smf_posterior_test', 'cgpcm_predict_quad_test',
            'cgpcm_predict_pair_test']
@@ -84,6 +84,8 @@ def lib():
     L.cgpcm_predict_f.argtypes = [vp, dp, dbl, dp, i64, dp, ctypes.c_int32, ctypes.c_int32, dp, dp]
     L.cgpcm_predict_f_batch.argtypes = [vp, dp, dbl, dp, i64, dp, ctypes.c_int32, ctypes.c_int32, dp, dp, dp, dp]
     L.cgpcm_predict_f_cov.argtypes = [vp, dp, dbl, dp, i64, dp, ctypes.c_int32, ctypes.c_int32, dp, dp, dp, dp, dp]
+    L.cgpcm_predict_logpdf.argtypes = [vp, dp, dbl, dp, dp, i64, dp, ctypes.c_int32, ctypes.c_int32, ctypes.c_int32,
+                                       dp, dp, dp]
     L.cgpcm_kernel_samples.argtypes = [vp, dp, dbl, dp, i64, dp, ctypes.c_int32, dp]
     L.cgpcm_filter_samples.argtypes = [vp, dp, dbl, dp, i64, dp, ctypes.c_int32, dp, dp]
     L.cgpcm_akm_sample.argtypes = [vp, dp, dbl, dp, i64, dp, dp, dp, dp]

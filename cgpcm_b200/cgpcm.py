@@ -740,6 +740,42 @@ class VCGPCM(CGPCM):
         return self._with_frozen_stats(lambda: self.engine.predict_f_cov(
             self._pack(), t, samples, smf=smf, reg=config.reg, noise=noise))[4]
 
+    def log_predictive_density(self, t, y, samples_h=50, joint=True, noise=True, per_sample=False):
+        """Log density of held-out values ``y`` at ``t`` under the mixture of the samples' predictive distributions
+        (``samples_h`` as in :meth:`predict_f_samples`).  ``noise=True``: ``y`` are observations, each sample's
+        predictive covariance plus ``s2 I``; ``noise=False``: ``y`` is the function itself, plus ``reg I``.
+
+        ``joint=True`` (at most 4096 inputs): the joint log density of the block, ``log mean_b N(y; m_b, C_b + d I)``
+        (:meth:`Engine.predict_logpdf`); ``per_sample=True`` returns ``(lp, lp_s[B], white[n, B])``, each sample's
+        joint log density and whitened residuals.  ``joint=False``: the log density of each point under the mixture of
+        the samples' marginals, ``log mean_b N(y_p; m_bp, v_bp + d)``, an array ``[n]`` (no limit on n);
+        ``per_sample=True`` returns ``(lp[n], lp_s[n, B])``."""
+        t = np.asarray(getattr(t, 'x', t), dtype=np.float64).ravel()
+        y = np.asarray(getattr(y, 'y', y), dtype=np.float64).ravel()
+        if y.shape != t.shape:
+            raise ValueError('y must have one value per input')
+        samples, smf = self._filter_batch(samples_h)
+        if joint:
+            lp, lp_s, white = self._with_frozen_stats(lambda: self.engine.predict_logpdf(
+                self._pack(), t, y, samples, smf=smf, reg=config.reg, noise=noise, white=per_sample))
+            return (lp, lp_s, white) if per_sample else lp
+        p = self._pack()
+        _, _, mean, var = self._with_frozen_stats(
+            lambda: self.engine.predict_f_batch(p, t, samples, smf=smf, reg=config.reg))
+        v = var + (np.exp(p[0]) if noise else config.reg)
+        bad = np.argwhere(~(v > 0))
+        if bad.size:
+            i, b = bad[0]
+            raise ValueError('predictive variance %g of sample %d at point %d is not positive' % (v[i, b], b, i))
+        lp_s = -.5 * (np.log(2 * np.pi * v) + (y[:, None] - mean) ** 2 / v)
+        # log mean_b exp(lp_s[:, b]), shifted by the largest term and added in ascending b
+        top = lp_s.max(1)
+        acc = np.zeros(t.shape[0])
+        for b in range(lp_s.shape[1]):
+            acc += np.exp(lp_s[:, b] - top)
+        lp = top + np.log(acc) - np.log(lp_s.shape[1])
+        return (lp, lp_s) if per_sample else lp
+
     def predict_k(self, t, samples_h=200, psd=False, normalise=True):
         """Predict the kernel, or the PSD via the kernel approximation, at lags ``t``
         (``src/core/cgpcm.py:610-661``): Monte-Carlo over filter samples (numeric ``samples_h``: draws from q(u)).

@@ -3079,12 +3079,16 @@ int pcov_tile(const cgpcm_handle* h) {
 //   per tile    of P x Q points with p >= q: the fold A*_p^T T_q (one GEMM), the pair blocks Bxx* (axx_pair_kernel), the
 //               centre statistics at the tile's lags (ahh_center_kernel) and, per batch, <Ahh_c, hh_b - iKh> (GEMM),
 //               <Bxx*, mx_b> (predict_qb_kernel) and pcov_finish_kernel;
-//   then        cov += C_b / B in ascending b, and per sample chol(C_b + reg I) (identity on the padding) and the draw.
+//   then        cov += C_b / B in ascending b, and per sample chol(C_b + reg I) (identity on the padding) and the draw;
+//   scoring     (y_host given, cgpcm_predict_logpdf) per sample the bordered K_b = [[C_b + d I, y - m_b], [.., c]]
+//               (pcov_border_kernel), its Cholesky factor, and per group pcov_score_kernel: lp_s[b] and the whitened
+//               residuals; d = s2 with noise = 1 (observations), reg with noise = 0 (f itself).
 // Every launch is shaped by the handle, n_star and the internal batch size, and no sum runs across samples except cov,
-// so a sample's mean, C_b and draw are bitwise the same in any batch and at any position.
+// so a sample's mean, C_b, draw, lp_s and whitened residuals are bitwise the same in any batch and at any position.
 int predict_cov_run(cgpcm_handle* h, const double* params_host, double reg, const double* tstar_host, long n_star,
                     const double* samples_host, int B, int smf, const double* noise_host, double* mean_s_out,
-                    double* cov_s_out, double* cov_out, double* draws_out) {
+                    double* cov_s_out, double* cov_out, double* draws_out, const double* y_host, int noise,
+                    double* lp_s_out, double* white_out) {
   const int nh = h->nh, nx = h->nx, nhp = h->nhp, nxp = h->nxp;
   const long ld = h->ld, l2 = ld * ld;
   const long np = 5 + nh + (long)nh * (nh + 1) / 2;
@@ -3092,8 +3096,13 @@ int predict_cov_run(cgpcm_handle* h, const double* params_host, double reg, cons
   if (check_finite(h, tstar_host, n_star, "non-finite test input")) return -4;
   if (check_samples(h, samples_host, B, nh)) return -4;
   if (noise_host && check_finite(h, noise_host, n_star * B, "non-finite noise")) return -4;
-  if (!h->frozen) { h->err = "cgpcm_predict_f_cov requires cgpcm_precompute"; return -1; }
+  if (y_host && check_finite(h, y_host, n_star, "non-finite y_star")) return -4;
+  if (!h->frozen) {
+    h->err = y_host ? "cgpcm_predict_logpdf requires cgpcm_precompute" : "cgpcm_predict_f_cov requires cgpcm_precompute";
+    return -1;
+  }
   const bool want_draws = draws_out && noise_host;
+  const bool want_score = y_host != nullptr;
   const Hyp hp = hyp_of(params_host);
   const double r = hp.r, c0 = hp.c0, s2f = hp.s2f, alpha = hp.alpha, gamma = hp.gamma;
   if (ensure_sweep_buffers(h)) return -2;
@@ -3114,7 +3123,10 @@ int predict_cov_run(cgpcm_handle* h, const double* params_host, double reg, cons
   const int nhl = round_up(nh, 2);
   const long KH = (long)nh * nhl;
   const int bcap = predict_bcap(h);
-  const double per = 8.0 * ((double)n2 + (double)KH + (double)nxp * nxp + (smf ? (double)l2 : 0.0));
+  const int ldk = round_up(n + 1, 8);    // the bordered matrix of the scoring stage
+  const long k2 = (long)ldk * ldk;
+  const double per = 8.0 * ((double)n2 + (double)KH + (double)nxp * nxp + (smf ? (double)l2 : 0.0) +
+                            (want_score ? (double)k2 : 0.0));
   const int gcap = std::max(bcap, std::min(round_up(B, bcap), (int)std::min(1e6, 4e9 / per) / bcap * bcap));
   const int nq = smf ? gcap : 1;         // q(z) slabs held at a time
   long wcols = 0;
@@ -3135,8 +3147,11 @@ int predict_cov_run(cgpcm_handle* h, const double* params_host, double reg, cons
   const size_t o_v = s.take((size_t)bcap * acols), o_y = s.take(acols);
   const size_t o_quad = s.take((size_t)npad * bcap), o_lin = s.take((size_t)npad * bcap);
   const size_t o_k = s.take(want_draws ? n2 : 0), o_f = s.take(want_draws ? npad : 0);
+  const size_t o_ys = s.take(want_score ? n : 0), o_kb = s.take(want_score ? (size_t)gcap * k2 : 0);
+  const size_t o_lps = s.take(want_score ? B : 0), o_white = s.take(want_score && white_out ? (size_t)n * B : 0);
   const size_t o_info = s.take(gcap + bcap, sizeof(int));
   CK(s.alloc());
+  double *d_ys = s.at(o_ys), *d_kb = s.at(o_kb), *d_lps = s.at(o_lps), *d_white = s.at(o_white);
   double *d_t = s.at(o_t), *d_A = s.at(o_a), *d_TA = s.at(o_ta), *d_mean = s.at(o_mean), *d_draw = s.at(o_draw);
   double *d_noise = s.at(o_noise), *d_cov = s.at(o_cov), *d_x = s.at(o_x), *d_g = s.at(o_g), *d_ac = s.at(o_ac);
   double *d_lag = s.at(o_lag), *d_AC = s.at(o_AC), *d_gf = s.at(o_gf), *d_qp = s.at(o_qp), *d_hs = s.at(o_hs);
@@ -3145,10 +3160,12 @@ int predict_cov_run(cgpcm_handle* h, const double* params_host, double reg, cons
   double *d_v = s.at(o_v), *d_y = s.at(o_y), *d_quad = s.at(o_quad), *d_lin = s.at(o_lin), *d_k = s.at(o_k);
   double* d_f = s.at(o_f);
   int* d_info = s.at<int>(o_info);
-  int* d_pinfo = d_info + bcap;          // per sample of the group: the factorisation of C_b + reg I
+  int* d_pinfo = d_info + bcap;          // per sample of the group: the factorisation of C_b + reg I, or of K_b
   if (begin_run(h)) return -2;
   CK(cudaMemcpyAsync(h->params_d, params_host, np * sizeof(double), cudaMemcpyHostToDevice, st));
   CK(cudaMemcpyAsync(d_t, tstar_host, n * sizeof(double), cudaMemcpyHostToDevice, st));
+  if (want_score) CK(cudaMemcpyAsync(d_ys, y_host, n * sizeof(double), cudaMemcpyHostToDevice, st));
+  const double d_add = noise ? hp.s2 : reg;    // S_b = C_b + d_add I
   if (cov_out) CK(cudaMemsetAsync(d_cov, 0, (size_t)n2 * sizeof(double), st));
   std::vector<double> noise_t;
   if (want_draws) {
@@ -3316,6 +3333,48 @@ int predict_cov_run(cgpcm_handle* h, const double* params_host, double reg, cons
       for (int b = 0; b < gn; ++b)
         if (inf[b]) return sample_pd_error(h, "C_b + reg I", g0 + b, inf[b] % 100000);
     }
+    if (want_score) {
+      CK(cudaMemsetAsync(d_pinfo, 0, (size_t)gn * sizeof(int), st));
+      pcov_border_kernel<<<148 * 8, 256, 0, st>>>(d_c, npad, n2, d_mean + g0, B, d_ys, n, d_add, gn, d_kb, ldk, k2);
+      L(h);
+      for (int b = 0; b < gn; ++b) {
+        cudaError_t e = potrf_lower(st, d_kb + (long)b * k2, ldk, ldk, d_pinfo + b, 8, h->M(M_XW));
+        L(h, 2 * ((ldk + LA_NB - 1) / LA_NB));
+        if (e != cudaSuccess) { h->err = "potrf launch failed"; return -2; }
+      }
+      pcov_score_kernel<<<gn, 256, 0, st>>>(d_kb, ldk, k2, n, d_lps + g0, white_out ? d_white + g0 : nullptr, B);
+      L(h);
+      CK(cudaMemcpyAsync(inf.data(), d_pinfo, (size_t)gn * sizeof(int), cudaMemcpyDeviceToHost, st));
+      CK(cudaStreamSynchronize(st));
+      for (int b = 0; b < gn; ++b) {
+        if (!inf[b]) continue;
+        int piv = inf[b] % 100000;
+        if (piv == n + 1) {
+          // The border pivot: potrf reports the last failed pivot of a panel, and a failed pivot of S_b can leave a
+          // non-finite z_b.  Factor S_b with an identity border so that the message names its own pivot.
+          CK(cudaMemsetAsync(d_pinfo + b, 0, sizeof(int), st));
+          pcov_border_kernel<<<148 * 8, 256, 0, st>>>(d_c + (long)b * n2, npad, n2, d_mean + g0 + b, B, nullptr, n,
+                                                      d_add, 1, d_kb + (long)b * k2, ldk, k2);
+          L(h);
+          cudaError_t e = potrf_lower(st, d_kb + (long)b * k2, ldk, ldk, d_pinfo + b, 8, h->M(M_XW));
+          if (e != cudaSuccess) { h->err = "potrf launch failed"; return -2; }
+          CK(cudaMemcpyAsync(&piv, d_pinfo + b, sizeof(int), cudaMemcpyDeviceToHost, st));
+          CK(cudaStreamSynchronize(st));
+          piv %= 100000;
+          if (!piv) {           // S_b is positive definite and |z_b|^2 overflows
+            char m[120];
+            snprintf(m, sizeof m, "the whitened residual of sample %d overflows", g0 + b);
+            h->err = m;
+            return -3;
+          }
+        }
+        return sample_pd_error(h, "C_b + d I", g0 + b, piv);
+      }
+    }
+  }
+  if (want_score) {
+    if (lp_s_out) CK(cudaMemcpyAsync(lp_s_out, d_lps, (size_t)B * sizeof(double), cudaMemcpyDefault, st));
+    if (white_out) CK(cudaMemcpyAsync(white_out, d_white, (size_t)n * B * sizeof(double), cudaMemcpyDefault, st));
   }
   if (mean_s_out) CK(cudaMemcpyAsync(mean_s_out, d_mean, (size_t)n * B * sizeof(double), cudaMemcpyDefault, st));
   if (want_draws) CK(cudaMemcpyAsync(draws_out, d_draw, (size_t)n * B * sizeof(double), cudaMemcpyDefault, st));
@@ -3436,7 +3495,38 @@ int cgpcm_predict_f_cov(cgpcm_handle* h, const double* params, double reg, const
     return -2;
   if (draws && to_host(h, noise, (long)n_star * n_samples, ns)) return -2;
   return predict_cov_run(h, host.data(), reg, ts.data(), n_star, smp.data(), n_samples, smf ? 1 : 0,
-                         draws ? ns.data() : nullptr, mean_s, cov_s, cov, draws);
+                         draws ? ns.data() : nullptr, mean_s, cov_s, cov, draws, nullptr, 0, nullptr, nullptr);
+}
+
+int cgpcm_predict_logpdf(cgpcm_handle* h, const double* params, double reg, const double* t_star,
+                         const double* y_star, int64_t n_star, const double* samples, int32_t n_samples, int32_t smf,
+                         int32_t noise, double* lp, double* lp_s, double* white) {
+  if (!h || !params || n_star < 0 || !samples || (n_star > 0 && (!t_star || !y_star))) return -1;
+  if (n_samples < 1) { h->err = "n_samples must be >= 1"; return -1; }
+  if (n_star > 4096) { h->err = "predict_logpdf: at most 4096 test inputs"; return -1; }
+  if (noise != 0 && noise != 1) { h->err = "predict_logpdf: noise must be 0 or 1"; return -1; }
+  if (int rc = check_call(h, h->t, reg)) return rc;
+  if (!h->frozen) { h->err = "cgpcm_predict_logpdf requires cgpcm_precompute"; return -1; }
+  CK(cudaSetDevice(h->device));
+  std::vector<double> lps(n_samples, 0.0);
+  if (n_star > 0) {
+    const long np = 5 + h->nh + (long)h->nh * (h->nh + 1) / 2;
+    std::vector<double> host, ts, ys, smp;
+    if (to_host(h, params, np, host) || to_host(h, t_star, n_star, ts) || to_host(h, y_star, n_star, ys) ||
+        to_host(h, samples, (long)n_samples * h->nh, smp))
+      return -2;
+    if (int rc = predict_cov_run(h, host.data(), reg, ts.data(), n_star, smp.data(), n_samples, smf ? 1 : 0, nullptr,
+                                 nullptr, nullptr, nullptr, nullptr, ys.data(), noise, lps.data(), white))
+      return rc;
+  }
+  // log (1 / B) sum_b exp(lp_s[b]), shifted by the largest term and added in ascending b
+  double mx = lps[0];
+  for (double v : lps) mx = std::max(mx, v);
+  double acc = 0.0;
+  for (double v : lps) acc += exp(v - mx);
+  const double mix = mx + log(acc) - log((double)n_samples);
+  if (put(h, lp, &mix, 1) || put(h, lp_s, lps.data(), n_samples)) return -2;
+  return 0;
 }
 
 int cgpcm_kernel_samples(cgpcm_handle* h, const double* params, double reg, const double* t, int64_t n,

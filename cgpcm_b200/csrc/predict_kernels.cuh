@@ -7,6 +7,7 @@
 // so that per sample and point only  v = Ahx*_n^T h,  v^T mx v  and  <Bxx*_n, mx>  remain:
 //     m2_n = s2_f (a + h^T Ahh h - tr(Ahh iKh) + <Bxx*_n, mx> + v^T mx v).
 #pragma once
+#include <cfloat>
 #include <cuda_runtime.h>
 
 #include "dgemm_dmma.cuh"
@@ -369,6 +370,62 @@ __global__ void pcov_finish_kernel(const double* __restrict__ qpart, int nrow, i
     Cb[(long)p * ldc + q] = v;
     Cb[(long)q * ldc + p] = v;
   }
+}
+
+// ---- Held-out scoring (cgpcm_predict_logpdf): log N(y; m_b, S_b), S_b = C_b + d I, through one Cholesky factorisation
+// of the bordered matrix
+//     K_b = [[S_b, r_b], [r_b^T, c]],   r_b = y - m_b,   L_K = [[L_b, 0], [z_b^T, l]],   L_b L_b^T = S_b,  z_b = L_b^-1 r_b
+// so that the factor's last row is the whitened residual and its first n diagonal entries give log det S_b.  c = DBL_MAX:
+// the border pivot c - |z_b|^2 is positive for any finite z_b short of overflow, so the factorisation fails only where
+// S_b does (a bound from d, such as c = 1 + 2 |r|^2 / d, needs d > 0, and d = reg = 0 is allowed), and nothing is ever
+// read from that pivot (c - l^2 would cancel).  Rows and columns past n + 1 are the identity.
+
+// K[b] (ldk x ldk, k2 apart) for samples b < nb of C (npad x npad, n2 apart) and the means m[p * ldm + b]; y == nullptr
+// writes r = 0 and c = 1 (S_b with an identity border).  Grid-stride, any grid.
+__global__ void pcov_border_kernel(const double* __restrict__ C, int npad, long n2, const double* __restrict__ m,
+                                   long ldm, const double* __restrict__ y, int n, double d, int nb,
+                                   double* __restrict__ K, int ldk, long k2) {
+  const long total = (long)nb * k2;
+  for (long idx = (long)blockIdx.x * blockDim.x + threadIdx.x; idx < total; idx += (long)gridDim.x * blockDim.x) {
+    const int b = (int)(idx / k2);
+    const long e = idx - (long)b * k2;
+    const int i = (int)(e / ldk), j = (int)(e - (long)i * ldk);
+    double v = (i == j) ? 1.0 : 0.0;
+    if (i < n && j < n) v = C[(long)b * n2 + (long)i * npad + j] + (i == j ? d : 0.0);
+    else if (i == n && j == n) v = y ? DBL_MAX : 1.0;
+    else if (i == n && j < n) v = y ? y[j] - m[(long)j * ldm + b] : 0.0;
+    else if (j == n && i < n) v = y ? y[i] - m[(long)i * ldm + b] : 0.0;
+    K[idx] = v;
+  }
+}
+
+// One CTA (256 threads) per sample b < gridDim.x of the factored K[b]: logdet = 2 sum log L_ii and q = sum z_i^2, each
+// thread over i = tid, tid + 256, .. in order, then a fixed tree; lp[b] = -(n log 2 pi + logdet + q) / 2 and
+// white[p * ldw + b] = z_p.
+__global__ void __launch_bounds__(256) pcov_score_kernel(const double* __restrict__ K, int ldk, long k2, int n,
+                                                         double* __restrict__ lp, double* __restrict__ white, long ldw) {
+  __shared__ double sl[256], sq[256];
+  const int b = blockIdx.x, tid = threadIdx.x;
+  const double* Kb = K + (long)b * k2;
+  const double* z = Kb + (long)n * ldk;
+  double l = 0.0, q = 0.0;
+  for (int i = tid; i < n; i += 256) {
+    const double zi = z[i];
+    l += log(Kb[(long)i * ldk + i]);
+    q += zi * zi;
+    if (white) white[(long)i * ldw + b] = zi;
+  }
+  sl[tid] = l;
+  sq[tid] = q;
+  __syncthreads();
+  for (int s = 128; s > 0; s >>= 1) {
+    if (tid < s) {
+      sl[tid] += sl[tid + s];
+      sq[tid] += sq[tid + s];
+    }
+    __syncthreads();
+  }
+  if (tid == 0) lp[b] = -0.5 * (n * 1.83787706640934548356 + 2.0 * sl[0] + sq[0]);    // log 2 pi
 }
 
 }  // namespace cg

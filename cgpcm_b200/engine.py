@@ -210,6 +210,30 @@ class Engine(object):
                                                      _lib.ptr(cov_s), _lib.ptr(cov), _lib.ptr(noise), _lib.ptr(draws)))
         return mean_s.mean(1), cov, mean_s, cov_s, draws
 
+    def predict_logpdf(self, params, t_star, y_star, samples, smf=True, reg=1e-8, noise=True, white=False):
+        """Joint log predictive density of the block ``y_star`` at ``t_star`` (at most 4096 inputs) for every filter
+        sample ([B, nh]) in one call: ``(lp, lp_s[B], white_s[n, B] or None)``.  ``lp_s[b] = log N(y_star; m_b, C_b +
+        d I)`` with ``m_b``, ``C_b`` the mean and covariance of :meth:`predict_f_cov` (``smf`` as there) and ``d`` the
+        noise variance ``s2`` (``noise=True``: ``y_star`` are observations) or ``reg`` (``noise=False``: ``y_star`` is
+        f itself); ``lp`` is the log density under the mixture of the samples, ``log mean_b exp(lp_s[b])``.
+        ``white=True`` also returns the whitened residuals ``L_b^-1 (y_star - m_b)``, ``L_b L_b^T = C_b + d I``.  A
+        sample's ``lp_s`` and residuals do not depend on the other samples of the call; needs the frozen statistics."""
+        t_star = np.ascontiguousarray(np.asarray(t_star, dtype=np.float64).ravel())
+        y_star = np.ascontiguousarray(np.asarray(y_star, dtype=np.float64).ravel())
+        samples = np.ascontiguousarray(np.asarray(samples, dtype=np.float64))
+        if samples.ndim == 1:
+            samples = samples.reshape(1, -1)
+        if samples.ndim != 2 or samples.shape[1] != self.nh or samples.shape[0] < 1 or \
+                int(params.shape[0]) != n_params(self.nh) or y_star.shape != t_star.shape:
+            raise ValueError('shape mismatch in predict_logpdf')
+        n, B = t_star.shape[0], samples.shape[0]
+        lp, lp_s = np.empty(1), np.empty(B)
+        white_s = np.empty((n, B)) if white else None
+        self._ck(_lib.lib().cgpcm_predict_logpdf(self._h, _lib.ptr(params), float(reg), _lib.ptr(t_star),
+                                                  _lib.ptr(y_star), n, _lib.ptr(samples), B, int(bool(smf)),
+                                                  int(bool(noise)), _lib.ptr(lp), _lib.ptr(lp_s), _lib.ptr(white_s)))
+        return float(lp[0]), lp_s, white_s
+
     def kernel_samples(self, params, t, samples, reg=1e-8):
         """Kernel samples ``k[n, b]`` of ``predict_k`` at lags ``t`` for filter ``samples`` ([B, nh])
         (``src/core/cgpcm.py:610-634``), before normalisation."""

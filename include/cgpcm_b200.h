@@ -185,6 +185,27 @@ int cgpcm_predict_f_cov(cgpcm_handle* h, const double* params, double reg, const
                         const double* samples, int32_t n_samples, int32_t smf, double* mean_s, double* cov_s,
                         double* cov, const double* noise, double* draws);
 
+/* Held-out scoring: the log predictive density of a block y_star[n_star] at the test inputs t_star, n_star <= 4096,
+ * per filter sample and for the mixture of the samples.  For sample b, with m_b and C_b the mean and covariance of f of
+ * cgpcm_predict_f_cov (smf as there) and S_b = C_b + d I, d = s2 = exp(params[0]) when noise = 1 (y_star are
+ * observations) and d = reg when noise = 0 (y_star is f itself):
+ *   lp_s[b]                      log N(y_star; m_b, S_b) = -(n log 2 pi + log det S_b + |z_b|^2) / 2,
+ *                                z_b = L_b^-1 (y_star - m_b), L_b L_b^T = S_b;
+ *   lp[0]                        log ((1 / n_samples) sum_b exp(lp_s[b])), a log-sum-exp shifted by the largest lp_s
+ *                                and added in ascending b (finite however negative the lp_s are);
+ *   white[p * n_samples + b]     z_b[p], the whitened residuals (standard normal when y_star is drawn from the
+ *                                sample's predictive distribution).
+ * One Cholesky factorisation per sample of the bordered matrix [[S_b, y - m_b], [(y - m_b)^T, c]] gives log det S_b and
+ * z_b together.  Every output may be NULL; host or device pointers.  Internal batch sizes depend on the handle's shape
+ * and n_star only and no sum runs across samples except lp: a sample's lp_s and whitened residuals are bitwise the same
+ * in any batch and at any position.  Uses the statistics frozen by cgpcm_precompute (-1 otherwise); -1 when n_samples
+ * < 1, n_star > 4096 or noise is not 0 or 1; -4 for a non-finite parameter, sample, test input or y_star; -3 when some
+ * P_b or some C_b + d I is not positive definite (cgpcm_last_error names the sample and the pivot); n_star = 0 writes
+ * lp = 0 and lp_s = 0 (the empty block has density 1). */
+int cgpcm_predict_logpdf(cgpcm_handle* h, const double* params, double reg, const double* t_star,
+                         const double* y_star, int64_t n_star, const double* samples, int32_t n_samples, int32_t smf,
+                         int32_t noise, double* lp, double* lp_s, double* white);
+
 /* The Monte-Carlo kernel samples of mod.predict_k(t, samples_h) (src/core/cgpcm.py:610-634; centre statistics
  * _a_center / _Ahh_center :164-166,190-192), before normalisation / FFT / percentiles (host post-processing):
  * out[p * n_samples + b] = s2_f (a_c(t_p) + tr((h_b h_b^T - iKh) Ahh_c(t_p))) for lags t[n] and filter samples
