@@ -24,7 +24,8 @@ EXPORTS = ['cgpcm_create', 'cgpcm_destroy', 'cgpcm_last_error', 'cgpcm_device_co
            'cgpcm_set_data', 'cgpcm_set_option', 'cgpcm_psi', 'cgpcm_precompute', 'cgpcm_frozen_mats', 'cgpcm_elbo_grad', 'cgpcm_elbo_smf', 'cgpcm_elbo_smf_batch', 'cgpcm_predict_f', 'cgpcm_predict_f_batch', 'cgpcm_predict_f_cov', 'cgpcm_predict_logpdf', 'cgpcm_kernel_samples', 'cgpcm_filter_samples', 'cgpcm_akm_sample', 'cgpcm_fpi', 'cgpcm_fpi_qz', 'cgpcm_elbo_qz',
            'cgpcm_last_timing', 'cgpcm_bvn_cdf', 'cgpcm_dgemm', 'cgpcm_dgemm_tri', 'cgpcm_dgemm_sym', 'cgpcm_cholinv', 'cgpcm_math_test', 'cgpcm_math_test_fast',
            'cgpcm_smf_c1_test', 'cgpcm_smf_algebra_test', 'cgpcm_smf_posterior_test', 'cgpcm_predict_quad_test',
-           'cgpcm_predict_pair_test']
+           'cgpcm_predict_pair_test', 'cgpcm_ahx_gen_test', 'cgpcm_ahx_dot_test', 'cgpcm_axx_sum_test',
+           'cgpcm_window_chol_test', 'cgpcm_sym_accum_test']
 
 
 def _sources():
@@ -107,6 +108,13 @@ def lib():
                                            dbl, dp, dp, dp, vp, vp]
     L.cgpcm_predict_quad_test.argtypes = [dp, i64, i32, dp, i64, dp, i64, dp, i32, i32, i32, i32, dp, dp, dp, vp]
     L.cgpcm_predict_pair_test.argtypes = [dp, i32, dp, i32, dp, i32, dp, i32, i32, dp, i64, i32, dp, vp]
+    L.cgpcm_ahx_gen_test.argtypes = [dp, dp, i32, i32, dp, i32, i32, dp, i32, i32, i32, dp, i32, i32, dbl, i32, i64, dp,
+                                     dp, vp]
+    L.cgpcm_ahx_dot_test.argtypes = [dp, dp, i32, i32, dp, i32, i32, dp, i32, i32, i32, dp, i32, i32, dbl, i32, i64, dp,
+                                     dp, dp, dp, vp]
+    L.cgpcm_axx_sum_test.argtypes = [dp, i32, i32, dp, i32, dp, i32, i32, dbl, i32, i32, i64, dp, vp]
+    L.cgpcm_window_chol_test.argtypes = [dp, i64, dbl, i32, dp, i32, dp, ctypes.POINTER(i32), vp]
+    L.cgpcm_sym_accum_test.argtypes = [i32, dp, dp, dp, i32, i64, dp, vp]
     for name in EXPORTS:
         if name != 'cgpcm_last_error':
             getattr(L, name).restype = ctypes.c_int

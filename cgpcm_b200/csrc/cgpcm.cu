@@ -541,23 +541,26 @@ cudaEvent_t prof_event(cgpcm_handle* h, int kind) {
   return h->pev[h->pev_used++];
 }
 
+// GEMM flop counters of one dgemm launch.  executed: the CTA tiles this launch computes (tiles strictly above the
+// diagonal are skipped when lower); algorithmic: M x N cells, or the M (M + 1) / 2 cells of the lower triangle of a
+// symmetric result
+void gemm_count(cgpcm_handle* h, int Mr, int Nr, int K, int lower) {
+  const int bm = pick_bm(Mr);
+  double cells = 0.0;
+  for (int m0 = 0; m0 < Mr; m0 += bm)
+    for (int n0 = 0; n0 < Nr; n0 += G_BN) {
+      if (lower && n0 > m0 + bm - 1) continue;
+      cells += (double)std::min(bm, Mr - m0) * std::min(G_BN, Nr - n0);
+    }
+  h->gemm_flops_exec += 2.0 * cells * K;
+  h->gemm_flops += 2.0 * K * ((lower && Mr == Nr) ? 0.5 * Mr * (Mr + 1.0) : (double)Mr * Nr);
+}
+
 int gemm(cgpcm_handle* h, bool a_kc, bool b_kc, bool c_tr, int Mr, int Nr, int K, double alpha, const double* A,
          long lda, const double* B, long ldb, double beta, double* C, long ldc, int splits = 1, long stride = 0,
          int lower = 0) {
-  {
-    // executed: the CTA tiles this launch computes (tiles strictly above the diagonal are skipped when lower);
-    // algorithmic: M x N cells, or the M (M + 1) / 2 cells of the lower triangle of a symmetric result
-    const int bm = pick_bm(Mr);
-    double cells = 0.0;
-    for (int m0 = 0; m0 < Mr; m0 += bm)
-      for (int n0 = 0; n0 < Nr; n0 += G_BN) {
-        if (lower && n0 > m0 + bm - 1) continue;
-        cells += (double)std::min(bm, Mr - m0) * std::min(G_BN, Nr - n0);
-      }
-    h->gemm_flops_exec += 2.0 * cells * K;
-    h->gemm_flops += 2.0 * K * ((lower && Mr == Nr) ? 0.5 * Mr * (Mr + 1.0) : (double)Mr * Nr);
-    h->gemm_launches++;
-  }
+  gemm_count(h, Mr, Nr, K, lower);
+  h->gemm_launches++;
   prof_gemm_begin(h);
   cudaError_t e;
   if (h->sl_opt && a_kc && b_kc == c_tr && splits <= 1 && !lower && beta == 0.0 && dgemm_sl_supported(Mr, Nr, K))
@@ -758,43 +761,120 @@ int ensure_ws(cgpcm_handle* h) {
 
 // ---- sweeps ---------------------------------------------------------------------------------------
 
-// sum_n Axx (and tangents) over this rank's observations -> M_AXX0..3
-int axx_sweep(cgpcm_handle* h, const PsiConst& c, const BvnTab& T, bool tangents, double* out4) {
-  const int nt = (h->nx + AXX_TILE - 1) / AXX_TILE;
+// ---- launches of the sweeps' kernels (handle-free: the sweeps and the C-ABI test hooks share them) -----------------
+
+// sum_n Axx (and tangents) of the n observations t -> out4 (1 or 4 ld x ld matrices): axx_sum_kernel into the slice
+// partials part ([slices][4][ld][ld]), then axx_reduce_kernel.  cheb: device room for the Chebyshev table of the
+// pair-hoisted branch.  Two launches.
+cudaError_t axx_launch(cudaStream_t st, const double* t, int n, bool sorted, const double* tx, int nx, double* part,
+                       long ld, int slices, const PsiConst& c, const BvnTab& T, double* cheb, bool tangents,
+                       double* out4) {
+  const int nt = (nx + AXX_TILE - 1) / AXX_TILE;
   const int ntiles = nt * nt;        // 16 inducing inputs x 16 separations per tile (psi_kernels.cuh)
   // pair-hoisted Genz branch: causal model, rho >= 0.925 (rho = gamma / A is always positive here)
   const bool hoist = c.causal && !c.causal_id && T.high && T.rho > 0.0 && T.as_ > 0.0 && T.ng == 20;
+  dim3 grid(ntiles, slices);
+  int deg = 0;
+  size_t smem = 0;
+  if (hoist) {
+    double B[(BVN_CHEB_MAXDEG + 1) * 20];
+    deg = bvn_make_cheb(T, B);
+    cudaError_t e = cudaMemcpyAsync(cheb, B, (size_t)(deg + 1) * 20 * sizeof(double), cudaMemcpyHostToDevice, st);
+    if (e != cudaSuccess) return e;
+    smem = (size_t)(deg + 1) * (20 + BVN_PAIR_THREADS) * sizeof(double);
+    static DeviceOnce attr_once;
+    unsigned long long attr_bit;
+    if (attr_once.need(&attr_bit)) {
+      const int mx = (BVN_CHEB_MAXDEG + 1) * (20 + BVN_PAIR_THREADS) * 8;
+      cudaFuncSetAttribute((const void*)axx_sum_kernel<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, mx);
+      cudaFuncSetAttribute((const void*)axx_sum_kernel<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, mx);
+      attr_once.done(attr_bit);
+    }
+  }
+#define CG_AXX(TG, HO) \
+  axx_sum_kernel<TG, HO><<<grid, 256, smem, st>>>(t, n, sorted ? 1 : 0, tx, nx, part, ld, c, T, cheb, deg)
+  if (tangents) { if (hoist) CG_AXX(true, true); else CG_AXX(true, false); }
+  else { if (hoist) CG_AXX(false, true); else CG_AXX(false, false); }
+#undef CG_AXX
+  axx_reduce_kernel<<<148 * 4, 256, 0, st>>>(part, slices, tangents ? 4 : 1, ld, nx, out4);
+  return cudaGetLastError();
+}
+
+// A[(i*nc + n)*kwp + k] = Ahx of the chunk's observations t[0 .. nv) at the window k_lo + k (ahx_gen_sep_kernel when
+// `sep`: default causal model only), and when Ypart != NULL the slice partials of sum_n y_n A.  One launch.
+void ahx_gen_launch(cudaStream_t st, bool sep, const double* t, const double* y, int nv, int nc, const double* th, int nh,
+                    int nhp, const double* tx, int nx, int k_lo, int kwp, double* A, double* Ypart, long ldy,
+                    long ypart_stride, const PsiConst& c) {
+  const int threads = std::min(256, round_up(kwp, 32));
+  dim3 grid(nhp, (nc + AHX_NSUB - 1) / AHX_NSUB);
+  if (sep) {
+    // default causal model: separable form, AHX_IB filter rows per CTA (psi_kernels.cuh)
+    grid.x = (nhp + AHX_IB - 1) / AHX_IB;
+    ahx_gen_sep_kernel<<<grid, threads, 0, st>>>(t, y, nv, nc, th, nh, nhp, tx, nx, k_lo, kwp, A, Ypart, ldy,
+                                                 ypart_stride, c);
+  } else {
+    ahx_gen_kernel<<<grid, threads, 0, st>>>(t, y, nv, nc, th, nh, tx, nx, k_lo, kwp, A, Ypart, ldy, ypart_stride, c);
+  }
+}
+
+// gpart[(slice * grid.x + cta) * 3 + theta] += sum (W + y Ybar) dA/dtheta over the chunk's block (ahx_dot_sep_kernel
+// when `sep`).  One launch.
+void ahx_dot_launch(cudaStream_t st, bool sep, const double* t, const double* y, int nv, int nc, const double* th, int nh,
+                    int nhp, const double* tx, int nx, int k_lo, int kwp, const double* A, const double* W,
+                    const double* Ybar, long ldy, double* gpart, const PsiConst& c) {
+  const int threads = std::min(256, round_up(kwp, 32));
+  dim3 grid(nhp, (nc + AHX_NSUB - 1) / AHX_NSUB);
+  if (sep) {
+    grid.x = (nhp + AHX_IB - 1) / AHX_IB;
+    ahx_dot_sep_kernel<<<grid, threads, 0, st>>>(t, y, nv, nc, th, nh, tx, nx, k_lo, kwp, A, W, Ybar, ldy, gpart, c);
+  } else {
+    ahx_dot_kernel<<<grid, threads, 0, st>>>(t, y, nv, nc, th, nh, tx, nx, k_lo, kwp, A, W, Ybar, ldy, gpart, c);
+  }
+}
+
+// The symmetric contractions' route: orders <= 40 (one warp block) stay on the tiled split-K kernel (154 us against
+// 204 us at the bench shape's cull = 80 window).
+inline bool sym_on_dgemm_sym(bool a_kc, bool b_kc, int Mr) {
+  return a_kc == b_kc && dgemm_sym_supported(Mr) && Mr > SY_BLK;
+}
+
+// Adds the lower triangle of op(A) op(B)^T (Mr x Mr) slice by slice into the K-slice buffers acc (stride ld * ld) at
+// element offset win; *splits = the slices the launch touched.  One launch.
+cudaError_t sym_accum_launch(cudaStream_t st, bool a_kc, bool b_kc, int Mr, int K, const double* A, long lda,
+                             const double* B, long ldb, double* acc, long ld, long win, int* splits) {
+  const long l2 = ld * ld;
+  double* C = acc + win;
+  if (sym_on_dgemm_sym(a_kc, b_kc, Mr)) {
+    *splits = dgemm_sym_splits(K);
+    return dgemm_sym(st, a_kc, Mr, K, A, lda, B, ldb, C, ld, l2, 1);
+  }
+  int s = std::min(pick_splits(Mr, Mr, K, true), SY_MAX_SPLITS);
+  // number of splits actually used by dgemm (it rounds the k range per split up to whole tiles)
+  int kt = (K + G_BK - 1) / G_BK;
+  int kt_per = (kt + s - 1) / s;
+  s = (kt + kt_per - 1) / kt_per;
+  *splits = s;
+  return dgemm(st, a_kc, b_kc, false, Mr, Mr, K, 1.0, A, lda, B, ldb, 1.0, C, ld, s, l2, 1);
+}
+
+// out (n x n at ld) = sum over the first `slices` K-slice buffers, in slice order, mirrored.  One launch.
+void sym_finish_launch(cudaStream_t st, const double* acc, long ld, int slices, int n, double* out) {
+  const long total = (long)n * n;
+  reduce_partials_kernel<<<(int)((total + 255) / 256), 256, 0, st>>>(acc, ld * ld, std::max(1, slices), out, n, n, ld,
+                                                                    ld, 0.0, 1);
+}
+
+// sum_n Axx (and tangents) over this rank's observations -> M_AXX0..3
+int axx_sweep(cgpcm_handle* h, const PsiConst& c, const BvnTab& T, bool tangents, double* out4) {
   // Observation slices (grid.y).  Fewer slices would amortise the per-pair set-up of the hoisted branch over more
   // observations, but measured slower (13 slices: 15.4 ms against 13.7 ms at the bench shape, 2.59 against 2.32 ms on an
   // 8-GPU shard): the per-CTA observation ranges are cut by the windows, and more, smaller CTAs balance better.
   int slices = h->axx_slices_opt > 0 ? h->axx_slices_opt : h->axx_slices;
-  dim3 grid(ntiles, slices);
   if (h->n_local > 0) {
-    int deg = 0;
-    size_t smem = 0;
-    if (hoist) {
-      double B[(BVN_CHEB_MAXDEG + 1) * 20];
-      deg = bvn_make_cheb(T, B);
-      CK(cudaMemcpyAsync(h->cheb_d, B, (size_t)(deg + 1) * 20 * sizeof(double), cudaMemcpyHostToDevice, h->st));
-      smem = (size_t)(deg + 1) * (20 + BVN_PAIR_THREADS) * sizeof(double);
-      static DeviceOnce attr_once;
-      unsigned long long attr_bit;
-      if (attr_once.need(&attr_bit)) {
-        const int mx = (BVN_CHEB_MAXDEG + 1) * (20 + BVN_PAIR_THREADS) * 8;
-        cudaFuncSetAttribute((const void*)axx_sum_kernel<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, mx);
-        cudaFuncSetAttribute((const void*)axx_sum_kernel<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, mx);
-        attr_once.done(attr_bit);
-      }
-    }
-#define CG_AXX(TG, HO)                                                                                            \
-  axx_sum_kernel<TG, HO><<<grid, 256, smem, h->st>>>(h->t, (int)h->n_local, h->t_sorted ? 1 : 0, h->tx, h->nx,    \
-                                                      h->axx_part, h->ld, c, T, h->cheb_d, deg)
-    if (tangents) { if (hoist) CG_AXX(true, true); else CG_AXX(true, false); }
-    else { if (hoist) CG_AXX(false, true); else CG_AXX(false, false); }
-#undef CG_AXX
-    L(h);
-    axx_reduce_kernel<<<148 * 4, 256, 0, h->st>>>(h->axx_part, slices, tangents ? 4 : 1, h->ld, h->nx, out4);
-    L(h);
+    prof_close(h);
+    CK(axx_launch(h->st, h->t, (int)h->n_local, h->t_sorted, h->tx, h->nx, h->axx_part, h->ld, slices, c, T, h->cheb_d,
+                  tangents, out4));
+    h->launches += 2;
   } else {
     zero(h, out4, 4 * h->ld * h->ld);
   }
@@ -823,22 +903,11 @@ int ensure_ypart(cgpcm_handle* h, int slices) {
 
 int gen_chunk(cgpcm_handle* h, const PsiConst& c, const Chunk& ch, bool with_y, double* dstA = nullptr) {
   if (!dstA) dstA = h->wsA;
-  const int threads = std::min(256, round_up(ch.kwp, 32));
-  dim3 grid(h->nhp, (ch.nc + AHX_NSUB - 1) / AHX_NSUB);
-  if ((int)grid.y > h->y_slices) { h->err = "internal: y_slices too small"; return -1; }
+  if ((ch.nc + AHX_NSUB - 1) / AHX_NSUB > h->y_slices) { h->err = "internal: y_slices too small"; return -1; }
   prof_close(h);
   if (h->profile) cudaEventRecord(prof_event(h, 1), h->st);
-  if (c.causal && !c.causal_id && h->sep_opt) {
-    // default causal model: separable form, AHX_IB filter rows per CTA (psi_kernels.cuh)
-    grid.x = (h->nhp + AHX_IB - 1) / AHX_IB;
-    ahx_gen_sep_kernel<<<grid, threads, 0, h->st>>>(h->t + ch.n0, h->y + ch.n0, ch.nv, ch.nc, h->th, h->nh, h->nhp, h->tx,
-                                                    h->nx, ch.k_lo, ch.kwp, dstA, with_y ? h->ypart : nullptr, h->ld,
-                                                    (long)h->nhp * h->ld, c);
-  } else {
-    ahx_gen_kernel<<<grid, threads, 0, h->st>>>(h->t + ch.n0, h->y + ch.n0, ch.nv, ch.nc, h->th, h->nh, h->tx, h->nx,
-                                                ch.k_lo, ch.kwp, dstA, with_y ? h->ypart : nullptr, h->ld,
-                                                (long)h->nhp * h->ld, c);
-  }
+  ahx_gen_launch(h->st, c.causal && !c.causal_id && h->sep_opt, h->t + ch.n0, h->y + ch.n0, ch.nv, ch.nc, h->th, h->nh,
+                 h->nhp, h->tx, h->nx, ch.k_lo, ch.kwp, dstA, with_y ? h->ypart : nullptr, h->ld, (long)h->nhp * h->ld, c);
   if (h->profile) cudaEventRecord(prof_event(h, 1), h->st);
   L(h);
   return 0;
@@ -857,40 +926,28 @@ int sym_begin(cgpcm_handle* h, int slot) {
 
 int gemm_splitk_sym(cgpcm_handle* h, bool a_kc, bool b_kc, int Mr, int K, const double* A, long lda, const double* B,
                     long ldb, int slot, long win) {
-  const long l2 = h->ld * h->ld;
-  double* C = h->symacc[slot] + win;
-  // orders <= 40 (one warp block) stay on the tiled split-K kernel: 154 us against 204 us at the bench shape's cull = 80 window
-  if (a_kc == b_kc && dgemm_sym_supported(Mr) && Mr > SY_BLK) {
-    const int splits = dgemm_sym_splits(K);
+  if (sym_on_dgemm_sym(a_kc, b_kc, Mr)) {
     h->gemm_flops_exec += 2.0 * K * dgemm_sym_cells(Mr);   // full + diagonal warp blocks of the launch's order
     h->gemm_flops += 2.0 * K * 0.5 * Mr * (Mr + 1.0);
-    h->gemm_launches++;
-    prof_gemm_begin(h);
-    cudaError_t e = dgemm_sym(h->st, a_kc, Mr, K, A, lda, B, ldb, C, h->ld, l2, 1);
-    h->launches++;
-    if (e != cudaSuccess) {
-      h->err = std::string("dgemm_sym launch failed: ") + cudaGetErrorString(e);
-      return -2;
-    }
-    h->sym_used[slot] = std::max(h->sym_used[slot], splits);
-    return 0;
+  } else {
+    gemm_count(h, Mr, Mr, K, 1);
   }
-  int splits = std::min(pick_splits(Mr, Mr, K, true), SY_MAX_SPLITS);
-  // number of splits actually used by dgemm (it rounds the k range per split up to whole tiles)
-  int kt = (K + G_BK - 1) / G_BK;
-  int kt_per = (kt + splits - 1) / splits;
-  splits = (kt + kt_per - 1) / kt_per;
-  if (gemm(h, a_kc, b_kc, false, Mr, Mr, K, 1.0, A, lda, B, ldb, 1.0, C, h->ld, splits, l2, 1)) return -2;
+  h->gemm_launches++;
+  prof_gemm_begin(h);
+  int splits = 1;
+  cudaError_t e = sym_accum_launch(h->st, a_kc, b_kc, Mr, K, A, lda, B, ldb, h->symacc[slot], h->ld, win, &splits);
+  h->launches++;
+  if (e != cudaSuccess) {
+    h->err = std::string("symmetric contraction launch failed: ") + cudaGetErrorString(e);
+    return -2;
+  }
   h->sym_used[slot] = std::max(h->sym_used[slot], splits);
   return 0;
 }
 
 int sym_finish(cgpcm_handle* h, int slot, int n, double* out) {
   prof_close(h);
-  const long total = (long)n * n;
-  reduce_partials_kernel<<<(int)((total + 255) / 256), 256, 0, h->st>>>(h->symacc[slot], h->ld * h->ld,
-                                                                        std::max(1, h->sym_used[slot]), out, n, n, h->ld,
-                                                                        h->ld, 0.0, 1);
+  sym_finish_launch(h->st, h->symacc[slot], h->ld, h->sym_used[slot], n, out);
   L(h);
   return 0;
 }
@@ -1062,19 +1119,9 @@ int backward_sweep(cgpcm_handle* h, const PsiConst& c, const std::vector<Chunk>&
       const double* Tb = st ? h->storeT + ch.off : h->wsT;
       if (!st && gemm(h, true, false, false, h->nhp, (int)cols, h->nhp, 1.0, Hm, h->ld, Ab, cols, 0.0, h->wsT, cols)) return -2;
       if (right_mul_sym(h, Tb, h->M(M_WX), ch, h->wsV)) return -2;
-      const int threads = std::min(256, round_up(ch.kwp, 32));
-      dim3 grid(h->nhp, (ch.nc + AHX_NSUB - 1) / AHX_NSUB);
       prof_close(h);
-      if (c.causal && !c.causal_id && h->sep_opt) {
-        grid.x = (h->nhp + AHX_IB - 1) / AHX_IB;
-        ahx_dot_sep_kernel<<<grid, threads, 0, h->st>>>(h->t + ch.n0, h->y + ch.n0, ch.nv, ch.nc, h->th, h->nh, h->tx,
-                                                        h->nx, ch.k_lo, ch.kwp, Ab, h->wsV, h->M(M_YBAR), h->ld,
-                                                        h->gpart, c);
-      } else {
-        ahx_dot_kernel<<<grid, threads, 0, h->st>>>(h->t + ch.n0, h->y + ch.n0, ch.nv, ch.nc, h->th, h->nh, h->tx,
-                                                    h->nx, ch.k_lo, ch.kwp, Ab, h->wsV, h->M(M_YBAR), h->ld, h->gpart,
-                                                    c);
-      }
+      ahx_dot_launch(h->st, c.causal && !c.causal_id && h->sep_opt, h->t + ch.n0, h->y + ch.n0, ch.nv, ch.nc, h->th,
+                     h->nh, h->nhp, h->tx, h->nx, ch.k_lo, ch.kwp, Ab, h->wsV, h->M(M_YBAR), h->ld, h->gpart, c);
       L(h);
     }
   }
@@ -1793,8 +1840,10 @@ int evaluate_once(cgpcm_handle* h, const double* params_host, int mode, uint32_t
       L(h);
     }
     CK(cudaStreamSynchronize(st));
-    // the precomputation factorises Kh, Kx and (option "tri") the window blocks of iKx, reported as Kx
-    static const char* names[] = {"?", "Kh", "Kx", "?", "?", "?", "Kx"};
+    // the precomputation factorises Kh, Kx and (option "tri") the window blocks of iKx; a failed window block (tag 6)
+    // makes evaluate() repeat the precomputation with the full blocks
+    static const char* names[] = {"?", "Kh", "Kx", "?", "?", "?", "iKx (a window block)"};
+    h->last_info_tag = info[0] / 100000;
     if (pd_error(h, info[0], names)) return -3;
     const double Ng = hs[S_COUNT + 0];
     const double a = (h->causal ? 0.5 : 1.0) * sqrt(3.14159265358979323846 / (2.0 * alpha));
@@ -3985,6 +4034,154 @@ int cgpcm_predict_pair_test(const double* tp, int np_, const double* tq, int nq,
   int rc = cudaGetLastError() == cudaSuccess ? 0 : -2;
   if (cudaStreamSynchronize(st) != cudaSuccess) rc = -2;
   return rc;
+}
+
+
+}  // extern "C"
+
+// ---- the sweeps' kernels under test (see the header) ----------------------------------------------------------------
+
+namespace {
+
+int psi_args(const double hyp[3], int causal, int causal_id, double cull, PsiConst* c) {
+  for (int i = 0; i < 3; ++i)
+    if (!std::isfinite(hyp[i]) || hyp[i] <= 0) return -4;
+  if (!std::isfinite(cull) || cull < 0) return -1;
+  psi_make_const(hyp[0], hyp[1], hyp[2], causal ? 1 : 0, cull, c, causal_id);
+  return 0;
+}
+
+bool chunk_ok(int n_valid, int nc, int nh, int nhp, int nx, int k_lo, int kwp, int64_t ld, int causal, int causal_id,
+              int sep) {
+  return n_valid >= 0 && n_valid <= nc && nc >= 8 && nc % 8 == 0 && nh >= 1 && nhp >= nh && nhp % 8 == 0 && nx >= 1 &&
+         kwp >= 8 && kwp % 8 == 0 && k_lo >= 0 && k_lo % 2 == 0 && ld % 8 == 0 && k_lo + kwp <= ld && nx <= ld &&
+         nhp <= ld && (!sep || (causal && !causal_id));
+}
+
+int drain(cudaStream_t st, int rc) {
+  if (cudaGetLastError() != cudaSuccess) rc = -2;
+  if (cudaStreamSynchronize(st) != cudaSuccess) rc = -2;
+  return rc;
+}
+
+}  // namespace
+
+extern "C" {
+
+int cgpcm_ahx_gen_test(const double* t, const double* y, int n_valid, int nc, const double* th, int nh, int nhp,
+                       const double* tx, int nx, int k_lo, int kwp, const double hyp[3], int causal, int causal_id,
+                       double cull, int sep, int64_t ld, double* A, double* ypart, void* stream) {
+  if (!t || !y || !th || !tx || !hyp || !A || !chunk_ok(n_valid, nc, nh, nhp, nx, k_lo, kwp, ld, causal, causal_id, sep))
+    return -1;
+  PsiConst c;
+  if (int rc = psi_args(hyp, causal, causal_id, cull, &c)) return rc;
+  cudaStream_t st = (cudaStream_t)stream;
+  const long ystride = (long)nhp * ld;
+  int rc = 0;
+  if (ypart && cudaMemsetAsync(ypart, 0, (size_t)((nc + AHX_NSUB - 1) / AHX_NSUB) * ystride * sizeof(double), st) !=
+                   cudaSuccess)
+    rc = -2;
+  if (!rc) ahx_gen_launch(st, sep != 0, t, y, n_valid, nc, th, nh, nhp, tx, nx, k_lo, kwp, A, ypart, ld, ystride, c);
+  return drain(st, rc);
+}
+
+int cgpcm_ahx_dot_test(const double* t, const double* y, int n_valid, int nc, const double* th, int nh, int nhp,
+                       const double* tx, int nx, int k_lo, int kwp, const double hyp[3], int causal, int causal_id,
+                       double cull, int sep, int64_t ld, const double* A, const double* W, const double* Ybar,
+                       double* g3, void* stream) {
+  if (!t || !y || !th || !tx || !hyp || !A || !W || !Ybar || !g3 ||
+      !chunk_ok(n_valid, nc, nh, nhp, nx, k_lo, kwp, ld, causal, causal_id, sep))
+    return -1;
+  PsiConst c;
+  if (int rc = psi_args(hyp, causal, causal_id, cull, &c)) return rc;
+  cudaStream_t st = (cudaStream_t)stream;
+  // CTA partials as the backward sweep sizes them: nhp x slices entries of 3
+  const long gneed = (long)nhp * ((nc + AHX_NSUB - 1) / AHX_NSUB);
+  Scratch s;
+  s.take(3 * gneed);
+  if (s.alloc() != cudaSuccess) { cudaGetLastError(); return -2; }
+  double* gpart = s.at(0);
+  int rc = cudaMemsetAsync(gpart, 0, 3 * gneed * sizeof(double), st) == cudaSuccess ? 0 : -2;
+  if (!rc) {
+    ahx_dot_launch(st, sep != 0, t, y, n_valid, nc, th, nh, nhp, tx, nx, k_lo, kwp, A, W, Ybar, ld, gpart, c);
+    sum3_kernel<<<1, 1024, 0, st>>>(gpart, gneed, g3);
+  }
+  return drain(st, rc);
+}
+
+int cgpcm_axx_sum_test(const double* t, int n, int sorted, const double* tx, int nx, const double hyp[3], int causal,
+                       int causal_id, double cull, int slices, int tangents, int64_t ld, double* out4, void* stream) {
+  if (!t || !tx || !hyp || !out4 || n < 1 || nx < 1 || ld < nx || slices < 1 || slices > AXX_MAX_SLICES) return -1;
+  PsiConst c;
+  if (int rc = psi_args(hyp, causal, causal_id, cull, &c)) return rc;
+  BvnTab T;
+  bvn_make_tab(hyp[1] / (hyp[0] + hyp[1] + hyp[2]), &T);
+  cudaStream_t st = (cudaStream_t)stream;
+  Scratch s;
+  const size_t o_part = s.take((size_t)slices * 4 * ld * ld), o_cheb = s.take((BVN_CHEB_MAXDEG + 1) * 20);
+  if (s.alloc() != cudaSuccess) { cudaGetLastError(); return -2; }
+  int rc = axx_launch(st, t, n, sorted != 0, tx, nx, s.at(o_part), ld, slices, c, T, s.at(o_cheb), tangents != 0,
+                      out4) == cudaSuccess ? 0 : -2;
+  return drain(st, rc);
+}
+
+int cgpcm_window_chol_test(const double* M, int64_t ld, double sign, int nwin, const int32_t* windows, int tag,
+                           double* out, int* info_host, void* stream) {
+  if (!M || !windows || !out || !info_host || nwin < 1 || ld < 1 || tag < 0 || tag > 20000) return -1;
+  std::vector<WinDesc> desc(nwin);
+  long off = 0;
+  int kw_max = 8;
+  for (int w = 0; w < nwin; ++w) {
+    const int k_lo = windows[3 * w], kw = windows[3 * w + 1], kv = windows[3 * w + 2];
+    if (kw < 8 || kw > 120 || kw % 8 || kv < 0 || kv > kw || k_lo < 0 || k_lo + kv > ld) return -1;
+    desc[w].k_lo = k_lo; desc[w].kw = kw; desc[w].kv = kv; desc[w].off = off;
+    off += (long)kw * kw;
+    kw_max = std::max(kw_max, kw);
+  }
+  cudaStream_t st = (cudaStream_t)stream;
+  Scratch s;
+  const size_t o_desc = s.take(nwin * sizeof(WinDesc), 1), o_info = s.take(1, sizeof(int));
+  if (s.alloc() != cudaSuccess) { cudaGetLastError(); return -2; }
+  int* info = s.at<int>(o_info);
+  int rc = 0;
+  if (cudaMemcpyAsync(s.at<WinDesc>(o_desc), desc.data(), nwin * sizeof(WinDesc), cudaMemcpyHostToDevice, st) !=
+          cudaSuccess || cudaMemsetAsync(info, 0, sizeof(int), st) != cudaSuccess)
+    rc = -2;
+  if (!rc && window_chol(st, M, ld, sign, s.at<WinDesc>(o_desc), nwin, kw_max, out, info, tag) != cudaSuccess) rc = -2;
+  if (!rc && cudaMemcpyAsync(info_host, info, sizeof(int), cudaMemcpyDeviceToHost, st) != cudaSuccess) rc = -2;
+  return drain(st, rc);
+}
+
+int cgpcm_sym_accum_test(int nwin, const int64_t* windows, const double* A, const double* B, int n, int64_t ld,
+                         double* out, void* stream) {
+  if (!windows || !A || !B || !out || nwin < 1 || n < 1 || ld < n || ld % 8) return -1;
+  for (int w = 0; w < nwin; ++w) {
+    const int64_t* v = windows + 6 * w;
+    const int64_t k_lo = v[1], order = v[2], K = v[3];
+    if (order < 8 || order % 8 || order > SY_MP || K < 2 || K % 2 || K > (1 << 30) || k_lo < 0 || k_lo + order > n ||
+        v[4] < 0 || v[5] < 0 || v[4] % 2 || v[5] % 2)
+      return -1;
+  }
+  cudaStream_t st = (cudaStream_t)stream;
+  Scratch s;
+  s.take((size_t)SY_MAX_SPLITS * ld * ld);
+  if (s.alloc() != cudaSuccess) { cudaGetLastError(); return -2; }
+  double* acc = s.at(0);
+  int rc = cudaMemsetAsync(acc, 0, (size_t)SY_MAX_SPLITS * ld * ld * sizeof(double), st) == cudaSuccess ? 0 : -2;
+  int used = 0;
+  for (int w = 0; w < nwin && !rc; ++w) {
+    const int64_t* v = windows + 6 * w;
+    const bool kc = v[0] != 0;
+    const int order = (int)v[2], K = (int)v[3];
+    const long lda = kc ? K : order;
+    int splits = 1;
+    if (sym_accum_launch(st, kc, kc, order, K, A + v[4], lda, B + v[5], lda, acc, ld, v[1] * ld + v[1], &splits) !=
+        cudaSuccess)
+      rc = -2;
+    used = std::max(used, splits);
+  }
+  if (!rc) sym_finish_launch(st, acc, ld, used, n, out);
+  return drain(st, rc);
 }
 
 }  // extern "C"

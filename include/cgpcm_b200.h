@@ -340,6 +340,44 @@ int cgpcm_predict_quad_test(const double* V, int64_t v_stride, int ldv, const do
 int cgpcm_predict_pair_test(const double* tp, int np, const double* tq, int nq, const double* tx, int nx,
                             const double hyp[3], int causal, int causal_id, const double* G, int64_t ldg, int gk,
                             double* X, void* stream);
+/* The kernels of the ELBO sweeps (csrc/psi_kernels.cuh, csrc/linalg.cuh, csrc/dgemm_sym.cuh) through the launch code the
+ * sweeps use.  Device pointers, except the descriptor arrays and hyp = (alpha, gamma, omega), which are on the host;
+ * stream: a cudaStream_t or NULL; each returns after the stream has drained.  -1 for bad shapes, -4 for a non-positive
+ * or non-finite hyper-parameter.  sep = 1 selects the separable kernels (default causal model only: causal = 1,
+ * causal_id = 0); cull = 0 evaluates every element (threshold 746).
+ * cgpcm_ahx_gen_test: one chunk of observations t[0 .. n_valid), n_valid <= nc, nc % 8 == 0, over the window of
+ * inducing inputs k_lo .. k_lo + kwp (k_lo even, kwp % 8 == 0, k_lo + kwp <= ld): A[(i * nc + n) * kwp + k] = Ahx for
+ * i < nhp (nhp % 8 == 0, nhp >= nh), 0 outside the valid nh x n_valid x nx box; when ypart is not NULL,
+ * ypart[s * nhp * ld + i * ld + k_lo + k] = sum over the observations n of slice s (16 per slice) of y_n A, the slices
+ * zeroed first ((nc + 15) / 16 slices of nhp x ld).
+ * cgpcm_ahx_dot_test: g3[theta] = sum over i < nh, n < n_valid, k_lo + k < nx, elements not culled, of
+ * (W[(i * nc + n) * kwp + k] + y_n Ybar[i * ld + k_lo + k]) dA/dtheta, theta = (alpha, gamma, omega), with A the block of
+ * cgpcm_ahx_gen_test; the same CTA partials and final sum as the backward sweep.
+ * cgpcm_axx_sum_test: out4[m * ld * ld + k * ld + l] = sum_n Axx[n] (m = 0) and its derivatives w.r.t. alpha, gamma,
+ * omega (m = 1..3, when tangents), k, l < nx, 0 elsewhere; `slices` observation slices (1..64); sorted = 1 declares t
+ * non-decreasing (each pair then visits only its own observation interval).  The pair-hoisted BVN branch is taken as
+ * the sweep takes it (causal model, rho = gamma / (alpha + gamma + omega) >= 0.925).
+ * cgpcm_window_chol_test: for window w of `windows` (host int32 [nwin][3] = k_lo, kw, kv; kw % 8 == 0, 8 <= kw <= 120,
+ * 0 <= kv <= kw, k_lo + kv <= ld), the upper-triangular S_w = L_w^T of sign * M[k_lo .. k_lo + kv, same] padded with
+ * the identity to kw x kw, dense at out + sum of kw^2 of the windows before it; all windows in one launch.
+ * *info_host = tag * 100000 + k_lo + j + 1 of a window whose pivot j was not positive (one of them), else 0.
+ * cgpcm_sym_accum_test: out (n x n at ld) = the sum of the windows' products op(A_w) op(B_w)^T, each order_w x order_w at
+ * (k_lo_w, k_lo_w), symmetric.  windows: host int64 [nwin][6] = (kc, k_lo, order, K, a_off, b_off); kc = 1:
+ * A_w[m][k] = A[a_off + m * K + k], kc = 0: A_w[m][k] = A[a_off + k * order + m], B_w likewise from B at b_off.  The
+ * windows are added into the sweep's zeroed K-slice buffers in list order, then summed and mirrored. */
+int cgpcm_ahx_gen_test(const double* t, const double* y, int n_valid, int nc, const double* th, int nh, int nhp,
+                       const double* tx, int nx, int k_lo, int kwp, const double hyp[3], int causal, int causal_id,
+                       double cull, int sep, int64_t ld, double* A, double* ypart, void* stream);
+int cgpcm_ahx_dot_test(const double* t, const double* y, int n_valid, int nc, const double* th, int nh, int nhp,
+                       const double* tx, int nx, int k_lo, int kwp, const double hyp[3], int causal, int causal_id,
+                       double cull, int sep, int64_t ld, const double* A, const double* W, const double* Ybar,
+                       double* g3, void* stream);
+int cgpcm_axx_sum_test(const double* t, int n, int sorted, const double* tx, int nx, const double hyp[3], int causal,
+                       int causal_id, double cull, int slices, int tangents, int64_t ld, double* out4, void* stream);
+int cgpcm_window_chol_test(const double* M, int64_t ld, double sign, int nwin, const int32_t* windows, int tag,
+                           double* out, int* info_host, void* stream);
+int cgpcm_sym_accum_test(int nwin, const int64_t* windows, const double* A, const double* B, int n, int64_t ld,
+                         double* out, void* stream);
 
 #ifdef __cplusplus
 }
