@@ -25,7 +25,7 @@ EXPORTS = ['cgpcm_create', 'cgpcm_destroy', 'cgpcm_last_error', 'cgpcm_device_co
            'cgpcm_last_timing', 'cgpcm_bvn_cdf', 'cgpcm_dgemm', 'cgpcm_dgemm_tri', 'cgpcm_dgemm_sym', 'cgpcm_cholinv', 'cgpcm_math_test', 'cgpcm_math_test_fast',
            'cgpcm_smf_c1_test', 'cgpcm_smf_algebra_test', 'cgpcm_smf_posterior_test', 'cgpcm_predict_quad_test',
            'cgpcm_predict_pair_test', 'cgpcm_ahx_gen_test', 'cgpcm_ahx_dot_test', 'cgpcm_axx_sum_test',
-           'cgpcm_window_chol_test', 'cgpcm_sym_accum_test']
+           'cgpcm_window_chol_test', 'cgpcm_sym_accum_test', 'cgpcm_potrf_test', 'cgpcm_trtri_test']
 
 
 def _sources():
@@ -115,6 +115,8 @@ def lib():
     L.cgpcm_axx_sum_test.argtypes = [dp, i32, i32, dp, i32, dp, i32, i32, dbl, i32, i32, i64, dp, vp]
     L.cgpcm_window_chol_test.argtypes = [dp, i64, dbl, i32, dp, i32, dp, ctypes.POINTER(i32), vp]
     L.cgpcm_sym_accum_test.argtypes = [i32, dp, dp, dp, i32, i64, dp, vp]
+    L.cgpcm_potrf_test.argtypes = [dp, i32, i64, i32, ctypes.POINTER(i32), vp]
+    L.cgpcm_trtri_test.argtypes = [dp, dp, i32, i64, vp]
     for name in EXPORTS:
         if name != 'cgpcm_last_error':
             getattr(L, name).restype = ctypes.c_int

@@ -3399,8 +3399,9 @@ int predict_cov_run(cgpcm_handle* h, const double* params_host, double reg, cons
         if (!inf[b]) continue;
         int piv = inf[b] % 100000;
         if (piv == n + 1) {
-          // The border pivot: potrf reports the last failed pivot of a panel, and a failed pivot of S_b can leave a
-          // non-finite z_b.  Factor S_b with an identity border so that the message names its own pivot.
+          // The border pivot: potrf reports the first failed pivot, so every pivot of S_b passed and only the border
+          // c - |z_b|^2 failed: |z_b|^2 overflows.  S_b is factorised alone with an identity border to confirm that
+          // before the overflow message (a failure there would be named by its own pivot).
           CK(cudaMemsetAsync(d_pinfo + b, 0, sizeof(int), st));
           pcov_border_kernel<<<148 * 8, 256, 0, st>>>(d_c + (long)b * n2, npad, n2, d_mean + g0 + b, B, nullptr, n,
                                                       d_add, 1, d_kb + (long)b * k2, ldk, k2);
@@ -4149,6 +4150,29 @@ int cgpcm_window_chol_test(const double* M, int64_t ld, double sign, int nwin, c
     rc = -2;
   if (!rc && window_chol(st, M, ld, sign, s.at<WinDesc>(o_desc), nwin, kw_max, out, info, tag) != cudaSuccess) rc = -2;
   if (!rc && cudaMemcpyAsync(info_host, info, sizeof(int), cudaMemcpyDeviceToHost, st) != cudaSuccess) rc = -2;
+  return drain(st, rc);
+}
+
+int cgpcm_potrf_test(double* A, int np, int64_t ld, int tag, int* info_host, void* stream) {
+  if (!A || !info_host || np < 8 || np % 8 || ld < np || ld % 2 || tag < 0 || tag > 20000) return -1;
+  cudaStream_t st = (cudaStream_t)stream;
+  Scratch s;
+  const size_t o_scr = s.take(LA_NB * LA_NB), o_info = s.take(1, sizeof(int));
+  if (s.alloc() != cudaSuccess) { cudaGetLastError(); return -2; }
+  int* info = s.at<int>(o_info);
+  int rc = cudaMemsetAsync(info, 0, sizeof(int), st) == cudaSuccess ? 0 : -2;
+  if (!rc && potrf_lower(st, A, np, ld, info, tag, s.at(o_scr)) != cudaSuccess) rc = -2;
+  if (!rc && cudaMemcpyAsync(info_host, info, sizeof(int), cudaMemcpyDeviceToHost, st) != cudaSuccess) rc = -2;
+  return drain(st, rc);
+}
+
+int cgpcm_trtri_test(const double* L, double* X, int np, int64_t ld, void* stream) {
+  if (!L || !X || np < 8 || np % 8 || ld < np || ld % 2) return -1;
+  cudaStream_t st = (cudaStream_t)stream;
+  Scratch s;
+  s.take((size_t)LA_NB * ld);
+  if (s.alloc() != cudaSuccess) { cudaGetLastError(); return -2; }
+  const int rc = trtri_lower(st, L, X, s.at(0), np, ld) == cudaSuccess ? 0 : -2;
   return drain(st, rc);
 }
 

@@ -10,9 +10,9 @@
 //   C_TR : C(m,n) at C[n*ldc + m]                    else C[m*ldc + n]
 // Requirements: M, N multiples of 8; K, lda, ldb, ldc even; 16-byte aligned pointers.
 //
-// Tiling: CTA tile = bm x 128 x 16 with bm <= 104 a multiple of 8 chosen by the caller so that M
-// splits evenly (M = 200 -> two tiles of 104/96 rows: 96 % useful instead of 78 % with 128-row
-// tiles).  8 warps side by side along N; each warp owns all (<= 13) 8-row blocks x two 8-column
+// Tiling: CTA tile = bm x 64 x 16 with bm = 32, 56 or 104 rows (pick_mb) chosen so that M splits
+// evenly (M = 200 -> two tiles of 104/96 rows: 96 % useful instead of 78 % with 128-row tiles).
+// 128 threads: 4 warps side by side along N; each warp owns all (<= 13) 8-row blocks x two 8-column
 // blocks = 26 DMMA per k4 step with 52 FP64 accumulators, so every SM sub-partition carries the
 // same tensor work.  Shared-memory strides are == 4 (mod 8) doubles: conflict-free fragment loads.
 // 3-stage cp.async pipeline (zero-filled at every edge).  Split-K over blockIdx.z writes partial

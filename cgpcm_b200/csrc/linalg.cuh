@@ -1,8 +1,10 @@
-// Small dense FP64 linear algebra on the device for the M x M part of the ELBO (M = nh, nx <= ~512):
-// the replacements of tf.cholesky / tf.cholesky_solve / tf.matrix_triangular_solve / log_det
-// (src/core/tf_util.py:98-105,134-138,271-278; used at src/core/cgpcm.py:214-229,535 and
-// src/core/distribution.py:60-76).  Everything runs on one stream, no host round trips; a failed
-// factorisation is reported through a device-side info word (checked once per evaluation).
+// Dense FP64 linear algebra on the device: the M x M part of the ELBO (M = nh, nx <= 4096), the replacements of
+// tf.cholesky / tf.cholesky_solve / tf.matrix_triangular_solve / log_det (src/core/tf_util.py:98-105,134-138,271-278;
+// used at src/core/cgpcm.py:214-229,535 and src/core/distribution.py:60-76), and the factorisations of the sampling
+// and scoring paths: order <= 8192 (filter draws), <= 4096 (AKM draws, predictive draws) and <= 4104 (the bordered
+// scoring matrix).  Everything runs on one stream, no host round trips; a failed factorisation is reported through a
+// device-side info word, tag * 100000 + the first non-positive pivot + 1 (the first failing launch sets it; checked
+// once per evaluation).
 //
 // All matrices are square row-major with leading dimension ld and a *padded* order np (multiple
 // of 8, np <= ld): callers put the identity on the padding block so that factor / inverse / logdet of
@@ -51,7 +53,7 @@ __global__ void __launch_bounds__(256) potrf_panel_kernel(double* __restrict__ A
   for (int j = 0; j < jb; ++j) {
     if (tid == 0) {
       double d = D[j][j];
-      if (!(d > 0.0)) { bad = j + 1; d = 1.0; }
+      if (!(d > 0.0)) { if (!bad) bad = j + 1; d = 1.0; }
       D[j][j] = sqrt(d);
     }
     __syncthreads();
@@ -152,7 +154,7 @@ __global__ void __launch_bounds__(256) window_chol_kernel(const double* __restri
   for (int j = 0; j < n; ++j) {
     if (tid == 0) {
       double dj = Wsm[j * P + j];
-      if (!(dj > 0.0)) { bad = j + 1; dj = 1.0; }
+      if (!(dj > 0.0)) { if (!bad) bad = j + 1; dj = 1.0; }
       Wsm[j * P + j] = sqrt(dj);
     }
     __syncthreads();

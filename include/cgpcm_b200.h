@@ -341,7 +341,7 @@ int cgpcm_predict_pair_test(const double* tp, int np, const double* tq, int nq, 
                             const double hyp[3], int causal, int causal_id, const double* G, int64_t ldg, int gk,
                             double* X, void* stream);
 /* The kernels of the ELBO sweeps (csrc/psi_kernels.cuh, csrc/linalg.cuh, csrc/dgemm_sym.cuh) through the launch code the
- * sweeps use.  Device pointers, except the descriptor arrays and hyp = (alpha, gamma, omega), which are on the host;
+ * sweeps use, and the dense factorisation under every entry point.  Device pointers, except the descriptor arrays and hyp = (alpha, gamma, omega), which are on the host;
  * stream: a cudaStream_t or NULL; each returns after the stream has drained.  -1 for bad shapes, -4 for a non-positive
  * or non-finite hyper-parameter.  sep = 1 selects the separable kernels (default causal model only: causal = 1,
  * causal_id = 0); cull = 0 evaluates every element (threshold 746).
@@ -360,11 +360,19 @@ int cgpcm_predict_pair_test(const double* tp, int np, const double* tq, int nq, 
  * cgpcm_window_chol_test: for window w of `windows` (host int32 [nwin][3] = k_lo, kw, kv; kw % 8 == 0, 8 <= kw <= 120,
  * 0 <= kv <= kw, k_lo + kv <= ld), the upper-triangular S_w = L_w^T of sign * M[k_lo .. k_lo + kv, same] padded with
  * the identity to kw x kw, dense at out + sum of kw^2 of the windows before it; all windows in one launch.
- * *info_host = tag * 100000 + k_lo + j + 1 of a window whose pivot j was not positive (one of them), else 0.
+ * *info_host = tag * 100000 + k_lo + j + 1 for the first pivot j that was not positive within a window (the window
+ * is any of those that have one), else 0.
  * cgpcm_sym_accum_test: out (n x n at ld) = the sum of the windows' products op(A_w) op(B_w)^T, each order_w x order_w at
  * (k_lo_w, k_lo_w), symmetric.  windows: host int64 [nwin][6] = (kc, k_lo, order, K, a_off, b_off); kc = 1:
  * A_w[m][k] = A[a_off + m * K + k], kc = 0: A_w[m][k] = A[a_off + k * order + m], B_w likewise from B at b_off.  The
- * windows are added into the sweep's zeroed K-slice buffers in list order, then summed and mirrored. */
+ * windows are added into the sweep's zeroed K-slice buffers in list order, then summed and mirrored.
+ * cgpcm_potrf_test: the blocked Cholesky factorisation (potrf_lower, csrc/linalg.cuh) as the sampling and scoring
+ * paths call it: A (np x np at ld, lower triangle read) -> L in place, upper triangle of the np x np block zeroed,
+ * nothing outside it touched; a 32 x 32 scratch slot of its own.  A non-positive pivot is replaced by 1 and the
+ * factorisation goes on; *info_host = tag * 100000 + j + 1 for the first such pivot j, else 0.  -1 unless
+ * np % 8 == 0, np <= ld and ld is even.
+ * cgpcm_trtri_test: X = L^-1 (trtri_lower) for the lower-triangular L (np x np at ld), X exactly lower triangular,
+ * nothing outside its np x np block touched; a workspace of 32 x ld of its own.  Shapes as cgpcm_potrf_test. */
 int cgpcm_ahx_gen_test(const double* t, const double* y, int n_valid, int nc, const double* th, int nh, int nhp,
                        const double* tx, int nx, int k_lo, int kwp, const double hyp[3], int causal, int causal_id,
                        double cull, int sep, int64_t ld, double* A, double* ypart, void* stream);
@@ -378,6 +386,8 @@ int cgpcm_window_chol_test(const double* M, int64_t ld, double sign, int nwin, c
                            double* out, int* info_host, void* stream);
 int cgpcm_sym_accum_test(int nwin, const int64_t* windows, const double* A, const double* B, int n, int64_t ld,
                          double* out, void* stream);
+int cgpcm_potrf_test(double* A, int np, int64_t ld, int tag, int* info_host, void* stream);
+int cgpcm_trtri_test(const double* L, double* X, int np, int64_t ld, void* stream);
 
 #ifdef __cplusplus
 }

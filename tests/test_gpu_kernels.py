@@ -147,25 +147,40 @@ def test_dgemm_sym(kc, M, K):
     assert np.array_equal(got, got.T)
 
 
-@pytest.mark.parametrize('n', [1, 5, 32, 33, 41, 150, 200, 301])
-def test_cholinv(n):
+@pytest.mark.parametrize('n,ld', [(1, 8), (1, 24), (5, 8), (32, 32), (33, 40), (41, 48), (41, 64), (150, 152),
+                                  (200, 200), (301, 304), (301, 320)])
+def test_cholinv(n, ld):
+    """cgpcm_cholinv against float64 bars: the factor's backward error |L L^T - A| <= 4 (n + 1) eps |L| |L|^T, the
+    residual and forward error of the inverse within 4 n eps cond(A), the padding rows / columns [n, np) of the inverse
+    exactly 0, and logdet within n eps of 2 sum log L_ii of the GPU's own factor and within 1e-12 of slogdet.  Every
+    element outside the logical n x n block starts as NaN: the identity padding must be put in by the call."""
+    import math
+    eps = np.finfo(np.float64).eps
     rng = np.random.default_rng(n)
     X = rng.standard_normal((n, n + 3))
     A = X @ X.T + 1e-3 * np.eye(n)
-    ld = (n + 7) // 8 * 8
-    buf = np.zeros((ld, ld))
+    np_ = (n + 7) // 8 * 8
+    buf = np.full((ld, ld), np.nan)
     buf[:n, :n] = A
     dA = torch.tensor(buf, device='cuda')
-    dI = torch.zeros_like(dA)
+    dI = torch.full_like(dA, np.nan)
     logdet = np.zeros(1)
     info = ctypes.c_int(0)
     rc = _lib.lib().cgpcm_cholinv(dA.data_ptr(), dI.data_ptr(), logdet.ctypes.data, n, ld, ctypes.byref(info))
     assert rc == 0 and info.value == 0
     L = dA.cpu().numpy()[:n, :n]
-    np.testing.assert_allclose(L, np.linalg.cholesky(A), rtol=1e-9, atol=1e-11)
-    inv = dI.cpu().numpy()[:n, :n]
-    np.testing.assert_allclose(inv @ A, np.eye(n), atol=1e-7)
-    np.testing.assert_allclose(inv, np.linalg.inv(A), rtol=1e-6, atol=1e-8 * np.abs(np.linalg.inv(A)).max())
+    assert np.all(np.triu(L, 1) == 0.0) and np.all(np.diag(L) > 0)
+    assert np.all(np.abs(L @ L.T - A) <= 4 * (n + 1) * eps * (np.abs(L) @ np.abs(L).T))
+    full = dI.cpu().numpy()
+    inv = full[:n, :n]
+    w = np.linalg.eigvalsh(A)
+    cond = w[-1] / w[0]
+    assert np.abs(A @ inv - np.eye(n)).max() <= 4 * n * eps * cond
+    ref = np.linalg.inv(A)
+    assert np.abs(inv - ref).max() <= 4 * n * eps * cond * np.abs(ref).max()
+    assert np.all(full[:np_, n:np_] == 0.0) and np.all(full[n:np_, :np_] == 0.0)
+    own = 2 * math.fsum(np.log(np.diag(L)))
+    assert abs(logdet[0] - own) <= (n + 2) * eps * 2 * math.fsum(np.abs(np.log(np.diag(L)))) + 1e-300
     assert logdet[0] == pytest.approx(np.linalg.slogdet(A)[1], rel=1e-12, abs=1e-12)
 
 
