@@ -22,7 +22,7 @@ MODE_FROZEN, MODE_FULL = 0, 1
 
 EXPORTS = ['cgpcm_create', 'cgpcm_destroy', 'cgpcm_last_error', 'cgpcm_device_count', 'cgpcm_comm_unique_id', 'cgpcm_comm_init',
            'cgpcm_set_data', 'cgpcm_set_option', 'cgpcm_psi', 'cgpcm_precompute', 'cgpcm_frozen_mats', 'cgpcm_elbo_grad', 'cgpcm_elbo_smf', 'cgpcm_elbo_smf_batch', 'cgpcm_predict_f', 'cgpcm_predict_f_batch', 'cgpcm_predict_f_cov', 'cgpcm_predict_logpdf', 'cgpcm_kernel_samples', 'cgpcm_filter_samples', 'cgpcm_akm_sample', 'cgpcm_fpi', 'cgpcm_fpi_qz', 'cgpcm_elbo_qz',
-           'cgpcm_last_timing', 'cgpcm_bvn_cdf', 'cgpcm_dgemm', 'cgpcm_dgemm_tri', 'cgpcm_dgemm_sym', 'cgpcm_cholinv', 'cgpcm_math_test', 'cgpcm_math_test_fast',
+           'cgpcm_last_timing', 'cgpcm_bvn_cdf', 'cgpcm_dgemm', 'cgpcm_dgemm_tri', 'cgpcm_dgemm_sym', 'cgpcm_cholinv', 'cgpcm_math_test', 'cgpcm_math_test_fast', 'cgpcm_math_test_tab',
            'cgpcm_smf_c1_test', 'cgpcm_smf_algebra_test', 'cgpcm_smf_posterior_test', 'cgpcm_predict_quad_test',
            'cgpcm_predict_pair_test', 'cgpcm_ahx_gen_test', 'cgpcm_ahx_dot_test', 'cgpcm_axx_sum_test',
            'cgpcm_window_chol_test', 'cgpcm_sym_accum_test', 'cgpcm_potrf_test', 'cgpcm_trtri_test']
@@ -101,6 +101,7 @@ def lib():
     L.cgpcm_cholinv.argtypes = [dp, dp, dp, i32, i64, ctypes.POINTER(i32)]
     L.cgpcm_math_test.argtypes = [dp, i64, dp, dp, ctypes.POINTER(i32)]
     L.cgpcm_math_test_fast.argtypes = [dp, i64, dp, dp]
+    L.cgpcm_math_test_tab.argtypes = [dp, i64, dp, dp, dp]
     L.cgpcm_smf_c1_test.argtypes = [dp, i64, i32, i32, dp, i32, i64, dp, vp]
     L.cgpcm_smf_algebra_test.argtypes = [dp, dp, dp, dp, dp, dp, i32, i32, i32, i64, i32, dbl, dbl, dbl, i32, i32, dp,
                                          vp, vp]

@@ -17,8 +17,10 @@
 //                      well conditioned); exp(-x^2) from the rounded square and its exact residual (fma);
 //                      one reciprocal (hardware approximation + 2 Newton steps) serves both divisions;
 //                      erfc(z) = 2 - erfc(-z) for z < 0.
+//   cg_erfcx_tab<U>(z) erfcx(z) for signed z in [-8, 3]: piecewise polynomial, 352 intervals of degree 10 (below).
 // Coefficients: computed with mpmath at 60 digits (tools/fit_cgmath.py), rounded to double; accuracy against mpmath is
-// tested in tests/test_gpu_kernels.py (cgpcm_math_test): <= 2 ulp (exp), <= 4 ulp (erfc) over the whole range.
+// tested in tests/test_gpu_kernels.py (cgpcm_math_test): <= 2 ulp (exp), <= 4 ulp (erfc) over the whole range, and in
+// tests/test_gpu_psi_tables.py (cgpcm_math_test_tab): <= 4.5 ulp (cg_erfcx_tab).
 #pragma once
 #include <cuda_runtime.h>
 
@@ -52,13 +54,16 @@ __constant__ double cg_erfc_c[27] = {CG_ERFC_C26, CG_ERFC_COEFS(CG_LIST)};
 // FLUSH = true: results below 2^-1021 (x < -708.05) are returned as 0 and the scaling is one integer add to the
 // exponent field instead of two exact multiplications (bit-identical for every normal result).  The Psi kernels use
 // it: an element below 5e-308 changes no bit of a sum whose terms are O(1).
-template <int U, bool FLUSH = false>
+// BIAS (FLUSH only): returns exp(x) 2^BIAS -- the same significand, BIAS added to the exponent -- so that factors down
+// to exp(-(1021 + BIAS) ln 2) stay normal; results below 2^-1021 are still returned as 0.
+template <int U, bool FLUSH = false, int BIAS = 0>
 __device__ __forceinline__ void cg_exp_neg(const double (&x)[U], double (&out)[U]) {
+  static_assert(BIAS == 0 || (FLUSH && BIAS > 0 && BIAS < 1000), "BIAS needs FLUSH");
   double r[U], p[U];
   int ni[U];
 #pragma unroll
   for (int u = 0; u < U; ++u) {
-    const double xc = fmax(x[u], -750.0);
+    const double xc = fmax(x[u], -750.0 - 0.6931471805599453 * BIAS);
     const double t = fma(xc, 0x1.71547652b82fep+0, 6755399441055744.0);      // x log2(e) + 1.5 * 2^52
     ni[u] = __double2loint(t);
     const double n = t - 6755399441055744.0;
@@ -74,8 +79,9 @@ __device__ __forceinline__ void cg_exp_neg(const double (&x)[U], double (&out)[U
   for (int u = 0; u < U; ++u) {
     if (FLUSH) {
       // p in [0.70, 1.42]: exponent field 1022 or 1023, so p 2^n is normal for n >= -1021
-      const double v = __hiloint2double(__double2hiint(p[u]) + (ni[u] << 20), __double2loint(p[u]));
-      out[u] = ni[u] >= -1021 ? v : 0.0;
+      const int nb = ni[u] + BIAS;
+      const double v = __hiloint2double(__double2hiint(p[u]) + (nb << 20), __double2loint(p[u]));
+      out[u] = nb >= -1021 ? v : 0.0;
     } else {
       const int k1 = ni[u] >> 1, k2 = ni[u] - k1;                             // both >= -541: normal powers of two
       const double s1 = __hiloint2double((1023 + k1) << 20, 0), s2 = __hiloint2double((1023 + k2) << 20, 0);
@@ -112,6 +118,77 @@ __device__ __forceinline__ void cg_erfcx_abs(const double (&z)[U], double (&out)
   }
 #pragma unroll
   for (int u = 0; u < U; ++u) out[u] = g[u] * inv[u];
+}
+
+// erfcx(z) = exp(z^2) erfc(z) for signed z in [CG_ERFCX_TAB_ZLO, CG_ERFCX_TAB_ZHI]: interval j = floor((z - ZLO) / W)
+// of CG_ERFCX_TAB_NI, polynomial of degree CG_ERFCX_TAB_DEG in x = z - c_j (c_j the interval's centre, so x is exact).
+// Each polynomial interpolates erfcx on its interval widened by W / 8 on both sides (tools/fit_cgmath.py, 60 digits):
+// <= 2 ulp before rounding of the Horner steps; tested against mpmath in tests/test_gpu_psi_tables.py.  Width and
+// degree: W = 1/32 keeps degree 10 within 2 ulp down to z = -8, where erfcx grows by e^{2|z| W} = 1.65 per interval
+// (W = 1/16 needs degree 12 there).  The coefficients are read through the L1 cache, coefficient-major: the lanes of
+// a warp step through consecutive intervals (ahx_gen_sep_kernel: 0.7 in z over a warp at the bench shape, 23
+// intervals), so a coefficient load of a warp touches one or two 128-byte lines.
+// The U arguments are evaluated in lock-step on the interval of the first one whose keep[u] is set, when every kept
+// argument lies on its widened interval (ahx_gen_sep_kernel: the U arguments are U consecutive observations at one
+// inducing input, so they nearly always share an interval): one load per coefficient for all U.  Otherwise each
+// argument is evaluated on its own interval.  Arguments outside the range give the value of the nearest end interval's
+// polynomial (finite or not): callers check the range, and results with keep[u] = false are to be discarded.
+constexpr double CG_ERFCX_TAB_ZLO = -8.0, CG_ERFCX_TAB_W = 1.0 / 32;
+constexpr int CG_ERFCX_TAB_NI = 352, CG_ERFCX_TAB_DEG = 10;
+constexpr double CG_ERFCX_TAB_ZHI = CG_ERFCX_TAB_ZLO + CG_ERFCX_TAB_NI * CG_ERFCX_TAB_W;     // 3
+__device__ double cg_erfcx_tab_c[(CG_ERFCX_TAB_DEG + 1) * CG_ERFCX_TAB_NI] = {
+#include "cgmath_erfcx_tab.inc"
+};
+
+__device__ __forceinline__ int cg_erfcx_tab_index(double z) {
+  const double s = fmin(fmax((z - CG_ERFCX_TAB_ZLO) * (1.0 / CG_ERFCX_TAB_W), 0.0), CG_ERFCX_TAB_NI - 1.0);
+  return (int)s;
+}
+
+__device__ __forceinline__ double cg_erfcx_tab_centre(int j) {
+  return fma((double)j, CG_ERFCX_TAB_W, CG_ERFCX_TAB_ZLO + 0.5 * CG_ERFCX_TAB_W);      // exact
+}
+
+template <int U>
+__device__ __forceinline__ void cg_erfcx_tab(const double (&z)[U], const bool (&keep)[U], double (&out)[U]) {
+  double zr = z[U - 1];
+#pragma unroll
+  for (int u = U - 2; u >= 0; --u) zr = keep[u] ? z[u] : zr;
+  const int j = cg_erfcx_tab_index(zr);
+  const double cj = cg_erfcx_tab_centre(j);
+  double x[U];
+  bool same = true;
+#pragma unroll
+  for (int u = 0; u < U; ++u) {
+    x[u] = z[u] - cj;
+    same = same && (!keep[u] || fabs(x[u]) <= (0.5 + 0.125) * CG_ERFCX_TAB_W);
+  }
+  if (same) {
+    const double* c = cg_erfcx_tab_c + j;
+    double p[U];
+    const double cd = __ldg(c);
+#pragma unroll
+    for (int u = 0; u < U; ++u) p[u] = cd;
+#pragma unroll
+    for (int k = 1; k <= CG_ERFCX_TAB_DEG; ++k) {
+      const double ck = __ldg(c + k * CG_ERFCX_TAB_NI);
+#pragma unroll
+      for (int u = 0; u < U; ++u) p[u] = fma(p[u], x[u], ck);
+    }
+#pragma unroll
+    for (int u = 0; u < U; ++u) out[u] = p[u];
+  } else {
+#pragma unroll
+    for (int u = 0; u < U; ++u) {
+      const int ju = cg_erfcx_tab_index(z[u]);
+      const double xu = z[u] - cg_erfcx_tab_centre(ju);
+      const double* c = cg_erfcx_tab_c + ju;
+      double p = __ldg(c);
+#pragma unroll
+      for (int k = 1; k <= CG_ERFCX_TAB_DEG; ++k) p = fma(p, xu, __ldg(c + k * CG_ERFCX_TAB_NI));
+      out[u] = p;
+    }
+  }
 }
 
 template <int U>

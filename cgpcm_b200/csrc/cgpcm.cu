@@ -800,18 +800,32 @@ cudaError_t axx_launch(cudaStream_t st, const double* t, int n, bool sorted, con
   return cudaGetLastError();
 }
 
+// Whether ahx_gen_sep_kernel<true> (table-driven erfcx) covers every element for the filter inducing inputs th[0 .. nh)
+// (host values) at the constants c.
+bool ahx_gen_tab(const PsiConst& c, const double* th_host, int nh) {
+  if (nh < 1) return false;
+  double lo = th_host[0], hi = th_host[0];
+  for (int i = 1; i < nh; ++i) { lo = std::min(lo, th_host[i]); hi = std::max(hi, th_host[i]); }
+  return psi_erfcx_tab_covers(c, lo, hi);
+}
+
 // A[(i*nc + n)*kwp + k] = Ahx of the chunk's observations t[0 .. nv) at the window k_lo + k (ahx_gen_sep_kernel when
-// `sep`: default causal model only), and when Ypart != NULL the slice partials of sum_n y_n A.  One launch.
-void ahx_gen_launch(cudaStream_t st, bool sep, const double* t, const double* y, int nv, int nc, const double* th, int nh,
-                    int nhp, const double* tx, int nx, int k_lo, int kwp, double* A, double* Ypart, long ldy,
-                    long ypart_stride, const PsiConst& c) {
+// `sep`: default causal model only; its table-driven erfcx when `tab`, see ahx_gen_tab), and when Ypart != NULL the
+// slice partials of sum_n y_n A.  One launch.
+void ahx_gen_launch(cudaStream_t st, bool sep, bool tab, const double* t, const double* y, int nv, int nc,
+                    const double* th, int nh, int nhp, const double* tx, int nx, int k_lo, int kwp, double* A,
+                    double* Ypart, long ldy, long ypart_stride, const PsiConst& c) {
   const int threads = std::min(256, round_up(kwp, 32));
   dim3 grid(nhp, (nc + AHX_NSUB - 1) / AHX_NSUB);
   if (sep) {
     // default causal model: separable form, AHX_IB filter rows per CTA (psi_kernels.cuh)
     grid.x = (nhp + AHX_IB - 1) / AHX_IB;
-    ahx_gen_sep_kernel<<<grid, threads, 0, st>>>(t, y, nv, nc, th, nh, nhp, tx, nx, k_lo, kwp, A, Ypart, ldy,
-                                                 ypart_stride, c);
+    if (tab)
+      ahx_gen_sep_kernel<true><<<grid, threads, 0, st>>>(t, y, nv, nc, th, nh, nhp, tx, nx, k_lo, kwp, A, Ypart, ldy,
+                                                         ypart_stride, c);
+    else
+      ahx_gen_sep_kernel<false><<<grid, threads, 0, st>>>(t, y, nv, nc, th, nh, nhp, tx, nx, k_lo, kwp, A, Ypart, ldy,
+                                                          ypart_stride, c);
   } else {
     ahx_gen_kernel<<<grid, threads, 0, st>>>(t, y, nv, nc, th, nh, tx, nx, k_lo, kwp, A, Ypart, ldy, ypart_stride, c);
   }
@@ -906,8 +920,10 @@ int gen_chunk(cgpcm_handle* h, const PsiConst& c, const Chunk& ch, bool with_y, 
   if ((ch.nc + AHX_NSUB - 1) / AHX_NSUB > h->y_slices) { h->err = "internal: y_slices too small"; return -1; }
   prof_close(h);
   if (h->profile) cudaEventRecord(prof_event(h, 1), h->st);
-  ahx_gen_launch(h->st, c.causal && !c.causal_id && h->sep_opt, h->t + ch.n0, h->y + ch.n0, ch.nv, ch.nc, h->th, h->nh,
-                 h->nhp, h->tx, h->nx, ch.k_lo, ch.kwp, dstA, with_y ? h->ypart : nullptr, h->ld, (long)h->nhp * h->ld, c);
+  const bool sep = c.causal && !c.causal_id && h->sep_opt;
+  ahx_gen_launch(h->st, sep, sep && ahx_gen_tab(c, h->h_th.data(), h->nh), h->t + ch.n0, h->y + ch.n0, ch.nv, ch.nc,
+                 h->th, h->nh, h->nhp, h->tx, h->nx, ch.k_lo, ch.kwp, dstA, with_y ? h->ypart : nullptr, h->ld,
+                 (long)h->nhp * h->ld, c);
   if (h->profile) cudaEventRecord(prof_event(h, 1), h->st);
   L(h);
   return 0;
@@ -3876,6 +3892,53 @@ int cgpcm_math_test_fast(const double* x, int64_t n, double* out_exp, double* ou
   return rc;
 }
 
+// out_exp[i] = cg_exp_neg<4, true, AHX_BIAS>(min(x[i], 0)), out_erfcx[i] = cg_erfcx_tab<4>(x[i]) with x in groups of 4
+// evaluated in lock-step as ahx_gen_sep_kernel<true> does (all kept)
+__global__ void math_test_tab_kernel(const double* __restrict__ x, long n, double* __restrict__ oe, double* __restrict__ oc) {
+  for (long i0 = ((long)blockIdx.x * blockDim.x + threadIdx.x) * 4; i0 < n; i0 += (long)gridDim.x * blockDim.x * 4) {
+    double xe[4], xc[4], e4[4], c4[4];
+    bool keep[4];
+#pragma unroll
+    for (int u = 0; u < 4; ++u) {
+      keep[u] = i0 + u < n;
+      const double v = keep[u] ? x[i0 + u] : 0.0;
+      xe[u] = fmin(v, 0.0);
+      xc[u] = v;
+    }
+    cg_exp_neg<4, true, AHX_BIAS>(xe, e4);
+    cg_erfcx_tab<4>(xc, keep, c4);
+#pragma unroll
+    for (int u = 0; u < 4; ++u) {
+      if (i0 + u >= n) break;
+      oe[i0 + u] = e4[u];
+      oc[i0 + u] = c4[u];
+    }
+  }
+}
+
+int cgpcm_math_test_tab(const double* x, int64_t n, double* out_exp, double* out_erfcx, double* params) {
+  if (!x || n < 1 || !out_exp || !out_erfcx || !params) return -1;
+  params[0] = CG_ERFCX_TAB_ZLO;
+  params[1] = CG_ERFCX_TAB_ZHI;
+  params[2] = AHX_BIAS;
+  double *dx = nullptr, *de = nullptr, *dc = nullptr;
+  int rc = 0;
+  if (cudaMalloc(&dx, n * sizeof(double)) != cudaSuccess || cudaMalloc(&de, n * sizeof(double)) != cudaSuccess ||
+      cudaMalloc(&dc, n * sizeof(double)) != cudaSuccess) rc = -2;
+  if (!rc) {
+    cudaMemcpy(dx, x, n * sizeof(double), cudaMemcpyDefault);
+    math_test_tab_kernel<<<148 * 4, 256>>>(dx, n, de, dc);
+    if (cudaDeviceSynchronize() != cudaSuccess) rc = -2;
+    cudaMemcpy(out_exp, de, n * sizeof(double), cudaMemcpyDefault);
+    cudaMemcpy(out_erfcx, dc, n * sizeof(double), cudaMemcpyDefault);
+  }
+  cudaGetLastError();
+  if (dx) cudaFree(dx);
+  if (de) cudaFree(de);
+  if (dc) cudaFree(dc);
+  return rc;
+}
+
 int cgpcm_cholinv(double* A, double* Ainv, double* logdet, int n, int64_t ld, int* info_host) {
   if (!A || n < 1 || ld < n || (ld % 8)) return -1;
   int np = round_up(n, 8);
@@ -4082,7 +4145,11 @@ int cgpcm_ahx_gen_test(const double* t, const double* y, int n_valid, int nc, co
   if (ypart && cudaMemsetAsync(ypart, 0, (size_t)((nc + AHX_NSUB - 1) / AHX_NSUB) * ystride * sizeof(double), st) !=
                    cudaSuccess)
     rc = -2;
-  if (!rc) ahx_gen_launch(st, sep != 0, t, y, n_valid, nc, th, nh, nhp, tx, nx, k_lo, kwp, A, ypart, ld, ystride, c);
+  std::vector<double> th_host(nh);
+  if (!rc && cudaMemcpy(th_host.data(), th, nh * sizeof(double), cudaMemcpyDefault) != cudaSuccess) rc = -2;
+  if (!rc)
+    ahx_gen_launch(st, sep != 0, sep != 0 && ahx_gen_tab(c, th_host.data(), nh), t, y, n_valid, nc, th, nh, nhp, tx,
+                   nx, k_lo, kwp, A, ypart, ld, ystride, c);
   return drain(st, rc);
 }
 

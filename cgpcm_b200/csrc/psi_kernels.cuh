@@ -330,18 +330,29 @@ __global__ void __launch_bounds__(256) ahx_gen_kernel(const double* __restrict__
 
 // ---- separable variants (default causal model, causal_id = false) -----------------------------------------------
 // Ahx[n,i,k] = pref exp(E) erfc(z) with E = c + z^2 and c = -(alpha + gamma) th_i^2 - omega d_nk^2: the Gaussian factor
-// of erfc(z) = exp(-z^2) erfcx(|z|) cancels the cross term of the envelope, and exp(c) = f_i g_nk with
+// of erfc(z) = exp(-z^2) erfcx(z) cancels the cross term of the envelope, and exp(c) = f_i g_nk with
 //   f_i = exp(-(alpha + gamma) th_i^2)   (one per filter inducing point),   g_nk = exp(-omega d_nk^2)   (one per (n, k)).
-// So   z >= 0:  Ahx = pref f_i g_nk erfcx(z)          z < 0:  Ahx = pref (2 exp(E) - f_i g_nk erfcx(-z))
-// (both factors are <= 1: nothing overflows, and where f_i g_nk underflows the term is below the subnormals anyway), and
-// the Gaussian factor exp(E - z^2) of the erfc derivative in the adjoint is f_i g_nk itself.  A CTA covers AHX_IB filter
-// rows of the same (n, k) block, so g_nk costs one exp per AHX_IB elements: ahx_gen spends one exp per element instead of
-// two, ahx_dot none.  Padding (k >= nx, n >= n_valid) is expressed as d = 1e160, whose envelope is exactly 0.
+// So   Ahx = pref f_i g_nk erfcx(z)   for either sign of z, and the Gaussian factor exp(E - z^2) of the erfc derivative in
+// the adjoint is f_i g_nk itself.  A CTA covers AHX_IB filter rows of the same (n, k) block, so g_nk costs one exp per
+// AHX_IB elements.  Padding (k >= nx, n >= n_valid) is expressed as d = 1e160, whose envelope is exactly 0.
+//
+// ahx_gen_sep_kernel<true> (the launch checks that every element with E >= -cull has z in the range of cg_erfcx_tab,
+// psi_erfcx_tab_covers): one table-driven erfcx per element and no other transcendental.  f_i g_nk alone underflows
+// where z^2 is large: an element with E >= -cull has ln(f_i g_nk) = E - z^2 >= -cull - z^2, down to -810 at cull 746
+// and z = -8.  So f_i and g_nk are carried as f_i 2^480 and g_nk 2^480 (cg_exp_neg with BIAS: the same significands),
+// which are normal down to e^-1040 each (the launch also checks cull + z^2 <= 1040), their product is at most
+// pref 2^960, and the element is ((pref f_i 2^480) (g_nk 2^480)) erfcx(z) 2^-960: the same three roundings as the
+// unscaled product, and the last scaling is exact unless the element is subnormal.
+// ahx_gen_sep_kernel<false> (z outside the table): z >= 0: pref f_i g_nk erfcx(z); z < 0: pref (2 exp(E) -
+// f_i g_nk erfcx(-z)), with erfcx(|z|) from cg_erfcx_abs and one exp(E) per element.
 constexpr int AHX_IB = 8;
 constexpr int AHX_US = 4;         // observations ahx_gen_sep_kernel evaluates in lock-step (8: 143 registers, 0.9 ms slower)
 constexpr double AHX_FAR = 1e160;
+constexpr int AHX_BIAS = 480;     // f_i and g_nk scaled by 2^AHX_BIAS each in ahx_gen_sep_kernel<true>
 
-struct AhxRow { double th, e0, e1, z0, pf, fx; };   // pf = pref f_i, fx = f_i / sqrt(A)
+static_assert(2 * AHX_BIAS == 960, "ahx_gen_sep_kernel<true> scales by 2^-960");
+
+struct AhxRow { double th, e0, e1, z0, pf, fx, pfs; };   // pf = pref f_i, fx = f_i / sqrt(A), pfs = pref f_i 2^AHX_BIAS
 
 __device__ __forceinline__ void ahx_row_init(AhxRow* rows, int i0, const double* __restrict__ th, int nh, const PsiConst& c) {
   if (threadIdx.x < AHX_IB) {
@@ -355,11 +366,49 @@ __device__ __forceinline__ void ahx_row_init(AhxRow* rows, int i0, const double*
     const double f = exp(-(c.alpha + c.gamma) * thi * thi);
     r.pf = c.pref_hx * f;
     r.fx = f * c.inv_sqrtA;
+    const double lf[1] = {-(c.alpha + c.gamma) * thi * thi};
+    double fs[1];
+    cg_exp_neg<1, true, AHX_BIAS>(lf, fs);
+    r.pfs = c.pref_hx * fs[0];
     rows[threadIdx.x] = r;
   }
   __syncthreads();
 }
 
+// z range of the elements with E >= -cull over filter inducing inputs th in [th_lo, th_hi] (host): for a fixed th those
+// elements are an interval of d around e_hd th / (2 e_dd), and z is linear in d, so the largest z is a concave and the
+// smallest a convex function of th on the th where the interval is not empty; golden-section search finds both.  The
+// interval is taken at cull + 1 (covers the rounding of E in the kernel).  True when cg_erfcx_tab covers the range and
+// the scaled factors of ahx_gen_sep_kernel<true> stay normal.
+inline bool psi_erfcx_tab_covers(const PsiConst& c, double th_lo, double th_hi) {
+  if (!c.causal || c.causal_id || !(th_lo <= th_hi)) return false;
+  const double cl = c.cull + 1.0;
+  const double k = c.e_hd / (2.0 * c.e_dd), m = c.e_hh - c.e_hd * k / 2.0;   // E = -e_dd (d - k th)^2 - m th^2
+  if (!(m > 0.0) || !(c.e_dd > 0.0)) return false;
+  const double tmax = sqrt(cl / m);                      // |th| beyond which no element is live
+  const double lo = fmax(th_lo, -tmax), hi = fmin(th_hi, tmax);
+  if (lo > hi) return true;                              // every element is culled
+  auto zext = [&](double t, double sgn) {                // sgn * z at the end of the live d interval that maximises it
+    const double r = sqrt(fmax(cl - m * t * t, 0.0) / c.e_dd);
+    const double d = k * t - sgn * r;
+    return sgn * (-(c.gamma * t + c.omega * d) * c.inv_sqrtA);
+  };
+  double zr[2];
+  for (int s = 0; s < 2; ++s) {
+    const double sgn = s ? -1.0 : 1.0, g = 0.6180339887498949;
+    double a = lo, b = hi;
+    for (int it = 0; it < 200 && b - a > 1e-15 * (fabs(a) + fabs(b)); ++it) {
+      const double x1 = b - g * (b - a), x2 = a + g * (b - a);
+      if (zext(x1, sgn) < zext(x2, sgn)) a = x1; else b = x2;
+    }
+    zr[s] = sgn * fmax(fmax(zext(a, sgn), zext(lo, sgn)), zext(hi, sgn));
+  }
+  const double zmax = zr[0], zmin = zr[1];
+  return zmin >= CG_ERFCX_TAB_ZLO && zmax <= CG_ERFCX_TAB_ZHI &&
+         c.cull + fmax(zmin * zmin, zmax * zmax) <= 1040.0;
+}
+
+template <bool TAB>
 __global__ void __launch_bounds__(256) ahx_gen_sep_kernel(const double* __restrict__ t, const double* __restrict__ y,
                                                           int n_valid, int nc, const double* __restrict__ th, int nh, int nhp,
                                                           const double* __restrict__ tx, int nx, int k_lo, int kwp,
@@ -388,7 +437,8 @@ __global__ void __launch_bounds__(256) ahx_gen_sep_kernel(const double* __restri
         yv[u] = live ? __ldg(y + n + u) : 0.0;
         w2[u] = -c.omega * d[u] * d[u];
       }
-      cg_exp_neg<AHX_US, true>(w2, gk);
+      if (TAB) cg_exp_neg<AHX_US, true, AHX_BIAS>(w2, gk);
+      else cg_exp_neg<AHX_US, true>(w2, gk);
       double* dst = A + ((long)i0 * nc + n) * kwp + k;
 #pragma unroll 1
       for (int ii = 0; ii < ib; ++ii, dst += (long)nc * kwp) {
@@ -402,7 +452,19 @@ __global__ void __launch_bounds__(256) ahx_gen_sep_kernel(const double* __restri
           any = any || E[u] >= -c.cull;
         }
         double ysum = 0.0;
-        if (any && i0 + ii < nh) {
+        if (TAB && any && i0 + ii < nh) {
+          bool keep[AHX_US];
+#pragma unroll
+          for (int u = 0; u < AHX_US; ++u) keep[u] = E[u] >= -c.cull;
+          cg_erfcx_tab<AHX_US>(z, keep, q);
+#pragma unroll
+          for (int u = 0; u < AHX_US; ++u) {
+            const double v = keep[u] ? ((r.pfs * gk[u]) * q[u]) * 0x1p-960 : 0.0;     // 2^-(2 AHX_BIAS)
+            ysum = fma(yv[u], v, ysum);
+            if (n + u < n1) dst[(long)u * kwp] = v;
+          }
+          ys[ii][threadIdx.x] += ysum;
+        } else if (!TAB && any && i0 + ii < nh) {
           cg_exp_neg<AHX_US, true>(E, ex);
           cg_erfcx_abs<AHX_US>(z, q);
 #pragma unroll

@@ -295,6 +295,11 @@ int cgpcm_math_test(const double* x, int64_t n, double* out_exp, double* out_erf
 /* cgpcm_math_test_fast: the variants the separable Psi kernels use: out_exp[i] = exp(min(x[i], 0)) with results below
  * 2^-1021 flushed to 0 (one integer add scales by 2^n), out_erfcx[i] = erfcx(|x[i]|) = exp(x^2) erfc(|x|). */
 int cgpcm_math_test_fast(const double* x, int64_t n, double* out_exp, double* out_erfcx);
+/* cgpcm_math_test_tab: the routines of the table-driven separable Ahx kernel: out_exp[i] = exp(min(x[i], 0)) 2^B
+ * (results below 2^-1021 flushed to 0) and out_erfcx[i] = erfcx(x[i]) from the piecewise table, x in groups of 4
+ * evaluated in lock-step (4 neighbours share one interval's coefficients when they fit on it).  params receives
+ * {table range low, table range high, B}; erfcx outside the range is not meaningful. */
+int cgpcm_math_test_tab(const double* x, int64_t n, double* out_exp, double* out_erfcx, double* params);
 /* The kernels of cgpcm_elbo_smf_batch (csrc/smf_batch.cuh) with the launch shapes that call uses.  Device pointers only,
  * except `windows`; stream: a cudaStream_t or NULL; both return after the stream has drained.
  * cgpcm_smf_c1_test: c1[b] (B slabs of ld x ld) = sum over the windows of W_w,b^T W_w,b placed at (k_lo, k_lo), lower
