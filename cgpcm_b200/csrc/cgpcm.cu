@@ -47,13 +47,14 @@ namespace {
 typedef struct ncclComm* ncclComm_t;
 typedef struct { char internal[128]; } ncclUniqueId;
 typedef int ncclResult_t;
-enum { NCCL_DOUBLE = 8, NCCL_SUM = 0 };
+enum { NCCL_INT32 = 2, NCCL_DOUBLE = 8, NCCL_SUM = 0, NCCL_MAX = 2 };
 
 struct NcclApi {
   void* lib = nullptr;
   ncclResult_t (*GetUniqueId)(ncclUniqueId*) = nullptr;
   ncclResult_t (*CommInitRank)(ncclComm_t*, int, ncclUniqueId, int) = nullptr;
   ncclResult_t (*AllReduce)(const void*, void*, size_t, int, int, ncclComm_t, cudaStream_t) = nullptr;
+  ncclResult_t (*AllGather)(const void*, void*, size_t, int, ncclComm_t, cudaStream_t) = nullptr;
   ncclResult_t (*CommDestroy)(ncclComm_t) = nullptr;
   const char* (*GetErrorString)(ncclResult_t) = nullptr;
   bool ok = false;
@@ -73,9 +74,10 @@ NcclApi& nccl() {
   api.GetUniqueId = (decltype(api.GetUniqueId))dlsym(api.lib, "ncclGetUniqueId");
   api.CommInitRank = (decltype(api.CommInitRank))dlsym(api.lib, "ncclCommInitRank");
   api.AllReduce = (decltype(api.AllReduce))dlsym(api.lib, "ncclAllReduce");
+  api.AllGather = (decltype(api.AllGather))dlsym(api.lib, "ncclAllGather");
   api.CommDestroy = (decltype(api.CommDestroy))dlsym(api.lib, "ncclCommDestroy");
   api.GetErrorString = (decltype(api.GetErrorString))dlsym(api.lib, "ncclGetErrorString");
-  api.ok = api.GetUniqueId && api.CommInitRank && api.AllReduce && api.CommDestroy;
+  api.ok = api.GetUniqueId && api.CommInitRank && api.AllReduce && api.AllGather && api.CommDestroy;
   return api;
 }
 
@@ -1242,11 +1244,22 @@ int q_sweep(cgpcm_handle* h, const PsiConst& c, const std::vector<Chunk>& chunks
   return 0;
 }
 
-int allreduce(cgpcm_handle* h, double* buf, long count) {
+int allreduce(cgpcm_handle* h, void* buf, long count, int type = NCCL_DOUBLE, int op = NCCL_SUM) {
   if (h->world <= 1 || !h->comm) return 0;
-  ncclResult_t r = nccl().AllReduce(buf, buf, (size_t)count, NCCL_DOUBLE, NCCL_SUM, h->comm, h->st);
+  ncclResult_t r = nccl().AllReduce(buf, buf, (size_t)count, type, op, h->comm, h->st);
   if (r != 0) {
     h->err = std::string("ncclAllReduce failed: ") + (nccl().GetErrorString ? nccl().GetErrorString(r) : "?");
+    return -2;
+  }
+  return 0;
+}
+
+// recv[r * count + i] = send_r[i] for every rank r (recv holds world * count doubles).
+int allgather(cgpcm_handle* h, const double* send, double* recv, long count) {
+  if (h->world <= 1 || !h->comm) return 0;
+  ncclResult_t r = nccl().AllGather(send, recv, (size_t)count, NCCL_DOUBLE, h->comm, h->st);
+  if (r != 0) {
+    h->err = std::string("ncclAllGather failed: ") + (nccl().GetErrorString ? nccl().GetErrorString(r) : "?");
     return -2;
   }
   return 0;
@@ -2951,13 +2964,30 @@ int smf_batch_run(cgpcm_handle* h, const double* params_host, double reg, const 
   return 0;
 }
 
-// Samples per internal batch of predict_batch_run: a function of the handle's shape only (every launch of the batch
-// is shaped for this many samples).  Per sample: the C1 partials and slab and the two slabs of smf_posterior_kernel
-// (SMF_SLICES + 3 ld x ld), and V_b of a test chunk (chunk x nxp), within ~1 GB.
-int predict_bcap(const cgpcm_handle* h) {
-  const double per = ((SMF_SLICES + 3.0) * (double)h->ld * h->ld + (double)h->chunk * h->nxp) * sizeof(double);
+// Samples per internal batch of predict_batch_run: a function of the handle's shape and the test chunk budget only
+// (every launch of the batch is shaped for this many samples).  Per sample: the C1 partials and slab and the two slabs
+// of smf_posterior_kernel (SMF_SLICES + 3 ld x ld), and V_b of a test chunk (chunk x nxp), within ~1 GB.
+int predict_bcap(const cgpcm_handle* h, int chunk) {
+  const double per = ((SMF_SLICES + 3.0) * (double)h->ld * h->ld + (double)chunk * h->nxp) * sizeof(double);
   const int b = (int)std::min(64.0, 1e9 / per) / 8 * 8;
   return std::max(8, b);
+}
+
+// Budget of the test chunks and sample batches of the batched prediction paths: the chunk the planner chose for this
+// rank's observations (plan_chunks).  With several ranks the largest over the ranks, so that every rank cuts the test
+// inputs and sizes its batches alike: a rank plans from its own observations only, and one without any keeps 512.
+int test_chunk(cgpcm_handle* h, int& chunk) {
+  chunk = h->chunk;
+  if (h->world <= 1) return 0;
+  Scratch s;
+  const size_t o = s.take(1, sizeof(int));
+  CK(s.alloc());
+  int* d = s.at<int>(o);
+  CK(cudaMemcpyAsync(d, &chunk, sizeof(int), cudaMemcpyHostToDevice, h->st));
+  if (allreduce(h, d, 1, NCCL_INT32, NCCL_MAX)) return -2;
+  CK(cudaMemcpyAsync(&chunk, d, sizeof(int), cudaMemcpyDeviceToHost, h->st));
+  CK(cudaStreamSynchronize(h->st));
+  return 0;
 }
 
 // The training side shared by all samples of the batched prediction paths: with smf = 0 the one q(z) of q(u)
@@ -3003,7 +3033,9 @@ void pad_mx(cgpcm_handle* h, const double* mx, int nb, double* mxp) {
 // stage of smf_batch_run and smf_posterior_kernel (P_b, xm_b, mx_b, q1_b).  Test side, per chunk of test points: A* and
 // Bxx* once (predict_chunk_blocks), then per batch V = H_B A* (small-left GEMM), Qb = <Bxx*, mx_b> (predict_qb_kernel),
 // v^T mx_b v and v . xm_b (predict_quad_kernel) and predict_finish_kernel.  With smf = 1 the samples go in groups whose
-// mx slabs fit ~1 GB; A* and Bxx* are rebuilt per group.
+// mx slabs fit ~1 GB; A* and Bxx* are rebuilt per group.  With several ranks every rank runs the training side (its
+// sums are all-reduced), test chunk ci is computed by rank ci % world only, and the outputs, zero where another rank
+// owns the chunk, are all-reduced once at the end: each element has one non-zero contributor, so the sum is exact.
 int predict_batch_run(cgpcm_handle* h, const double* params_host, double reg, const double* tstar_host, long n_star,
                       const double* samples_host, int B, int smf, double* mu_out, double* var_out, double* mean_s_out,
                       double* var_s_out) {
@@ -3027,9 +3059,11 @@ int predict_batch_run(cgpcm_handle* h, const double* params_host, double reg, co
   plan_chunks(h, h->fc, chunks);
   if (ensure_ypart(h, y_slices_used(chunks))) return -2;
   cudaStream_t st = h->st;
-  const int TC = std::min<long>(h->chunk, n_star);
+  int tchunk;
+  if (test_chunk(h, tchunk)) return -2;
+  const int TC = std::min<long>(tchunk, n_star);
   const int TCP = round_up(TC, 8);
-  const int bcap = predict_bcap(h);
+  const int bcap = predict_bcap(h, tchunk);
   const int gcap = smf ? std::max(bcap, std::min(round_up(B, bcap), (int)(1e9 / (l2 * 8.0)) / bcap * bcap))
                        : round_up(B, bcap);
   const int nq = smf ? gcap : 1;         // q(z) slabs held at a time
@@ -3057,6 +3091,7 @@ int predict_batch_run(cgpcm_handle* h, const double* params_host, double reg, co
   CK(cudaMemcpyAsync(h->params_d, params_host, np * sizeof(double), cudaMemcpyHostToDevice, st));
   CK(cudaMemcpyAsync(d_t, tstar_host, n_star * sizeof(double), cudaMemcpyHostToDevice, st));
   CK(cudaMemsetAsync(d_acc, 0, (size_t)2 * n_star * sizeof(double), st));
+  if (h->world > 1 && per_sample) CK(cudaMemsetAsync(d_ps, 0, (size_t)2 * n_star * B * sizeof(double), st));
   if (prior_stage(h, c, reg, true)) return -2;
   if ((smf || !h->gram_valid) && plan_store(h, chunks, false)) return -2;
   if (predict_qu(h, reg)) return -2;
@@ -3084,6 +3119,7 @@ int predict_batch_run(cgpcm_handle* h, const double* params_host, double reg, co
     }
     // ---- test side of the group, chunk by chunk
     for (long p0 = 0; p0 < n_star; p0 += TC) {
+      if ((p0 / TC) % h->world != h->rank) continue;
       const int nv = (int)std::min<long>(TC, n_star - p0);
       const long cols = (long)round_up(nv, 8) * nxp;
       if (predict_chunk_blocks(h, cd, T, d_t + p0, nv, d_x)) return -2;
@@ -3118,6 +3154,8 @@ int predict_batch_run(cgpcm_handle* h, const double* params_host, double reg, co
     }
     CK(cudaGetLastError());
   }
+  if (allreduce(h, d_acc, 2 * n_star)) return -2;
+  if (per_sample && allreduce(h, d_ps, 2 * n_star * B)) return -2;
   if (mu_out) CK(cudaMemcpyAsync(mu_out, d_acc, n_star * sizeof(double), cudaMemcpyDefault, st));
   if (var_out) CK(cudaMemcpyAsync(var_out, d_acc + n_star, n_star * sizeof(double), cudaMemcpyDefault, st));
   if (mean_s_out) CK(cudaMemcpyAsync(mean_s_out, d_ps, n_star * B * sizeof(double), cudaMemcpyDefault, st));
@@ -3150,6 +3188,13 @@ int pcov_tile(const cgpcm_handle* h) {
 //               residuals; d = s2 with noise = 1 (observations), reg with noise = 0 (f itself).
 // Every launch is shaped by the handle, n_star and the internal batch size, and no sum runs across samples except cov,
 // so a sample's mean, C_b, draw, lp_s and whitened residuals are bitwise the same in any batch and at any position.
+// Several ranks: every rank runs the training side, A*, T, V, the means and R_b.  Pair tile k is computed by rank
+// k % world only and the tiles of the group's C_b are gathered (pcov_pack_kernel, ncclAllGather, pcov_unpack_kernel),
+// so every rank holds every C_b and adds cov.  Sample b of a group is factorised (draw, score) by rank b % world only;
+// draws, lp_s and whitened residuals, zero where another rank owns the sample, are all-reduced once at the end, and
+// the info words per group before any rank decides, so that every rank returns the same code and message.  The
+// tiles, groups and launch shapes do not depend on the world size (the batch size only on the test chunk budget,
+// test_chunk), so no output changes a bit with it.
 int predict_cov_run(cgpcm_handle* h, const double* params_host, double reg, const double* tstar_host, long n_star,
                     const double* samples_host, int B, int smf, const double* noise_host, double* mean_s_out,
                     double* cov_s_out, double* cov_out, double* draws_out, const double* y_host, int noise,
@@ -3187,7 +3232,9 @@ int predict_cov_run(cgpcm_handle* h, const double* params_host, double reg, cons
   const int TPP = TP * TP;               // pairs of a full tile (a multiple of 8)
   const int nhl = round_up(nh, 2);
   const long KH = (long)nh * nhl;
-  const int bcap = predict_bcap(h);
+  int tchunk;
+  if (test_chunk(h, tchunk)) return -2;
+  const int bcap = predict_bcap(h, tchunk);
   const int ldk = round_up(n + 1, 8);    // the bordered matrix of the scoring stage
   const long k2 = (long)ldk * ldk;
   const double per = 8.0 * ((double)n2 + (double)KH + (double)nxp * nxp + (smf ? (double)l2 : 0.0) +
@@ -3197,6 +3244,10 @@ int predict_cov_run(cgpcm_handle* h, const double* params_host, double reg, cons
   long wcols = 0;
   for (const Chunk& ch : chunks) wcols = std::max<long>(wcols, (long)ch.nc * ch.kwp);
   const long acols = (long)npad * nxp;   // columns of A* / T: [i][p][k]
+  const int ntile = (n + TP - 1) / TP;
+  const long ntp = (long)ntile * (ntile + 1) / 2;            // pair tiles p >= q
+  const int rank = h->rank, world = h->world;
+  const long slots = world > 1 ? (ntp + world - 1) / world : 0;   // tiles per rank in the gather
   Scratch s;
   const size_t o_t = s.take(n), o_a = s.take((size_t)nhp * acols), o_ta = s.take((size_t)nhp * acols);
   const size_t o_mean = s.take((size_t)n * B), o_draw = s.take(want_draws ? (size_t)n * B : 0);
@@ -3215,7 +3266,9 @@ int predict_cov_run(cgpcm_handle* h, const double* params_host, double reg, cons
   const size_t o_ys = s.take(want_score ? n : 0), o_kb = s.take(want_score ? (size_t)gcap * k2 : 0);
   const size_t o_lps = s.take(want_score ? B : 0), o_white = s.take(want_score && white_out ? (size_t)n * B : 0);
   const size_t o_info = s.take(gcap + bcap, sizeof(int));
+  const size_t o_pk = s.take((size_t)slots * gcap * TPP), o_pg = s.take((size_t)world * slots * gcap * TPP);
   CK(s.alloc());
+  double *d_pk = s.at(o_pk), *d_pg = s.at(o_pg);
   double *d_ys = s.at(o_ys), *d_kb = s.at(o_kb), *d_lps = s.at(o_lps), *d_white = s.at(o_white);
   double *d_t = s.at(o_t), *d_A = s.at(o_a), *d_TA = s.at(o_ta), *d_mean = s.at(o_mean), *d_draw = s.at(o_draw);
   double *d_noise = s.at(o_noise), *d_cov = s.at(o_cov), *d_x = s.at(o_x), *d_g = s.at(o_g), *d_ac = s.at(o_ac);
@@ -3232,6 +3285,11 @@ int predict_cov_run(cgpcm_handle* h, const double* params_host, double reg, cons
   if (want_score) CK(cudaMemcpyAsync(d_ys, y_host, n * sizeof(double), cudaMemcpyHostToDevice, st));
   const double d_add = noise ? hp.s2 : reg;    // S_b = C_b + d_add I
   if (cov_out) CK(cudaMemsetAsync(d_cov, 0, (size_t)n2 * sizeof(double), st));
+  if (world > 1) {                       // the per-sample outputs another rank owns stay 0 for the final all-reduce
+    if (want_draws) CK(cudaMemsetAsync(d_draw, 0, (size_t)n * B * sizeof(double), st));
+    if (want_score) CK(cudaMemsetAsync(d_lps, 0, (size_t)B * sizeof(double), st));
+    if (want_score && white_out) CK(cudaMemsetAsync(d_white, 0, (size_t)n * B * sizeof(double), st));
+  }
   std::vector<double> noise_t;
   if (want_draws) {
     // noise[p][b] -> one zero-padded column per sample
@@ -3256,7 +3314,6 @@ int predict_cov_run(cgpcm_handle* h, const double* params_host, double reg, cons
   if (gemm(h, true, false, false, nhp, (int)acols, nhp, 1.0, h->M(M_IKH), ld, d_A, acols, 0.0, d_TA, acols)) return -2;
   std::vector<int> inf(gcap);
   const double w = 1.0 / B;
-  const int ntile = (n + TP - 1) / TP;
   for (int g0 = 0; g0 < B; g0 += gcap) {
     const int gn = std::min(gcap, B - g0);
     const int nbat = (gn + bcap - 1) / bcap;
@@ -3309,9 +3366,10 @@ int predict_cov_run(cgpcm_handle* h, const double* params_host, double reg, cons
         if (gemm(h, true, true, false, npad, npad, nxp, 1.0, d_y, nxp, Vb, nxp, 0.0, Cb, npad)) return -2;
       }
     }
-    // ---- pair tiles p >= q
-    for (int pt = 0; pt < ntile; ++pt)
-      for (int qt = 0; qt <= pt; ++qt) {
+    // ---- pair tiles p >= q; tile k on rank k % world
+    for (int pt = 0, k = 0; pt < ntile; ++pt)
+      for (int qt = 0; qt <= pt; ++qt, ++k) {
+        if (k % world != rank) continue;
         const int p0 = pt * TP, q0 = qt * TP;
         const int P = std::min(TP, n - p0), Q = std::min(TP, n - q0);
         const int npairs = P * Q, npp = round_up(npairs, 8);
@@ -3352,6 +3410,13 @@ int predict_cov_run(cgpcm_handle* h, const double* params_host, double reg, cons
         }
       }
     CK(cudaGetLastError());
+    if (world > 1) {
+      pcov_pack_kernel<<<148 * 8, 256, 0, st>>>(d_c, n2, npad, gn, n, TP, ntp, rank, world, slots, d_pk);
+      L(h);
+      if (allgather(h, d_pk, d_pg, slots * gn * TPP)) return -2;
+      pcov_unpack_kernel<<<148 * 8, 256, 0, st>>>(d_pg, world, slots, gn, n, TP, ntp, d_c, n2, npad);
+      L(h);
+    }
     // ---- cov += C_b / B in ascending b; the per-sample outputs
     if (cov_out) {
       const double* C = d_c;
@@ -3371,6 +3436,7 @@ int predict_cov_run(cgpcm_handle* h, const double* params_host, double reg, cons
     if (want_draws) {
       CK(cudaMemsetAsync(d_pinfo, 0, (size_t)gn * sizeof(int), st));
       for (int b = 0; b < gn; ++b) {
+        if (b % world != rank) continue;
         const double* Cb = d_c + (long)b * n2;
         double* Kp = d_k;
         const int nn = n, ldn = npad;
@@ -3393,6 +3459,7 @@ int predict_cov_run(cgpcm_handle* h, const double* params_host, double reg, cons
         ew(st, n, [=] __device__(long p) { dr[p * Bn] = mean[p * Bn] + fv[p]; });
         L(h);
       }
+      if (allreduce(h, d_pinfo, gn, NCCL_INT32)) return -2;
       CK(cudaMemcpyAsync(inf.data(), d_pinfo, (size_t)gn * sizeof(int), cudaMemcpyDeviceToHost, st));
       CK(cudaStreamSynchronize(st));
       for (int b = 0; b < gn; ++b)
@@ -3403,12 +3470,15 @@ int predict_cov_run(cgpcm_handle* h, const double* params_host, double reg, cons
       pcov_border_kernel<<<148 * 8, 256, 0, st>>>(d_c, npad, n2, d_mean + g0, B, d_ys, n, d_add, gn, d_kb, ldk, k2);
       L(h);
       for (int b = 0; b < gn; ++b) {
+        if (b % world != rank) continue;
         cudaError_t e = potrf_lower(st, d_kb + (long)b * k2, ldk, ldk, d_pinfo + b, 8, h->M(M_XW));
         L(h, 2 * ((ldk + LA_NB - 1) / LA_NB));
         if (e != cudaSuccess) { h->err = "potrf launch failed"; return -2; }
       }
-      pcov_score_kernel<<<gn, 256, 0, st>>>(d_kb, ldk, k2, n, d_lps + g0, white_out ? d_white + g0 : nullptr, B);
+      pcov_score_kernel<<<gn, 256, 0, st>>>(d_kb, ldk, k2, n, d_lps + g0, white_out ? d_white + g0 : nullptr, B, rank,
+                                            world);
       L(h);
+      if (allreduce(h, d_pinfo, gn, NCCL_INT32)) return -2;
       CK(cudaMemcpyAsync(inf.data(), d_pinfo, (size_t)gn * sizeof(int), cudaMemcpyDeviceToHost, st));
       CK(cudaStreamSynchronize(st));
       for (int b = 0; b < gn; ++b) {
@@ -3417,13 +3487,17 @@ int predict_cov_run(cgpcm_handle* h, const double* params_host, double reg, cons
         if (piv == n + 1) {
           // The border pivot: potrf reports the first failed pivot, so every pivot of S_b passed and only the border
           // c - |z_b|^2 failed: |z_b|^2 overflows.  S_b is factorised alone with an identity border to confirm that
-          // before the overflow message (a failure there would be named by its own pivot).
+          // before the overflow message (a failure there would be named by its own pivot).  The owner of the sample
+          // factorises; every rank receives its info word.
           CK(cudaMemsetAsync(d_pinfo + b, 0, sizeof(int), st));
-          pcov_border_kernel<<<148 * 8, 256, 0, st>>>(d_c + (long)b * n2, npad, n2, d_mean + g0 + b, B, nullptr, n,
-                                                      d_add, 1, d_kb + (long)b * k2, ldk, k2);
-          L(h);
-          cudaError_t e = potrf_lower(st, d_kb + (long)b * k2, ldk, ldk, d_pinfo + b, 8, h->M(M_XW));
-          if (e != cudaSuccess) { h->err = "potrf launch failed"; return -2; }
+          if (b % world == rank) {
+            pcov_border_kernel<<<148 * 8, 256, 0, st>>>(d_c + (long)b * n2, npad, n2, d_mean + g0 + b, B, nullptr, n,
+                                                        d_add, 1, d_kb + (long)b * k2, ldk, k2);
+            L(h);
+            cudaError_t e = potrf_lower(st, d_kb + (long)b * k2, ldk, ldk, d_pinfo + b, 8, h->M(M_XW));
+            if (e != cudaSuccess) { h->err = "potrf launch failed"; return -2; }
+          }
+          if (allreduce(h, d_pinfo + b, 1, NCCL_INT32)) return -2;
           CK(cudaMemcpyAsync(&piv, d_pinfo + b, sizeof(int), cudaMemcpyDeviceToHost, st));
           CK(cudaStreamSynchronize(st));
           piv %= 100000;
@@ -3438,6 +3512,9 @@ int predict_cov_run(cgpcm_handle* h, const double* params_host, double reg, cons
       }
     }
   }
+  if (want_score && allreduce(h, d_lps, B)) return -2;
+  if (want_score && white_out && allreduce(h, d_white, (long)n * B)) return -2;
+  if (want_draws && allreduce(h, d_draw, (long)n * B)) return -2;
   if (want_score) {
     if (lp_s_out) CK(cudaMemcpyAsync(lp_s_out, d_lps, (size_t)B * sizeof(double), cudaMemcpyDefault, st));
     if (white_out) CK(cudaMemcpyAsync(white_out, d_white, (size_t)n * B * sizeof(double), cudaMemcpyDefault, st));

@@ -372,6 +372,62 @@ __global__ void pcov_finish_kernel(const double* __restrict__ qpart, int nrow, i
   }
 }
 
+// ---- Several ranks: pair tile k (numbered k = pt (pt + 1) / 2 + qt in the order predict_cov_run visits them) is
+// computed by rank k % world only.  The owner packs its tiles of the group's nb covariance slabs into `slots` slots of
+// nb x tpp doubles (slot j holds tile rank + j world: [j][b][e], e = i Q + j as pcov_finish_kernel numbers the pairs,
+// zero past the tile and for slots past the last tile); one ncclAllGather lays the ranks' buffers out as [rank][slot],
+// and pcov_unpack_kernel writes every tile back into C and mirrors it.  The values are moved, never summed, so C is
+// the same on every rank as in a run on one rank.
+__device__ inline void pcov_tile_of(long k, int tp, int n, int& p0, int& q0, int& P, int& Q) {
+  int pt = (int)((sqrt(8.0 * (double)k + 1.0) - 1.0) * 0.5);
+  while ((long)(pt + 1) * (pt + 2) / 2 <= k) ++pt;
+  while ((long)pt * (pt + 1) / 2 > k) --pt;
+  const int qt = (int)(k - (long)pt * (pt + 1) / 2);
+  p0 = pt * tp;
+  q0 = qt * tp;
+  P = min(tp, n - p0);
+  Q = min(tp, n - q0);
+}
+
+__global__ void pcov_pack_kernel(const double* __restrict__ C, long cstride, long ldc, int nb, int n, int tp, long ntiles,
+                                 int rank, int world, long slots, double* __restrict__ out) {
+  const long tpp = (long)tp * tp;
+  const long total = slots * nb * tpp;
+  for (long idx = (long)blockIdx.x * blockDim.x + threadIdx.x; idx < total; idx += (long)gridDim.x * blockDim.x) {
+    const long j = idx / (nb * tpp);
+    const long r = idx - j * nb * tpp;
+    const int b = (int)(r / tpp), e = (int)(r - (long)b * tpp);
+    const long k = rank + j * world;
+    double v = 0.0;
+    if (k < ntiles) {
+      int p0, q0, P, Q;
+      pcov_tile_of(k, tp, n, p0, q0, P, Q);
+      if (e < P * Q) v = C[(long)b * cstride + (long)(p0 + e / Q) * ldc + q0 + e % Q];
+    }
+    out[idx] = v;
+  }
+}
+
+__global__ void pcov_unpack_kernel(const double* __restrict__ in, int world, long slots, int nb, int n, int tp,
+                                   long ntiles, double* __restrict__ C, long cstride, long ldc) {
+  const long tpp = (long)tp * tp;
+  const long total = ntiles * nb * tpp;
+  for (long idx = (long)blockIdx.x * blockDim.x + threadIdx.x; idx < total; idx += (long)gridDim.x * blockDim.x) {
+    const long k = idx / (nb * tpp);
+    const long r = idx - k * nb * tpp;
+    const int b = (int)(r / tpp), e = (int)(r - (long)b * tpp);
+    int p0, q0, P, Q;
+    pcov_tile_of(k, tp, n, p0, q0, P, Q);
+    if (e >= P * Q) continue;
+    const int p = p0 + e / Q, q = q0 + e % Q;
+    if (p < q) continue;
+    const double v = in[((k % world) * slots + k / world) * nb * tpp + r];
+    double* Cb = C + (long)b * cstride;
+    Cb[(long)p * ldc + q] = v;
+    Cb[(long)q * ldc + p] = v;
+  }
+}
+
 // ---- Held-out scoring (cgpcm_predict_logpdf): log N(y; m_b, S_b), S_b = C_b + d I, through one Cholesky factorisation
 // of the bordered matrix
 //     K_b = [[S_b, r_b], [r_b^T, c]],   r_b = y - m_b,   L_K = [[L_b, 0], [z_b^T, l]],   L_b L_b^T = S_b,  z_b = L_b^-1 r_b
@@ -401,11 +457,13 @@ __global__ void pcov_border_kernel(const double* __restrict__ C, int npad, long 
 
 // One CTA (256 threads) per sample b < gridDim.x of the factored K[b]: logdet = 2 sum log L_ii and q = sum z_i^2, each
 // thread over i = tid, tid + 256, .. in order, then a fixed tree; lp[b] = -(n log 2 pi + logdet + q) / 2 and
-// white[p * ldw + b] = z_p.
+// white[p * ldw + b] = z_p.  With several ranks only the samples b % world == rank, which this rank factorised.
 __global__ void __launch_bounds__(256) pcov_score_kernel(const double* __restrict__ K, int ldk, long k2, int n,
-                                                         double* __restrict__ lp, double* __restrict__ white, long ldw) {
+                                                         double* __restrict__ lp, double* __restrict__ white, long ldw,
+                                                         int rank, int world) {
   __shared__ double sl[256], sq[256];
   const int b = blockIdx.x, tid = threadIdx.x;
+  if (b % world != rank) return;
   const double* Kb = K + (long)b * k2;
   const double* z = Kb + (long)n * ldk;
   double l = 0.0, q = 0.0;

@@ -155,7 +155,11 @@ int cgpcm_predict_f(cgpcm_handle* h, const double* params, double reg, const dou
  * a sample's mean_s / var_s are bitwise the same whatever other samples share the call and in any position.  Uses the
  * statistics frozen by cgpcm_precompute (-1 otherwise); -1 when n_samples < 1; -4 for a non-finite parameter, sample or
  * test input; -3 when some P_b is not positive definite (cgpcm_last_error names the sample and the pivot); n_star = 0
- * returns 0 and writes nothing. */
+ * returns 0 and writes nothing.
+ * With several ranks (cgpcm_comm_init) this call is collective: every rank must make it with the same arguments except
+ * its own observations, and every rank receives the full outputs.  Test chunk c is computed by rank c % world and the
+ * outputs are all-reduced with one non-zero contributor per element, so they are bitwise those of one rank holding
+ * the same training sums. */
 int cgpcm_predict_f_batch(cgpcm_handle* h, const double* params, double reg, const double* t_star, int64_t n_star,
                           const double* samples, int32_t n_samples, int32_t smf, double* mean, double* var,
                           double* mean_s, double* var_s);
@@ -180,7 +184,12 @@ int cgpcm_predict_f_batch(cgpcm_handle* h, const double* params, double reg, con
  * the same in any batch and at any position.  Uses the statistics frozen by cgpcm_precompute (-1 otherwise); -1 when
  * n_samples < 1 or n_star > 4096; -4 for a non-finite parameter, sample, test input or noise; -3 when some P_b or some
  * C_b + reg I is not positive definite (cgpcm_last_error names the sample and the pivot); n_star = 0 returns 0 and
- * writes nothing. */
+ * writes nothing.
+ * With several ranks (cgpcm_comm_init) this call is collective: every rank must make it with the same arguments except
+ * its own observations, and every rank receives the full outputs.  The pair tiles of the C_b are split across the
+ * ranks (tile k on rank k % world) and gathered, and sample b of each internal group is factorised on rank b % world;
+ * the outputs are bitwise those of one rank holding the same training sums, and every rank returns the same code and
+ * cgpcm_last_error. */
 int cgpcm_predict_f_cov(cgpcm_handle* h, const double* params, double reg, const double* t_star, int64_t n_star,
                         const double* samples, int32_t n_samples, int32_t smf, double* mean_s, double* cov_s,
                         double* cov, const double* noise, double* draws);
@@ -201,7 +210,9 @@ int cgpcm_predict_f_cov(cgpcm_handle* h, const double* params, double reg, const
  * in any batch and at any position.  Uses the statistics frozen by cgpcm_precompute (-1 otherwise); -1 when n_samples
  * < 1, n_star > 4096 or noise is not 0 or 1; -4 for a non-finite parameter, sample, test input or y_star; -3 when some
  * P_b or some C_b + d I is not positive definite (cgpcm_last_error names the sample and the pivot); n_star = 0 writes
- * lp = 0 and lp_s = 0 (the empty block has density 1). */
+ * lp = 0 and lp_s = 0 (the empty block has density 1).
+ * With several ranks: collective, as cgpcm_predict_f_cov, with the same split of the pair tiles and of the
+ * factorisations; every rank receives lp, lp_s and white, and returns the same code and cgpcm_last_error. */
 int cgpcm_predict_logpdf(cgpcm_handle* h, const double* params, double reg, const double* t_star,
                          const double* y_star, int64_t n_star, const double* samples, int32_t n_samples, int32_t smf,
                          int32_t noise, double* lp, double* lp_s, double* white);
